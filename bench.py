@@ -2,6 +2,7 @@
 """bench.py -- IVF-PQ batched search throughput (BASELINE.json's metric) on 1..8 B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c5|c5s|c3|tiny] [--impl reference]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the search hot path (probe selection -> query-only LUT -> fused ADC list scan +
 top-k [-> all-gather + mergeTopK at N > 1]) over ONE batch of nq synthetic queries against a device-resident
@@ -17,6 +18,11 @@ through the public API with pinned HOST query/result buffers (H2D + D2H inside t
 (query, probed list) of list length x M code bytes, SURVEY.md 8d); `cpu_baseline` = the oracle (C
 restatement of the reference arithmetic, OpenMP over queries) on a bounded sample of the same queries.
 `--impl reference` times only that CPU path (all host threads) on the same index.
+
+`--dump-outputs DIR` writes what the last timed step returned to its caller as DIR/<name>.npy (float32; ids as float64,
+which holds every id exactly): the inputs depend only on the workload and fixed seeds, so two builds of the
+project can be compared output for output.  An output above DUMP_LIMIT bytes is cut to a fixed, seeded sample of rows,
+whose row numbers are written beside it.
 """
 from __future__ import annotations
 
@@ -61,6 +67,25 @@ PRESETS = {
 CHUNK = 1_000_000
 GT_QUERIES = 256
 SEED = 123
+DUMP_LIMIT = 60_000_000                                               # bytes written by --dump-outputs, in all (< 64 MB)
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes name -> host array as out_dir/<name>.npy: integers wider than 16 bits as float64 (exact up to 2^53), the rest
+    as float32.  When the whole set would exceed DUMP_LIMIT, every array keeps the same fixed, seeded sample of rows,
+    listed in rows.npy."""
+    arrays = {name: a.astype(np.float64 if np.issubdtype(a.dtype, np.integer) and a.dtype.itemsize > 2 else np.float32)
+              for name, a in arrays.items()}
+    n = next(iter(arrays.values())).shape[0]
+    row_bytes = sum(a.nbytes for a in arrays.values()) // max(n, 1)
+    if row_bytes * n > DUMP_LIMIT:
+        rows = np.sort(np.random.default_rng(SEED).choice(n, DUMP_LIMIT // (row_bytes + 8), replace=False))
+        arrays = {name: a[rows] for name, a in arrays.items()}
+        arrays["rows"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    log(f"[bench] wrote {sorted(arrays)} ({sum(a.nbytes for a in arrays.values())} bytes) to {out_dir}")
 
 
 def log(*a):
@@ -348,6 +373,7 @@ def run_side_workload(args, cfg, K, W):
         cpu = {"value": nq / cpu_dt, "unit": unit, "cores": cores, "kind": "port",
                "sample": f"all {nq} queries against the full base, oracle/ C restatement of L2Sqr + selectTopK ({cpu_dt:.1f} s)"}
         check = lambda: bool(np.array_equal(o_pin[1], ci) and np.array_equal(o_pin[0].view(np.uint32), cd.view(np.uint32)))   # noqa: E731
+        outputs = lambda: {"distances": od.cpu().numpy(), "ids": oi.cpu().numpy()}   # noqa: E731
         detail["parity_with_cpu_baseline"] = "ids and distance bits equal"
         # two TF32 tensor-core passes dominate the step; TF32 runs at half the bf16 rate
         peak = float(peaks.get("bf16_tflops_sustained", 1385.9)) / 2.0
@@ -393,6 +419,7 @@ def run_side_workload(args, cfg, K, W):
         cpu = {"value": ns / cpu_dt, "unit": unit, "cores": cores, "kind": kind,
                "sample": f"all {ns} vectors, {what} ({cpu_dt:.1f} s)"}
         check = lambda: bool(np.array_equal(c_pin[:ns], ref))        # noqa: E731
+        outputs = lambda: {"codes": codes.cpu().numpy()}             # noqa: E731
         detail["parity_with_cpu_baseline"] = "codes bit-identical on all vectors"
         peak = float(peaks.get("hbm_gbs", 6650.0))
         roof = {"kernel": "pq_tc_encode_kernel (tcgen05 shortlist + exact finalists)", "bound": "hbm", "unit": "GB/s", "peak": peak,
@@ -412,6 +439,7 @@ def run_side_workload(args, cfg, K, W):
     torch.cuda.synchronize()
     launches = int(L.vix_kernel_launches(0))
     ms = e0.elapsed_time(e1) / K
+    last = outputs() if args.dump_outputs else None
     _lib.check(L.vix_set_async(0))
     for _ in range(W):
         api()
@@ -442,6 +470,8 @@ def run_side_workload(args, cfg, K, W):
                 "ms_per_step": None, "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "f32",
                 "data": "synthetic", "config": line["config"], "cpu_baseline": cpu,
                 "e2e": {"value": cpu["value"], "unit": unit, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}
+    if last is not None:
+        dump_outputs(args.dump_outputs, last)
     emit(line)
     return 0
 
@@ -474,9 +504,15 @@ def main():
     ap.add_argument("--profile", action="store_true",
                     help="bracket the timed steps with cudaProfilerStart/Stop (for ncu --profile-from-start off) "
                          "and skip the e2e / CPU legs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned as DIR/<name>.npy (float32 / float64, at most 64 MB)")
     args = ap.parse_args()
     cfg = dict(PRESETS[args.workload])
-    K, W = max(1, args.steps), max(3, args.warmup)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path; --impl reference has none")
+    K, W = args.steps, max(3, args.warmup)
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -587,6 +623,7 @@ def main():
     barrier()
     if args.profile:
         torch.cuda.profiler.stop()
+    last = {"distances": res_d.cpu().numpy(), "ids": res_i.cpu().numpy()} if args.dump_outputs and rank == 0 else None
     launches = int(L.vix_kernel_launches(0))
     ms_total = e0.elapsed_time(e1)
     scan_ms = coarse_ms = kern_ms = 0.0
@@ -740,6 +777,8 @@ def main():
     if world == 1 and not args.no_cpu_baseline and not args.profile:
         info, _, _ = cpu_search_arm(cfg, idx, q_host, gpu_ids=np.asarray(h_i))
         line["cpu_baseline"] = info
+    if last is not None:
+        dump_outputs(args.dump_outputs, last)
     emit(line)
     if dist:
         dist.barrier()

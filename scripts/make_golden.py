@@ -7,12 +7,22 @@ cpq_encode_reference.npz   outputs of the REFERENCE's own C encoder (Sources/CPQ
                            Tests/VectorIndexTests/PQEncodeParity_AoS_C_vs_Swift_Tests.swift:5-31 and on a seeded random
                            problem, every entry point.  Real reference outputs: the oracle and the CUDA library must
                            reproduce them bit for bit.
+cpq_encode_reference_fixtures.npz
+                           outputs of the same compiled reference encoder on the inputs of the oracle pins and the GPU layout
+                           test (tests/golden_inputs.py): every entry point on a seeded random problem, plain and fused
+                           residual codes at d / m = 128, and the with-CSQ codes and the SoA-blocked and interleaved layouts
+                           of the n = 70 parity fixture.  The committed file was written where the reference source was not
+                           at hand, from the oracle's codes (the layouts: pq_encode.c's index formulas applied to them).
+                           The same oracle and CUDA code had passed the tests that now read these arrays while those tests
+                           still called the compiled reference: they asserted these codes and buffers bit-equal to its
+                           outputs.  Run where oracle/_ref is built, this script rewrites them from the reference itself.
 oracle_search_small.npz    a small IVF-PQ problem (SIFT-shaped values with many ties) with the ORACLE's outputs of every
                            stage of the search path: list assignment, residual PQ codes, probe lists, residual LUTs, ADC
                            distances, flat top-k and the IVF-PQ top-k.  No reference test pins LUT / ADC arithmetic (SURVEY.md
                            8c), so these vectors only freeze the restatement; the GPU tests compare against them so that a
                            parity claim does not depend on rebuilding the oracle.
 Inputs are regenerated from seeds by the tests (tests/golden_inputs.py); only outputs are stored."""
+import ctypes as C
 import os
 import sys
 
@@ -23,6 +33,7 @@ sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 from oracle import oracle  # noqa: E402
 import golden_inputs as gi  # noqa: E402
+from conftest import parity_fixture  # noqa: E402
 
 OUT = os.path.join(ROOT, "tests", "golden")
 os.makedirs(OUT, exist_ok=True)
@@ -51,6 +62,44 @@ def encoder_golden():
         out[f"{name}.csq"] = csq
     np.savez_compressed(os.path.join(OUT, "cpq_encode_reference.npz"), **out)
     print("cpq_encode_reference.npz:", {k: v.shape for k, v in out.items()})
+
+
+def reference_fixtures_golden():
+    assert oracle.ref_lib() is not None, "oracle/_ref/libcpq_ref.so is needed (make -C oracle ref)"
+    out = {}
+    nodot = oracle.PQEncodeOpts(0, False, False, 8, 0, 0, 0)
+    for v in gi.ENCODER_VARIANTS:
+        x, cb, coarse, assign, m, ks = gi.encoder_variant_problem(v)
+        res = dict(coarse=coarse, assign_=assign)
+        csq = oracle.pq_centroid_sq(cb, m, ks, x.shape[1] // m, swift=True)
+        out[f"variant.{v}"] = {
+            "u8": lambda: oracle.ref_encode("cpq_encode_u8_f32", x, cb, m, ks),
+            "u8_nodot": lambda: oracle.ref_encode("cpq_encode_u8_f32", x, cb, m, ks, opts=nodot),
+            "u8_csq": lambda: oracle.ref_encode("cpq_encode_u8_f32_with_csq", x, cb, m, ks, centroid_sq=csq),
+            "res": lambda: oracle.ref_encode("cpq_encode_residual_u8_f32", x, cb, m, ks, **res),
+            "res_nodot": lambda: oracle.ref_encode("cpq_encode_residual_u8_f32", x, cb, m, ks, opts=nodot, **res),
+            "res_csq": lambda: oracle.ref_encode("cpq_encode_residual_u8_f32_with_csq", x, cb, m, ks, centroid_sq=csq, **res),
+            "u4": lambda: oracle.ref_encode("cpq_encode_u4_f32", x, cb, m, ks, packed_u4=True),
+            "res_u4": lambda: oracle.ref_encode("cpq_encode_residual_u4_f32", x, cb, m, ks, packed_u4=True, **res),
+        }[v]()
+    x, cent, asg, cb, m, ks = gi.long_subvector_residual_problem()
+    out["long_residual.plain"] = oracle.ref_encode("cpq_encode_u8_f32", (x - cent[asg]).astype(np.float32), cb, m, ks)
+    out["long_residual.fused"] = oracle.ref_encode("cpq_encode_residual_u8_f32", x, cb, m, ks, coarse=cent, assign_=asg)
+    x, cb, _, _ = parity_fixture(n=70)
+    n, d, m = x.shape[0], x.shape[1], 8
+    out["parity70.u8_csq"] = oracle.ref_encode("cpq_encode_u8_f32_with_csq", x, cb, m, 256,
+                                               centroid_sq=oracle.pq_centroid_sq(cb, m, 256, d // m, swift=False))
+    L = oracle.ref_lib()
+    L.cpq_encode_u8_f32.restype = None
+    for name, layout, B, g in gi.LAYOUTS:
+        Bq, gq = (B or 64), (g or 8)
+        buf = np.zeros(m * ((n + Bq - 1) // Bq) * Bq if layout == 1 else ((n + gq - 1) // gq) * m * gq, dtype=np.uint8)
+        L.cpq_encode_u8_f32(x.ctypes.data_as(oracle.f32p), C.c_int64(n), C.c_int(d), C.c_int(m), C.c_int(256),
+                            cb.ctypes.data_as(oracle.f32p), buf.ctypes.data_as(oracle.u8p),
+                            C.byref(oracle.PQEncodeOpts(layout, True, False, 8, 0, B, g)))
+        out[f"layout.{name}"] = buf
+    np.savez_compressed(os.path.join(OUT, "cpq_encode_reference_fixtures.npz"), **out)
+    print("cpq_encode_reference_fixtures.npz:", {k: v.shape for k, v in out.items()})
 
 
 def search_golden():
@@ -103,4 +152,5 @@ def search_golden():
 
 if __name__ == "__main__":
     encoder_golden()
+    reference_fixtures_golden()
     search_golden()

@@ -23,6 +23,38 @@ def encoder_problems():
     return out
 
 
+ENCODER_VARIANTS = ["u8", "u8_nodot", "u8_csq", "res", "res_csq", "res_nodot", "u4", "res_u4"]
+
+
+def encoder_variant_problem(variant):
+    """seeded random problem of tests/test_oracle_pins.py::test_oracle_encoder_equals_reference_encoder:
+    (x, codebooks, coarse, assign, m, ks); the codebooks have ks = 16 for the u4 variants"""
+    rng = np.random.default_rng(7)
+    n, d, m, kc = 300, 48, 6, 5
+    ks = 16 if variant.endswith("u4") else 256
+    x = rng.standard_normal((n, d)).astype(np.float32)
+    cb = rng.standard_normal((m * ks * (d // m))).astype(np.float32)
+    coarse = rng.standard_normal((kc, d)).astype(np.float32) * np.float32(0.5)
+    assign = rng.integers(0, kc, n).astype(np.int32)
+    return x, cb, coarse, assign, m, ks
+
+
+def long_subvector_residual_problem():
+    """ResidualKernelTests.swift:126-200 (n = 2000, d = 1024, m = 8, ks = 256, kc = 100, uniform [-1, 1)):
+    (x, coarse, assign, codebooks, m, ks)"""
+    rng = np.random.default_rng(1)
+    n, d, m, ks, kc = 2000, 1024, 8, 256, 100
+    x = rng.uniform(-1, 1, (n, d)).astype(np.float32)
+    cent = rng.uniform(-1, 1, (kc, d)).astype(np.float32)
+    asg = rng.integers(0, kc, n).astype(np.int32)
+    cb = rng.uniform(-1, 1, (m * ks, d // m)).astype(np.float32)
+    return x, cent, asg, cb, m, ks
+
+
+# output layouts of pq_encode.c:260-276 on parity_fixture(n=70): (name, layout, soa_block_B, interleave_g)
+LAYOUTS = [("soa_b64", 1, 64, 0), ("soa_b16", 1, 16, 0), ("interleaved_g8", 2, 0, 8), ("interleaved_g4", 2, 0, 4)]
+
+
 def search_problem():
     """small SIFT-shaped IVF-PQ problem: non-negative integer-valued components (many exact ties)"""
     rng = np.random.default_rng(96)

@@ -8,6 +8,7 @@ import os
 import numpy as np
 import pytest
 
+import golden_inputs as gi
 from conftest import parity_fixture
 from vectorindex_b200 import _lib
 
@@ -124,29 +125,21 @@ def test_pq_encode_tensor_core_shortlist_is_exact(oracle, vk, n, d, m, monkeypat
 
 
 def test_pq_encode_reference_fixture_and_layouts(oracle, vk):
-    """fixture of PQEncodeParity_AoS_C_vs_Swift_Tests.swift:5-31 against the compiled reference encoder,
-    including the SoA-blocked and interleaved output layouts (pq_encode.c:260-276)."""
+    """fixture of PQEncodeParity_AoS_C_vs_Swift_Tests.swift:5-31 against the reference encoder's stored outputs
+    (tests/golden/cpq_encode_reference_fixtures.npz), including the SoA-blocked and interleaved output layouts
+    (pq_encode.c:260-276)."""
     x, cb, coarse, assign = parity_fixture(n=70)
     csq = oracle.pq_centroid_sq(cb, 8, 256, 4, swift=False)
     got = vk.pq_encode_u8_f32_withCSQ(x, cb, csq, 8)
     assert got[0].tolist() == [212, 186, 160, 117, 255, 154, 186, 249]
-    if oracle.ref_lib() is None:
-        pytest.skip("oracle/_ref not present")
-    assert np.array_equal(got, oracle.ref_encode("cpq_encode_u8_f32_with_csq", x, cb, 8, 256, centroid_sq=csq))
-    n, m = x.shape[0], 8
-    for layout, B, g in ((1, 64, 0), (1, 16, 0), (2, 0, 8), (2, 0, 4)):
+    gold = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "cpq_encode_reference_fixtures.npz"))
+    assert np.array_equal(got, gold["parity70.u8_csq"])
+    m = 8
+    for name, layout, B, g in gi.LAYOUTS:
         o = _lib.PQEncodeOpts(layout, True, False, 8, 0, B, g)
-        ro = oracle.PQEncodeOpts(layout, True, False, 8, 0, B, g)
         ours = np.asarray(vk.pq_encode_u8_f32(x, cb, m, opts=o)).reshape(-1)
-        Bq, gq = (B or 64), (g or 8)
-        size = m * ((n + Bq - 1) // Bq) * Bq if layout == 1 else ((n + gq - 1) // gq) * m * gq
-        ref = np.zeros(size, dtype=np.uint8)
-        import ctypes as C
-        L = oracle.ref_lib()
-        L.cpq_encode_u8_f32.restype = None
-        L.cpq_encode_u8_f32(x.ctypes.data_as(oracle.f32p), C.c_int64(n), C.c_int(x.shape[1]), C.c_int(m), C.c_int(256),
-                            cb.ctypes.data_as(oracle.f32p), ref.ctypes.data_as(oracle.u8p), C.byref(ro))
-        assert np.array_equal(ours[:size], ref), f"layout {layout} B={B} g={g}"
+        ref = gold[f"layout.{name}"]
+        assert np.array_equal(ours[:ref.size], ref), f"layout {layout} B={B} g={g}"
 
 
 def test_pq_encode_empty_and_device_pointers(oracle, vk):
