@@ -763,6 +763,14 @@ query_prep_kernel(const float* __restrict__ queries, int64_t nq, int d, const fl
     float sq = 1.0f;
     if (g > 0.0f) { int e = 0; frexpf(g, &e); sq = ldexpf(1.0f, 10 - e); }
     const float s_c = tmeta[1], rmax = tmeta[2];                // of the decode table (per codebooks; meta is this launch's)
+    // The filter scales its bounds by s_q s_c (tc_scan_kernel).  Queries and codebooks both below 2^-50 make that product
+    // overflow (2^64 x 2^64 at 2^-54) although every distance is a normal fp32 number: s_q is lowered to keep it at most
+    // 2^126.  A smaller s_q only leaves more of the fp16 row subnormal, which the 6e-8 sqrt(d) rmax / s_q term of eps
+    // bounds; a product still not normal (s_c itself not finite, or both data above 2^73) hands the queries back below.
+    // tau and h_v themselves (sc times a distance) may still overflow when a distance exceeds 2^128 / sc; the sign makes
+    // that harmless: +inf rejects vectors that are that far anyway, -inf passes everything (at worst the log overflows
+    // and the queries are handed back).
+    if (sq * s_c > 0x1p126f) sq = 0x1p126f / s_c;
     if (q == 0 && lane == 0) { meta[0] = sq; meta[1] = s_c; }
     for (int e = lane; e < d; e += 32) qh[q * d + e] = __float2half_rn(__ldg(queries + q * d + e) * sq);
     if (lane == 0) {
@@ -774,8 +782,9 @@ query_prep_kernel(const float* __restrict__ queries, int64_t nq, int d, const fl
         const float eta = 1.05f * 0.0009765625f + (float)d * 4.8e-7f;
         const float eps = eta * qn * rmax + 6e-8f * sqrtf((float)d) * (rmax / sq + qn / s_c) + 2e-6f * qn * rmax;
         const float u = -0.5f * thr - eps - 2e-6f * fabsf(thr);
+        const float sc = sq * s_c;
         const bool fine = thr == thr && fabsf(thr) < __int_as_float(0x7f800000) && u == u && fabsf(u) < __int_as_float(0x7f800000) &&
-                          qn * sq < 60000.0f;
+                          qn * sq < 60000.0f && sc >= 0x1p-126f && sc <= 0x1p126f;
         uq[q] = fine ? u : 0.0f;
         flag[q] = fine ? 0 : 1;
     }
