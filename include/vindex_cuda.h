@@ -453,6 +453,12 @@ int vix_index_trace_get(vix_index_t* h, int i, vix_search_stats* out);
 int vix_debug_tc_scores_f32(const float* queries, int64_t nq, const float* centroids, int kc, int d, int metric,
                             const float* centroid_norms, float* out);
 
+/* Test hook: the list-major tensor-core scan's decode layout of an IVF-PQ index's codes (vix_scan.cuh), as the next search
+ * reads it (the lists are rebuilt first if rows were added).  *bytes_out = list slots x m, or 0 when the index keeps no such
+ * layout (only L2 indexes with ks = 256, d = 2 m and m in {16, 32, 48, 64} do); out (host or device, nullable) receives
+ * the bytes when cap holds them. */
+int vix_debug_tc_codes(vix_index_t* h, uint8_t* out, int64_t cap, int64_t* bytes_out);
+
 /* a16  AccelerableIndex-shaped convenience (AccelerableIndex.swift:15-127): candidates [c x d]
  * contiguous in, (indices into candidates, distances) out, per query. */
 int vix_accel_rank_candidates_f32(const float* queries, int64_t nq, const float* candidates, int64_t c,

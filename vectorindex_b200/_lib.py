@@ -95,7 +95,7 @@ _EXPORTS = [
     "vix_index_search_with_probes_keys_peers",
     "vix_comm_unique_id", "vix_comm_create", "vix_comm_destroy", "vix_comm_rank", "vix_comm_world",
     "vix_comm_uses_peer_memory", "vix_comm_trace", "vix_comm_trace_get", "vix_sharded_query_block", "vix_sharded_add", "vix_sharded_search",
-    "vix_index_encode", "vix_index_add_encoded", "vix_debug_tc_scores_f32", "vix_accel_rank_candidates_f32",
+    "vix_index_encode", "vix_index_add_encoded", "vix_debug_tc_scores_f32", "vix_debug_tc_codes", "vix_accel_rank_candidates_f32",
     "cpq_encode_u8_f32", "cpq_encode_u8_f32_with_csq", "cpq_encode_u4_f32", "cpq_encode_residual_u8_f32",
     "cpq_encode_residual_u8_f32_with_csq", "cpq_encode_residual_u4_f32", "cpq_pack_u4_bulk", "cpq_unpack_u4_bulk",
 ]

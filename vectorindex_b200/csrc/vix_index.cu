@@ -164,6 +164,29 @@ fill_slots_pq_kernel(const int32_t* __restrict__ slot_row, int64_t nslots, const
     if (lane == 0) { slot_ids[g] = ids[row]; slot_tx[g] = (float)acc; }
 }
 
+// The decode layout (vix_scan.cuh) from the AoS rows: one thread per 16-byte piece (chunk, group, thread t = 4 r + c of the
+// decoding warp), which gathers four bytes of each of the slots r + 8 v and writes them with one coalesced store.
+__global__ void __launch_bounds__(256)
+fill_tc_codes_kernel(const int32_t* __restrict__ slot_row, int64_t npieces, const uint8_t* __restrict__ codes, int m,
+                     uint4* __restrict__ tc_codes) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= npieces) return;
+    const int64_t ch = i / (2 * m);
+    const int rem = (int)(i - ch * 2 * m), grp = rem >> 5, r = (rem >> 2) & 7, c = rem & 3;
+    uint32_t w[4];
+#pragma unroll
+    for (int v = 0; v < 4; ++v) {
+        const int row = slot_row[ch * 32 + r + 8 * v];
+        w[v] = 0;
+        if (row >= 0) {
+            const uint8_t* src = codes + (int64_t)row * m + 16 * grp + c;
+#pragma unroll
+            for (int s = 0; s < 4; ++s) w[v] |= (uint32_t)src[4 * (s ^ (r & 3))] << (8 * s);
+        }
+    }
+    tc_codes[i] = make_uint4(w[0], w[1], w[2], w[3]);
+}
+
 __global__ void fill_slots_flat_kernel(const int32_t* __restrict__ slot_row, int64_t nslots,
                                        const float* __restrict__ vecs, const int64_t* __restrict__ ids, int d,
                                        float* __restrict__ slot_vecs, int64_t* __restrict__ slot_ids) {
@@ -237,12 +260,21 @@ int build_lists(vix_index* h) {
         const int rotated = (scan_layout(m).fast && h->p.ks == 256) ? 1 : 0;
         VIX_TRY(h->slot_codes.resize((size_t)nslots * h->code_bytes() + 16, false));
         VIX_TRY(h->slot_tx.resize((size_t)nslots, false));
+        const bool tc = tc_codes_shape(h->p.metric, m, h->p.ks, h->p.d / m);
+        if (tc) VIX_TRY(h->tc_codes.resize((size_t)nslots * m, false));
+        else h->tc_codes.free_all();
         if (nslots > 0) {
             int64_t threads = nslots * 32;
             fill_slots_pq_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, s>>>(
                 h->slot_row.ptr, nslots, h->codes.ptr, h->ids.ptr, h->assign.ptr, h->coarse.ptr, h->codebooks.ptr,
                 h->p.d, m, h->p.ks, rotated, h->p.metric, h->slot_codes.ptr, h->slot_ids.ptr, h->slot_tx.ptr);
             VIX_LAUNCH_CHECK();
+            if (tc) {
+                const int64_t npieces = nslots * m / 16;
+                fill_tc_codes_kernel<<<(unsigned)((npieces + 255) / 256), 256, 0, s>>>(
+                    h->slot_row.ptr, npieces, h->codes.ptr, m, reinterpret_cast<uint4*>(h->tc_codes.ptr));
+                VIX_LAUNCH_CHECK();
+            }
         }
     } else {
         VIX_TRY(h->slot_vecs.resize((size_t)nslots * h->p.d, false));
@@ -735,6 +767,7 @@ int index_search_locked(vix_index* h, const float* queries, int64_t nq, int k, i
             a.probes = pp; a.nprobe = nprobe; a.coarse = h->coarse.ptr; a.kc = h->kc; a.codebooks = h->codebooks.ptr;
             a.list_off = h->list_off.ptr; a.list_len = h->list_len.ptr;
             a.slot_codes = h->slot_codes.ptr; a.slot_tx = h->slot_tx.ptr; a.slot_ids = h->slot_ids.ptr;
+            a.tc_codes = h->tc_codes.ptr;
             a.metric = h->p.metric; a.k = k; a.out_dist = dd.dev; a.out_ids = di.dev;
             a.scanned = stats ? scanned.ptr : (traced ? h->trace_scanned.ptr + h->trace_n : nullptr);
             a.phase_cycles = stats ? scanned.ptr + 1 : nullptr;
@@ -1058,6 +1091,20 @@ int vix_index_export_lists(vix_index_t* h, int64_t* list_offsets, uint8_t* codes
     VIX_TRY(dids.commit());
     if (assignments_in_add_order && n > 0)
         VIX_CUDA(cudaMemcpyAsync(assignments_in_add_order, h->assign.ptr, (size_t)n * 4, cudaMemcpyDefault, ctx().stream));
+    return finish(true);
+}
+
+int vix_debug_tc_codes(vix_index_t* h, uint8_t* out, int64_t cap, int64_t* bytes_out) {
+    VIX_REQUIRE(h && bytes_out, VIX_ERR_NULL_PTR, "vix_debug_tc_codes: null pointer");
+    std::lock_guard<std::mutex> lk(h->mu);
+    VIX_REQUIRE(h->p.kind == VIX_INDEX_IVF_PQ && h->has_coarse, VIX_ERR_NOT_TRAINED, "vix_debug_tc_codes: not a trained IVF-PQ index");
+    if (h->dirty) VIX_TRY(build_lists(h));
+    const int64_t bytes = h->tc_codes.ptr ? h->nslots * h->p.m : 0;
+    *bytes_out = bytes;
+    if (out && bytes) {
+        VIX_REQUIRE(cap >= bytes, VIX_ERR_INVALID_PARAM, "vix_debug_tc_codes: %lld bytes do not fit %lld", (long long)bytes, (long long)cap);
+        VIX_CUDA(cudaMemcpyAsync(out, h->tc_codes.ptr, (size_t)bytes, cudaMemcpyDefault, ctx().stream));
+    }
     return finish(true);
 }
 

@@ -107,6 +107,8 @@ struct vix_index {
     DevBuf<int32_t> list_len;           // [kc]
     DevBuf<int32_t> slot_row;           // [nslots] add-order row of a slot, -1 for padding
     DevBuf<uint8_t> slot_codes;         // [nslots x m] scan layout (vix_scan.cuh)
+    DevBuf<uint8_t> tc_codes;           // [nslots x m] the list-major scan's decode layout of the same codes (vix_scan.cuh),
+                                        // only when the index can take that path (tc_codes_shape)
     DevBuf<float> slot_tx;              // [nslots]  ||r^||^2 + 2<c, r^>  (L2) / 0 (IP)
     DevBuf<int64_t> slot_ids;           // [nslots]
     DevBuf<float> slot_vecs;            // IVF_FLAT: [nslots x d]

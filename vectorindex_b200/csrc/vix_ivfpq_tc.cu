@@ -14,9 +14,10 @@
 //
 //   decode   32 vectors per warp, one vector per lane = one TMEM lane: 16 G look-ups into ONE query-independent table (the
 //            codebooks as fp16 pairs, two replicas, T[code][64 slots] x 2 sub-tables = 128 KB of shared memory) in the
-//            rotated order of the stored codes, so the 32 look-ups of a warp instruction hit 32 banks; a four-stage exchange
-//            network puts the 16 values of a group back into sub-quantiser order and tcgen05.st writes them as 16 TMEM
-//            columns: the A operand never touches shared memory.  Paid once per LIST VISIT, not per (query, list).
+//            order of the index's decode layout of the codes (vix_scan.cuh), so the 32 look-ups of a warp instruction hit 32
+//            banks; a two-stage exchange network puts each value into its column and two tcgen05.st .16x128b per group
+//            write them as 16 TMEM columns: the A operand never touches shared memory.  Paid once per LIST VISIT, not per
+//            (query, list).
 //   MMA      tcgen05.mma kind::f16 M128 N16..64 K16, A from TMEM, B = the fp16 rows of the queries probing the list
 //            (gathered into a 128B-swizzled shared-memory tile): D[vector][query] = <r^, q>, fp32 accumulators in TMEM.
 //   filter   one thread per vector row: D >= tau_q + h_v  <=>  bias + t_x - 2 <q, r^> <= thr_q + eps_q, where thr_q is an
@@ -100,7 +101,7 @@ struct Small {                                           // the bookkeeping in f
 };
 
 struct Args {
-    const uint8_t* slot_codes; const float* slot_tx;
+    const uint8_t* tc_codes; const float* slot_tx;      // the decode layout of the codes (vix_scan.cuh)
     const int64_t* list_off; const int32_t* list_len; int kc;
     const int32_t* pair_off;       // [kc + 1]
     const int32_t* order;          // [*n_order] the lists with pairs, most work first (list_order_*_kernel)
@@ -222,43 +223,51 @@ __device__ __forceinline__ uint32_t lds_tab(uint32_t addr) {
     asm volatile("ld.shared.b32 %0, [%1+%2];" : "=r"(v) : "r"(addr), "n"(IMM));
     return v;
 }
-__device__ __forceinline__ void tmem_st16(uint32_t taddr, const uint32_t (&r)[16]) {
+// .16x128b.x4: register 2 k + e of thread 4 i + c goes to TMEM lane i + 8 e, column 4 k + c (16 lanes x 16 columns)
+__device__ __forceinline__ void tmem_st16x128_x4(uint32_t taddr, const uint32_t (&r)[8]) {
     asm volatile(
-        "tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], "
-        "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};"
-        ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]), "r"(r[8]),
-          "r"(r[9]), "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]), "r"(r[14]), "r"(r[15])
+        "tcgen05.st.sync.aligned.16x128b.x4.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};"
+        ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7])
         : "memory");
 }
 __device__ __forceinline__ void tmem_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 
-// one group of 16 sub-quantisers of one vector (= one lane = one TMEM lane): 16 look-ups in the ROTATED order of the stored
-// codes (byte b holds sub-quantiser b ^ rot, rot = slot & 15: the 16 lanes of a half-warp ask for 16 different table slots,
-// the two half-warps read two replicas -- no bank conflicts), then the values are put back into sub-quantiser order with a
-// four-stage exchange network (register i <-> i ^ 2^s where bit s of rot is set) and leave as 16 TMEM columns.
+// one group of 16 sub-quantisers of the four slots r + 8 v (v = 0..3) of thread t = 4 r + c: 16 look-ups in the order of the
+// decode layout (vix_scan.cuh: byte s of word v holds sub-quantiser 4 (s ^ q) + c, q = r & 3).  For one (v, s) the 16
+// threads of a half-warp (q, c all different) ask for 16 different table slots and the two half-warps (h = r >> 2) read two
+// replicas: the 32 look-ups hit 32 banks.  (One replica per half-warp is why some exchange remains: without one, the lanes
+// that share a TMEM column in a store would all want the same slot.)  A two-stage exchange network (register s <-> s ^ 2^b where
+// bit b of q is set) puts each slot's four values into column order (register k = sub-quantiser 4 k + c), and two
+// tcgen05.st .16x128b write the slots r, r + 8 and r + 16, r + 24: TMEM lane = slot of the chunk, column = sub-quantiser.
 template <int IMM>
-__device__ __forceinline__ void decode16(const uint4& w, const uint32_t (&pre)[8], uint32_t taddr, bool b0, bool b1, bool b2, bool b3) {
+__device__ __forceinline__ void decode16(const uint4& w, uint32_t pre0, uint32_t pre1, uint32_t taddr, bool q0, bool q1) {
     const uint32_t x[4] = {w.x, w.y, w.z, w.w};
-    uint32_t r[16];
+    uint32_t r[4][4];
 #pragma unroll
-    for (int i = 0; i < 4; ++i) {
-        r[4 * i + 0] = lds_tab<IMM>(__byte_perm(x[i], pre[2 * i + 0], 0x7604));
-        r[4 * i + 1] = lds_tab<IMM>(__byte_perm(x[i], pre[2 * i + 0], 0x7615));
-        r[4 * i + 2] = lds_tab<IMM>(__byte_perm(x[i], pre[2 * i + 1], 0x7624));
-        r[4 * i + 3] = lds_tab<IMM>(__byte_perm(x[i], pre[2 * i + 1], 0x7635));
+    for (int v = 0; v < 4; ++v) {
+        r[v][0] = lds_tab<IMM>(__byte_perm(x[v], pre0, 0x7604));
+        r[v][1] = lds_tab<IMM>(__byte_perm(x[v], pre0, 0x7615));
+        r[v][2] = lds_tab<IMM>(__byte_perm(x[v], pre1, 0x7624));
+        r[v][3] = lds_tab<IMM>(__byte_perm(x[v], pre1, 0x7635));
     }
 #pragma unroll
-    for (int s = 0; s < 4; ++s) {
-        const bool bit = s == 0 ? b0 : s == 1 ? b1 : s == 2 ? b2 : b3;
+    for (int v = 0; v < 4; ++v) {
 #pragma unroll
-        for (int i = 0; i < 16; ++i) {
-            if ((i >> s) & 1) continue;
-            const uint32_t lo = r[i], hi = r[i | (1 << s)];
-            r[i] = bit ? hi : lo;
-            r[i | (1 << s)] = bit ? lo : hi;
+        for (int b = 0; b < 2; ++b) {
+            const bool bit = b == 0 ? q0 : q1;
+#pragma unroll
+            for (int i = 0; i < 4; ++i) {
+                if ((i >> b) & 1) continue;
+                const uint32_t lo = r[v][i], hi = r[v][i | (1 << b)];
+                r[v][i] = bit ? hi : lo;
+                r[v][i | (1 << b)] = bit ? lo : hi;
+            }
         }
     }
-    tmem_st16(taddr, r);
+    const uint32_t s01[8] = {r[0][0], r[1][0], r[0][1], r[1][1], r[0][2], r[1][2], r[0][3], r[1][3]};
+    const uint32_t s23[8] = {r[2][0], r[3][0], r[2][1], r[3][1], r[2][2], r[3][2], r[2][3], r[3][3]};
+    tmem_st16x128_x4(taddr, s01);
+    tmem_st16x128_x4(taddr + (16u << 16), s23);
 }
 
 template <int G>
@@ -306,14 +315,16 @@ tc_scan_kernel(Args a) {
         // this warp's rows of the operand stage: TMEM lanes [32 wi, 32 wi + 32) (the lanes a warp may touch: warp % 4 == wi),
         // lane = slot of the chunk; columns kACol0 + 64 stage + sub-quantiser
         const uint32_t a_taddr0 = tmem_base + ((32u * (uint32_t)wi) << 16) + (uint32_t)kACol0;
-        const bool rb0 = lane & 1, rb1 = lane & 2, rb2 = lane & 4, rb3 = lane & 8;       // bits of rot = slot & 15
-        uint32_t pre0[8];
+        // thread 4 r + c looks up byte s of each code word in table slot 16 h + 4 (s ^ q) + c, q = r & 3; pre holds the four
+        // byte offsets of those slots
+        const uint32_t q = ((uint32_t)lane >> 2) & 3u, c4 = 4u * ((uint32_t)lane & 3u);
+        const bool q0 = q & 1u, q1 = q & 2u;
+        uint32_t pre[2];
 #pragma unroll
-        for (int b = 0; b < 16; b += 2) {
-            const uint32_t c0 = 64u * h + 4u * ((uint32_t)(b ^ lane) & 15u);
-            const uint32_t c1 = 64u * h + 4u * ((uint32_t)((b + 1) ^ lane) & 15u);
-            pre0[b >> 1] = c0 | (c1 << 8);
-            asm volatile("" : "+r"(pre0[b >> 1]));
+        for (uint32_t s = 0; s < 4; s += 2) {
+            const uint32_t b0 = 64u * h + 16u * (s ^ q) + c4, b1 = 64u * h + 16u * ((s + 1) ^ q) + c4;
+            pre[s >> 1] = b0 | (b1 << 8);
+            asm volatile("" : "+r"(pre[s >> 1]));
         }
         // The warp walks its units (tile t of item it with (units before the item + t) % 3 == grp) with the NEXT unit's codes
         // already in flight while it decodes the current one (two register buffers, loop unrolled by two).  Moving on may
@@ -347,7 +358,7 @@ tc_scan_kernel(Args a) {
         };
         auto load = [&](uint4 (&w)[G], int ch) {
             if (ch < nch) {
-                const uint4* src = reinterpret_cast<const uint4*>(a.slot_codes + (size_t)(fc + ch) * (512u * G)) + lane;
+                const uint4* src = reinterpret_cast<const uint4*>(a.tc_codes + (size_t)(fc + ch) * (512u * G)) + lane;
 #pragma unroll
                 for (int s = 0; s < G; ++s) w[s] = __ldg(src + 32 * s);
             }
@@ -359,10 +370,10 @@ tc_scan_kernel(Args a) {
             if (use > 0 && !mbar_wait(&S.a_empty[st], (uint32_t)(use - 1) & 1u, a.error, a.error_host, VIX_DG(1))) return false;
             if (live) {
                 // group g: sub-table g / 2, slots 32 (g % 2) + 16 h + ..: the immediates are compile-time
-                decode16<(int)kTabAbs>(w[0], pre0, a_taddr, rb0, rb1, rb2, rb3);
-                if (G > 1) decode16<(int)kTabAbs + 128>(w[G > 1 ? 1 : 0], pre0, a_taddr + 16, rb0, rb1, rb2, rb3);
-                if (G > 2) decode16<(int)kTabAbs + 65536>(w[G > 2 ? 2 : 0], pre0, a_taddr + 32, rb0, rb1, rb2, rb3);
-                if (G > 3) decode16<(int)kTabAbs + 65536 + 128>(w[G > 3 ? 3 : 0], pre0, a_taddr + 48, rb0, rb1, rb2, rb3);
+                decode16<(int)kTabAbs>(w[0], pre[0], pre[1], a_taddr, q0, q1);
+                if (G > 1) decode16<(int)kTabAbs + 128>(w[G > 1 ? 1 : 0], pre[0], pre[1], a_taddr + 16, q0, q1);
+                if (G > 2) decode16<(int)kTabAbs + 65536>(w[G > 2 ? 2 : 0], pre[0], pre[1], a_taddr + 32, q0, q1);
+                if (G > 3) decode16<(int)kTabAbs + 65536 + 128>(w[G > 3 ? 3 : 0], pre[0], pre[1], a_taddr + 48, q0, q1);
                 tmem_wait_st();
             }
             fence_before_sync();
@@ -1153,6 +1164,7 @@ static StageTimes* stage_times() {
 }  // namespace tcs
 
 bool tc_decode_table_shape(int m, int ks, int dsub) { return dsub == 2 && ks == 256 && (m == 16 || m == 32 || m == 48 || m == 64); }
+bool tc_codes_shape(int metric, int m, int ks, int dsub) { return metric == VIX_METRIC_L2 && tc_decode_table_shape(m, ks, dsub); }
 int tc_decode_table(const float* codebooks, int m, uint32_t* table, float* meta) {
     tcs::table_kernel<<<1, 1024, 0, ctx().stream>>>(codebooks, m, table, meta);
     VIX_LAUNCH_CHECK();
@@ -1162,7 +1174,7 @@ int tc_decode_table(const float* codebooks, int m, uint32_t* table, float* meta)
 bool tc_scan_supported(const ScanArgs& a) {
     const char* env = getenv("VIX_TC_SCAN");
     if (env && env[0] == '0') return false;
-    if (a.metric != VIX_METRIC_L2 || !tc_decode_table_shape(a.m, a.ks, a.dsub)) return false;
+    if (!tc_codes_shape(a.metric, a.m, a.ks, a.dsub)) return false;
     if (a.filter || a.phase_cycles || a.nq_dev || a.k > 64) return false;
     if (a.nq * (int64_t)a.nprobe >= (1LL << 32) || a.nq < 1) return false;
     if (!(env && env[0] == '1') && a.nq * (int64_t)a.nprobe < 32768) return false;
@@ -1300,7 +1312,7 @@ int launch_ivfpq_scan_tc(ScanArgs& a) {
     VIX_TRY(cand.alloc((size_t)grid * kEpiWarps * log_cap));
     VIX_CUDA(cudaMemsetAsync(log_cnt.ptr, 0, (size_t)grid * kEpiWarps * sizeof(int), s));
     Args t{};
-    t.slot_codes = a.slot_codes; t.slot_tx = a.slot_tx; t.list_off = a.list_off; t.list_len = a.list_len; t.kc = a.kc;
+    t.tc_codes = a.tc_codes; t.slot_tx = a.slot_tx; t.list_off = a.list_off; t.list_len = a.list_len; t.kc = a.kc;
     t.pair_off = off.ptr; t.order = order.ptr; t.n_order = counters.ptr + 5; t.pairs = pairs.ptr; t.bias = bias.ptr; t.qh = qh.ptr;
     t.uq = uq.ptr; t.table = table_ptr;
     t.scales = meta.ptr; t.nprobe = a.nprobe; t.d = d; t.m = m;

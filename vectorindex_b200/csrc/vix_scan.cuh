@@ -26,6 +26,7 @@ struct ScanArgs {
                                                   // built once per codebooks (tc_decode_table); absent -> built per launch
     const int64_t* list_off; const int32_t* list_len;
     const uint8_t* slot_codes; const float* slot_tx; const int64_t* slot_ids;
+    const uint8_t* tc_codes;                      // the decode layout of slot_codes (below); the list-major path needs it
     // optional id filter (IDFilter.swift:115-135): ids outside [0, filter_cap) never pass; allowlist keeps set bits,
     // denylist keeps clear bits.  Applied BEFORE selection (pre-filter, IVFIndex.swift:813, 1034).
     const uint64_t* filter; int64_t filter_cap; int filter_deny;
@@ -64,6 +65,12 @@ int launch_probe_bias(const ScanArgs& a, float* bias, const int* only_flagged = 
 // [kTcTableWords] fp16 pairs, meta [4] floats ([1] the table's scale, [2] the bound of a decoded residual's norm)
 constexpr size_t kTcTableWords = 2 * 256 * 64;
 bool tc_decode_table_shape(int m, int ks, int dsub);
+// The decode layout: a second copy of the codes that only the list-major scan's decoders read (the rotated layout above
+// stays the one every exact key is computed from).  Chunk-blocked like the rotated layout -- the 512-byte block of chunk
+// and group grp at the same offset -- but inside a block thread t = 4 r + c (r = 0..7, c = 0..3) of the decoding warp owns
+// bytes [16 t, 16 t + 16), and byte 4 v + s holds the code of slot r + 8 v, sub-quantiser 16 grp + 4 (s ^ (r & 3)) + c.
+// Built for L2 indexes of the decode table's shape (tc_codes_shape), which are the only ones the list-major path takes.
+bool tc_codes_shape(int metric, int m, int ks, int dsub);
 int tc_decode_table(const float* codebooks, int m, uint32_t* table, float* meta);
 
 }  // namespace vix
