@@ -16,12 +16,13 @@
  *     (a mutex per handle: one add / search enqueues at a time, the reference's actor isolation, IVFIndex.swift:13).
  *     Device work of calls issued from different threads is ordered only by their streams: every search owns its
  *     work queue and scratch (stream-ordered allocations), so concurrent asynchronous searches of one handle on
- *     different streams are independent; a call that CHANGES the handle (add, train, set_*, clear, the lazy list
- *     rebuild of the first search after an add) must not overlap other calls still running on another stream --
- *     synchronise (vix_synchronize) before it;
+ *     different streams are independent; a call that CHANGES the handle (add, remove, train, set_*, clear, the lazy list
+ *     rebuild of the first search after an add or a removal) must not overlap other calls still running on another
+ *     stream -- synchronise (vix_synchronize) before it;
  *   - ids live in [0, 2^32 - 1) (the reference's top-k id type is Int32, TopK.swift:59), checked for host AND device
  *     id arrays; adding an id that is already stored APPENDS a second row (the reference's Dictionary store replaces,
- *     IVFIndex.swift:42): callers that need replacement delete / rebuild; duplicates are returned as separate results;
+ *     IVFIndex.swift:42): callers that need replacement call vix_index_remove with the id, then add the new row;
+ *     duplicates are returned as separate results;
  *   - list ids (assignments handed to vix_index_add_encoded, probe lists handed to *_with_probes*) outside [0, kc) are
  *     rejected (assignments) or skipped like the -1 padding (probes); rows whose scores are all NaN get no list:
  *     IVF_FLAT keeps them unreachable as the reference does (IVFIndex.swift:376-435 "guard best >= 0"), IVF_PQ add fails.
@@ -305,8 +306,19 @@ int vix_index_set_codebooks(vix_index_t* h, const float* codebooks, const float*
 int vix_index_get_coarse(vix_index_t* h, float* centroids_out, int* kc_out);
 int vix_index_get_codebooks(vix_index_t* h, float* codebooks_out, float* centroid_norms_out);
 
-/* batchInsert: ids NULL => consecutive ids continuing from the current count */
+/* batchInsert: ids NULL => consecutive ids continuing after the last automatic id this handle handed out, counting every
+ * row added since the handle was created, cleared or imported into.  Without removals that is the current count; after
+ * one, automatic ids never repeat an id that may still be stored. */
 int vix_index_add(vix_index_t* h, const float* x, const int64_t* ids, int64_t n);
+/* remove(id:): remove every stored row whose id is in ids[0..n) (host or device array; duplicates and ids that are not
+ * stored are allowed).  A row stored twice under one id is removed twice.  *removed_out (nullable, host) = rows removed.
+ * Ids are checked as by add (VIX_ERR_INVALID_PARAM outside [0, 2^32 - 1)) before anything changes: a call rejected for
+ * its input removes nothing.  The remaining rows keep their order, so the index then equals one built by adding only them: same lists,
+ * same slots, same search results.  The rows are compacted on the device (one extra copy of the largest row array at
+ * the peak) and the lists are rebuilt by the next call that reads them, as after an add; a call that matches no row
+ * changes nothing.  Every index kind.  On a shard it removes what THIS rank holds: a sharded host passes the same ids to
+ * every rank and sums the counts itself. */
+int vix_index_remove(vix_index_t* h, const int64_t* ids, int64_t n, int64_t* removed_out);
 /* import of prebuilt inverted lists in the reference's AoS list format (Kernels/IVFAppend.swift:
  * 220-236): CSR offsets[kc+1], codes[N x m], ids[N] */
 int vix_index_import_lists(vix_index_t* h, const int64_t* list_offsets, const uint8_t* codes,

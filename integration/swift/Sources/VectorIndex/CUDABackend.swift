@@ -70,6 +70,12 @@ public final class CUDAIVFPQIndex {
     public func batchInsert(_ x: [Float], ids: [Int64]) throws {
         try _vixCheck(vix_index_add(h, x, ids, Int64(ids.count)), "vix_index_add")
     }
+    /// remove(id:) for a batch: every stored row whose id is listed goes; returns the number of rows removed
+    public func batchRemove(ids: [Int64]) throws -> Int {
+        var removed: Int64 = 0
+        try _vixCheck(vix_index_remove(h, ids, Int64(ids.count), &removed), "vix_index_remove")
+        return Int(removed)
+    }
     /// ascending by API distance, padded with id -1 / NaN; k <= 0 leaves the outputs untouched (IVFIndex.swift:866)
     public func batchSearch(_ q: [Float], nq: Int, k: Int) throws -> ([Float], [Int64]) {
         var dist = [Float](repeating: .nan, count: nq * k); var ids = [Int64](repeating: -1, count: nq * k)

@@ -87,7 +87,7 @@ _EXPORTS = [
     "vix_ivf_assign_metric_f32", "vix_pq_query_subnorms_f32", "vix_pq_lut_batch_l2_f32", "vix_pq_lut_residual_l2_f32", "vix_adc_scan_u8",
     "vix_adc_scan_u4", "vix_kmeanspp_seed_f32", "vix_kmeans_minibatch_f32", "vix_pq_train_f32", "vix_pq_train_streaming_f32",
     "vix_index_params_default", "vix_index_create", "vix_index_destroy", "vix_index_train", "vix_index_set_coarse",
-    "vix_index_set_codebooks", "vix_index_get_coarse", "vix_index_get_codebooks", "vix_index_add",
+    "vix_index_set_codebooks", "vix_index_get_coarse", "vix_index_get_codebooks", "vix_index_add", "vix_index_remove",
     "vix_index_import_lists", "vix_index_count", "vix_index_list_sizes", "vix_index_export_lists", "vix_index_clear",
     "vix_index_search", "vix_index_search_ex", "vix_index_search_rerank", "vix_index_trace", "vix_index_trace_get", "vix_index_probe_range", "vix_index_search_with_probes",
     "vix_index_search_with_probes_ex", "vix_index_search_filtered", "vix_index_probe_range_keys", "vix_merge_probe_keys",

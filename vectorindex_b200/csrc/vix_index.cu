@@ -643,12 +643,16 @@ static int index_add_locked(vix_index* h, const float* x, const int64_t* ids, in
         VIX_REQUIRE(h->has_pq, VIX_ERR_NOT_TRAINED, "index_add: PQ codebooks not trained / set");
     }
     if (ids) VIX_TRY(is_device_ptr(ids) ? check_ids_device(ids, n) : check_ids_host(ids, n));
-    if (!ids) VIX_REQUIRE(h->n + n < 0xFFFFFFFFLL, VIX_ERR_INVALID_PARAM, "automatic ids exceed 2^32 - 1");
+    if (!ids) VIX_REQUIRE(h->next_auto_id + n < 0xFFFFFFFFLL, VIX_ERR_INVALID_PARAM, "automatic ids exceed 2^32 - 1");
 
     const int64_t n0 = h->n;
     VIX_TRY(h->ids.resize((size_t)(n0 + n)));
     if (ids) VIX_CUDA(cudaMemcpyAsync(h->ids.ptr + n0, ids, (size_t)n * 8, cudaMemcpyDefault, s));
-    else { iota64_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(h->ids.ptr + n0, n, n0); VIX_LAUNCH_CHECK(); }
+    else {
+        // (after a removal the count no longer names an unused id: automatic ids continue from the last one handed out)
+        iota64_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(h->ids.ptr + n0, n, h->next_auto_id);
+        VIX_LAUNCH_CHECK();
+    }
 
     if (h->p.kind == VIX_INDEX_FLAT || h->p.kind == VIX_INDEX_IVF_FLAT) {
         VIX_TRY(h->vecs.resize((size_t)(n0 + n) * d));
@@ -687,8 +691,138 @@ static int index_add_locked(vix_index* h, const float* x, const int64_t* ids, in
         }
     }
     h->n = n0 + n;
+    h->next_auto_id += n;
     h->dirty = true;
     return finish(true);
+}
+
+// ------------------------------------------------------------------------------------------------
+// removal: compaction of the add-order rows.  The lists and the decode layout are derived from these rows, so they are
+// only marked dirty here and build_lists() rebuilds them, as after an add.
+// ------------------------------------------------------------------------------------------------
+// ids in [0, 2^32 - 1) (checked): the low 32 bits are the whole id, so the sort key is 4 bytes whatever the ids are
+__global__ void ids_to_keys_kernel(const int64_t* __restrict__ ids, int64_t n, uint32_t* __restrict__ keys) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) keys[i] = (uint32_t)ids[i];
+}
+
+// keep[i] = 0 when the id of row i is in the sorted set (binary search), 1 otherwise; keep[n] = 0 closes the scan
+__global__ void mark_removed_kernel(const int64_t* __restrict__ row_ids, int64_t n, const uint32_t* __restrict__ sorted,
+                                    int64_t ns, int32_t* __restrict__ keep) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i > n) return;
+    if (i == n) { keep[n] = 0; return; }
+    const uint32_t id = (uint32_t)row_ids[i];
+    int64_t lo = 0, hi = ns;
+    while (lo < hi) {
+        const int64_t mid = (lo + hi) >> 1;
+        if (__ldg(sorted + mid) < id) lo = mid + 1; else hi = mid;
+    }
+    keep[i] = (lo < ns && __ldg(sorted + lo) == id) ? 0 : 1;
+}
+
+// dst row pos[r] = src row r for every kept row; rows of w units U, one thread per unit (reads coalesced, writes in runs)
+template <typename U>
+__global__ void __launch_bounds__(256)
+compact_rows_kernel(const U* __restrict__ src, int64_t n, int w, const int32_t* __restrict__ keep,
+                    const int32_t* __restrict__ pos, U* __restrict__ dst) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int64_t units = n * w;
+    if (i >= units) return;
+    const int64_t row = units <= 0xFFFFFFFFLL ? (int64_t)((uint32_t)i / (uint32_t)w) : i / w;
+    if (__ldg(keep + row)) dst[(int64_t)__ldg(pos + row) * w + (i - row * w)] = src[i];
+}
+
+template <typename U>
+static int launch_compact(const void* src, int64_t n, int64_t row_bytes, const int32_t* keep, const int32_t* pos, void* dst) {
+    const int w = (int)(row_bytes / (int64_t)sizeof(U));
+    const int64_t blocks = (n * w + 255) / 256;
+    compact_rows_kernel<U><<<(unsigned)blocks, 256, 0, ctx().stream>>>(static_cast<const U*>(src), n, w, keep, pos,
+                                                                        static_cast<U*>(dst));
+    VIX_LAUNCH_CHECK();
+    return VIX_OK;
+}
+
+// the kept rows of one add-order array (row_bytes per row) into an exactly sized new array, swapped in
+template <typename T>
+static int compact_array(DevBuf<T>& buf, int64_t n, int64_t row_elems, int64_t kept, const int32_t* keep, const int32_t* pos) {
+    if (kept == 0) { buf.size = 0; return VIX_OK; }
+    const int64_t row_bytes = row_elems * (int64_t)sizeof(T);
+    T* out = nullptr;
+    VIX_CUDA(cudaMalloc(reinterpret_cast<void**>(&out), (size_t)(kept * row_bytes)));
+    int rc;
+    if (row_bytes % 16 == 0) rc = launch_compact<uint4>(buf.ptr, n, row_bytes, keep, pos, out);         // (cudaMalloc: 256 B aligned)
+    else if (row_bytes % 8 == 0) rc = launch_compact<uint2>(buf.ptr, n, row_bytes, keep, pos, out);
+    else if (row_bytes % 4 == 0) rc = launch_compact<uint32_t>(buf.ptr, n, row_bytes, keep, pos, out);
+    else if (row_bytes % 2 == 0) rc = launch_compact<uint16_t>(buf.ptr, n, row_bytes, keep, pos, out);
+    else rc = launch_compact<uint8_t>(buf.ptr, n, row_bytes, keep, pos, out);
+    cudaError_t e = rc == VIX_OK ? cudaStreamSynchronize(ctx().stream) : cudaSuccess;
+    if (rc != VIX_OK || e != cudaSuccess) { cudaFree(out); if (rc != VIX_OK) return rc; VIX_CUDA(e); }
+    buf.adopt(out, (size_t)(kept * row_elems));
+    return VIX_OK;
+}
+
+static int index_remove_locked(vix_index* h, const int64_t* ids, int64_t n, int64_t* removed) {
+    *removed = 0;
+    if (n == 0) return VIX_OK;
+    // the id contract of add, checked before anything changes
+    const bool dev_ids = is_device_ptr(ids);
+    VIX_TRY(dev_ids ? check_ids_device(ids, n) : check_ids_host(ids, n));
+    const int64_t rows = h->n;
+    if (rows == 0) return VIX_OK;
+    cudaStream_t s = ctx().stream;
+    In<int64_t> did;
+    VIX_TRY(did.stage(ids, (size_t)n));
+    // 1. the requested ids, sorted (4-byte keys: scratch independent of the id range)
+    Scratch<uint32_t> keys_in, keys;
+    VIX_TRY(keys_in.alloc((size_t)n));
+    VIX_TRY(keys.alloc((size_t)n));
+    ids_to_keys_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(did.dev, n, keys_in.ptr);
+    VIX_LAUNCH_CHECK();
+    size_t sort_bytes = 0, scan_bytes = 0;
+    VIX_CUDA(cub::DeviceRadixSort::SortKeys(nullptr, sort_bytes, keys_in.ptr, keys.ptr, (int)n, 0, 32, s));
+    Scratch<int32_t> keep, pos;
+    VIX_TRY(keep.alloc((size_t)rows + 1));
+    VIX_TRY(pos.alloc((size_t)rows + 1));
+    VIX_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, keep.ptr, pos.ptr, (int)(rows + 1), s));
+    Scratch<unsigned char> tmp;
+    VIX_TRY(tmp.alloc((sort_bytes > scan_bytes ? sort_bytes : scan_bytes) + 16));
+    VIX_CUDA(cub::DeviceRadixSort::SortKeys(tmp.ptr, sort_bytes, keys_in.ptr, keys.ptr, (int)n, 0, 32, s));
+    ctx().launches += 1;
+    // 2. per stored row: keep flag; 3. new positions of the kept rows, and their number
+    mark_removed_kernel<<<(unsigned)((rows + 1 + 255) / 256), 256, 0, s>>>(h->ids.ptr, rows, keys.ptr, n, keep.ptr);
+    VIX_LAUNCH_CHECK();
+    VIX_CUDA(cub::DeviceScan::ExclusiveSum(tmp.ptr, scan_bytes, keep.ptr, pos.ptr, (int)(rows + 1), s));
+    ctx().launches += 1;
+    int32_t kept32 = 0;
+    VIX_CUDA(cudaMemcpyAsync(&kept32, pos.ptr + rows, 4, cudaMemcpyDeviceToHost, s));
+    VIX_CUDA(cudaStreamSynchronize(s));
+    const int64_t kept = kept32;
+    if (kept == rows) return VIX_OK;                              // nothing matched: the handle is untouched (lists stay built)
+    // 4. gather the kept rows of every add-order array, largest first: once its copy is made, the memory it frees holds
+    //    every later copy, so a call that gets past the first allocation completes
+    struct Part { int which; int64_t bytes; };
+    Part parts[4];
+    int np = 0;
+    parts[np++] = {0, rows * 8};
+    if (h->assign.size == (size_t)rows) parts[np++] = {1, rows * 4};
+    if (h->p.kind == VIX_INDEX_IVF_PQ) parts[np++] = {2, rows * (int64_t)h->code_bytes()};
+    else parts[np++] = {3, rows * (int64_t)h->p.d * 4};
+    for (int a = 1; a < np; ++a)
+        for (int b = a; b > 0 && parts[b].bytes > parts[b - 1].bytes; --b) { Part t = parts[b]; parts[b] = parts[b - 1]; parts[b - 1] = t; }
+    for (int a = 0; a < np; ++a) {
+        switch (parts[a].which) {
+            case 0: VIX_TRY(compact_array(h->ids, rows, 1, kept, keep.ptr, pos.ptr)); break;
+            case 1: VIX_TRY(compact_array(h->assign, rows, 1, kept, keep.ptr, pos.ptr)); break;
+            case 2: VIX_TRY(compact_array(h->codes, rows, h->code_bytes(), kept, keep.ptr, pos.ptr)); break;
+            default: VIX_TRY(compact_array(h->vecs, rows, h->p.d, kept, keep.ptr, pos.ptr)); break;
+        }
+    }
+    // 5. the lists, the scan layouts and the decode layout follow at the next call that reads them
+    h->n = kept;
+    h->dirty = true;
+    *removed = rows - kept;
+    return VIX_OK;
 }
 
 int index_search_locked(vix_index* h, const float* queries, int64_t nq, int k, int nprobe, float* out_dist,
@@ -1042,6 +1176,7 @@ int vix_index_import_lists(vix_index_t* h, const int64_t* list_offsets, const ui
     expand_assign_kernel<<<kc, 128, 0, ctx().stream>>>(doff.ptr, kc, h->assign.ptr);
     VIX_LAUNCH_CHECK();
     h->n = n;
+    h->next_auto_id = n;
     h->dirty = true;
     return finish(true);
 }
@@ -1112,8 +1247,21 @@ int vix_index_clear(vix_index_t* h) {
     VIX_REQUIRE(h, VIX_ERR_NULL_PTR, "vix_index_clear: null handle");
     std::lock_guard<std::mutex> lk(h->mu);
     h->n = 0;
+    h->next_auto_id = 0;
     h->vecs.size = h->ids.size = h->assign.size = h->codes.size = 0;
     h->dirty = true;
+    return VIX_OK;
+}
+
+int vix_index_remove(vix_index_t* h, const int64_t* ids, int64_t n, int64_t* removed_out) {
+    if (removed_out) *removed_out = 0;
+    VIX_TRY(ensure_device());
+    VIX_REQUIRE(h && (ids || n == 0), VIX_ERR_NULL_PTR, "vix_index_remove: null pointer");
+    VIX_REQUIRE(n >= 0 && n < 0x7FFFFFFFLL, VIX_ERR_INVALID_PARAM, "vix_index_remove: n must lie in [0, 2^31 - 1)");
+    std::lock_guard<std::mutex> lk(h->mu);
+    int64_t removed = 0;
+    VIX_TRY(index_remove_locked(h, ids, n, &removed));
+    if (removed_out) *removed_out = removed;
     return VIX_OK;
 }
 
@@ -1461,6 +1609,7 @@ int index_add_encoded_locked(vix_index* h, const int32_t* assign, const uint8_t*
     VIX_CUDA(cudaMemcpyAsync(h->assign.ptr + n0, assign, (size_t)n * 4, cudaMemcpyDefault, s));
     VIX_CUDA(cudaMemcpyAsync(h->codes.ptr + (size_t)n0 * h->code_bytes(), codes, (size_t)n * h->code_bytes(), cudaMemcpyDefault, s));
     h->n = n0 + n;
+    h->next_auto_id += n;
     h->dirty = true;
     return finish(true);
 }

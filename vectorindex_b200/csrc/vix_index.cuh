@@ -77,6 +77,8 @@ struct DevBuf {
         return VIX_OK;
     }
     void free_all() { if (ptr) cudaFree(ptr); ptr = nullptr; size = cap = 0; }
+    // take over a cudaMalloc'ed array of n elements (the old one is freed)
+    void adopt(T* p, size_t n) { free_all(); ptr = p; size = cap = n; }
     ~DevBuf() { free_all(); }
 };
 
@@ -96,11 +98,12 @@ struct vix_index {
     bool has_coarse = false, has_pq = false;
     // rows in add order
     int64_t n = 0;
+    int64_t next_auto_id = 0;           // first id of an add without ids: grows with every add, equals n until a removal
     DevBuf<float> vecs;                 // FLAT / IVF_FLAT: [n x d]
     DevBuf<int64_t> ids;                // [n]
     DevBuf<int32_t> assign;             // IVF: [n]
     DevBuf<uint8_t> codes;              // IVF_PQ: [n x m] AoS (the reference's interchange format)
-    // inverted lists, rebuilt lazily after adds ("slots": rows sorted by list, list starts 32-aligned)
+    // inverted lists, rebuilt lazily after adds and removals ("slots": rows sorted by list, list starts 32-aligned)
     bool dirty = true;
     int64_t nslots = 0;
     DevBuf<int64_t> list_off;           // [kc + 1] slot offsets (32-aligned)

@@ -145,6 +145,18 @@ class _Index:
 
     add = batch_insert
 
+    def batch_remove(self, ids) -> int:
+        """Removes every stored row whose id is in ``ids`` (numpy or torch, host or device; duplicates and ids that are not
+        stored are allowed; a row stored twice is removed twice).  Returns the number of rows removed.  The index then
+        answers exactly as one built from the remaining rows in their order."""
+        i = as_input(ids, np.int64).reshape(-1)
+        removed = C.c_int64(0)
+        check(lib().vix_index_remove(self._h, ptr(i, np.int64), C.c_int64(int(i.shape[0])), C.byref(removed)))
+        return int(removed.value)
+
+    def remove(self, id_: int) -> int:
+        return self.batch_remove(np.array([id_], dtype=np.int64))
+
     def clear(self):
         check(lib().vix_index_clear(self._h))
 
@@ -740,6 +752,18 @@ class ShardedIVFPQIndex:
                 r_assign, r_codes, r_ids = r_assign.numpy(), r_codes.numpy(), r_ids.numpy()
             self.local.add_encoded(r_assign, r_codes, r_ids)
 
+    def remove(self, ids) -> int:
+        """Collective: every rank passes the SAME ids (as for ``batch_search``) and removes the rows of them it holds;
+        returns the number of rows removed on all ranks together."""
+        n = self.local.batch_remove(ids)
+        if self.world == 1:
+            return n
+        import torch
+        import torch.distributed as dist
+        t = torch.tensor([n], dtype=torch.int64, device=self._comm_device())
+        dist.all_reduce(t, group=self.group)
+        return int(t.item())
+
     # ---- search
     def query_block(self, nq: int):
         """Rows of the batch whose probe lists THIS rank computes: (first row, rows, rows per rank)."""
@@ -884,6 +908,10 @@ class ReplicatedIVFPQIndex(ShardedIVFPQIndex):
 
     def set_list_bounds(self, bounds):
         raise ValueError("a replicated index has no list partition")
+
+    def remove(self, ids) -> int:
+        """Every replica removes the rows locally (no exchange); returns this replica's count, which is every replica's."""
+        return self.local.batch_remove(ids)
 
     def add(self, vectors, ids):
         import torch
