@@ -32,7 +32,6 @@
  *                            d = 2 m, ks = 256, nq x nprobe >= 32768)
  *   VIX_TC_SCAN_DEBUG=1      per launch (synchronises): queries handed back, finalists per query
  *   VIX_TC_SCAN_TIMES=1      CUDA events between the stages of every list-major launch, summed, printed at exit
- *   VIX_SCAN_DUAL=2          two query pipelines per SM in the query-major scan (an error where the shape cannot)
  *   VIX_DISABLE_TC, VIX_DISABLE_PQ_TC, VIX_DISABLE_LUT_IMAGE
  *                            exact CUDA-core kernels instead of the tensor-core shortlists / per-query tables built inside
  *                            the scan instead of batch-wide (the parity tests compare both ways)
@@ -377,29 +376,6 @@ int vix_index_probe_range(vix_index_t* h, const float* queries, int64_t nq, int 
                           int32_t* list_ids_out /* [nq x nprobe] */, float* list_scores_out /* nullable */);
 int vix_index_search_with_probes(vix_index_t* h, const float* queries, int64_t nq, int k, const int32_t* probes,
                                  int nprobe, float* out_dist, int64_t* out_ids);
-/* Packed records for the two exchange steps: key = orderable(score) << 32 | id (score = probe score, resp. API
- * distance; both ascend), so ascending key order is mergeTopK's (score, then smaller id) order (TopKMerge.swift:66-71).
- * ONE all-gather of 8-byte keys per step; the merges read the gathered [world x nq x kk] layout directly.
- *   vix_index_probe_range_keys  -> all-gather -> vix_merge_probe_keys   = the global probe lists [nq x nprobe]
- *   vix_index_search_with_probes_keys -> all-gather -> vix_merge_result_keys = the merged [nq x k] result
- * Unused slots are 0xFFFFFFFFFFFFFFFF (keys) / id -1, NaN (merged outputs). */
-int vix_index_probe_range_keys(vix_index_t* h, const float* queries, int64_t nq, int nprobe, int list_begin, int list_count,
-                               uint64_t* keys_out /* [nq x nprobe] */);
-int vix_merge_probe_keys(const uint64_t* keys_all /* [world x nq x nprobe] */, int world, int64_t nq, int nprobe,
-                         int32_t* probes_out /* [nq x nprobe] */);
-int vix_index_search_with_probes_keys(vix_index_t* h, const float* queries, int64_t nq, int k, const int32_t* probes,
-                                      int nprobe, uint64_t* keys_out /* [nq x k] */);
-int vix_merge_result_keys(const uint64_t* keys_all /* [world x nq x k] */, int world, int64_t nq, int k,
-                          float* out_dist, int64_t* out_ids /* [nq x k] */);
-/* The same two exchanges over PEER MEMORY (NVLink / NVSwitch) instead of NCCL: every rank owns a buffer of `world` slots
- * that is mapped into all peers (symmetric memory); peer_bufs_dev is a DEVICE array of the `world` buffer addresses.  A
- * rank's kernels store its block straight into slot `rank` of every peer's buffer; the caller then runs ONE barrier across
- * the ranks on the stream and merges from its own buffer (vix_merge_result_keys / the gathered probe ids).
- *   vix_peer_scatter_block                   any device block of a multiple of 16 bytes (the probe-list ids of the rank's query block)
- *   vix_index_search_with_probes_keys_peers  the fused scan, its local top-k packed and stored by the same call */
-int vix_peer_scatter_block(const void* src, size_t bytes, void* const* peer_bufs_dev, int world, int rank);
-int vix_index_search_with_probes_keys_peers(vix_index_t* h, const float* queries, int64_t nq, int k, const int32_t* probes,
-                                            int nprobe, void* const* peer_bufs_dev, int world, int rank);
 
 /* ---- the whole sharded step behind the C ABI: one process per GPU, one communicator per process ------------------
  * north_star: "the database shards by inverted list across the GPUs of one box; queries are broadcast, each GPU produces

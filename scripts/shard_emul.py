@@ -68,20 +68,3 @@ print(f"scan stage {st.ms_scan:.3f} ms, {st.code_bytes_scanned / 1e9:.3f} GB of 
       f"tail {st.cycles_tail / nq:.0f}); pieces per query: select {st.cycles_select / nq:.0f} probe table "
       f"{st.cycles_probe_table / nq:.0f} lut {st.cycles_lut / nq:.0f}; merge candidates per query "
       f"{st.merge_candidates / nq:.1f}")
-
-# A/B of the two-pipeline scan (VIX_SCAN_DUAL, read by the library per launch): same results, time per step
-ref = None
-for mode in ("0", "2"):
-    os.environ["VIX_SCAN_DUAL"] = mode
-    for _ in range(2):
-        dd, ii = idx.search_with_probes(q, k, probes)
-    a0, a1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    a0.record()
-    for _ in range(5):
-        dd, ii = idx.search_with_probes(q, k, probes)
-    a1.record()
-    torch.cuda.synchronize()
-    same = "" if ref is None else f"; equals one pipeline: ids {bool(torch.equal(ii, ref[1]))}, distance bits {bool(torch.equal(dd.view(torch.int32), ref[0].view(torch.int32)))}"
-    ref = ref or (dd.clone(), ii.clone())
-    print(f"VIX_SCAN_DUAL={mode}: search_with_probes {a0.elapsed_time(a1) / 5:.3f} ms per step{same}", flush=True)
-os.environ.pop("VIX_SCAN_DUAL", None)

@@ -1,6 +1,6 @@
 """One rank of the multi-GPU parity check (launched by tests/test_sharded_gpu.py under torch.distributed.run, one process
 per GPU): the native sharded step (vix_sharded_add / vix_sharded_search behind ShardedIVFPQIndex) against a single-GPU
-index holding all rows, against the oracle, and against the Python exchange path (VIX_PY_SHARDED=1)."""
+index holding all rows and against the oracle, over peer memory or, with VIX_NO_P2P=1, over NCCL all-gathers."""
 import os
 import sys
 
@@ -17,6 +17,44 @@ def same_as_single(si, sd, fi, fd, what):
     for r in diff:                                                          # ids may swap only at a tie inside the tolerance
         assert set(si[r]) == set(fi[r]) or abs(sd[r][-1] - fd[r][-1]) <= 2e-6 * abs(fd[r][-1]), f"{what}: row {r}"
     assert diff.size <= max(1, si.shape[0] // 50), f"{what}: {diff.size} rows differ in ids"
+
+
+def padded_shard_case(rank, world):
+    """The last rank owns one list of 4 vectors, so every query's local top-10 there is mostly padding keys: the merged
+    result must still equal a single-GPU index holding the same rows."""
+    import torch
+    from vectorindex_b200.index import IVFPQIndex, ShardedIVFPQIndex
+
+    n, d, m, kc, nq, k, nprobe, few = 6000, 96, 48, 64, 200, 10, 9, 4
+    rng = np.random.default_rng(8)
+    centres = rng.standard_normal((kc, d)).astype(np.float32)
+    home = np.concatenate([rng.integers(0, kc - 1, n - few), np.full(few, kc - 1)])     # list kc - 1 gets `few` rows
+    xb = (centres[home] + 0.3 * rng.standard_normal((n, d))).astype(np.float32)
+    qhome = np.concatenate([np.full(20, kc - 1), rng.integers(0, kc, nq - 20)])         # 20 queries probe the small list
+    q = (centres[qhome] + 0.3 * rng.standard_normal((nq, d))).astype(np.float32)
+    cb = (0.3 * rng.standard_normal((m, 256, d // m))).astype(np.float32)
+    ids = np.arange(n, dtype=np.int64) * 5 + 2
+    full = IVFPQIndex(d, "euclidean", nlist=kc, nprobe=nprobe, m=m)
+    full.set_coarse(centres)
+    full.set_codebooks(cb)
+    full.batch_insert(xb, ids)
+    assert np.bincount(full.export_lists()[3], minlength=kc)[kc - 1] == few
+    fd, fi = full.batch_search(q, k)
+    local = IVFPQIndex(d, "euclidean", nlist=kc, nprobe=nprobe, m=m)
+    local.set_coarse(centres)
+    local.set_codebooks(cb)
+    sh = ShardedIVFPQIndex.wrap(local, kc, nprobe)
+    sh.set_list_bounds(np.concatenate([np.linspace(0, kc - 1, world).round(), [kc]]).astype(np.int64))
+    mine = np.arange(rank, n, world)
+    sh.add(torch.from_numpy(xb[mine]).cuda(), torch.from_numpy(ids[mine]).cuda())
+    if rank == world - 1:
+        assert local.count == few, local.count
+    sd, si = sh.batch_search(q, k)
+    assert (si >= 0).all() and np.array_equal(si, fi), "padded shard: ids"
+    same_as_single(si, sd, fi, fd, "padded shard")
+    if rank == 0:
+        print(f"ok padded shard: world {world}, the last rank holds {few} rows", flush=True)
+    sh.comm.close()
 
 
 def main():
@@ -97,6 +135,7 @@ def main():
         if rank == 0:
             print(f"ok {metric}: world {world}, peer memory {peer}, {n} rows, top-k overlap with the oracle {same:.4f}", flush=True)
         sh.comm.close()
+    padded_shard_case(rank, world)
     dist.barrier()
     dist.destroy_process_group()
 

@@ -700,33 +700,6 @@ def test_batchwide_tables_equal_in_kernel_tables(oracle, monkeypatch, d, metric)
     assert np.array_equal(i1, i2) and np.array_equal(bits(d1), bits(d2))
 
 
-@pytest.mark.parametrize("d,m,metric,nq,k,filtered", [
-    (96, 48, "euclidean", 700, 10, False),     # C5-shaped: three shared 64 KB tables
-    (128, 16, "euclidean", 333, 10, False),    # one table, both pipelines in its two half rows
-    (128, 32, "dotProduct", 301, 32, False),   # k = 32: the queues hold k + 32 entries, a flush per accepted chunk
-    (96, 48, "euclidean", 1, 5, False),        # one query: the second pipeline finds no work
-    (128, 32, "euclidean", 257, 10, True),     # id filter
-])
-def test_two_pipeline_scan_equals_one_pipeline(oracle, monkeypatch, d, m, metric, nq, k, filtered):
-    """ivfpq_scan_kernel<G, FILTER, false, 2> (two query pipelines of 8 warps per CTA) looks up the same tables in the same
-    order as the one-pipeline kernel and selects by the same total order: identical ids and distance bits."""
-    from vectorindex_b200.index import IDFilter, IVFPQIndex
-    n, kc, nprobe = 30000, 48, 12
-    xb, q, coarse, cb, norms = _make_ivfpq_problem(oracle, n, d, m, kc, nq, seed=d + m + k)
-    idx = IVFPQIndex(d, metric, nlist=kc, nprobe=nprobe, m=m)
-    idx.set_coarse(coarse); idx.set_codebooks(cb, norms)
-    idx.batch_insert(xb)
-    flt = None
-    if filtered:
-        flt = IDFilter(n, "allow")
-        flt.set(np.arange(0, n, 3))
-    monkeypatch.delenv("VIX_SCAN_DUAL", raising=False)
-    d1, i1 = idx.batch_search(q, k, filter=flt)
-    monkeypatch.setenv("VIX_SCAN_DUAL", "2")                         # 2: a launch that cannot take two pipelines is an error
-    d2, i2 = idx.batch_search(q, k, filter=flt)
-    assert np.array_equal(i1, i2) and np.array_equal(bits(d1), bits(d2))
-
-
 @pytest.mark.parametrize("d,m,n,kc,nq,nprobe,k,kind", [
     (96, 48, 60000, 64, 600, 12, 10, "unit"),      # C5-shaped: three groups of 16 sub-quantisers (the last one read through its replica)
     (32, 16, 30000, 40, 300, 8, 10, "gauss"),      # one group
@@ -797,82 +770,6 @@ def test_sharded_pieces_emulated_on_one_gpu(oracle):
     md, mi = vk.mergeTopK(dd, ii, k, 0)
     assert np.array_equal(mi, si)
     assert np.array_equal(bits(md), bits(sd))
-
-
-@pytest.mark.parametrize("metric", ["euclidean", "dotProduct"])
-def test_sharded_key_exchange_emulated_on_one_gpu(oracle, metric):
-    """The packed-record exchange of the NCCL path (probe_range_keys -> gather -> merge_probe_keys ->
-    search_with_probes_keys -> gather -> merge_result_keys), three list-block shards emulated in one process with the
-    all-gathers replaced by np.stack: probe lists, ids and distance bits equal the single index's."""
-    from vectorindex_b200.index import IVFPQIndex, list_block, list_owner, merge_probe_keys, merge_result_keys
-    n, d, m, kc, nq, k, nprobe, world = 7000, 64, 16, 45, 40, 10, 7, 3
-    xb, q, coarse, cb, norms = _make_ivfpq_problem(oracle, n, d, m, kc, nq, seed=17)
-    ids = np.arange(n, dtype=np.int64) * 3 + 1
-    single = IVFPQIndex(d, metric, nlist=kc, nprobe=nprobe, m=m)
-    single.set_coarse(coarse); single.set_codebooks(cb, norms)
-    single.batch_insert(xb, ids)
-    sd, si, sp = single.batch_search(q, k, return_probes=True)
-    shards = []
-    for r in range(world):
-        ix = IVFPQIndex(d, metric, nlist=kc, nprobe=nprobe, m=m)
-        ix.set_coarse(coarse); ix.set_codebooks(cb, norms)
-        shards.append(ix)
-    asg, codes = shards[0].encode(xb)
-    owner = list_owner(asg.astype(np.int64), kc, world)
-    for r in range(world):
-        sel = owner == r
-        shards[r].add_encoded(asg[sel], codes[sel], ids[sel])
-    pk = np.stack([shards[r].probe_range_keys(q, nprobe, *list_block(kc, r, world)) for r in range(world)])
-    assert pk.dtype == np.uint64 and pk.shape == (world, nq, nprobe)
-    gp = merge_probe_keys(pk)
-    assert gp.dtype == np.int32 and np.array_equal(gp, sp)
-    rk = np.stack([shards[r].search_with_probes_keys(q, k, gp) for r in range(world)])
-    md, mi = merge_result_keys(rk)
-    assert np.array_equal(mi, si)
-    assert np.array_equal(bits(md), bits(sd))
-    # fewer than k vectors in the probed lists of a shard -> padded keys, merged result unaffected
-    tiny = IVFPQIndex(d, metric, nlist=kc, nprobe=nprobe, m=m)
-    tiny.set_coarse(coarse); tiny.set_codebooks(cb, norms)
-    tiny.add_encoded(asg[:3], codes[:3], ids[:3])
-    tk = tiny.search_with_probes_keys(q, k, gp)
-    assert (tk == np.uint64(0xFFFFFFFFFFFFFFFF)).sum() >= nq * (k - 3)
-    md2, mi2 = merge_result_keys(np.stack([tk, np.full_like(tk, 0xFFFFFFFFFFFFFFFF)]))
-    assert np.array_equal(mi2 >= 0, ~np.isnan(md2))
-
-
-def test_peer_memory_exchange_entry_points_on_one_gpu(oracle):
-    """vix_peer_scatter_block / vix_index_search_with_probes_keys_peers with two "peers" that are two buffers of the same
-    GPU (on a multi-GPU box they are symmetric-memory mappings of the other ranks): every peer's slot `rank` receives the
-    block, and the packed keys equal those of vix_index_search_with_probes_keys."""
-    import ctypes as C
-    import torch
-    from vectorindex_b200._lib import check, lib, ptr
-    from vectorindex_b200.index import IVFPQIndex
-    dev = torch.device("cuda", 0)
-    world, rank = 2, 1
-    block = torch.arange(4 * 1024, dtype=torch.int32, device=dev)
-    bufs = [torch.full((world, block.numel()), -7, dtype=torch.int32, device=dev) for _ in range(world)]
-    table = torch.tensor([b.data_ptr() for b in bufs], dtype=torch.int64, device=dev)
-    check(lib().vix_peer_scatter_block(ptr(block), C.c_size_t(block.numel() * 4), C.c_void_p(table.data_ptr()), C.c_int(world),
-                                       C.c_int(rank)))
-    torch.cuda.synchronize()
-    for b in bufs:
-        assert torch.equal(b[rank], block) and (b[0] == -7).all()
-    n, d, m, kc, nq, k, nprobe = 5000, 64, 16, 24, 40, 10, 5
-    xb, q, coarse, cb, norms = _make_ivfpq_problem(oracle, n, d, m, kc, nq, seed=8)
-    idx = IVFPQIndex(d, "euclidean", nlist=kc, nprobe=nprobe, m=m)
-    idx.set_coarse(coarse); idx.set_codebooks(cb, norms)
-    idx.batch_insert(xb)
-    _, _, probes = idx.batch_search(q, k, return_probes=True)
-    want = torch.from_numpy(idx.search_with_probes_keys(q, k, probes).view(np.int64)).to(dev)
-    kb = [torch.zeros((world, nq, k), dtype=torch.int64, device=dev) for _ in range(world)]
-    ktab = torch.tensor([b.data_ptr() for b in kb], dtype=torch.int64, device=dev)
-    qd, pd = torch.from_numpy(q).to(dev), torch.from_numpy(probes).to(dev)
-    check(lib().vix_index_search_with_probes_keys_peers(idx._h, ptr(qd), C.c_int64(nq), C.c_int(k), ptr(pd), C.c_int(nprobe),
-                                                        C.c_void_p(ktab.data_ptr()), C.c_int(world), C.c_int(rank)))
-    torch.cuda.synchronize()
-    for b in kb:
-        assert torch.equal(b[rank], want) and (b[0] == 0).all()
 
 
 @pytest.mark.parametrize("mode", ["allow", "deny"])

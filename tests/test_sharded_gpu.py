@@ -81,4 +81,4 @@ def test_two_ranks_under_torchrun(no_p2p):
            "--master-port", "29533", os.path.join(ROOT, "tests", "mp_sharded_check.py")]
     out = subprocess.run(cmd, capture_output=True, text=True, timeout=900, env=env)
     assert out.returncode == 0, out.stdout[-3000:] + out.stderr[-3000:]
-    assert "ok euclidean" in out.stdout and "ok dotProduct" in out.stdout
+    assert "ok euclidean" in out.stdout and "ok dotProduct" in out.stdout and "ok padded shard" in out.stdout

@@ -90,9 +90,7 @@ _EXPORTS = [
     "vix_index_set_codebooks", "vix_index_get_coarse", "vix_index_get_codebooks", "vix_index_add", "vix_index_remove",
     "vix_index_import_lists", "vix_index_count", "vix_index_list_sizes", "vix_index_export_lists", "vix_index_clear",
     "vix_index_search", "vix_index_search_ex", "vix_index_search_rerank", "vix_index_trace", "vix_index_trace_get", "vix_index_probe_range", "vix_index_search_with_probes",
-    "vix_index_search_with_probes_ex", "vix_index_search_filtered", "vix_index_probe_range_keys", "vix_merge_probe_keys",
-    "vix_index_search_with_probes_keys", "vix_merge_result_keys", "vix_peer_scatter_block",
-    "vix_index_search_with_probes_keys_peers",
+    "vix_index_search_with_probes_ex", "vix_index_search_filtered",
     "vix_comm_unique_id", "vix_comm_create", "vix_comm_destroy", "vix_comm_rank", "vix_comm_world",
     "vix_comm_uses_peer_memory", "vix_comm_trace", "vix_comm_trace_get", "vix_sharded_query_block", "vix_sharded_add", "vix_sharded_search",
     "vix_index_encode", "vix_index_add_encoded", "vix_debug_tc_scores_f32", "vix_debug_tc_codes", "vix_accel_rank_candidates_f32",

@@ -489,7 +489,7 @@ bool supported(int64_t nA, int64_t nB, int d, const float* A, const float* B) {
 
 // rows resident (ARES) when both A buffers and the B ring fit: d <= 128
 // (d <= 96: both A buffers + three 32 KB B stages; at d = 128 only two B stages would be left, so A streams there)
-static bool a_resident(int kblocks) { return kblocks <= 3 && getenv("VIX_TC_NO_ARES") == nullptr; }
+static bool a_resident(int kblocks) { return kblocks <= 3; }
 static int ring_stages(int kblocks) {
     if (!a_resident(kblocks)) return kStages;
     const size_t left = 227 * 1024 - 12 * 1024 - (size_t)2 * kblocks * kM * kKB * 4;
@@ -510,11 +510,9 @@ static int launch(const float* A, int64_t nA, const float* B, int nB, int d, Arg
     a.kblocks = (d + kKB - 1) / kKB;
     a.ntiles = (nB + kN - 1) / kN;
     a.mtiles = (int)((nA + kM - 1) / kM);
-    // column splits: enough work items for ~3 waves of the SMs; in MODE_MIN a split is a whole number of groups
-    // (eight waves: with three, the last wave of C5's probe stage ran a fifth of the SMs)
-    const char* wv = getenv("VIX_TC_WAVES");
-    const int waves = wv ? atoi(wv) : 8;
-    int nsplit = (waves * num_sms() + a.mtiles - 1) / a.mtiles;
+    // column splits: enough work items for eight waves of the SMs (with three, the last wave of C5's probe stage ran a
+    // fifth of the SMs); in MODE_MIN a split is a whole number of groups
+    int nsplit = (8 * num_sms() + a.mtiles - 1) / a.mtiles;
     if (nsplit < 1) nsplit = 1;
     if (nsplit > a.ntiles) nsplit = a.ntiles;
     int tps = (a.ntiles + nsplit - 1) / nsplit;

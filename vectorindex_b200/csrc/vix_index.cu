@@ -1337,226 +1337,6 @@ int vix_index_probe_range(vix_index_t* h, const float* queries, int64_t nq, int 
     return finish(di.is_host() || ds.is_host());
 }
 
-// ---- packed records for the two exchange steps of a sharded search ------------------------------------------
-// key = orderable(score) << 32 | id: ascending key order is the (score, then smaller id) order of mergeTopK
-// (TopKMerge.swift:66-71), so ONE all-gather of 8-byte keys per step replaces separate score / id gathers and
-// the merge is a selection of the smallest keys.  order_max (inner product) keys hold the complemented score,
-// exactly as the selection queues of the scan do.
-__global__ void pack_keys_kernel(const float* __restrict__ score, const int32_t* __restrict__ id32,
-                                 const int64_t* __restrict__ id64, int64_t total, int negate, int order_max,
-                                 u64* __restrict__ keys) {
-    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= total) return;
-    const int64_t id = id32 ? (int64_t)id32[i] : id64[i];
-    const float sc = negate ? -score[i] : score[i];
-    keys[i] = id < 0 ? kEmptyKey : make_key(sc, (uint32_t)id, order_max);
-}
-
-// keys_all: [world][nq][kk] as all-gathered; one CTA per query selects the kk smallest of its world x kk keys
-__global__ void merge_shard_keys_kernel(const u64* __restrict__ keys_all, int world, int64_t nq, int kk, int P2,
-                                        int order_max, int negate, int32_t* __restrict__ out_id32,
-                                        float* __restrict__ out_score, int64_t* __restrict__ out_id64) {
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    u64* s = reinterpret_cast<u64*>(smem_raw);
-    const int64_t row = blockIdx.x;
-    const int nin = world * kk;
-    for (int i = threadIdx.x; i < P2; i += blockDim.x) {
-        u64 key = kEmptyKey;
-        if (i < nin) { const int r = i / kk, j = i - r * kk; key = keys_all[((size_t)r * nq + row) * kk + j]; }
-        s[i] = key;
-    }
-    __syncthreads();
-    bitonic_sort_keys<false>(s, P2, threadIdx.x, blockDim.x);
-    for (int i = threadIdx.x; i < kk; i += blockDim.x) {
-        const u64 key = s[i];
-        const size_t o = (size_t)row * kk + i;
-        if (key == kEmptyKey) {
-            if (out_id32) out_id32[o] = -1;
-            if (out_score) out_score[o] = __int_as_float(0x7fc00000);
-            if (out_id64) out_id64[o] = -1;
-        } else {
-            const float sc = key_score(key, order_max);
-            if (out_id32) out_id32[o] = (int32_t)key_id(key);
-            if (out_score) out_score[o] = negate ? -sc : sc;
-            if (out_id64) out_id64[o] = (int64_t)key_id(key);
-        }
-    }
-}
-
-}  // extern "C"
-namespace vix {
-int merge_shard_keys(const u64* keys_all, int world, int64_t nq, int kk, int order_max, int negate,
-                            int32_t* out_id32, float* out_score, int64_t* out_id64) {
-    const int P2 = next_pow2(world * kk < 2 ? 2 : world * kk);
-    const size_t smem = (size_t)P2 * 8;
-    VIX_REQUIRE(smem <= 200 * 1024, VIX_ERR_UNSUPPORTED, "shard merge: %d keys per query exceed shared memory", world * kk);
-    VIX_CUDA(cudaFuncSetAttribute(merge_shard_keys_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    const int threads = P2 / 2 < 32 ? 32 : (P2 / 2 > 256 ? 256 : P2 / 2);
-    merge_shard_keys_kernel<<<(unsigned)nq, threads, smem, ctx().stream>>>(keys_all, world, nq, kk, P2, order_max, negate,
-                                                                         out_id32, out_score, out_id64);
-    VIX_LAUNCH_CHECK();
-    return VIX_OK;
-}
-}  // namespace vix
-extern "C" {
-
-int vix_index_probe_range_keys(vix_index_t* h, const float* queries, int64_t nq, int nprobe, int list_begin, int list_count,
-                               uint64_t* keys_out) {
-    VIX_TRY(ensure_device());
-    VIX_REQUIRE(h && queries && keys_out, VIX_ERR_NULL_PTR, "vix_index_probe_range_keys: null pointer");
-    std::lock_guard<std::mutex> lk(h->mu);
-    VIX_REQUIRE(h->has_coarse, VIX_ERR_NOT_TRAINED, "vix_index_probe_range_keys: not trained");
-    VIX_REQUIRE(h->p.metric != VIX_METRIC_COSINE, VIX_ERR_UNSUPPORTED, "vix_index_probe_range_keys: cosine indexes are not sharded");
-    VIX_REQUIRE(nprobe > 0 && nprobe <= VIX_MAX_K, VIX_ERR_INVALID_K, "vix_index_probe_range_keys: nprobe");
-    VIX_REQUIRE(list_begin >= 0 && list_count > 0 && list_begin + list_count <= h->kc, VIX_ERR_INVALID_PARAM,
-                "vix_index_probe_range_keys: list range [%d, %d) outside [0, %d)", list_begin, list_begin + list_count, h->kc);
-    if (nq <= 0) return VIX_OK;
-    const int d = h->p.d;
-    const int64_t total = nq * (int64_t)nprobe;
-    In<float> dq;
-    Out<u64> dk;
-    Scratch<int32_t> ids;
-    Scratch<float> sc;
-    VIX_TRY(dq.stage(queries, (size_t)nq * d));
-    VIX_TRY(dk.stage(reinterpret_cast<u64*>(keys_out), (size_t)total));
-    VIX_TRY(ids.alloc((size_t)total));
-    VIX_TRY(sc.alloc((size_t)total));
-    VIX_TRY(probe_select_fast_device(dq.dev, nq, h->coarse.ptr + (size_t)list_begin * d, list_count, d, h->p.metric, nprobe,
-                                     h->coarse_norms.ptr + list_begin, ids.ptr, sc.ptr, h->coarse_norm_max.ptr));
-    if (list_begin > 0) {
-        offset_ids_kernel<<<(unsigned)((total + 255) / 256), 256, 0, ctx().stream>>>(ids.ptr, total, list_begin);
-        VIX_LAUNCH_CHECK();
-    }
-    // probe scores are "smaller is better" for both metrics (CentroidBatchScore.swift:54-64): plain ascending keys
-    pack_keys_kernel<<<(unsigned)((total + 255) / 256), 256, 0, ctx().stream>>>(sc.ptr, ids.ptr, nullptr, total, 0, 0, dk.dev);
-    VIX_LAUNCH_CHECK();
-    VIX_TRY(dk.commit());
-    return finish(dk.is_host());
-}
-
-int vix_merge_probe_keys(const uint64_t* keys_all, int world, int64_t nq, int nprobe, int32_t* probes_out) {
-    VIX_TRY(ensure_device());
-    VIX_REQUIRE(keys_all && probes_out, VIX_ERR_NULL_PTR, "vix_merge_probe_keys: null pointer");
-    VIX_REQUIRE(world > 0 && nprobe > 0, VIX_ERR_INVALID_K, "vix_merge_probe_keys: world / nprobe must be > 0");
-    if (nq <= 0) return VIX_OK;
-    In<u64> dk;
-    Out<int32_t> dp;
-    VIX_TRY(dk.stage(reinterpret_cast<const u64*>(keys_all), (size_t)world * nq * nprobe));
-    VIX_TRY(dp.stage(probes_out, (size_t)nq * nprobe));
-    VIX_TRY(merge_shard_keys(dk.dev, world, nq, nprobe, 0, 0, dp.dev, nullptr, nullptr));
-    VIX_TRY(dp.commit());
-    return finish(dp.is_host());
-}
-
-int vix_index_search_with_probes_keys(vix_index_t* h, const float* queries, int64_t nq, int k, const int32_t* probes,
-                                      int nprobe, uint64_t* keys_out) {
-    VIX_TRY(ensure_device());
-    VIX_REQUIRE(h && probes && keys_out, VIX_ERR_NULL_PTR, "vix_index_search_with_probes_keys: null pointer");
-    VIX_REQUIRE(nprobe > 0, VIX_ERR_INVALID_K, "vix_index_search_with_probes_keys: nprobe must be > 0");
-    std::lock_guard<std::mutex> lk(h->mu);
-    VIX_REQUIRE(h->p.kind != VIX_INDEX_FLAT && h->has_coarse, VIX_ERR_NOT_TRAINED, "vix_index_search_with_probes_keys: IVF index not trained");
-    if (nq <= 0 || k <= 0) return VIX_OK;
-    const int64_t total = nq * (int64_t)k;
-    Out<u64> dk;
-    Scratch<float> dist;
-    Scratch<int64_t> ids;
-    VIX_TRY(dk.stage(reinterpret_cast<u64*>(keys_out), (size_t)total));
-    VIX_TRY(dist.alloc((size_t)total));
-    VIX_TRY(ids.alloc((size_t)total));
-    In<float> dq;                                      // staged once here: the search below then sees a device pointer
-    VIX_TRY(dq.stage(queries, (size_t)nq * h->p.d));
-    In<int32_t> dpr;
-    VIX_TRY(dpr.stage(probes, (size_t)nq * nprobe));
-    VIX_TRY(index_search_locked(h, dq.dev, nq, k, nprobe, dist.ptr, ids.ptr, nullptr, nullptr, dpr.dev));
-    // API distances ascend for both metrics (inner product: -dot, DistanceUtils.swift:40-46)
-    pack_keys_kernel<<<(unsigned)((total + 255) / 256), 256, 0, ctx().stream>>>(dist.ptr, nullptr, ids.ptr, total, 0, 0, dk.dev);
-    VIX_LAUNCH_CHECK();
-    VIX_TRY(dk.commit());
-    return finish(dk.is_host());
-}
-
-// ---- the exchange steps over PEER MEMORY (NVLink / NVSwitch) instead of NCCL ------------------------------------
-// Every rank owns a buffer of `world` slots mapped into all peers (symmetric memory: torch's _SymmetricMemory in this
-// repo, cuMemMap'ed / IPC allocations from another host); `peer_bufs` is a DEVICE array of the `world` buffer addresses.
-// A rank stores its block straight into slot `rank` of every peer's buffer -- the all-gather IS the producing kernel's
-// store pattern -- and the caller then runs one barrier across the ranks on the stream.
-__global__ void peer_scatter_kernel(const uint4* __restrict__ src, int64_t n16, void* const* __restrict__ peer_bufs,
-                                    int world, int64_t slot16) {
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n16; i += (int64_t)gridDim.x * blockDim.x) {
-        const uint4 v = src[i];
-        for (int p = 0; p < world; ++p) reinterpret_cast<uint4*>(peer_bufs[p])[slot16 + i] = v;
-    }
-}
-
-// the local top-k of a sharded search packed into keys and stored into slot `rank` of every peer's [world x nq x k] buffer
-__global__ void pack_keys_to_peers_kernel(const float* __restrict__ score, const int64_t* __restrict__ id64, int64_t total,
-                                          void* const* __restrict__ peer_bufs, int world, int64_t slot) {
-    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= total) return;
-    const int64_t id = id64[i];
-    const u64 key = id < 0 ? kEmptyKey : make_key(score[i], (uint32_t)id, 0);
-    for (int p = 0; p < world; ++p) reinterpret_cast<u64*>(peer_bufs[p])[slot + i] = key;
-}
-
-int vix_peer_scatter_block(const void* src, size_t bytes, void* const* peer_bufs_dev, int world, int rank) {
-    VIX_TRY(ensure_device());
-    VIX_REQUIRE(src && peer_bufs_dev, VIX_ERR_NULL_PTR, "vix_peer_scatter_block: null pointer");
-    VIX_REQUIRE(world > 0 && rank >= 0 && rank < world, VIX_ERR_INVALID_PARAM, "vix_peer_scatter_block: rank / world");
-    VIX_REQUIRE(bytes % 16 == 0 && is_device_ptr(src), VIX_ERR_INVALID_PARAM,
-                "vix_peer_scatter_block: the block must be a device buffer of a multiple of 16 bytes");
-    if (bytes == 0) return VIX_OK;
-    const int64_t n16 = (int64_t)(bytes / 16);
-    const int64_t want = (n16 + 255) / 256;
-    const unsigned grid = (unsigned)(want < 4 * num_sms() ? want : 4 * num_sms());
-    peer_scatter_kernel<<<grid, 256, 0, ctx().stream>>>(static_cast<const uint4*>(src), n16, peer_bufs_dev, world,
-                                                        (int64_t)rank * n16);
-    VIX_LAUNCH_CHECK();
-    return finish(false);
-}
-
-int vix_index_search_with_probes_keys_peers(vix_index_t* h, const float* queries, int64_t nq, int k, const int32_t* probes,
-                                            int nprobe, void* const* peer_bufs_dev, int world, int rank) {
-    VIX_TRY(ensure_device());
-    VIX_REQUIRE(h && probes && peer_bufs_dev, VIX_ERR_NULL_PTR, "vix_index_search_with_probes_keys_peers: null pointer");
-    VIX_REQUIRE(nprobe > 0, VIX_ERR_INVALID_K, "vix_index_search_with_probes_keys_peers: nprobe must be > 0");
-    VIX_REQUIRE(world > 0 && rank >= 0 && rank < world, VIX_ERR_INVALID_PARAM, "vix_index_search_with_probes_keys_peers: rank / world");
-    std::lock_guard<std::mutex> lk(h->mu);
-    VIX_REQUIRE(h->p.kind != VIX_INDEX_FLAT && h->has_coarse, VIX_ERR_NOT_TRAINED,
-                "vix_index_search_with_probes_keys_peers: IVF index not trained");
-    if (nq <= 0 || k <= 0) return VIX_OK;
-    const int64_t total = nq * (int64_t)k;
-    Scratch<float> dist;
-    Scratch<int64_t> ids;
-    VIX_TRY(dist.alloc((size_t)total));
-    VIX_TRY(ids.alloc((size_t)total));
-    In<float> dq;
-    VIX_TRY(dq.stage(queries, (size_t)nq * h->p.d));
-    In<int32_t> dpr;
-    VIX_TRY(dpr.stage(probes, (size_t)nq * nprobe));
-    VIX_TRY(index_search_locked(h, dq.dev, nq, k, nprobe, dist.ptr, ids.ptr, nullptr, nullptr, dpr.dev));
-    pack_keys_to_peers_kernel<<<(unsigned)((total + 255) / 256), 256, 0, ctx().stream>>>(dist.ptr, ids.ptr, total, peer_bufs_dev,
-                                                                                       world, (int64_t)rank * total);
-    VIX_LAUNCH_CHECK();
-    return finish(false);
-}
-
-int vix_merge_result_keys(const uint64_t* keys_all, int world, int64_t nq, int k, float* out_dist, int64_t* out_ids) {
-    VIX_TRY(ensure_device());
-    VIX_REQUIRE(keys_all && out_dist && out_ids, VIX_ERR_NULL_PTR, "vix_merge_result_keys: null pointer");
-    VIX_REQUIRE(world > 0 && k > 0, VIX_ERR_INVALID_K, "vix_merge_result_keys: world / k must be > 0");
-    if (nq <= 0) return VIX_OK;
-    In<u64> dk;
-    Out<float> dd;
-    Out<int64_t> di;
-    VIX_TRY(dk.stage(reinterpret_cast<const u64*>(keys_all), (size_t)world * nq * k));
-    VIX_TRY(dd.stage(out_dist, (size_t)nq * k));
-    VIX_TRY(di.stage(out_ids, (size_t)nq * k));
-    VIX_TRY(merge_shard_keys(dk.dev, world, nq, k, 0, 0, nullptr, dd.dev, di.dev));
-    VIX_TRY(dd.commit());
-    VIX_TRY(di.commit());
-    return finish(dd.is_host() || di.is_host());
-}
-
 int vix_index_encode(vix_index_t* h, const float* x, int64_t n, int32_t* assign_out, uint8_t* codes_out) {
     VIX_TRY(ensure_device());
     VIX_REQUIRE(h && x && assign_out, VIX_ERR_NULL_PTR, "vix_index_encode: null pointer");

@@ -142,9 +142,6 @@ int index_search_locked(vix_index* h, const float* queries, int64_t nq, int k, i
 int assign_lists_device(vix_index* h, const float* x, int64_t n, int32_t* assign);
 // number of assignments outside [0, kc) in a device array (synchronises the stream)
 int count_invalid_assign(const int32_t* assign, int64_t n, int kc, unsigned long long* out);
-// keys_all [world][nq][kk] -> the kk smallest keys per query (device pointers)
-int merge_shard_keys(const u64* keys_all, int world, int64_t nq, int kk, int order_max, int negate,
-                     int32_t* out_id32, float* out_score, int64_t* out_id64);
 // append already encoded rows (device or host pointers) to an IVF-PQ index whose mutex the caller holds
 int index_add_encoded_locked(vix_index* h, const int32_t* assign, const uint8_t* codes, const int64_t* ids, int64_t n);
 int build_lists(vix_index* h);

@@ -82,18 +82,12 @@ __device__ __forceinline__ void lookup2(uint32_t a0, uint32_t a1, unsigned long 
         : "r"(a0), "r"(a1), "n"(IMM));
 }
 
-// Two query pipelines per CTA (PIPES == 2, see ivfpq_scan_kernel): the tables cannot start at a 64 KB boundary of the
-// shared window any more (3 x 64 KB + bookkeeping > 227 KB), so they start at the FIXED shared address kDualTab, which
-// travels in the LDS immediate, and end exactly at the end of the 228 KB window.
-constexpr uint32_t kDualTab = 36 * 1024;
-constexpr int kDualWarps = 8;                    // warps per pipeline
-
 // one group of 16 sub-quantisers: 16 look-ups of one lane, 4 running sums kept as two f32x2 pairs (s0, s1), (s2, s3).
-// PIPES == 1: table T / 2, half row T % 2.  PIPES == 2: table T, half row = pipeline (part of the lane constants).
-template <int T, int PIPES = 1>
+// Group T: table T / 2, half row T % 2.
+template <int T>
 __device__ __forceinline__ void lookup16(const uint4& w, const uint32_t (&pre)[8], unsigned long long& s01,
                                          unsigned long long& s23) {
-    constexpr int IMM = PIPES == 1 ? (T & 1) * 128 + (T >> 1) * 65536 : (int)kDualTab + T * 65536;
+    constexpr int IMM = (T & 1) * 128 + (T >> 1) * 65536;
     const uint32_t x[4] = {w.x, w.y, w.z, w.w};
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
@@ -213,10 +207,9 @@ __device__ VIX_SCAN_FN void build_probe_table(const float* __restrict__ q, int d
 // codebooks_t is [256][M][dsub], so the M threads of a code read consecutive memory.  The build is bound by the
 // latency of those (L2-resident) reads, so as many codes as the registers hold are in flight per thread: all of
 // a thread's codes at dsub = 2 (one round trip), eight otherwise.  The two replicas of an entry are written in
-// opposite order by the two half-warps, so a warp-wide store touches 32 different banks.
-// PIPE < 0: the one-pipeline layout (group t16 in table t16 / 2, half row t16 % 2); PIPE = 0 / 1: the two-pipeline layout
-// (group t16 in table t16, half row PIPE).
-template <int M, int PIPE = -1>
+// opposite order by the two half-warps, so a warp-wide store touches 32 different banks.  Group t16 goes to table t16 / 2,
+// half row t16 % 2.
+template <int M>
 __device__ VIX_SCAN_FN void build_lut(float* __restrict__ s_lut, const float* __restrict__ q,
                                       const float* __restrict__ codebooks_t, int dsub, float lut_scale, int t, int nthr) {
     const int ngroups = nthr / M;
@@ -224,9 +217,7 @@ __device__ VIX_SCAN_FN void build_lut(float* __restrict__ s_lut, const float* __
     const int j = t % M, c0 = t / M;
     const int rep_first = (threadIdx.x & 31) >> 4;
     const int t16 = j >> 4;
-    float* col;
-    if constexpr (PIPE < 0) col = s_lut + (t16 >> 1) * 16384 + (t16 & 1) * 32 + (j & 15);
-    else col = s_lut + t16 * 16384 + PIPE * 32 + (j & 15);
+    float* col = s_lut + (t16 >> 1) * 16384 + (t16 & 1) * 32 + (j & 15);
     float* colA = col + 16 * rep_first;
     float* colB = col + 16 * (rep_first ^ 1);
     constexpr int U = 8;
@@ -394,39 +385,21 @@ __device__ __noinline__ uint32_t flush_queue(u64* wq, int Pw, int k, int cnt, bo
 
 // m = 16 G; FILTER: an id filter is active; STATS: the phase counters of vix_search_stats are kept (separate
 // instantiations, so the production kernel pays neither in instructions nor in registers).
-//
-// PIPES == 2 (opt-in, VIX_SCAN_DUAL=1; G <= 3): the 16 warps form TWO independent query pipelines of 8 warps, each with
-// its own bookkeeping, work items, threshold, selection queues and named barrier, so the per-query serial part of one
-// (table build between two barriers) hides behind the other's scan -- what matters when a query's share of the lists is
-// short (one rank of a sharded index).  Tables: group t of pipeline p is the half row p of table t (3 x 64 KB at M = 48,
-// [A g0 | B g0][A g1 | B g1][A g2 | B g2]); the half-row select rides in the lane constants, so both pipelines run the
-// same instruction stream.  `tid`, `warp`, `nwarps` below are pipeline-local.
-template <int G, bool FILTER, bool STATS, int PIPES = 1>
+template <int G, bool FILTER, bool STATS>
 __global__ void __launch_bounds__(kFastThreads, 1)
 ivfpq_scan_kernel(ScanArgs a) {
     constexpr int m = 16 * G;
-    constexpr int NTAB = PIPES == 1 ? (G + 1) / 2 : G;
+    constexpr int NTAB = (G + 1) / 2;
     constexpr int kGrab = 4;                             // largest run of chunks handed to a warp at once
-    static_assert(PIPES == 1 || (PIPES == 2 && G <= 3), "two pipelines: at most three 64 KB tables");
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    const int pipe = PIPES == 1 ? 0 : (int)(threadIdx.x >> 8);
-    const int tid = PIPES == 1 ? (int)threadIdx.x : (int)(threadIdx.x & 255u), lane = tid & 31, warp = tid >> 5;
-    const int nwarps = PIPES == 1 ? (int)(blockDim.x >> 5) : kDualWarps;
-    const int nthreads = PIPES == 1 ? (int)blockDim.x : 32 * kDualWarps;
-    // barrier of one pipeline: the whole CTA, or the pipeline's 256 threads on named barrier 1 + pipe
-    auto pipe_sync = [&]() {
-        if constexpr (PIPES == 1) __syncthreads();
-        else asm volatile("bar.sync %0, %1;" ::"r"(pipe + 1), "n"(32 * kDualWarps) : "memory");
-    };
+    const int tid = (int)threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int nwarps = (int)(blockDim.x >> 5);
 
-    // ---- shared-memory map: bookkeeping first (one block per pipeline), then the tables ----
+    // ---- shared-memory map: bookkeeping first, then the tables ----
     // probe tables, double buffered (the next query's is built while this one is scanned):
     // [bias nprobe][first slot / 32 nprobe][length nprobe][chunk prefix nprobe + 1]
     const int pt_words = 4 * a.nprobe + 1;
-    const uint32_t book_bytes = (uint32_t)((2 * pt_words + 2 * a.d + 8) * 4 + 15) & ~15u;     // everything before s_wq
-    const uint32_t pipe_bytes = book_bytes + 3u * (uint32_t)nwarps * (uint32_t)a.Pw * 8u;      // one pipeline's block
-    unsigned char* mbase = PIPES == 1 ? smem_raw : smem_raw + (size_t)pipe * pipe_bytes;
-    int* s_pt = reinterpret_cast<int*>(mbase);                            // [2][pt_words]
+    int* s_pt = reinterpret_cast<int*>(smem_raw);                         // [2][pt_words]
     float* s_qv = reinterpret_cast<float*>(s_pt + 2 * pt_words);          // [2][d] the queries themselves
     int* s_np = reinterpret_cast<int*>(s_qv + 2 * a.d);                   // [2] non-empty probes of the query
     int* s_item = s_np + 2;                                               // [2] work items (double buffered)
@@ -437,12 +410,10 @@ ivfpq_scan_kernel(ScanArgs a) {
     u64* s_cand = s_wq + (size_t)nwarps * a.Pw;                           // [2][nwarps * Pw] published candidates
     unsigned char* misc_end = reinterpret_cast<unsigned char*>(s_cand + 2 * (size_t)nwarps * a.Pw);
     const uint32_t dyn_abs = (uint32_t)__cvta_generic_to_shared(smem_raw);
-    // PIPES == 1: tables at the first 64 KB boundary behind the bookkeeping (the address travels in the lane constants);
-    // PIPES == 2: tables at the fixed address kDualTab (it travels in the LDS immediate; lane constants carry no base)
-    const uint32_t tab_abs = PIPES == 1 ? (dyn_abs + (uint32_t)(misc_end - smem_raw) + 65535u) & ~65535u : kDualTab;
+    // tables at the first 64 KB boundary behind the bookkeeping (the address travels in the lane constants)
+    const uint32_t tab_abs = (dyn_abs + (uint32_t)(misc_end - smem_raw) + 65535u) & ~65535u;
     float* s_lut = reinterpret_cast<float*>(smem_raw + (tab_abs - dyn_abs)); // NTAB x [256][64]
-    if (PIPES == 1 ? tab_abs - dyn_abs + NTAB * 65536u > (uint32_t)a.smem_bytes
-                   : (dyn_abs + 2u * pipe_bytes > kDualTab || kDualTab - dyn_abs + NTAB * 65536u > (uint32_t)a.smem_bytes)) {
+    if (tab_abs - dyn_abs + NTAB * 65536u > (uint32_t)a.smem_bytes) {
         if (threadIdx.x == 0 && blockIdx.x == 0 && a.status) *a.status = 1;
         return;
     }
@@ -459,14 +430,13 @@ ivfpq_scan_kernel(ScanArgs a) {
 
     // per-lane look-up constants
     // (byte b of a group: slot byte offset 4 * (16 * replica + ((b ^ lane) & 15)); packed two per register under
-    // the table address, whose low 16 bits are zero; two pipelines: no address, + 128 = the half row of pipeline 1)
+    // the table address, whose low 16 bits are zero)
     uint32_t pre[8];
 #pragma unroll
     for (int b = 0; b < 16; b += 2) {
-        const uint32_t half = PIPES == 1 ? 0u : 128u * (uint32_t)pipe;
-        const uint32_t c0 = 4u * (16u * (lane >> 4) + ((b ^ lane) & 15)) + half;
-        const uint32_t c1 = 4u * (16u * (lane >> 4) + (((b + 1) ^ lane) & 15)) + half;
-        pre[b >> 1] = (PIPES == 1 ? tab_abs : 0u) | c0 | (c1 << 8);
+        const uint32_t c0 = 4u * (16u * (lane >> 4) + ((b ^ lane) & 15));
+        const uint32_t c1 = 4u * (16u * (lane >> 4) + (((b + 1) ^ lane) & 15));
+        pre[b >> 1] = tab_abs | c0 | (c1 << 8);
         asm volatile("" : "+r"(pre[b >> 1]));  // opaque: keep the constants in registers, never recompute them
     }
 
@@ -484,12 +454,12 @@ ivfpq_scan_kernel(ScanArgs a) {
     };
 
     if (tid == 32) { s_item[0] = atomicAdd(a.work_counter, 1); s_ncand[0] = 0; s_ncand[1] = 0; }
-    pipe_sync();
+    __syncthreads();
     if (warp == 1) {
         probe_table(s_item[0], 0);
         if (lane == 0) s_item[1] = atomicAdd(a.work_counter, 1);
     }
-    pipe_sync();
+    __syncthreads();
     int buf = 0;
     bool have_prev = false;
     int64_t prev_qi = 0;
@@ -512,17 +482,12 @@ ivfpq_scan_kernel(ScanArgs a) {
             if (tid == 32) { *cta_thr = 0xFFFFFFFFu; *s_next = nwarps * kGrab; }
             const long long t0 = STATS ? clock64() : 0;
             if (nchunks > 0) {
-                if constexpr (PIPES == 1) {
-                    if (a.lut_image) copy_lut_image(s_lut, a.lut_image + (size_t)qi * (NTAB * 8192), NTAB * 2048, tid, (int)blockDim.x);
-                    else build_lut<m>(s_lut, q, a.codebooks_t, a.dsub, lut_scale, tid, (int)blockDim.x);
-                } else {                                   // (the launcher never combines table images with two pipelines)
-                    if (pipe == 0) build_lut<m, 0>(s_lut, q, a.codebooks_t, a.dsub, lut_scale, tid, nthreads);
-                    else build_lut<m, 1>(s_lut, q, a.codebooks_t, a.dsub, lut_scale, tid, nthreads);
-                }
+                if (a.lut_image) copy_lut_image(s_lut, a.lut_image + (size_t)qi * (NTAB * 8192), NTAB * 2048, tid, (int)blockDim.x);
+                else build_lut<m>(s_lut, q, a.codebooks_t, a.dsub, lut_scale, tid, (int)blockDim.x);
             }
             if (STATS && a.phase_cycles && tid == 64) atomicAdd(a.phase_cycles + 5, (unsigned long long)(clock64() - t0));
         }
-        pipe_sync();                                   // (1) table ready; s_item[buf] has been read by everybody
+        __syncthreads();                               // (1) table ready; s_item[buf] has been read by everybody
         // ---- warp 0 first selects the k best of the candidates published for the PREVIOUS query and warp 1 builds
         //      the NEXT query's probe table; the other warps are already scanning, and chunks are handed out
         //      dynamically, so nobody waits for either
@@ -614,10 +579,10 @@ ivfpq_scan_kernel(ScanArgs a) {
             VIX_ADVANCE()
 #endif
             unsigned long long s01 = 0ull, s23 = 0ull;     // (s0, s1), (s2, s3) as f32x2 pairs
-            lookup16<0, PIPES>(wc[0], pre, s01, s23);
-            if (G > 1) lookup16<1, PIPES>(wc[G > 1 ? 1 : 0], pre, s01, s23);
-            if (G > 2) lookup16<2, PIPES>(wc[G > 2 ? 2 : 0], pre, s01, s23);
-            if (G > 3) lookup16<3, PIPES>(wc[G > 3 ? 3 : 0], pre, s01, s23);
+            lookup16<0>(wc[0], pre, s01, s23);
+            if (G > 1) lookup16<1>(wc[G > 1 ? 1 : 0], pre, s01, s23);
+            if (G > 2) lookup16<2>(wc[G > 2 ? 2 : 0], pre, s01, s23);
+            if (G > 3) lookup16<3>(wc[G > 3 ? 3 : 0], pre, s01, s23);
             const float s0 = __uint_as_float((uint32_t)s01), s1 = __uint_as_float((uint32_t)(s01 >> 32));
             const float s2 = __uint_as_float((uint32_t)s23), s3 = __uint_as_float((uint32_t)(s23 >> 32));
 #ifdef VIX_SCAN_NOPREFETCH
@@ -715,7 +680,7 @@ ivfpq_scan_kernel(ScanArgs a) {
             }
         }
         if (STATS) { const long long t = clock64(); cyc_scan += (unsigned long long)(t - t_mark); t_mark = t; }
-        pipe_sync();                                   // (2) scan finished everywhere, candidates published
+        __syncthreads();                               // (2) scan finished everywhere, candidates published
         if (STATS) { const long long t = clock64(); cyc_tail += (unsigned long long)(t - t_mark); t_mark = t; }
         have_prev = true;
         prev_qi = qi;
@@ -891,46 +856,8 @@ static size_t generic_smem_bytes(const ScanArgs& a) {
     return s;
 }
 
-// Two query pipelines per CTA (opt-in: VIX_SCAN_DUAL=1, or =2 to make a launch that cannot take them an error).  Taken
-// when three 64 KB tables are enough (m <= 48), the tables are built in the kernel, k <= 32 (the queues shrink to
-// next_pow2(k + 32) entries) and both pipelines' bookkeeping fits in front of the tables (`taken`); anything else runs
-// the one-pipeline kernel.
-template <int G, bool FILTER>
-static int launch_dual(ScanArgs& a, bool& taken) {
-    taken = false;
-    const char* const env = getenv("VIX_SCAN_DUAL");                   // read per launch: one process can compare both
-    if (!env || (env[0] != '1' && env[0] != '2')) return VIX_OK;
-    const bool required = env[0] == '2';
-    const int Pw = next_pow2(a.k + 32);
-    const size_t book = ((size_t)(2 * (4 * a.nprobe + 1) + 2 * a.d + 8) * 4 + 15) & ~(size_t)15;
-    const size_t pipe_bytes = book + 3 * (size_t)kDualWarps * Pw * 8;  // = the kernel's pipe_bytes
-    const bool fits = G <= 3 && !a.phase_cycles && !a.lut_image && a.k <= 32 && 1024 + 2 * pipe_bytes <= kDualTab;
-    VIX_REQUIRE(fits || !required, VIX_ERR_UNSUPPORTED,
-                "ivfpq scan: VIX_SCAN_DUAL=2, but m = %d, k = %d, nprobe = %d, d = %d cannot run as two pipelines", a.m, a.k,
-                a.nprobe, a.d);
-    if (!fits) return VIX_OK;
-    if constexpr (G <= 3) {
-        taken = true;
-        a.Pw = Pw;
-        const size_t smem = 227 * 1024;                                // the tables end at the end of the window
-        a.smem_bytes = (int)smem;
-        auto kern = ivfpq_scan_kernel<G, FILTER, false, 2>;
-        VIX_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        int64_t grid = num_sms();
-        if (2 * grid > a.nq) grid = (a.nq + 1) / 2;
-        if (a.ev_kernel[0]) VIX_CUDA(cudaEventRecord(a.ev_kernel[0], ctx().stream));
-        kern<<<(unsigned)grid, kFastThreads, smem, ctx().stream>>>(a);
-        VIX_LAUNCH_CHECK();
-        if (a.ev_kernel[1]) VIX_CUDA(cudaEventRecord(a.ev_kernel[1], ctx().stream));
-    }
-    return VIX_OK;
-}
-
 template <int G, bool FILTER>
 static int launch_fast(ScanArgs& a) {
-    bool dual = false;
-    VIX_TRY((launch_dual<G, FILTER>(a, dual)));
-    if (dual) return VIX_OK;
     const bool stats = a.phase_cycles != nullptr;
     constexpr int NTAB = (G + 1) / 2;
     // as many warps as the per-warp selection queues leave room for (24 unless k is large)

@@ -276,6 +276,45 @@ __global__ void pack_result_keys_kernel(const float* __restrict__ dist, const in
     for (int p = 0; p < world; ++p) reinterpret_cast<u64*>(static_cast<char*>(peer_base[p]) + off)[i] = key;
 }
 
+// keys_all: [world][nq][k] as gathered; one CTA per query selects the k smallest of its world x k keys (padding keys
+// come out as NaN / id -1)
+__global__ void merge_shard_keys_kernel(const u64* __restrict__ keys_all, int world, int64_t nq, int k, int P2,
+                                        float* __restrict__ out_dist, int64_t* __restrict__ out_ids) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    u64* s = reinterpret_cast<u64*>(smem_raw);
+    const int64_t row = blockIdx.x;
+    const int nin = world * k;
+    for (int i = threadIdx.x; i < P2; i += blockDim.x) {
+        u64 key = kEmptyKey;
+        if (i < nin) { const int r = i / k, j = i - r * k; key = keys_all[((size_t)r * nq + row) * k + j]; }
+        s[i] = key;
+    }
+    __syncthreads();
+    bitonic_sort_keys<false>(s, P2, threadIdx.x, blockDim.x);
+    for (int i = threadIdx.x; i < k; i += blockDim.x) {
+        const u64 key = s[i];
+        const size_t o = (size_t)row * k + i;
+        if (key == kEmptyKey) {
+            out_dist[o] = __int_as_float(0x7fc00000);
+            out_ids[o] = -1;
+        } else {
+            out_dist[o] = key_score(key, 0);
+            out_ids[o] = (int64_t)key_id(key);
+        }
+    }
+}
+
+static int merge_shard_keys(const u64* keys_all, int world, int64_t nq, int k, float* out_dist, int64_t* out_ids) {
+    const int P2 = next_pow2(world * k < 2 ? 2 : world * k);
+    const size_t smem = (size_t)P2 * 8;
+    VIX_REQUIRE(smem <= 200 * 1024, VIX_ERR_UNSUPPORTED, "shard merge: %d keys per query exceed shared memory", world * k);
+    VIX_CUDA(cudaFuncSetAttribute(merge_shard_keys_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const int threads = P2 / 2 < 32 ? 32 : (P2 / 2 > 256 ? 256 : P2 / 2);
+    merge_shard_keys_kernel<<<(unsigned)nq, threads, smem, ctx().stream>>>(keys_all, world, nq, k, P2, out_dist, out_ids);
+    VIX_LAUNCH_CHECK();
+    return VIX_OK;
+}
+
 // The list-major scan's bounds (vix_scan.cuh: scan_thr_hook_t) over peer memory: a rank finds a finite bound only for the
 // queries whose first probed list it owns, so the minimum over the ranks is a store of those into every peer's bound
 // array, a barrier, and a minimum with what arrived here -- which is reset on the way (the next writers are behind the
@@ -488,7 +527,7 @@ int vix_sharded_search(vix_index_t* h, vix_comm_t* c, const float* queries, int6
                                                                               c->off_results + (size_t)rank * total * 8, nullptr);
         VIX_LAUNCH_CHECK();
         VIX_TRY(peer_barrier(c));
-        VIX_TRY(merge_shard_keys(rbuf, world, nq, k, 0, 0, nullptr, dd.dev, di.dev));
+        VIX_TRY(merge_shard_keys(rbuf, world, nq, k, dd.dev, di.dev));
     } else {
         // NCCL carries the two exchanges
         In<float> dq;
@@ -523,7 +562,7 @@ int vix_sharded_search(vix_index_t* h, vix_comm_t* c, const float* queries, int6
                                                                               kall + (size_t)rank * total);
         VIX_LAUNCH_CHECK();
         VIX_NCCL(g_nccl.AllGather(kall + (size_t)rank * total, kall, (size_t)total, ncclUint64, c->comm, s));
-        VIX_TRY(merge_shard_keys(kall, world, nq, k, 0, 0, nullptr, dd.dev, di.dev));
+        VIX_TRY(merge_shard_keys(kall, world, nq, k, dd.dev, di.dev));
     }
     mark(3);
     VIX_TRY(dd.commit());

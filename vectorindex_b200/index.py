@@ -319,28 +319,6 @@ class IVFPQIndex(IVFIndex):
                                                  C.c_int(nprobe), ptr(dist, np.float32), ptr(ids, np.int64)))
         return dist, ids
 
-    def probe_range_keys(self, queries, nprobe, list_begin, list_count):
-        """probe_range as packed records: key = orderable(score) << 32 | list id, [nq x nprobe] (numpy uint64 / torch
-        int64 carrying the same bits) -- what one all-gather of the sharded search exchanges"""
-        q = as_input(queries, np.float32)
-        self._check_dim(q, "probe_range_keys")
-        nq = int(q.shape[0])
-        keys = empty_like_input(q, (nq, nprobe), np.uint64)
-        check(lib().vix_index_probe_range_keys(self._h, ptr(q, np.float32), C.c_int64(nq), C.c_int(nprobe), C.c_int(list_begin),
-                                               C.c_int(list_count), ptr(keys, np.uint64)))
-        return keys
-
-    def search_with_probes_keys(self, queries, k, probes):
-        """search_with_probes as packed records: key = orderable(distance) << 32 | id, [nq x k]"""
-        q = as_input(queries, np.float32)
-        self._check_dim(q, "search_with_probes_keys")
-        pr = as_input(probes, np.int32)
-        nq, nprobe = int(q.shape[0]), int(pr.shape[1])
-        keys = empty_like_input(q, (nq, k), np.uint64)
-        check(lib().vix_index_search_with_probes_keys(self._h, ptr(q, np.float32), C.c_int64(nq), C.c_int(k), ptr(pr, np.int32),
-                                                      C.c_int(nprobe), ptr(keys, np.uint64)))
-        return keys
-
     def encode(self, vectors):
         """(list assignment, PQ codes) of a batch without storing it (bit-exact, same kernels as batch_insert)"""
         x = as_input(vectors, np.float32)
@@ -430,27 +408,6 @@ def merge_shard_results(dist_all, ids_all, k, metric=METRIC_L2):
         sc = np.ascontiguousarray(np.transpose(dist_all, (1, 0, 2)))
         idm = np.ascontiguousarray(np.transpose(ids_all, (1, 0, 2)))
     return mergeTopK(sc, idm, k, 0)
-
-
-def merge_probe_keys(keys_all):
-    """[world x nq x nprobe] gathered probe keys -> the global probe lists [nq x nprobe] int32 (mergeTopK order)"""
-    keys_all = as_input(keys_all, np.uint64)
-    world, nq, nprobe = (int(v) for v in keys_all.shape)
-    probes = empty_like_input(keys_all, (nq, nprobe), np.int32)
-    check(lib().vix_merge_probe_keys(ptr(keys_all, np.uint64), C.c_int(world), C.c_int64(nq), C.c_int(nprobe),
-                                     ptr(probes, np.int32)))
-    return probes
-
-
-def merge_result_keys(keys_all):
-    """[world x nq x k] gathered result keys -> merged (distances [nq x k] f32, ids [nq x k] int64)"""
-    keys_all = as_input(keys_all, np.uint64)
-    world, nq, k = (int(v) for v in keys_all.shape)
-    dist = empty_like_input(keys_all, (nq, k), np.float32)
-    ids = empty_like_input(keys_all, (nq, k), np.int64)
-    check(lib().vix_merge_result_keys(ptr(keys_all, np.uint64), C.c_int(world), C.c_int64(nq), C.c_int(k),
-                                      ptr(dist, np.float32), ptr(ids, np.int64)))
-    return dist, ids
 
 
 def merge_shard_results_host(dist_all, ids_all, k):
@@ -576,8 +533,7 @@ class ShardedIVFPQIndex:
     def _native(self):
         """The product path: the whole sharded step inside the library (vix_sharded_search / vix_sharded_add over a
         ``vix_comm_t``).  The Python exchange below remains for CPU ranks (gloo tests with an oracle-backed local index)."""
-        import os
-        if self.world <= 1 or not self._nccl() or not hasattr(self.local, "_h") or os.environ.get("VIX_PY_SHARDED"):
+        if self.world <= 1 or not self._nccl() or not hasattr(self.local, "_h"):
             return None
         if self.__dict__.get("comm") is None:
             self.comm = Comm.from_torch(self.group)
@@ -604,89 +560,6 @@ class ShardedIVFPQIndex:
             # enqueued behind it on the same stream); pageable sources are staged by torch and stay safe
             a = a.to(torch.device("cuda", torch.cuda.current_device()), non_blocking=a.is_pinned())
         return a.contiguous()
-
-    # ---- exchanges over peer memory (NVLink / NVSwitch) -------------------------------------------------------
-    def _p2p(self):
-        """Symmetric-memory state, or None (then NCCL all-gathers carry the exchanges): torch's _SymmetricMemory maps a
-        buffer of every rank into all peers; the library's kernels store into the peers directly."""
-        import os
-        st = self.__dict__.get("_p2p_state", "unset")
-        if st != "unset":
-            return st
-        st = None
-        if self.world > 1 and self._nccl() and hasattr(self.local, "_h"):
-            # decided ONCE and by ALL ranks together (all-reduce MIN of a local capability flag): a rank that cannot map
-            # peer memory must not leave the others waiting in a barrier; a failure inside a step is an error, not a
-            # reason to change the exchange on one rank only
-            import torch
-            import torch.distributed as dist
-            symm, ok = None, 0
-            if not os.environ.get("VIX_NO_P2P"):
-                try:
-                    import torch.distributed._symmetric_memory as symm
-                    t = symm.empty((16,), dtype=torch.int32, device=self._comm_device())
-                    ok = 1 if t is not None else 0
-                except Exception:  # noqa: BLE001
-                    symm, ok = None, 0
-            flag = torch.tensor([ok], dtype=torch.int32, device=self._comm_device())
-            dist.all_reduce(flag, op=dist.ReduceOp.MIN, group=self.group)
-            if int(flag.item()) == 1:
-                st = {"symm": symm, "bufs": {}}
-        self._p2p_state = st
-        return st
-
-    def _symm_buffer(self, tag, shape, dtype):
-        """(tensor, handle) of a symmetric buffer, double buffered: consecutive uses of a tag alternate between two
-        allocations, and between two uses of the same one lies the barrier of the other exchange, so a fast rank never
-        overwrites what a slow peer is still merging."""
-        import torch.distributed as dist
-        st = self._p2p_state
-        ent = st["bufs"].get((tag, shape, dtype))
-        if ent is None:
-            pairs = []
-            for _ in range(2):
-                t = st["symm"].empty(shape, dtype=dtype, device=self._comm_device())
-                pairs.append((t, st["symm"].rendezvous(t, self.group if self.group is not None else dist.group.WORLD)))
-            ent = st["bufs"][(tag, shape, dtype)] = {"pairs": pairs, "i": 0}
-        ent["i"] ^= 1
-        return ent["pairs"][ent["i"]]
-
-    # a peer that never arrives makes the barrier kernel trap after this long (an error instead of a hung box)
-    _BARRIER_TIMEOUT_MS = 120_000
-
-    def _search_over_peer_memory(self, queries, k, nprobe, mark):
-        """One sharded search step whose two exchanges are stores into peer memory by the producing kernels + one
-        barrier each (vix_peer_scatter_block, vix_index_search_with_probes_keys_peers)."""
-        import torch
-        nq = int(queries.shape[0])
-        lo, cnt, per = self.query_block(nq)
-        if (per * nprobe) % 4:
-            raise ValueError("probe block is not a multiple of 16 bytes")
-        q = as_input(queries, np.float32)
-        # probe lists of this rank's query block -> slot `rank` of every peer's [world * per x nprobe] buffer
-        pbuf, ph = self._symm_buffer("probes", (self.world * per, nprobe), torch.int32)
-        if cnt == per:
-            block = self.local.probe_range(q[lo:lo + cnt], nprobe, 0, self.kc)[0]
-        else:
-            block = torch.full((per, nprobe), -1, dtype=torch.int32, device=pbuf.device)
-            if cnt > 0:
-                block[:cnt] = self.local.probe_range(q[lo:lo + cnt], nprobe, 0, self.kc)[0]
-        check(lib().vix_peer_scatter_block(ptr(block, np.int32), C.c_size_t(per * nprobe * 4), C.c_void_p(int(ph.buffer_ptrs_dev)),
-                                           C.c_int(self.world), C.c_int(self.rank)))
-        ph.barrier(0, self._BARRIER_TIMEOUT_MS)
-        probes = pbuf[:nq]
-        mark("probe_select+gather")
-        # fused scan; its local top-k leaves as packed keys for slot `rank` of every peer's [world x nq x k] buffer
-        kbuf, kh = self._symm_buffer("results", (self.world, nq, k), torch.int64)
-        check(lib().vix_index_search_with_probes_keys_peers(self.local._h, ptr(q, np.float32), C.c_int64(nq), C.c_int(k),
-                                                            ptr(probes, np.int32), C.c_int(nprobe),
-                                                            C.c_void_p(int(kh.buffer_ptrs_dev)), C.c_int(self.world),
-                                                            C.c_int(self.rank)))
-        mark("scan")
-        kh.barrier(0, self._BARRIER_TIMEOUT_MS)
-        out = merge_result_keys(kbuf)
-        mark("gather+merge")
-        return out
 
     def _to_host(self, t):
         """device tensor -> numpy array through a pinned staging buffer kept with the index (one D2H at full PCIe rate,
@@ -832,48 +705,10 @@ class ShardedIVFPQIndex:
             return md, mi
         if self.world > 1 and was_numpy and self._nccl():
             queries = self._to_comm(np.ascontiguousarray(queries, dtype=np.float32))
-        marks = [] if getattr(self, "phase_times", None) is not None and self._nccl() else None
-
-        def mark(name):
-            if marks is not None:
-                e = torch.cuda.Event(enable_timing=True)
-                e.record()
-                marks.append((name, e))
-
-        mark("start")
-        if self.world > 1 and self._nccl() and hasattr(self.local, "probe_range_keys"):
-            # device path: probe lists by query block + one all-gather of list ids; local top-k as packed 8-byte records,
-            # one all-gather, merge straight from the gathered layout
-            # every intermediate lives on the device and the stages are ordered by the stream, so the library calls
-            # need not synchronise one by one (the copy of the merged result to the host, below, does it once)
-            was_async = lib().vix_get_async()
-            lib().vix_set_async(1)
-            try:
-                md = None
-                if self._p2p() is not None:
-                    md, mi = self._search_over_peer_memory(queries, k, nprobe, mark)
-                if md is None:
-                    probes = self.global_probes(queries, nprobe)
-                    mark("probe_select+gather")
-                    rk = self.local.search_with_probes_keys(queries, k, probes)
-                    mark("scan")
-                    md, mi = merge_result_keys(self._all_gather(rk))
-                    mark("gather+merge")
-            finally:
-                lib().vix_set_async(was_async)
-            if marks:
-                torch.cuda.synchronize()
-                for (_, a), (name, b) in zip(marks[:-1], marks[1:]):
-                    self.phase_times[name] = self.phase_times.get(name, 0.0) + a.elapsed_time(b)
-            if was_numpy:
-                md, mi = self._to_host(md), self._to_host(mi)
-            return md, mi
         probes = self.global_probes(queries, nprobe)
-        mark("probe_select+gather")
         if not self._nccl() and _lib._is_torch(probes):
             probes = probes.numpy()
         d_loc, i_loc = self.local.search_with_probes(queries, k, probes)
-        mark("scan")
         if self.world == 1:
             return d_loc, i_loc
         d_all, i_all = self._all_gather(self._to_comm(d_loc)), self._all_gather(self._to_comm(i_loc))
@@ -881,11 +716,6 @@ class ShardedIVFPQIndex:
             md, mi = merge_shard_results(d_all, i_all, k)
         else:
             md, mi = merge_shard_results_host(d_all.numpy(), i_all.numpy(), k)
-        mark("gather+merge")
-        if marks:
-            torch.cuda.synchronize()
-            for (_, a), (name, b) in zip(marks[:-1], marks[1:]):
-                self.phase_times[name] = self.phase_times.get(name, 0.0) + a.elapsed_time(b)
         if was_numpy and _lib._is_torch(md):
             md, mi = md.cpu().numpy(), mi.cpu().numpy()
         return md, mi
