@@ -25,12 +25,12 @@
 //   warp 1      MMA issuer: one elected lane issues tcgen05.mma M128 N128 K8 (4 per K-block); tcgen05.commit
 //               releases ring slots and publishes finished accumulators; two accumulator buffers in TMEM
 //   warps 2-5   epilogue: tcgen05.ld (32 lanes x 32 columns), fused ||c||^2 term, group minima / emission
-// Every mbarrier wait is bounded (a stuck pipeline raises an error flag instead of hanging the GPU).
+// PTX wrappers: vix_tcgen05.cuh.  Every mbarrier wait is bounded (mbar_wait there: a stuck pipeline raises an error flag).
 #include "vix_common.cuh"
 #include "vix_exact.cuh"
+#include "vix_tcgen05.cuh"
 #include "vix_topk.cuh"
 
-#include <cuda.h>
 #include <stdlib.h>
 
 #include <algorithm>
@@ -53,7 +53,7 @@ constexpr int kStageBytes = (kM + kN) * kKB * 4;       // 48 KB
 constexpr int kEpiWarps = 8;                          // two per TMEM lane quarter: each takes 128 of the 256 columns, 64 at a time
 constexpr int kThreads = 64 + 32 * kEpiWarps;
 constexpr int kTmemCols = 512;                         // two fp32 accumulators of 256 columns
-constexpr uint32_t kIdesc = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(kN >> 3) << 17) | ((uint32_t)(kM >> 4) << 24);
+constexpr uint32_t kIdesc = idesc_tf32(kM, kN);
 
 enum Mode { MODE_WRITE = 0, MODE_MIN = 1, MODE_EMIT = 2 };
 
@@ -77,123 +77,6 @@ struct Args {
     int* error;            // device flag, set to 1 when a barrier wait times out (the other waits then give up too)
     int* error_host;       // optional mapped host copy of the flag (raised once, never polled by the device)
 };
-
-// ---------------------------------------------------------------------------------------------- PTX wrappers
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
-    uint32_t ok;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok)
-        : "r"(smem_u32(bar)), "r"(parity)
-        : "memory");
-    return ok != 0;
-}
-// bounded wait: ~2 s at 2 GHz, then raise the error flag and give up
-__device__ __forceinline__ bool mbar_wait(uint64_t* bar, uint32_t parity, int* error, int* error_host) {
-    if (mbar_try_wait(bar, parity)) return true;
-    const long long t0 = clock64();
-    while (!mbar_try_wait(bar, parity)) {
-        if (clock64() - t0 > 4000000000LL || *reinterpret_cast<volatile int*>(error) != 0) {
-            atomicExch(error, 1);
-            if (error_host) { *reinterpret_cast<volatile int*>(error_host) = 1; __threadfence_system(); }
-            return false;
-        }
-    }
-    return true;
-}
-__device__ __forceinline__ void tma_load_2d(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-        ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1)
-        : "memory");
-}
-__device__ __forceinline__ void tmem_alloc(uint32_t* slot, uint32_t ncols) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(slot)), "r"(ncols));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-}
-__device__ __forceinline__ void tmem_dealloc(uint32_t addr, uint32_t ncols) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(addr), "r"(ncols));
-}
-__device__ __forceinline__ void fence_before_sync() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void fence_after_sync() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void mma_tf32(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(kIdesc), "r"(accumulate)
-        : "memory");
-}
-__device__ __forceinline__ void mma_commit(uint64_t* bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, float (&v)[32]) {
-    uint32_t r[32];
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-        "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-          "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-          "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-          "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-        : "r"(taddr));
-    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-    for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]);
-}
-
-// The same load in two halves: `issue` starts it, `wait` makes the registers readable (it names them as in/out operands,
-// so no use can be scheduled in front of it).  Both 32-column loads of a tile are issued before the first wait.
-__device__ __forceinline__ void tmem_ld32_issue(uint32_t taddr, uint32_t (&r)[32]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-        "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-          "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-          "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-          "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-        : "r"(taddr));
-}
-__device__ __forceinline__ void tmem_ld32_wait(uint32_t (&r)[32], uint32_t (&q)[32]) {
-    asm volatile("tcgen05.wait::ld.sync.aligned;"
-                 : "+r"(r[0]), "+r"(r[1]), "+r"(r[2]), "+r"(r[3]), "+r"(r[4]), "+r"(r[5]), "+r"(r[6]), "+r"(r[7]), "+r"(r[8]),
-                   "+r"(r[9]), "+r"(r[10]), "+r"(r[11]), "+r"(r[12]), "+r"(r[13]), "+r"(r[14]), "+r"(r[15]), "+r"(r[16]),
-                   "+r"(r[17]), "+r"(r[18]), "+r"(r[19]), "+r"(r[20]), "+r"(r[21]), "+r"(r[22]), "+r"(r[23]), "+r"(r[24]),
-                   "+r"(r[25]), "+r"(r[26]), "+r"(r[27]), "+r"(r[28]), "+r"(r[29]), "+r"(r[30]), "+r"(r[31])
-                 :: "memory");
-    asm volatile(""
-                 : "+r"(q[0]), "+r"(q[1]), "+r"(q[2]), "+r"(q[3]), "+r"(q[4]), "+r"(q[5]), "+r"(q[6]), "+r"(q[7]), "+r"(q[8]),
-                   "+r"(q[9]), "+r"(q[10]), "+r"(q[11]), "+r"(q[12]), "+r"(q[13]), "+r"(q[14]), "+r"(q[15]), "+r"(q[16]),
-                   "+r"(q[17]), "+r"(q[18]), "+r"(q[19]), "+r"(q[20]), "+r"(q[21]), "+r"(q[22]), "+r"(q[23]), "+r"(q[24]),
-                   "+r"(q[25]), "+r"(q[26]), "+r"(q[27]), "+r"(q[28]), "+r"(q[29]), "+r"(q[30]), "+r"(q[31])
-                 :: "memory");
-}
-
-// K-major operand tile [rows][32 tf32] = rows x 128 B, 128B swizzle (8-row atoms of 1024 B): SBO = 1024 B
-__device__ __forceinline__ uint64_t make_desc(uint32_t smem_addr) {
-    uint64_t d = 0;
-    d |= (uint64_t)((smem_addr >> 4) & 0x3FFF);        // start address
-    d |= (uint64_t)0 << 16;                            // leading byte offset (unused for swizzled K-major)
-    d |= (uint64_t)(1024 >> 4) << 32;                  // stride byte offset
-    d |= (uint64_t)1 << 46;                            // descriptor version (Blackwell)
-    d |= (uint64_t)2 << 61;                            // SWIZZLE_128B
-    return d;
-}
 
 // ---------------------------------------------------------------------------------------------- the kernel
 // ARES: the row tile of A (kblocks x 16 KB, d <= 128) stays RESIDENT in shared memory for all the column tiles of a work
@@ -226,7 +109,7 @@ tc_score_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant_
         for (int s = 0; s < kStagesMax; ++s) { mbar_init(full + s, 1); mbar_init(empty + s, 1); }
         for (int b = 0; b < 2; ++b) { mbar_init(tfull + b, 1); mbar_init(tempty + b, kEpiWarps); }
         for (int b = 0; b < 2; ++b) { mbar_init(afull + b, 1); mbar_init(aempty + b, 1); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
     }
     if (warp == 1) tmem_alloc(tmem_slot, kTmemCols);
     fence_before_sync();
@@ -293,10 +176,10 @@ tc_score_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant_
                         fence_after_sync();
                         const uint32_t sS = smem_u32(ring + (size_t)stage * kRingStage);
                         const uint32_t sA = ARES ? smem_u32(a_res + (size_t)ab * a_bytes + (size_t)kb * kTileBytes) : sS;
-                        const uint64_t da = make_desc(sA), db = make_desc(ARES ? sS : sS + kTileBytes);
+                        const uint64_t da = make_desc_sw128(sA), db = make_desc_sw128(ARES ? sS : sS + kTileBytes);
 #pragma unroll
                         for (int k = 0; k < kKB / 8; ++k)      // K = 8 tf32 (32 B) per instruction: +2 in 16 B units
-                            mma_tf32(tmem_d, da + 2 * k, db + 2 * k, (kb | k) ? 1u : 0u);
+                            mma_tf32(tmem_d, da + 2 * k, db + 2 * k, kIdesc, (kb | k) ? 1u : 0u);
                         mma_commit(empty + stage);             // frees the ring slot when these MMAs retire
                         if (++stage == a.nstages) { stage = 0; phase ^= 1; }
                     }
@@ -462,7 +345,6 @@ static EncodeTiledFn encode_fn() {
     return fn;
 }
 
-// rows x d fp32 row-major, box = 32 columns (128 B) x box_rows rows, 128B swizzle, zero fill out of bounds
 int make_map_rows(CUtensorMap* map, const float* ptr, int64_t rows, int d, int box_rows) {
     EncodeTiledFn fn = encode_fn();
     VIX_REQUIRE(fn != nullptr, VIX_ERR_CUDA, "cuTensorMapEncodeTiled is not available from this driver");

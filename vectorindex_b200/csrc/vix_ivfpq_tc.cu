@@ -36,7 +36,7 @@
 //   warps 20-21  MMA issuers (one lane each, alternating tiles)
 //   warp 22      work: takes the next list from a global counter -- the lists with pairs in work-descending order, so that no
 //                long list ends up as the kernel's tail --, publishes the item, gathers the B tile + tau
-// Every mbarrier wait is bounded (a stuck pipeline raises the error flag instead of hanging the GPU).
+// PTX wrappers: vix_tcgen05.cuh.  Every mbarrier wait is bounded (mbar_wait_sleep there: a stuck pipeline raises the error flag).
 #include <cuda_fp16.h>
 #include <stdlib.h>
 
@@ -48,6 +48,7 @@
 #include "vix_common.cuh"
 #include "vix_scan.cuh"
 #include "vix_scan_select.cuh"
+#include "vix_tcgen05.cuh"
 
 namespace vix {
 
@@ -84,7 +85,6 @@ constexpr int kAStageCols = 64;                          // one operand stage: 1
 constexpr int kTmemCols = 512;
 static_assert(kACol0 + kStagesA * kAStageCols <= kTmemCols, "TMEM columns");
 constexpr int kSeedChunks = 8;                           // the seed looks at the first 256 vectors of a query's first list
-constexpr uint32_t kIdescF16 = (1u << 4) | ((uint32_t)(128 >> 4) << 24);   // A, B fp16 (format 0), D fp32, K-major both
 
 struct Item { int first_chunk, nchunks, len, n, pair_begin, pad0, pad1, pad2; };
 
@@ -122,116 +122,17 @@ struct Args {
     unsigned long long* diag;      // VIX_TCS_DIAG builds: waiting cycles per role and barrier kind
 };
 
-// ---------------------------------------------------------------------------------------------- PTX wrappers
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
-    uint32_t ok;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-    return ok != 0;
-}
-// the same with a suspend-time hint: the thread sleeps in hardware until the phase completes or ~`ns` have passed, instead
-// of coming back at once and spinning (23 warps share four schedulers; a spinning warp takes issue slots from the decoders)
-__device__ __forceinline__ bool mbar_try_wait_sleep(uint64_t* bar, uint32_t parity, uint32_t ns) {
-    uint32_t ok;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity), "r"(ns) : "memory");
-    return ok != 0;
-}
 #ifdef VIX_TCS_DIAG
 #define VIX_DG(i) dg[i]
 #else
 #define VIX_DG(i) dg_none
 #endif
-__device__ __forceinline__ bool mbar_wait(uint64_t* bar, uint32_t parity, int* error, int* error_host, unsigned long long& waited) {
-#ifdef VIX_TCS_DIAG
-    const long long w0 = clock64();
-    struct Acc { unsigned long long& w; long long t; __device__ ~Acc() { w += (unsigned long long)(clock64() - t); } } acc{waited, w0};
-#endif
-    if (mbar_try_wait(bar, parity)) return true;
-    // try_wait suspends the thread in hardware until the phase completes or a time limit passes, so the loop is not a busy
-    // spin; the clock and the (global) error flag are looked at only every 64th return -- a global load per iteration would
-    // add its ~600 clocks to EVERY hand-over of the pipeline
-    const long long t0 = clock64();
-    for (uint32_t spins = 1;; ++spins) {
-        if (mbar_try_wait_sleep(bar, parity, 4000u)) return true;
-        if ((spins & 63u) == 0 && (clock64() - t0 > 4000000000LL || *reinterpret_cast<volatile int*>(error) != 0)) {
-            atomicExch(error, 1);
-            if (error_host) { *reinterpret_cast<volatile int*>(error_host) = 1; __threadfence_system(); }
-            return false;
-        }
-    }
-}
-__device__ __forceinline__ void tmem_alloc(uint32_t* slot, uint32_t ncols) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(slot)), "r"(ncols));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-}
-__device__ __forceinline__ void tmem_dealloc(uint32_t addr, uint32_t ncols) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(addr), "r"(ncols));
-}
-__device__ __forceinline__ void fence_before_sync() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void fence_after_sync() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void fence_async_proxy() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-// A operand in TMEM (rows = lanes, 32-bit columns of two halves), B from shared memory
-__device__ __forceinline__ void mma_f16_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
-        ::"r"(tmem_d), "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-__device__ __forceinline__ void mma_commit(uint64_t* bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, float (&v)[16]) {
-    uint32_t r[16];
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
-        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-          "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-        : "r"(taddr));
-    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-    for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(r[i]);
-}
-// K-major operand tile, rows of 128 B, 128B swizzle (8-row atoms of 1024 B): SBO = 1024 B
-__device__ __forceinline__ uint64_t make_desc(uint32_t smem_addr) {
-    uint64_t d = 0;
-    d |= (uint64_t)((smem_addr >> 4) & 0x3FFF);
-    d |= (uint64_t)(1024 >> 4) << 32;
-    d |= (uint64_t)1 << 46;
-    d |= (uint64_t)2 << 61;
-    return d;
-}
 template <int IMM>
 __device__ __forceinline__ uint32_t lds_tab(uint32_t addr) {
     uint32_t v;
     asm volatile("ld.shared.b32 %0, [%1+%2];" : "=r"(v) : "r"(addr), "n"(IMM));
     return v;
 }
-// .16x128b.x4: register 2 k + e of thread 4 i + c goes to TMEM lane i + 8 e, column 4 k + c (16 lanes x 16 columns)
-__device__ __forceinline__ void tmem_st16x128_x4(uint32_t taddr, const uint32_t (&r)[8]) {
-    asm volatile(
-        "tcgen05.st.sync.aligned.16x128b.x4.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};"
-        ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7])
-        : "memory");
-}
-__device__ __forceinline__ void tmem_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
-
 // one group of 16 sub-quantisers of the four slots r + 8 v (v = 0..3) of thread t = 4 r + c: 16 look-ups in the order of the
 // decode layout (vix_scan.cuh: byte s of word v holds sub-quantiser 4 (s ^ q) + c, q = r & 3).  For one (v, s) the 16
 // threads of a half-warp (q, c all different) ask for 16 different table slots and the two half-warps (h = r >> 2) read two
@@ -291,7 +192,7 @@ tc_scan_kernel(Args a) {
         for (int i = 0; i < kStagesA; ++i) { mbar_init(&S.a_full[i], 128); mbar_init(&S.a_empty[i], 1); }
         for (int i = 0; i < 2; ++i) { mbar_init(&S.b_full[i], 32); mbar_init(&S.b_empty[i], kEpiWarps); }
         for (int i = 0; i < kDBufs; ++i) { mbar_init(&S.d_full[i], 1); mbar_init(&S.d_empty[i], 4); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
     }
     if (warp == kMmaWarp) tmem_alloc(&S.tmem_slot, kTmemCols);
     if (threadIdx.x == 32) S.mma_seq = 0;
@@ -347,7 +248,7 @@ tc_scan_kernel(Args a) {
                 }
                 slot = it % kItemRing;
                 const uint32_t par = (uint32_t)(it / kItemRing) & 1u;
-                if (blocking) { if (!mbar_wait(&S.item_full[slot], par, a.error, a.error_host, VIX_DG(0))) return 0; }
+                if (blocking) { if (!mbar_wait_sleep(&S.item_full[slot], par, a.error, a.error_host, VIX_DG(0))) return 0; }
                 else if (!__all_sync(0xFFFFFFFFu, mbar_try_wait(&S.item_full[slot], par))) return 2;
                 fc = S.items[slot].first_chunk; nch = S.items[slot].nchunks;
                 if (nch < 0) return 0;
@@ -367,7 +268,7 @@ tc_scan_kernel(Args a) {
             const int st = (int)(unit % kStagesA);
             const long long use = unit / kStagesA;
             const uint32_t a_taddr = a_taddr0 + (uint32_t)(st * kAStageCols);
-            if (use > 0 && !mbar_wait(&S.a_empty[st], (uint32_t)(use - 1) & 1u, a.error, a.error_host, VIX_DG(1))) return false;
+            if (use > 0 && !mbar_wait_sleep(&S.a_empty[st], (uint32_t)(use - 1) & 1u, a.error, a.error_host, VIX_DG(1))) return false;
             if (live) {
                 // group g: sub-table g / 2, slots 32 (g % 2) + 16 h + ..: the immediates are compile-time
                 decode16<(int)kTabAbs>(w[0], pre[0], pre[1], a_taddr, q0, q1);
@@ -414,13 +315,13 @@ tc_scan_kernel(Args a) {
             long long u = 0;
             for (;;) {
                 const int slot = it % kItemRing;
-                if (!mbar_wait(&S.item_full[slot], (uint32_t)(it / kItemRing) & 1u, a.error, a.error_host, VIX_DG(0))) break;
+                if (!mbar_wait_sleep(&S.item_full[slot], (uint32_t)(it / kItemRing) & 1u, a.error, a.error_host, VIX_DG(0))) break;
                 const int nch = S.items[slot].nchunks, n = S.items[slot].n;
                 if (nch < 0) break;
                 const int nt = (nch + 3) >> 2;
-                const uint32_t idesc = kIdescF16 | ((uint32_t)(((n + 15) & ~15) >> 3) << 17);
+                const uint32_t idesc = idesc_f16(128, (n + 15) & ~15);
                 const int buf = it & 1;
-                if (!mbar_wait(&S.b_full[buf], (uint32_t)(it >> 1) & 1u, a.error, a.error_host, VIX_DG(1))) break;
+                if (!mbar_wait_sleep(&S.b_full[buf], (uint32_t)(it >> 1) & 1u, a.error, a.error_host, VIX_DG(1))) break;
                 bool ok = true;
                 for (int t = 0; t < nt; ++t, ++u) {
                     if ((int)(u % kMmaWarps) != me) continue;
@@ -434,8 +335,8 @@ tc_scan_kernel(Args a) {
                         }
                         if (!ok) { atomicExch(a.error, 1); break; }
                     }
-                    if (!mbar_wait(&S.a_full[st], (uint32_t)(u / kStagesA) & 1u, a.error, a.error_host, VIX_DG(2))) { ok = false; break; }
-                    if (u >= kDBufs && !mbar_wait(&S.d_empty[db], (uint32_t)(u / kDBufs - 1) & 1u, a.error, a.error_host, VIX_DG(3))) { ok = false; break; }
+                    if (!mbar_wait_sleep(&S.a_full[st], (uint32_t)(u / kStagesA) & 1u, a.error, a.error_host, VIX_DG(2))) { ok = false; break; }
+                    if (u >= kDBufs && !mbar_wait_sleep(&S.d_empty[db], (uint32_t)(u / kDBufs - 1) & 1u, a.error, a.error_host, VIX_DG(3))) { ok = false; break; }
                     *reinterpret_cast<volatile uint32_t*>(&S.mma_seq) = (uint32_t)(u + 1);
                     fence_after_sync();
 #ifdef VIX_TCS_DIAG
@@ -444,7 +345,7 @@ tc_scan_kernel(Args a) {
                     const uint32_t dcol = tmem_base + (uint32_t)(db * kDStride);
 #pragma unroll
                     for (int ks = 0; ks < kKSteps; ++ks) {
-                        const uint64_t bd = make_desc(kBBase + (uint32_t)buf * kBBuf + (uint32_t)(ks >> 2) * kBAtom) + (uint64_t)(2 * (ks & 3));
+                        const uint64_t bd = make_desc_sw128(kBBase + (uint32_t)buf * kBBuf + (uint32_t)(ks >> 2) * kBAtom) + (uint64_t)(2 * (ks & 3));
                         // A from TMEM: 8 columns (16 halves) of the stage per K-step
                         mma_f16_ts(dcol, tmem_base + (uint32_t)(kACol0 + st * kAStageCols + 8 * ks), bd, idesc, ks > 0 ? 1u : 0u);
                     }
@@ -477,7 +378,7 @@ tc_scan_kernel(Args a) {
         long long u = 0;
         for (;;) {
             const int slot = it % kItemRing;
-            if (!mbar_wait(&S.item_full[slot], (uint32_t)(it / kItemRing) & 1u, a.error, a.error_host, VIX_DG(0))) break;
+            if (!mbar_wait_sleep(&S.item_full[slot], (uint32_t)(it / kItemRing) & 1u, a.error, a.error_host, VIX_DG(0))) break;
             const int fc = S.items[slot].first_chunk, nch = S.items[slot].nchunks, len = S.items[slot].len, n = S.items[slot].n;
             if (nch < 0) break;
             const int nt = (nch + 3) >> 2;
@@ -490,7 +391,7 @@ tc_scan_kernel(Args a) {
             // this set's tiles of the item: t0, t0 + kEpiSets, ... ((u + t) % kEpiSets == eset)
             const int t0 = (int)(((long long)eset - u % kEpiSets + kEpiSets) % kEpiSets);
             float tx_next = load_tx(t0);
-            if (!mbar_wait(&S.b_full[buf], (uint32_t)(it >> 1) & 1u, a.error, a.error_host, VIX_DG(1))) break;
+            if (!mbar_wait_sleep(&S.b_full[buf], (uint32_t)(it >> 1) & 1u, a.error, a.error_host, VIX_DG(1))) break;
             const float* tau = S.tau[buf];
             bool ok = true;
             for (int t = t0; t < nt; t += kEpiSets) {
@@ -502,7 +403,7 @@ tc_scan_kernel(Args a) {
                 const uint32_t g = ((uint32_t)(fc + ch) << 5) + sl;
                 const float tx = tx_next;
                 tx_next = t + kEpiSets < nt ? load_tx(t + kEpiSets) : 0.0f;
-                if (!mbar_wait(&S.d_full[db], (uint32_t)(uu / kDBufs) & 1u, a.error, a.error_host, VIX_DG(2))) { ok = false; break; }
+                if (!mbar_wait_sleep(&S.d_full[db], (uint32_t)(uu / kDBufs) & 1u, a.error, a.error_host, VIX_DG(2))) { ok = false; break; }
                 fence_after_sync();
                 const float hv = sc * (0.5f * tx - 1.5e-6f * fabsf(tx));
                 for (int cb = 0; cb < n; cb += 16) {
@@ -544,7 +445,7 @@ tc_scan_kernel(Args a) {
         const int n_order = *a.n_order;
         auto publish = [&](int fc, int nch, int len, int n, int pb) {
             const int slot = it % kItemRing;
-            if (it >= kItemRing && !mbar_wait(&S.item_empty[slot], (uint32_t)(it / kItemRing - 1) & 1u, a.error, a.error_host, VIX_DG(0))) return false;
+            if (it >= kItemRing && !mbar_wait_sleep(&S.item_empty[slot], (uint32_t)(it / kItemRing - 1) & 1u, a.error, a.error_host, VIX_DG(0))) return false;
             if (lane == 0) {
                 Item& I = S.items[slot];
                 I.first_chunk = fc; I.nchunks = nch; I.len = len; I.n = n; I.pair_begin = pb;
@@ -567,7 +468,7 @@ tc_scan_kernel(Args a) {
                 const int n = min(kNQ, pe - g0);
                 if (!publish(fc, nch, len, n, g0)) { ok = false; break; }
                 const int buf = it & 1;
-                if (it >= 2 && !mbar_wait(&S.b_empty[buf], (uint32_t)((it >> 1) - 1) & 1u, a.error, a.error_host, VIX_DG(1))) { ok = false; break; }
+                if (it >= 2 && !mbar_wait_sleep(&S.b_empty[buf], (uint32_t)((it >> 1) - 1) & 1u, a.error, a.error_host, VIX_DG(1))) { ok = false; break; }
                 const uint32_t bbase = kBBase + (uint32_t)buf * kBBuf;
                 for (int idx = lane; idx < n * CH; idx += 32) {
                     const int c = idx / CH, chn = idx - c * CH;

@@ -22,20 +22,15 @@
 // Warp roles as in vix_gemm.cu: warp 0 TMA producer (3-stage ring of A 16 KB | B 32 KB), warp 1 MMA issuer, warps 2-17 two
 // epilogue teams of eight warps, one team per TMEM accumulator buffer (2 x 256 columns), two threads per (vector,
 // sub-space) with 128 codewords each; codes are staged per row tile in shared memory and leave as one contiguous
-// [128 x m] byte slab.  Residual variants: r = x - g is materialised once (the
-// shortlist's A operand); the exact stage reads x and g and follows the reference's residual arithmetic.
+// [128 x m] byte slab.  Residual variants: r = x - g is materialised once (the shortlist's A operand); the exact stage reads x
+// and g and follows the reference's residual arithmetic.  PTX wrappers, bounded mbarrier waits (mbar_wait): vix_tcgen05.cuh.
 #include "vix_common.cuh"
 #include "vix_pq_encode.cuh"
+#include "vix_tcgen05.cuh"
 
-#include <cuda.h>
 #include <stdlib.h>
 
 namespace vix {
-
-namespace tc {
-int make_map_rows(CUtensorMap* map, const float* ptr, int64_t rows, int d, int box_rows);
-bool supported(int64_t nA, int64_t nB, int d, const float* A, const float* B);
-}
 
 namespace pqtc {
 
@@ -44,7 +39,7 @@ constexpr int kStages = 3;
 constexpr int kStageBytes = (kM + kN) * kKB * 4;       // 48 KB
 constexpr int kThreads = 64 + 512;                     // producer, MMA issuer, 2 teams x 2 column halves x 4 epilogue warps
 constexpr int kCap = 4;                                // finalists kept per (vector, sub-space)
-constexpr uint32_t kIdesc = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(kN >> 3) << 17) | ((uint32_t)(kM >> 4) << 24);
+constexpr uint32_t kIdesc = idesc_tf32(kM, kN);
 
 struct Args {
     const float* x;                 // [n x d] the rows (exact arithmetic)
@@ -61,98 +56,10 @@ struct Args {
     int* error_host;
 };
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ bool mbar_try_wait(uint64_t* bar, uint32_t parity) {
-    uint32_t ok;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-    return ok != 0;
-}
-// bounded wait: a stuck pipeline raises the error flag instead of hanging the GPU
-__device__ __forceinline__ bool mbar_wait(uint64_t* bar, uint32_t parity, int* error, int* error_host) {
-    if (mbar_try_wait(bar, parity)) return true;
-    const long long t0 = clock64();
-    while (!mbar_try_wait(bar, parity)) {
-        if (clock64() - t0 > 4000000000LL || *reinterpret_cast<volatile int*>(error) != 0) {
-            atomicExch(error, 1);
-            if (error_host) { *reinterpret_cast<volatile int*>(error_host) = 1; __threadfence_system(); }
-            return false;
-        }
-    }
-    return true;
-}
-__device__ __forceinline__ void tma_load_2d(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-        ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(smem_u32(bar)), "r"(c0), "r"(c1)
-        : "memory");
-}
-__device__ __forceinline__ void tmem_alloc(uint32_t* slot, uint32_t ncols) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(slot)), "r"(ncols));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-}
-__device__ __forceinline__ void tmem_dealloc(uint32_t addr, uint32_t ncols) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(addr), "r"(ncols));
-}
-__device__ __forceinline__ void fence_before_sync() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void fence_after_sync() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void mma_tf32(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(kIdesc), "r"(accumulate)
-        : "memory");
-}
-__device__ __forceinline__ void mma_commit(uint64_t* bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-// tcgen05.ld is asynchronous: `issue` starts the load of 32 columns into r, `wait` makes them readable.  The wait names
-// every register of the load as an in/out operand, so the compiler cannot schedule a use of r in front of it.
-__device__ __forceinline__ void tmem_ld32_issue(uint32_t taddr, uint32_t (&r)[32]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-        "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-          "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-          "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-          "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-        : "r"(taddr));
-}
-__device__ __forceinline__ void tmem_ld32_wait(uint32_t (&r)[32]) {
-    asm volatile("tcgen05.wait::ld.sync.aligned;"
-                 : "+r"(r[0]), "+r"(r[1]), "+r"(r[2]), "+r"(r[3]), "+r"(r[4]), "+r"(r[5]), "+r"(r[6]), "+r"(r[7]), "+r"(r[8]),
-                   "+r"(r[9]), "+r"(r[10]), "+r"(r[11]), "+r"(r[12]), "+r"(r[13]), "+r"(r[14]), "+r"(r[15]), "+r"(r[16]),
-                   "+r"(r[17]), "+r"(r[18]), "+r"(r[19]), "+r"(r[20]), "+r"(r[21]), "+r"(r[22]), "+r"(r[23]), "+r"(r[24]),
-                   "+r"(r[25]), "+r"(r[26]), "+r"(r[27]), "+r"(r[28]), "+r"(r[29]), "+r"(r[30]), "+r"(r[31])
-                 :: "memory");
-}
 __device__ __forceinline__ float4 lds_f4(uint32_t addr) {
     float4 v;
     asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(addr));
     return v;
-}
-// K-major operand tile [rows][32 tf32] = rows x 128 B, 128B swizzle (8-row atoms of 1024 B): SBO = 1024 B
-__device__ __forceinline__ uint64_t make_desc(uint32_t smem_addr) {
-    uint64_t d = 0;
-    d |= (uint64_t)((smem_addr >> 4) & 0x3FFF);
-    d |= (uint64_t)(1024 >> 4) << 32;
-    d |= (uint64_t)1 << 46;
-    d |= (uint64_t)2 << 61;
-    return d;
 }
 
 template <int MODE, int DSUB>
@@ -176,7 +83,7 @@ pq_tc_encode_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_const
     if (warp == 0 && lane == 0) {
         for (int s = 0; s < kStages; ++s) { mbar_init(full + s, 1); mbar_init(empty + s, 1); }
         for (int b = 0; b < 2; ++b) { mbar_init(tfull + b, 1); mbar_init(tempty + b, 8); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init_fence();
     }
     for (int e = threadIdx.x; e < a.m * 256; e += kThreads) s_csq[e] = a.csq[e];
     if (warp == 1) tmem_alloc(tmem_slot, 512);
@@ -213,7 +120,7 @@ pq_tc_encode_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_const
                     if (!mbar_wait(full + stage, phase, a.error, a.error_host)) { ok = false; break; }
                     fence_after_sync();
                     const uint32_t sA = smem_u32(ring + (size_t)stage * kStageBytes);
-                    const uint64_t da = make_desc(sA), db = make_desc(sA + kM * kKB * 4);
+                    const uint64_t da = make_desc_sw128(sA), db = make_desc_sw128(sA + kM * kKB * 4);
                     const int nsub = min(per_group, a.m - g * per_group);
                     for (int s = 0; s < nsub; ++s) {
                         if (!mbar_wait(tempty + acc, aphase ^ 1, a.error, a.error_host)) { ok = false; break; }
@@ -221,7 +128,7 @@ pq_tc_encode_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_const
                         const uint32_t tmem_d = tmem_base + (uint32_t)acc * kN;
 #pragma unroll
                         for (int k = 0; k < kSteps; ++k)               // 8 tf32 = 32 B per step: +2 in 16-byte units
-                            mma_tf32(tmem_d, da + 2 * (s * kSteps + k), db + 2 * (s * kSteps + k), k ? 1u : 0u);
+                            mma_tf32(tmem_d, da + 2 * (s * kSteps + k), db + 2 * (s * kSteps + k), kIdesc, k ? 1u : 0u);
                         mma_commit(tfull + acc);
                         if (++acc == 2) { acc = 0; aphase ^= 1; }
                     }
