@@ -98,6 +98,14 @@ int         vix_synchronize(void);           /* wait for the calling thread's st
 int64_t     vix_kernel_launches(int reset);  /* kernels launched by this thread (bench bookkeeping) */
 int64_t     vix_scan_tc_launches(void);      /* IVF-PQ searches of this process that took the list-major tensor-core
                                                 scan (csrc/vix_ivfpq_tc.cu) rather than the query-major one (tests, bench) */
+/* the tensor-core shortlist of the GEMM-shaped stages (csrc/vix_gemm.cu), per kind: coarse probe selection, flat search,
+ * IVF list assignment (vix_index_add, k-means, vix_ivf_assign_f32) */
+typedef enum { VIX_SHORTLIST_PROBE = 0, VIX_SHORTLIST_FLAT = 1, VIX_SHORTLIST_ASSIGN = 2 } vix_shortlist_kind;
+int64_t     vix_tc_shortlist_calls(int kind);       /* calls of this process that took the shortlist rather than the exact
+                                                       CUDA-core kernel alone (-1: no such kind) */
+int64_t     vix_tc_shortlist_exact_rows(int kind);  /* rows of those calls whose shortlist overflowed or was empty and that the
+                                                       exact kernel computed instead; flat and assignment only (probe
+                                                       selection hands them over on the device and counts 0) */
 
 /* ------------------------------------------------------------------------------------------------ */
 /* a1-a3  Flat scoring.  Replaces @_cdecl l2sqr_f32_block / ip_f32_block                            */

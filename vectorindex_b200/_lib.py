@@ -81,7 +81,7 @@ _LIB = None
 # symbol -> (restype, is_status)
 _EXPORTS = [
     "vix_version", "vix_last_error", "vix_clear_error", "vix_device_count", "vix_set_device", "vix_set_stream", "vix_set_async", "vix_get_async",
-    "vix_synchronize", "vix_kernel_launches", "vix_scan_tc_launches",
+    "vix_synchronize", "vix_kernel_launches", "vix_scan_tc_launches", "vix_tc_shortlist_calls", "vix_tc_shortlist_exact_rows",
     "vix_l2sqr_f32_block", "vix_ip_f32_block", "vix_row_norms_f32", "vix_flat_search_f32", "vix_select_topk_f32",
     "vix_merge_topk_f32", "vix_rerank_exact_topk_f32", "vix_centroid_batch_score_f32", "vix_ivf_select_nprobe_batch_f32", "vix_ivf_assign_f32",
     "vix_ivf_assign_metric_f32", "vix_pq_query_subnorms_f32", "vix_pq_lut_batch_l2_f32", "vix_pq_lut_residual_l2_f32", "vix_adc_scan_u8",
@@ -115,6 +115,8 @@ def lib() -> C.CDLL:
         L.vix_last_error.restype = C.c_char_p
         L.vix_kernel_launches.restype = C.c_int64
         L.vix_scan_tc_launches.restype = C.c_int64
+        L.vix_tc_shortlist_calls.restype = C.c_int64
+        L.vix_tc_shortlist_exact_rows.restype = C.c_int64
         L.vix_index_count.restype = C.c_int64
         L.vix_index_destroy.restype = None
         L.vix_index_params_default.restype = None

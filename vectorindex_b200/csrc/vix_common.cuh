@@ -178,6 +178,16 @@ __device__ __forceinline__ float key_score(u64 key, int order_max) {
     return f32_from_orderable(u);
 }
 __device__ __forceinline__ uint32_t key_id(u64 key) { return (uint32_t)(key & 0xFFFFFFFFull); }
+// A CentroidBatchScore value (probe selection) of centroid c as the selection returns it.  make_key folds -0 into +0; the
+// sign of a zero score follows from the metric: IP is -s with s summed from +0 in round-to-nearest (never -0), so a zero
+// is -0; L2 is -2 s + ||c||^2, a zero is ||c||^2 itself when that is a zero (s = +0, -2 s = -0) and +0 otherwise (exact
+// cancellation).
+__device__ __forceinline__ float cbs_signed_zero(float s, uint32_t c, int metric, const float* cnorm) {
+    if (s != 0.0f) return s;
+    if (metric != VIX_METRIC_L2) return -0.0f;
+    const float cn = cnorm ? cnorm[c] : 0.0f;
+    return cn == 0.0f ? cn : 0.0f;
+}
 
 // idFilterPass (Operations/Filtering/IDFilter.swift:115-135): out-of-range ids are dropped in either mode
 __device__ __forceinline__ bool id_filter_pass(const uint64_t* __restrict__ words, int64_t cap, int deny, int64_t id) {

@@ -12,12 +12,23 @@
 //           columns of a row to its minimum; nothing else leaves the SM.
 //   select  T_q = (k-th smallest group minimum of row q) + 2 eps_q.  k different groups hold a score
 //           <= that minimum, so the exact k-th best score is <= T_q - eps_q, and every member of the exact
-//           top k has S~ <= T_q  (eps_q bounds |S~ - S| for the row: TF32 truncation + accumulation).
+//           top k has S~ <= T_q.  eps_q bounds |S~ - S| for every column of the row, S being the score in
+//           the reference's own fp32 evaluation (up to a constant per row: the flat scan's ||q||^2):
+//             eps_q = rel ||q|| max||c|| + rel2 (||q||^2 + max||c||^2)          (shortlist_margin)
+//           rel   the dot product: TF32 operand truncation 2 * 2^-10 + fp32 accumulation d * 2^-21 (x 2 for L2);
+//           rel2  L2 only: the fp32 rounding that scales with the squared norms, not with ||q|| ||c|| -- the
+//                 epilogue's fmaf, ||c||^2 summed in another order than the reference's (row_norms against
+//                 Km12, the direct (q - x)^2 sum or the fused form), the reference's own sums (each within
+//                 d u (||q|| + ||c||)^2 <= 2 d u (||q||^2 + ||c||^2), u = 2^-24) and the addition forming T_q:
+//                 (3 d + 8) u, taken as 4 (d + 3) u.  Without it a row with ||q|| << max||c|| (a zero row:
+//                 eps = 0) keeps only the columns whose ROUNDED norm is the smallest and can miss the column
+//                 whose reference distance is smallest.  Both carry a factor 1.25 of slack.
+//           IP scores have no squared-norm term; their fp32 rounding is within rel's accumulation share.
 //   pass 2  the same contraction again (cheaper than keeping 10^9 scores); the epilogue emits the columns
 //           with S~ <= T_q into a per-row candidate list (expected ~1.2 k entries).
 //   exact   the candidates are rescored in the reference's operation order by the exact CUDA-core
-//           kernels and selected by (score, index); rows whose list overflowed fall back to the exact
-//           kernel entirely.
+//           kernels and selected by (score, index); rows whose list overflowed, or is empty (a NaN in the
+//           row makes T_q NaN), fall back to the exact kernel entirely.
 //
 // Kernel structure (one CTA per SM, persistent over (row tile, column split) work items):
 //   warp 0      TMA producer: A (128 rows x 32 tf32) and B (128 columns x 32 tf32) K-blocks, 128B swizzle,
@@ -34,6 +45,7 @@
 #include <stdlib.h>
 
 #include <algorithm>
+#include <atomic>
 #include <mutex>
 
 namespace vix {
@@ -431,6 +443,17 @@ static int launch(const float* A, int64_t nA, const float* B, int nB, int d, Arg
 }
 
 // ---------------------------------------------------------------------------------------------- thresholds
+// eps_q = rel ||q|| max||c|| + rel2 (||q||^2 + max||c||^2): the bound on |S~ - S| of the header, for all three consumers
+struct Margin { float rel, rel2; };
+static Margin shortlist_margin(int d, int metric) {
+    const bool l2 = metric == VIX_METRIC_L2;
+    return {(l2 ? 2.0f : 1.0f) * 1.25f * (2.0f / 1024.0f + (float)d / 2097152.0f),
+            l2 ? 1.25f * (float)(d + 3) / 4194304.0f : 0.0f};
+}
+__device__ __forceinline__ float shortlist_eps(Margin m, float anorm, float bnorm_max) {
+    return m.rel * sqrtf(anorm) * bnorm_max + m.rel2 * (anorm + bnorm_max * bnorm_max);
+}
+
 // T_q = (k-th smallest group minimum of the row) + margin_q.  One WARP per row: the <= 32 VPL minima of the row stay in
 // registers as order-preserving 32-bit keys and the k-th smallest is found by a radix select, one bit per step
 // (how many keys share the prefix found so far and have a 0 in this bit?) with warp ballots -- no shared memory, no
@@ -438,7 +461,7 @@ static int launch(const float* A, int64_t nA, const float* B, int nB, int d, Arg
 template <int VPL>
 __global__ void __launch_bounds__(256)
 threshold_kernel(const float* __restrict__ gmin, int64_t nrows, int ngroups, int k, const float* __restrict__ anorm,
-                 const float* __restrict__ bnorm_max, float rel, float* __restrict__ thr) {
+                 const float* __restrict__ bnorm_max, Margin margin, float* __restrict__ thr) {
     const int lane = threadIdx.x & 31;
     const int64_t row = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     if (row >= nrows) return;
@@ -462,19 +485,18 @@ threshold_kernel(const float* __restrict__ gmin, int64_t nrows, int ngroups, int
         }
         kth = f32_from_orderable(prefix);
     }
-    // |S~ - S| <= rel * ||q|| * max||c||  (TF32 operand truncation 2 * 2^-10 + fp32 accumulation, with margin)
-    if (lane == 0) thr[row] = kth + 2.0f * rel * sqrtf(anorm[row]) * bnorm_max[0];
+    if (lane == 0) thr[row] = kth + 2.0f * shortlist_eps(margin, anorm[row], bnorm_max[0]);
 }
 
 static int launch_threshold(const float* gmin, int64_t nrows, int ngroups, int k, const float* anorm, const float* bnorm_max,
-                            float rel, float* thr) {
+                            Margin margin, float* thr) {
     const unsigned grid = (unsigned)((nrows * 32 + 255) / 256);
     cudaStream_t s = ctx().stream;
-    if (ngroups <= 256) threshold_kernel<8><<<grid, 256, 0, s>>>(gmin, nrows, ngroups, k, anorm, bnorm_max, rel, thr);
-    else if (ngroups <= 512) threshold_kernel<16><<<grid, 256, 0, s>>>(gmin, nrows, ngroups, k, anorm, bnorm_max, rel, thr);
-    else if (ngroups <= 1024) threshold_kernel<32><<<grid, 256, 0, s>>>(gmin, nrows, ngroups, k, anorm, bnorm_max, rel, thr);
-    else if (ngroups <= 2048) threshold_kernel<64><<<grid, 256, 0, s>>>(gmin, nrows, ngroups, k, anorm, bnorm_max, rel, thr);
-    else if (ngroups <= 4096) threshold_kernel<128><<<grid, 256, 0, s>>>(gmin, nrows, ngroups, k, anorm, bnorm_max, rel, thr);
+    if (ngroups <= 256) threshold_kernel<8><<<grid, 256, 0, s>>>(gmin, nrows, ngroups, k, anorm, bnorm_max, margin, thr);
+    else if (ngroups <= 512) threshold_kernel<16><<<grid, 256, 0, s>>>(gmin, nrows, ngroups, k, anorm, bnorm_max, margin, thr);
+    else if (ngroups <= 1024) threshold_kernel<32><<<grid, 256, 0, s>>>(gmin, nrows, ngroups, k, anorm, bnorm_max, margin, thr);
+    else if (ngroups <= 2048) threshold_kernel<64><<<grid, 256, 0, s>>>(gmin, nrows, ngroups, k, anorm, bnorm_max, margin, thr);
+    else if (ngroups <= 4096) threshold_kernel<128><<<grid, 256, 0, s>>>(gmin, nrows, ngroups, k, anorm, bnorm_max, margin, thr);
     else { set_error("threshold: %d groups per row (> 4096)", ngroups); return VIX_ERR_UNSUPPORTED; }
     VIX_LAUNCH_CHECK();
     return VIX_OK;
@@ -498,7 +520,8 @@ __global__ void max_sqrt_kernel(const float* __restrict__ x, int64_t n, float* _
 // are read 32 floats at a time with coalesced 128-byte loads (all 32 in flight) into a padded shared tile, and
 // lane i then walks row i of the tile -- one sequential chain per candidate, the same operations in the same order
 // as a thread reading its row straight from global memory, at a thirtieth of the L1 traffic.  Nothing in the
-// kernel synchronises more than a warp.  Rows whose candidate list overflowed are flagged for the exact kernel below.
+// kernel synchronises more than a warp.  Rows whose candidate list overflowed or is empty are flagged for the exact kernel
+// below.
 constexpr int kRescoreWarps = 8;
 __global__ void __launch_bounds__(32 * kRescoreWarps)
 rescore_probe_kernel(const float* __restrict__ A, int64_t nA, const float* __restrict__ B, int d, int metric,
@@ -515,7 +538,7 @@ rescore_probe_kernel(const float* __restrict__ A, int64_t nA, const float* __res
     const int64_t row = (int64_t)blockIdx.x * kRescoreWarps + warp;
     if (row >= nA) return;
     const int n = cand_cnt[row];
-    if (n > cap) {
+    if (n > cap || n == 0) {                                           // overflowed, or empty (T_q NaN)
         if (lane == 0) overflow_rows[atomicAdd(n_overflow, 1)] = (int)row;
         return;
     }
@@ -552,11 +575,11 @@ rescore_probe_kernel(const float* __restrict__ A, int64_t nA, const float* __res
         const u64 key = i < P ? keys[i] : kEmptyKey;
         const size_t o = (size_t)row * k + i;
         if (key == kEmptyKey) { out_idx[o] = -1; if (out_scores) out_scores[o] = __int_as_float(0x7fc00000); }
-        else { out_idx[o] = (int32_t)key_id(key); if (out_scores) out_scores[o] = key_score(key, 0); }
+        else { out_idx[o] = (int32_t)key_id(key); if (out_scores) out_scores[o] = cbs_signed_zero(key_score(key, 0), key_id(key), metric, bnorm); }
     }
 }
 
-// The rows whose shortlist overflowed (normally none), without a host round trip: a fixed grid walks the list the
+// The rows whose shortlist overflowed or is empty (normally none), without a host round trip: a fixed grid walks the list the
 // kernel above left on the device; one CTA per row scores EVERY column in the same operation order and selects by
 // (score, index) with a CTA-wide queue.
 __global__ void __launch_bounds__(256)
@@ -590,19 +613,19 @@ probe_overflow_rows_kernel(const float* __restrict__ A, const float* __restrict_
             const u64 key = keys[i];
             const size_t o = (size_t)row * k + i;
             if (key == kEmptyKey) { out_idx[o] = -1; if (out_scores) out_scores[o] = __int_as_float(0x7fc00000); }
-            else { out_idx[o] = (int32_t)key_id(key); if (out_scores) out_scores[o] = key_score(key, 0); }
+            else { out_idx[o] = (int32_t)key_id(key); if (out_scores) out_scores[o] = cbs_signed_zero(key_score(key, 0), key_id(key), metric, bnorm); }
         }
     }
 }
 
 // k = 1 (assignment): T = (smallest group minimum) + margin, one thread per row
 __global__ void threshold_min_kernel(const float* __restrict__ gmin, int64_t n, int ngroups, const float* __restrict__ anorm,
-                                     const float* __restrict__ bnorm_max, float rel, float* __restrict__ thr) {
+                                     const float* __restrict__ bnorm_max, Margin margin, float* __restrict__ thr) {
     const int64_t row = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (row >= n) return;
     float m = INFINITY;
     for (int g = 0; g < ngroups; ++g) m = fminf(m, gmin[row * ngroups + g]);
-    thr[row] = m + 2.0f * rel * sqrtf(anorm[row]) * bnorm_max[0];
+    thr[row] = m + 2.0f * shortlist_eps(margin, anorm[row], bnorm_max[0]);
 }
 
 // IVF list assignment from the shortlist: one thread per vector evaluates the reference's exact distance
@@ -656,7 +679,7 @@ rescore_flat_kernel(const float* __restrict__ A, const float* __restrict__ B, in
     float* sq = reinterpret_cast<float*>(keys + P);
     const int64_t row = blockIdx.x;
     const int n = cand_cnt[row];
-    if (n > cap) {
+    if (n > cap || n == 0) {                                           // overflowed, or empty (T_q NaN)
         if (threadIdx.x == 0) overflow_rows[atomicAdd(n_overflow, 1)] = (int)row;
         return;
     }
@@ -719,6 +742,9 @@ __global__ void scatter_probe_rows_kernel(const int32_t* __restrict__ idx, const
     }
 }
 
+// route evidence per shortlist kind (vix_tc_shortlist_calls / vix_tc_shortlist_exact_rows)
+static std::atomic<long long> g_calls[3], g_exact_rows[3];
+
 // number of group minima per row for a given group width (see the MODE_MIN epilogue)
 static int num_groups(int64_t nB, int gcols) {
     if (gcols < kN) return (int)((nB + gcols - 1) / gcols);
@@ -777,6 +803,7 @@ int probe_select_fast_device(const float* q, int64_t nq, const float* c, int kc,
         return probe_select_device(q, nq, c, kc, d, metric, nprobe, cnorm, nullptr, out_idx, out_scores);
     cudaStream_t s = ctx().stream;
     VIX_TRY(check_pipeline_error());                   // a pipeline that gave up in an earlier asynchronous call
+    tc::g_calls[VIX_SHORTLIST_PROBE].fetch_add(1);     // (its exact rows stay on the device: no host round trip here)
     int* pipe_flag = pipeline_error_flag();
     VIX_REQUIRE(pipe_flag != nullptr, VIX_ERR_OOM, "cannot allocate the mapped pipeline-error flag");
     Scratch<float> gmin, thr, qn, cn_tmp, cmax;
@@ -806,9 +833,7 @@ int probe_select_fast_device(const float* q, int64_t nq, const float* c, int kc,
     a.metric = metric; a.bnorm = (metric == VIX_METRIC_L2) ? cn : nullptr; a.error = flags.ptr; a.error_host = pipe_flag;
     a.mode = tc::MODE_MIN; a.gcols = gcols; a.ngroups = ngroups; a.gmin = gmin.ptr;
     VIX_TRY(tc::launch(q, nq, c, kc, d, a));
-    // |S~ - S|: dot error (2 * 2^-10 truncation + d * 2^-22 accumulation) * ||q|| ||c||, doubled for the L2 score
-    const float rel = ((metric == VIX_METRIC_L2) ? 2.0f : 1.0f) * 1.25f * (2.0f / 1024.0f + (float)d / 4194304.0f);
-    VIX_TRY(tc::launch_threshold(gmin.ptr, nq, ngroups, keff, qn.ptr, cmaxp, rel, thr.ptr));
+    VIX_TRY(tc::launch_threshold(gmin.ptr, nq, ngroups, keff, qn.ptr, cmaxp, tc::shortlist_margin(d, metric), thr.ptr));
     a.mode = tc::MODE_EMIT; a.thr = thr.ptr; a.cand_cnt = cand_cnt.ptr; a.cand_idx = cand_idx.ptr; a.cap = cap;
     VIX_TRY(tc::launch(q, nq, c, kc, d, a));
     {
@@ -846,6 +871,7 @@ int flat_search_auto_device(const float* q, int64_t nq, const float* xb, int64_t
                         nq >= 16 && tc::supported(nq, n, d, q, xb) && ngroups64 >= 2 * keff && keff <= 256 && d <= 4096 &&
                         (metric == VIX_METRIC_L2 || metric == VIX_METRIC_IP);
     if (!use_tc) return flat_search_device(q, nq, xb, n, d, metric, k, xb_norm, out_dist, out_ids, raw_scores);
+    tc::g_calls[VIX_SHORTLIST_FLAT].fetch_add(1);
     cudaStream_t s = ctx().stream;
     const int ngroups = (int)ngroups64;
     const int nb = (int)n;
@@ -872,8 +898,7 @@ int flat_search_auto_device(const float* q, int64_t nq, const float* xb, int64_t
     a.metric = metric; a.bnorm = (metric == VIX_METRIC_L2) ? xn.ptr : nullptr; a.error = flags.ptr;
     a.mode = tc::MODE_MIN; a.gcols = gcols; a.ngroups = ngroups; a.gmin = gmin.ptr;
     VIX_TRY(tc::launch(q, nq, xb, nb, d, a));
-    const float rel = ((metric == VIX_METRIC_L2) ? 2.0f : 1.0f) * 1.25f * (2.0f / 1024.0f + (float)d / 2097152.0f);
-    VIX_TRY(tc::launch_threshold(gmin.ptr, nq, ngroups, keff, qn.ptr, xmax.ptr, rel, thr.ptr));
+    VIX_TRY(tc::launch_threshold(gmin.ptr, nq, ngroups, keff, qn.ptr, xmax.ptr, tc::shortlist_margin(d, metric), thr.ptr));
     a.mode = tc::MODE_EMIT; a.thr = thr.ptr; a.cand_cnt = cand_cnt.ptr; a.cand_idx = cand_idx.ptr; a.cap = cap;
     VIX_TRY(tc::launch(q, nq, xb, nb, d, a));
     {
@@ -889,6 +914,7 @@ int flat_search_auto_device(const float* q, int64_t nq, const float* xb, int64_t
     VIX_CUDA(cudaMemcpyAsync(hflags, flags.ptr, 8, cudaMemcpyDeviceToHost, s));
     VIX_CUDA(cudaStreamSynchronize(s));
     VIX_REQUIRE(hflags[0] == 0, VIX_ERR_CUDA, "tensor-core pipeline timed out");
+    tc::g_exact_rows[VIX_SHORTLIST_FLAT].fetch_add(hflags[1]);
     if (hflags[1] > 0) {
         const int m = hflags[1];
         Scratch<float> sub, sub_d;
@@ -913,6 +939,7 @@ int ivf_assign_auto_device(const float* x, int64_t n, int d, const float* c, int
     const bool use_tc = getenv("VIX_DISABLE_TC") == nullptr && tc::supported(n, kc, d, x, c) && kc >= 1024 && n >= 1024 &&
                         d <= 4096 && n < (1LL << 31);
     if (!use_tc) return ivf_assign_device(x, n, d, c, kc, assign, dist);
+    tc::g_calls[VIX_SHORTLIST_ASSIGN].fetch_add(1);
     cudaStream_t s = ctx().stream;
     const int gcols = tc::choose_gcols(kc, 1);
     const int ngroups = tc::num_groups(kc, gcols);
@@ -939,9 +966,8 @@ int ivf_assign_auto_device(const float* x, int64_t n, int d, const float* c, int
     a.metric = VIX_METRIC_L2; a.bnorm = cn.ptr; a.error = flags.ptr;
     a.mode = tc::MODE_MIN; a.gcols = gcols; a.ngroups = ngroups; a.gmin = gmin.ptr;
     VIX_TRY(tc::launch(x, n, c, kc, d, a));
-    // TF32 shortlist error + the rounding of the exact fp32 evaluation itself (see DESIGN.md)
-    const float rel = 2.0f * 1.25f * (2.0f / 1024.0f + (float)d / 2097152.0f);
-    tc::threshold_min_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(gmin.ptr, n, ngroups, xn.ptr, cmax.ptr, rel, thr.ptr);
+    tc::threshold_min_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(gmin.ptr, n, ngroups, xn.ptr, cmax.ptr,
+                                                                       tc::shortlist_margin(d, VIX_METRIC_L2), thr.ptr);
     VIX_LAUNCH_CHECK();
     a.mode = tc::MODE_EMIT; a.thr = thr.ptr; a.cand_cnt = cand_cnt.ptr; a.cand_idx = cand_idx.ptr; a.cap = cap;
     VIX_TRY(tc::launch(x, n, c, kc, d, a));
@@ -952,6 +978,7 @@ int ivf_assign_auto_device(const float* x, int64_t n, int d, const float* c, int
     VIX_CUDA(cudaMemcpyAsync(hflags, flags.ptr, 8, cudaMemcpyDeviceToHost, s));
     VIX_CUDA(cudaStreamSynchronize(s));
     VIX_REQUIRE(hflags[0] == 0, VIX_ERR_CUDA, "tensor-core pipeline timed out");
+    tc::g_exact_rows[VIX_SHORTLIST_ASSIGN].fetch_add(hflags[1]);
     if (hflags[1] > 0) {
         const int m = hflags[1];
         Scratch<float> sub, sub_dist;
@@ -984,6 +1011,14 @@ int vix_debug_tc_scores_f32(const float* queries, int64_t nq, const float* centr
                     (centroid_norms == nullptr || is_device_ptr(centroid_norms)),
                 VIX_ERR_INVALID_PARAM, "vix_debug_tc_scores_f32: device pointers only");
     return tc_scores_device(queries, nq, centroids, kc, d, metric, centroid_norms, out);
+}
+
+int64_t vix_tc_shortlist_calls(int kind) {
+    return kind >= 0 && kind < 3 ? (int64_t)tc::g_calls[kind].load() : -1;
+}
+
+int64_t vix_tc_shortlist_exact_rows(int kind) {
+    return kind >= 0 && kind < 3 ? (int64_t)tc::g_exact_rows[kind].load() : -1;
 }
 
 }  // extern "C"

@@ -575,9 +575,30 @@ int centroid_batch_score_cosine_device(const float* q, int64_t nq, const float* 
 
 // batchSearch probe stage (IVFIndex.swift:905-927): CentroidBatchScore row + ordered prefix.
 // Outputs [nq x nprobe] padded with -1 / NaN beyond min(nprobe, kc).
+// the selections below carry their scores in keys (make_key: -0 folded into +0); put back the sign of the zero scores
+__global__ void probe_zero_sign_kernel(const int32_t* __restrict__ idx, float* __restrict__ scores, int64_t n, int metric,
+                                       const float* __restrict__ cnorm) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n && idx[i] >= 0) scores[i] = cbs_signed_zero(scores[i], (uint32_t)idx[i], metric, cnorm);
+}
+
+static int probe_select_keys(const float* q, int64_t nq, const float* c, int kc, int d, int metric, int nprobe,
+                             const float* cnorm, const uint64_t* disabled, int32_t* out_idx, float* out_scores);
+
 int probe_select_device(const float* q, int64_t nq, const float* c, int kc, int d, int metric, int nprobe,
                         const float* cnorm, const uint64_t* disabled, int32_t* out_idx, float* out_scores) {
     if (nq == 0 || nprobe <= 0) return VIX_OK;
+    VIX_TRY(probe_select_keys(q, nq, c, kc, d, metric, nprobe, cnorm, disabled, out_idx, out_scores));
+    if (out_scores) {
+        const int64_t n = nq * (int64_t)nprobe;
+        probe_zero_sign_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx().stream>>>(out_idx, out_scores, n, metric, cnorm);
+        VIX_LAUNCH_CHECK();
+    }
+    return VIX_OK;
+}
+
+static int probe_select_keys(const float* q, int64_t nq, const float* c, int kc, int d, int metric, int nprobe,
+                             const float* cnorm, const uint64_t* disabled, int32_t* out_idx, float* out_scores) {
     TilePlan plan;
     if (!plan_tile(d, EPI_TOPK, nprobe, &plan)) {
         // rows too long for the tiled engine: the CentroidBatchScore block of a tile of queries, then the ordered prefix
