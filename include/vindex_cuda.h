@@ -32,6 +32,12 @@
  *                            d = 2 m, ks = 256, nq x nprobe >= 32768)
  *   VIX_TC_SCAN_DEBUG=1      per launch (synchronises): queries handed back, finalists per query
  *   VIX_TC_SCAN_TIMES=1      CUDA events between the stages of every list-major launch, summed, printed at exit
+ *   VIX_SCAN_DEBUG=1         per query-major IVF-PQ scan launch (no synchronisation), one stderr line "[vix scan] ...": the
+ *                            kernel (fast G = m / 16, or generic), filter and stats instantiation, warps, Pw, P2, the
+ *                            table source (image: batch-wide lut_image_kernel; kernel: built in the scan), the bias source
+ *                            (kernel: in the scan; rows: probe_bias_rows_kernel; pairs: probe_bias_kernel; given: by the
+ *                            list-major scan), the locality order (yes / no) and the work items (query count, or device:
+ *                            the queries the list-major scan hands back)
  *   VIX_DISABLE_TC, VIX_DISABLE_PQ_TC, VIX_DISABLE_LUT_IMAGE
  *                            exact CUDA-core kernels instead of the tensor-core shortlists / per-query tables built inside
  *                            the scan instead of batch-wide (the parity tests compare both ways)
@@ -337,8 +343,17 @@ int     vix_index_export_lists(vix_index_t* h, int64_t* list_offsets, uint8_t* c
 int     vix_index_clear(vix_index_t* h);
 
 /* batchSearch: out_dist/out_ids [nq x k] ascending by API distance, padded with id -1 / NaN.
- * nprobe <= 0 => the index's configured nprobe.  k <= 0 => VIX_OK with nothing written
- * (IVFIndex.swift:866).  With sharding the result is this shard's local top-k (merge with
+ * nprobe <= 0 => the index's configured nprobe; nprobe > VIX_MAX_K => VIX_ERR_INVALID_K.  k <= 0 => VIX_OK with nothing written
+ * (IVFIndex.swift:866).  IVF-PQ probes: -1, ids outside [0, kc) and empty lists are skipped; a list probed twice in one
+ * row is scanned twice, so its vectors can come back twice (both copies with the same distance bits).  Shared-memory
+ * limits of the query-major scan, refused with VIX_ERR_UNSUPPORTED before any kernel runs: m in {48, 64} (ks = 256)
+ * with k > 448 needs 4 nprobe + d <= 1912; the generic kernel (other m, or ks = 16) needs
+ * 4 (m ks + d + 4 nprobe) + 64 next_pow2(k + 32) + 8 next_pow2(8 k) <= 227 KB.
+ * Non-finite values (IVF-PQ): results rank by (distance, id), NaN after every number, equal distances by the smaller id
+ * (the oracle keeps its scan order among equal or NaN distances).  A NaN query component makes every probed distance
+ * NaN (the row is the k smallest probed ids); an infinite one can give NaN where the oracle gives +-inf, because the scan
+ * adds the per-probe and per-code terms of its decomposition (+inf + -inf); a query whose L2 distances overflow gets +inf.
+ * With sharding the result is this shard's local top-k (merge with
  * vix_merge_topk_f32 after an all-gather). */
 int vix_index_search(vix_index_t* h, const float* queries, int64_t nq, int k, int nprobe,
                      float* out_dist, int64_t* out_ids);

@@ -4,6 +4,7 @@ distances within 1e-5 relative; top-k id sets equal except at ties inside that t
 kernel restates the reference's summation order (flat scan, probe scores, LUT, materialising ADC) the
 comparison is bit-exact as well."""
 import os
+import re
 
 import numpy as np
 import pytest
@@ -633,22 +634,40 @@ def _make_ivfpq_problem(oracle, n, d, m, kc, nq, seed, sift=False, unit=False):
     return xb, q, coarse, cb, norms
 
 
+# the route each row takes in the query-major scan (VIX_SCAN_DEBUG=1): "fast G table bias" or "generic"
+STAGEWISE_ROUTE = {
+    (20000, 128, 16): "fast 1 kernel kernel",
+    (12000, 96, 48): "fast 3 kernel kernel",
+    (8000, 64, 8): "generic",
+    (6000, 48, 12): "generic",
+    (6000, 160, 80): "generic",
+    (6000, 192, 96): "generic",
+    (5000, 256, 128): "generic",
+    (8000, 128, 32): "fast 2 kernel kernel",
+    (9000, 128, 64): "fast 4 kernel kernel",
+    (6000, 512, 64): "fast 4 image kernel",
+    (5000, 768, 64): "fast 4 image kernel",
+    (4000, 640, 64): "fast 4 image kernel",
+    (3000, 1664, 64): "fast 4 kernel kernel",
+}
+
+
 @pytest.mark.parametrize("n,d,m,kc,nprobe,metric,kind", [
-    (20000, 128, 16, 64, 8, 0, "sift"),      # C3-shaped, fast path m=16
-    (12000, 96, 48, 50, 6, 0, "unit"),       # C5-shaped, m=48 (dsub=2)
-    (8000, 64, 8, 30, 5, 0, "gauss"),        # m=8: four vector blocks per warp pass
-    (6000, 48, 12, 20, 5, 0, "gauss"),       # generic m (not 32 F + {0, 8, 16}): AoS fallback kernel
-    (6000, 160, 80, 24, 5, 0, "gauss"),      # m=80 = 2 full passes + 16 left over (two 64 KB tables)
-    (6000, 192, 96, 24, 5, 1, "unit"),       # m=96 inner product
-    (5000, 256, 128, 16, 4, 0, "gauss"),     # m=128: largest table
-    (8000, 128, 32, 40, 40, 0, "gauss"),     # nprobe == kc: exhaustive
-    (9000, 128, 64, 32, 6, 1, "unit"),       # C4-shaped inner product, m=64
-    (6000, 512, 64, 24, 5, 0, "gauss"),      # 512 KB of codebooks: tables built batch-wide (lut_image_kernel), dsub=8
-    (5000, 768, 64, 16, 4, 1, "unit"),       # C4's d / m: dsub=12, inner product, batch-wide tables + batch-wide bias
-    (4000, 640, 64, 16, 4, 0, "gauss"),      # dsub=10: scalar codebook reads in the batch-wide table build
-    (3000, 1664, 64, 12, 4, 0, "gauss"),     # d=1664 (near the exact engine's limit): the staged queries leave room for 15 of 16 warps; dsub=26
+    (20000, 128, 16, 64, 8, 0, "sift"),            # C3-shaped, fast kernel m=16
+    (12000, 96, 48, 50, 6, 0, "unit"),             # C5-shaped, m=48 (dsub=2)
+    (8000, 64, 8, 30, 5, 0, "gauss"),              # m=8: generic kernel (the fast one takes m = 16, 32, 48, 64)
+    (6000, 48, 12, 20, 5, 0, "gauss"),             # m=12: generic kernel
+    (6000, 160, 80, 24, 5, 0, "gauss"),            # m=80: generic kernel, 80 KB table
+    (6000, 192, 96, 24, 5, 1, "unit"),             # m=96 inner product: generic kernel
+    (5000, 256, 128, 16, 4, 0, "gauss"),           # m=128: generic kernel, largest table (128 KB)
+    (8000, 128, 32, 40, 40, 0, "gauss"),           # nprobe == kc: exhaustive
+    (9000, 128, 64, 32, 6, 1, "unit"),             # C4-shaped inner product, m=64
+    (6000, 512, 64, 24, 5, 0, "gauss"),            # 512 KB of codebooks: tables built batch-wide (lut_image_kernel), dsub=8
+    (5000, 768, 64, 16, 4, 1, "unit"),             # C4's d / m: dsub=12, inner product, batch-wide tables (d x nprobe = 3072: bias in the scan)
+    (4000, 640, 64, 16, 4, 0, "gauss"),            # dsub=10: scalar codebook reads in the batch-wide table build
+    (3000, 1664, 64, 12, 4, 0, "gauss"),           # d=1664 (near the exact engine's limit): staged queries still leave room for 16 warps; dsub=26 (tables in the scan)
 ])
-def test_ivfpq_index_stagewise_parity(oracle, n, d, m, kc, nprobe, metric, kind):
+def test_ivfpq_index_stagewise_parity(oracle, monkeypatch, capfd, n, d, m, kc, nprobe, metric, kind):
     from vectorindex_b200.index import IVFPQIndex
     nq, k = 64, 10
     xb, q, coarse, cb, norms = _make_ivfpq_problem(oracle, n, d, m, kc, nq, seed=n + m, sift=(kind == "sift"),
@@ -670,9 +689,17 @@ def test_ivfpq_index_stagewise_parity(oracle, n, d, m, kc, nprobe, metric, kind)
     assert np.array_equal(lids, ids[order])
     assert np.array_equal(codes, ocodes[order])
     assert np.array_equal(idx.list_sizes(), np.diff(ooff))
-    # search: probes exact, distances 1e-5, id sets up to ties
+    # the route of the search (VIX_SCAN_DEBUG line of the query-major scan): kernel, G, table source, bias source
     od, oi, op = oracle.ivfpq_search(q, coarse, cb, norms, off, codes, lids, m, 256, nprobe, k, metric)
+    capfd.readouterr()
+    monkeypatch.setenv("VIX_SCAN_DEBUG", "1")
     gd, gi, gp = idx.batch_search(q, k, return_probes=True)
+    monkeypatch.delenv("VIX_SCAN_DEBUG")
+    lines = re.findall(r"\[vix scan\] kernel (fast G (\d)|generic),.*table (\w+), bias (\w+)", capfd.readouterr().err)
+    assert len(lines) == 1, lines
+    got = "generic" if lines[0][0] == "generic" else f"fast {lines[0][1]} {lines[0][2]} {lines[0][3]}"
+    assert got == STAGEWISE_ROUTE[(n, d, m)]
+    # search: probes exact, distances 1e-5, id sets up to ties
     assert np.array_equal(gp, op)
     scale = float(np.nanmax(np.abs(od)))
     assert_topk_close(gd, gi, od, oi, rtol=RTOL, atol=RTOL * scale * (1.0 if metric == 1 else 0.0))

@@ -6,20 +6,19 @@ sets them too (search_with_probes), so the route of every query is known before 
     VIX_TC_SCAN_DEBUG=1 gives the queries handed back to the query-major scan, the finalists (most per query) and the log
     capacity, and that no pipeline wait timed out;
   - bit equality with the query-major scan (vix_ivfpq_scan.cu), which the rest of the suite pins to the oracle;
-  - a float64 reference of ||q - c_l - r^||^2 that shares no code with either scan or the oracle (ref64).
+  - a float64 reference of ||q - c_l - r^||^2 that shares no code with either scan or the oracle (pq_ref64.ref64).
 """
-import collections
 import re
 
 import numpy as np
 import pytest
 
+from pq_ref64 import RTOL, assert_ref64, ref64
 from test_gpu_parity import _make_ivfpq_problem, assert_topk_close, bits
 from vectorindex_b200 import _lib
 
 pytestmark = pytest.mark.gpu
 
-RTOL = 1e-5
 TINY = float(np.finfo(np.float32).tiny)
 LOG_CAP = 4096            # records of one filter warp's log at small batches (launch_ivfpq_scan_tc: at least 4096)
 ROUTE = re.compile(r"\[vix tc scan\] nq (\d+), handed back (\d+), candidates (\d+) \(max (\d+) per query; (\d+) per log\), "
@@ -81,56 +80,6 @@ class Lists:
 
     def handed_back(self, probes, k):
         return int(self.flagged(probes, k).sum())
-
-
-def ref64(q, coarse, cb, probes, off, codes, lids, k):
-    """float64 top-k of ||q - c_l - r^||^2, r^ = (cb_j[code_j])_j, over the vectors of the probed lists (-1 and probes outside
-    [0, kc) skipped), by (distance, id).  Returns (dist [nq x k], ids [nq x k], per query (d64, ids, tol) of every probed
-    vector).  tol is what the fp32 decomposition bias + t_x - 2 <q, r^> of both scans may be off by:
-    1e-5 (||q - c||^2 + |t_x| + 2 ||q|| ||r^||)."""
-    q64, c64, cb64 = (np.asarray(a, np.float64) for a in (q, coarse, cb))
-    kc, m = c64.shape[0], cb64.shape[0]
-    rhat = cb64[np.arange(m), codes.astype(np.intp)].reshape(len(codes), -1)
-    lens = np.diff(off)
-    nq = q64.shape[0]
-    dist, ids, cand = np.full((nq, k), np.nan), np.full((nq, k), -1, np.int64), []
-    for r in range(nq):
-        ls = [int(l) for l in probes[r] if 0 <= l < kc and lens[l] > 0]
-        rows = np.concatenate([np.arange(off[l], off[l + 1]) for l in ls]) if ls else np.zeros(0, np.intp)
-        cl = c64[np.repeat(np.array(ls, np.intp), lens[ls])] if ls else np.zeros((0, c64.shape[1]))
-        rr = rhat[rows]
-        qc = q64[r] - cl
-        d64 = ((qc - rr) ** 2).sum(1)
-        tx = (rr * rr).sum(1) + 2.0 * (cl * rr).sum(1)
-        tol = RTOL * ((qc * qc).sum(1) + np.abs(tx) + 2.0 * np.linalg.norm(q64[r]) * np.linalg.norm(rr, axis=1))
-        idr = lids[rows]
-        o = np.lexsort((idr, d64))[:k]
-        dist[r, :o.size], ids[r, :o.size] = d64[o], idr[o]
-        cand.append((d64, idr, tol, o))
-    return dist, ids, cand
-
-
-def assert_ref64(gd, gi, ref):
-    """as many results as min(k, vectors probed), each distance within tol of the float64 value of its id, the id set that
-    of the reference except for ties at the k-th distance within tol (ids stored twice counted twice)"""
-    _, _, cand = ref
-    k = gd.shape[1]
-    for r, (d64, idr, tol, o) in enumerate(cand):
-        nv = min(k, d64.size)
-        assert (gi[r, :nv] >= 0).all() and (gi[r, nv:] == -1).all() and np.isnan(gd[r, nv:]).all(), \
-            f"row {r}: {(gi[r] >= 0).sum()} results, {d64.size} vectors probed, k {k}"
-        if nv == 0:
-            continue
-        assert (np.diff(gd[r, :nv]) >= 0).all(), f"row {r}: distances not ascending"
-        kth, tk = d64[o[nv - 1]], tol[o[nv - 1]]
-        for i, g in zip(gi[r, :nv].tolist(), gd[r, :nv].astype(np.float64).tolist()):
-            sel = idr == i
-            assert sel.any(), f"row {r}: id {i} is not in a probed list"
-            assert (np.abs(d64[sel] - g) <= tol[sel]).any(), f"row {r} id {i}: {g} vs float64 {d64[sel].min()}"
-            assert (d64[sel] - tol[sel] <= kth + tk).any(), f"row {r} id {i}: {g} beyond the k-th distance {kth}"
-        got = collections.Counter(gi[r, :nv].tolist())
-        for i, c in collections.Counter(idr[d64 + tol < kth - tk].tolist()).items():
-            assert got[i] >= c, f"row {r}: id {i} (clearly inside the top {k}) missing"
 
 
 def tc_launches():

@@ -871,7 +871,8 @@ int index_search_locked(vix_index* h, const float* queries, int64_t nq, int k, i
         if (traced) for (int e = 1; e < 5; ++e) VIX_CUDA(cudaEventRecord(tev[e], s));
     } else {
         if (nprobe <= 0) nprobe = h->p.nprobe;
-        VIX_REQUIRE(nprobe > 0, VIX_ERR_INVALID_K, "index_search: nprobe must be > 0");
+        VIX_REQUIRE(nprobe > 0 && nprobe <= VIX_MAX_K, VIX_ERR_INVALID_K, "index_search: nprobe = %d (1 .. %d)", nprobe,
+                    VIX_MAX_K);
         if (h->dirty) VIX_TRY(build_lists(h));
         VIX_TRY(dp.stage(out_probes, out_probes ? (size_t)nq * nprobe : 0));
         Scratch<int32_t> probes;

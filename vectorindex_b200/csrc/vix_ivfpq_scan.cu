@@ -180,6 +180,24 @@ __device__ VIX_SCAN_FN void build_probe_table(const float* __restrict__ q, int d
             carry += __shfl_sync(0xFFFFFFFFu, inc, 31);
         }
     }
+    // probes 256 .. VIX_MAX_K - 1 (rare): the same rounds, one at a time
+    for (int p0 = 256; p0 < nprobe; p0 += 32) {
+        const int pp = p0 + lane;
+        const int l = (pp < nprobe) ? __ldg(qprobes + pp) : -1;
+        const bool ok = (unsigned)l < (unsigned)kc;
+        const int len = ok ? __ldg(list_len + l) : 0;
+        const int nch = (len + 31) >> 5;
+        int inc = nch;
+        for (int o = 1; o < 32; o <<= 1) { const int t = __shfl_up_sync(0xFFFFFFFFu, inc, o); if (lane >= o) inc += t; }
+        const unsigned ball = __ballot_sync(0xFFFFFFFFu, nch > 0);
+        if (nch > 0) {
+            const int p = np + __popc(ball & ((1u << lane) - 1u));
+            s_start[p] = (int)(__ldg(list_off + l) >> 5); s_len[p] = len; s_pref[p] = carry + inc - nch;
+            if (qbias) s_bias[p] = __ldg(qbias + pp); else s_list[p] = l;
+        }
+        np += __popc(ball);
+        carry += __shfl_sync(0xFFFFFFFFu, inc, 31);
+    }
     if (lane == 0) { s_pref[np] = carry; *s_np = np; }
     __syncwarp();
     if (qbias) return;                                     // precomputed batch-wide (probe_bias_kernel)
@@ -734,11 +752,11 @@ ivfpq_scan_generic_kernel(ScanArgs a) {
     for (int64_t qi = blockIdx.x; qi < a.nq; qi += gridDim.x) {
         __syncthreads();
         for (int e = tid; e < a.d; e += kScanThreads) s_q[e] = a.queries[qi * (int64_t)a.d + e];
-        if (tid < a.nprobe) {
-            const int l = a.probes[qi * (int64_t)a.nprobe + tid];
+        for (int p = tid; p < a.nprobe; p += kScanThreads) {
+            const int l = a.probes[qi * (int64_t)a.nprobe + p];
             const bool ok = (unsigned)l < (unsigned)a.kc;
-            s_start[tid] = ok ? (int)(a.list_off[l] >> 5) : 0;
-            s_len[tid] = ok ? a.list_len[l] : 0;
+            s_start[p] = ok ? (int)(a.list_off[l] >> 5) : 0;
+            s_len[p] = ok ? a.list_len[l] : 0;
         }
         __syncthreads();
         if (tid == 0) {
@@ -856,34 +874,41 @@ static size_t generic_smem_bytes(const ScanArgs& a) {
     return s;
 }
 
-template <int G, bool FILTER>
-static int launch_fast(ScanArgs& a) {
-    const bool stats = a.phase_cycles != nullptr;
-    constexpr int NTAB = (G + 1) / 2;
-    // as many warps as the per-warp selection queues leave room for (24 unless k is large)
-    // The tables start at a 64 KB boundary of the shared window; the bookkeeping (probe tables, queries, selection queues)
-    // sits in front of them, behind the <= 1 KB the system keeps at the start of the window.  Two tables must start at
-    // 64 KB (they end at 192 of 227 KB); one table may also start at 128 KB.  Large d / nprobe / k are paid for with
-    // fewer warps (smaller queues).
-    const size_t misc_limit = (NTAB == 2) ? 65536 - 1024 : 100 * 1024;
-    int nwarps = kFastThreads / 32;
+// Warps and shared memory of the fast kernel for (m, d, k, nprobe), with a.Pw set.  The tables start at a 64 KB boundary of
+// the shared window; the bookkeeping (probe tables, queries, selection queues) sits in front of them, behind the <= 1 KB
+// the system keeps at the start of the window.  Two tables must start at 64 KB (they end at 192 of 227 KB); one table
+// may also start at 128 KB.  Large d / nprobe / k are paid for with fewer warps (smaller queues): 16 unless k is large,
+// at least 3 while that fits, and 2 (warps 0 and 1 carry every role of the pipeline) when only that fits -- two
+// tables with k > 448 (Pw = 1024).  nwarps = 0: not even that fits (two tables, k > 448 and 4 nprobe + d > 1912).
+struct FastPlan { int nwarps; size_t misc, misc_limit, smem; };
+static FastPlan fast_plan(const ScanArgs& a) {
+    const int NTAB = (a.m / 16 + 1) / 2;
+    FastPlan f;
+    f.misc_limit = (NTAB == 2) ? 65536 - 1024 : 100 * 1024;
     auto misc_bytes = [&](int w) {
         return 2 * ((size_t)a.nprobe * 16 + 4) + 2 * (size_t)a.d * 4 + 40 + 16 + 3 * (size_t)w * a.Pw * 8;
     };
-    while (nwarps > 3 && (3 * (size_t)nwarps * a.Pw * 8 > 56 * 1024 || misc_bytes(nwarps) > misc_limit)) --nwarps;
-    const size_t misc = misc_bytes(nwarps);
-    VIX_REQUIRE(misc <= misc_limit, VIX_ERR_UNSUPPORTED,
-                "ivfpq scan: d = %d, k = %d, nprobe = %d need %zu bytes of bookkeeping shared memory (limit %zu)", a.d, a.k,
-                a.nprobe, misc, misc_limit);
-    size_t smem = misc + 65535 + (size_t)NTAB * 65536;
-    if (smem > 227 * 1024) smem = 227 * 1024;
+    f.nwarps = kFastThreads / 32;
+    while (f.nwarps > 3 && (3 * (size_t)f.nwarps * a.Pw * 8 > 56 * 1024 || misc_bytes(f.nwarps) > f.misc_limit)) --f.nwarps;
+    if (misc_bytes(f.nwarps) > f.misc_limit) f.nwarps = 2;
+    f.misc = misc_bytes(f.nwarps);
+    if (f.misc > f.misc_limit) f.nwarps = 0;
+    f.smem = f.misc + 65535 + (size_t)NTAB * 65536;
+    if (f.smem > 227 * 1024) f.smem = 227 * 1024;
+    return f;
+}
+
+template <int G, bool FILTER>
+static int launch_fast(ScanArgs& a, const FastPlan& f) {
+    const bool stats = a.phase_cycles != nullptr;
+    const size_t smem = f.smem;
     a.smem_bytes = (int)smem;
     auto kern = stats ? ivfpq_scan_kernel<G, FILTER, true> : ivfpq_scan_kernel<G, FILTER, false>;
     VIX_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int64_t grid = num_sms();
     if (grid > a.nq) grid = a.nq;
     if (a.ev_kernel[0]) VIX_CUDA(cudaEventRecord(a.ev_kernel[0], ctx().stream));
-    kern<<<(unsigned)grid, 32 * nwarps, smem, ctx().stream>>>(a);
+    kern<<<(unsigned)grid, 32 * f.nwarps, smem, ctx().stream>>>(a);
     VIX_LAUNCH_CHECK();
     if (a.ev_kernel[1]) VIX_CUDA(cudaEventRecord(a.ev_kernel[1], ctx().stream));
     return VIX_OK;
@@ -958,13 +983,18 @@ int launch_ivfpq_scan(ScanArgs& a) {
 // query-major: one look-up table per query
 int launch_ivfpq_scan_classic(ScanArgs& a) {
     const ScanLayout L = scan_layout(a.m);
+    const bool debug = getenv("VIX_SCAN_DEBUG") != nullptr;
+    VIX_REQUIRE(a.nprobe > 0 && a.nprobe <= VIX_MAX_K, VIX_ERR_INVALID_K, "ivfpq scan: nprobe = %d (1 .. %d)", a.nprobe, VIX_MAX_K);
     if (!L.fast || a.ks != 256) {
         a.Pw = next_pow2(a.k + 32);
         a.P2 = next_pow2(kScanWarps * a.k);
         const size_t smem = generic_smem_bytes(a);
         VIX_REQUIRE(smem <= 227 * 1024, VIX_ERR_UNSUPPORTED,
                     "ivfpq scan: m = %d, k = %d, nprobe = %d need %zu bytes of shared memory", a.m, a.k, a.nprobe, smem);
-        VIX_REQUIRE(a.nprobe <= kScanThreads, VIX_ERR_INVALID_K, "ivfpq scan: nprobe > %d", kScanThreads);
+        if (debug)
+            fprintf(stderr, "[vix scan] kernel generic, filter %d, stats %d, warps %d, Pw %d, P2 %d, table kernel, bias kernel, "
+                    "order no, items %lld\n", a.filter != nullptr, a.phase_cycles != nullptr, kScanWarps, a.Pw, a.P2,
+                    (long long)a.nq);
         VIX_CUDA(cudaFuncSetAttribute(ivfpq_scan_generic_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         int occ = 1;
         VIX_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, ivfpq_scan_generic_kernel, kScanThreads, smem));
@@ -978,7 +1008,10 @@ int launch_ivfpq_scan_classic(ScanArgs& a) {
     }
     a.Pw = next_pow2(a.k + 64);
     a.P2 = 0;
-    VIX_REQUIRE(a.nprobe <= 256, VIX_ERR_INVALID_K, "ivfpq scan: nprobe > 256");
+    const FastPlan plan = fast_plan(a);
+    VIX_REQUIRE(plan.nwarps > 0, VIX_ERR_UNSUPPORTED,
+                "ivfpq scan: d = %d, k = %d, nprobe = %d need %zu bytes of bookkeeping shared memory (limit %zu)", a.d, a.k,
+                a.nprobe, plan.misc, plan.misc_limit);
     VIX_REQUIRE(a.work_counter != nullptr, VIX_ERR_NULL_PTR, "ivfpq scan: work counter missing");
     VIX_CUDA(cudaMemsetAsync(a.work_counter, 0, 2 * sizeof(int), ctx().stream));
     // a kernel that finds its shared-memory layout does not fit refuses loudly: it raises the mapped host flag that the
@@ -986,7 +1019,9 @@ int launch_ivfpq_scan_classic(ScanArgs& a) {
     int* const loud = pipeline_error_flag();
     a.status = loud ? loud : a.work_counter + 1;
     Scratch<float> bias;
+    const char* bias_src = a.bias ? "given" : "kernel";
     if (!a.bias && (int64_t)a.d * a.nprobe > 8192) {
+        bias_src = (size_t)a.d * 4 * 8 <= 48 * 1024 ? "rows" : "pairs";      // launch_probe_bias's choice
         // one staging warp per CTA cannot hide this much bias arithmetic behind a query's scan: do it batch-wide
         VIX_TRY(bias.alloc((size_t)(a.nq * (int64_t)a.nprobe)));
         VIX_TRY(launch_probe_bias(a, bias.ptr));
@@ -1012,11 +1047,19 @@ int launch_ivfpq_scan_classic(ScanArgs& a) {
         VIX_LAUNCH_CHECK();
         a.lut_image = image.ptr;
     }
+    if (debug) {
+        // work items: the batch, or (queries handed back by the list-major scan) a count only the device knows
+        char items[32] = "device";
+        if (!a.nq_dev) snprintf(items, sizeof items, "%lld", (long long)a.nq);
+        fprintf(stderr, "[vix scan] kernel fast G %d, filter %d, stats %d, warps %d, Pw %d, P2 %d, table %s, bias %s, "
+                "order %s, items %s\n", a.m / 16, a.filter != nullptr, a.phase_cycles != nullptr, plan.nwarps, a.Pw, a.P2,
+                a.lut_image ? "image" : "kernel", bias_src, a.order && !a.nq_dev ? "yes" : "no", items);
+    }
     switch (a.m) {
-        case 16: return a.filter ? launch_fast<1, true>(a) : launch_fast<1, false>(a);
-        case 32: return a.filter ? launch_fast<2, true>(a) : launch_fast<2, false>(a);
-        case 48: return a.filter ? launch_fast<3, true>(a) : launch_fast<3, false>(a);
-        case 64: return a.filter ? launch_fast<4, true>(a) : launch_fast<4, false>(a);
+        case 16: return a.filter ? launch_fast<1, true>(a, plan) : launch_fast<1, false>(a, plan);
+        case 32: return a.filter ? launch_fast<2, true>(a, plan) : launch_fast<2, false>(a, plan);
+        case 48: return a.filter ? launch_fast<3, true>(a, plan) : launch_fast<3, false>(a, plan);
+        case 64: return a.filter ? launch_fast<4, true>(a, plan) : launch_fast<4, false>(a, plan);
     }
     set_error("ivfpq scan: unsupported m = %d", a.m);
     return VIX_ERR_UNSUPPORTED;
