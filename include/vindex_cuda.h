@@ -37,7 +37,9 @@
  *                            table source (image: batch-wide lut_image_kernel; kernel: built in the scan), the bias source
  *                            (kernel: in the scan; rows: probe_bias_rows_kernel; pairs: probe_bias_kernel; given: by the
  *                            list-major scan), the locality order (yes / no) and the work items (query count, or device:
- *                            the queries the list-major scan hands back)
+ *                            the queries the list-major scan hands back); and per vix_index_range_search call one line
+ *                            "[vix range] kind K, kernel fast G n | generic | ivfflat | flat, filter 0|1, passes 1|2, total T,
+ *                            max_row M, sorted_long L" (L: rows longer than the in-shared-memory sort, merged in global memory)
  *   VIX_DISABLE_TC, VIX_DISABLE_PQ_TC, VIX_DISABLE_LUT_IMAGE
  *                            exact CUDA-core kernels instead of the tensor-core shortlists / per-query tables built inside
  *                            the scan instead of batch-wide (the parity tests compare both ways)
@@ -376,6 +378,36 @@ typedef struct {
 int vix_index_search_ex(vix_index_t* h, const float* queries, int64_t nq, int k, int nprobe,
                         float* out_dist, int64_t* out_ids, int32_t* out_probes /* [nq x nprobe] nullable */,
                         vix_search_stats* stats /* nullable */);
+
+/* Range search (Kernel #07, Operations/RangeQuery/RangeQuery.swift; rangeScanADC_u8 / _u4): for every query, EVERY stored
+ * vector whose API distance is <= radius, sorted ascending by (distance, id), as CSR in a result object the library owns.
+ *   - candidates: FLAT every stored row; IVF_FLAT / IVF_PQ the rows of the nprobe probed lists, chosen exactly as
+ *     vix_index_search chooses them (nprobe <= 0 => the configured nprobe; nprobe > VIX_MAX_K => VIX_ERR_INVALID_K; -1, ids
+ *     outside [0, kc) and empty lists skipped); an IVF_FLAT index without centroids scans every row, as its search does;
+ *   - distance: what vix_index_search returns for the same (query, vector) -- FLAT / IVF_FLAT: L2 sqrt(L2^2), IP -dot,
+ *     cosine 1 - similarity; IVF_PQ: L2 the ADC squared distance (no sqrt), IP -score -- bit for bit (IVF_PQ always takes
+ *     the query-major scan); the test is the IEEE comparison distance <= radius on that value: NaN distances never pass,
+ *     a NaN radius is VIX_ERR_INVALID_PARAM, +inf returns every candidate with a number for its distance, negative radii
+ *     are valid (an IP radius of -0.8 keeps dot >= 0.8);
+ *   - filter_words (nullable): the id filter of vix_index_search_filtered, applied before the radius test;
+ *   - a row stored twice, or a list probed twice, comes back twice; a dirty handle rebuilds its lists first, as search
+ *     does; on a shard the result is what THIS rank holds (no cross-rank merge).
+ * The call synchronises its stream once, even in asynchronous mode: the size of the answer depends on the data.  It
+ * normally scans once; when the answer outgrows the capacity the handle remembers from its previous call, the scan runs a
+ * second time with the exact capacity.  A result that does not fit in device memory returns VIX_ERR_OOM with nothing
+ * allocated and the handle unchanged.  nq == 0 gives an empty result (lims = {0}).  *out must be released with
+ * vix_range_result_destroy.  VIX_SCAN_DEBUG=1 prints one "[vix range] ..." line per call (kind, kernel, filter, passes,
+ * total, longest row, rows sorted in global memory). */
+typedef struct vix_range_result vix_range_result_t;
+int     vix_index_range_search(vix_index_t* h, const float* queries, int64_t nq, float radius, int nprobe,
+                               const uint64_t* filter_words /* nullable */, int64_t filter_capacity, int filter_mode,
+                               vix_range_result_t** out);
+int64_t vix_range_result_nq(const vix_range_result_t* r);
+int64_t vix_range_result_total(const vix_range_result_t* r);
+/* CSR: lims [nq + 1] (lims[0] = 0), dist / ids [total]; each nullable; host or device pointers (host outputs are valid when
+ * the call returns, device outputs as the usual asynchronous-mode rules say) */
+int     vix_range_result_get(const vix_range_result_t* r, int64_t* lims, float* dist, int64_t* ids);
+void    vix_range_result_destroy(vix_range_result_t* r);   /* NULL is a no-op */
 
 /* Search with an id filter: IDFilterBitset / idFilterPass of Operations/Filtering/IDFilter.swift:13-135 -- a bitset over
  * the dense id domain [0, capacity); ids outside the domain never pass; VIX_FILTER_ALLOW keeps ids whose bit is 1,

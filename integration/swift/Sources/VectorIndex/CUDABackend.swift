@@ -89,6 +89,19 @@ public final class CUDAIVFPQIndex {
                                                 Int32(VIX_FILTER_ALLOW.rawValue), &dist, &ids), "vix_index_search_filtered")
         return (dist, ids)
     }
+    /// RangeQuery.swift (Kernel #07): every vector within `radius` of each query, per query ascending by (distance, id), as
+    /// CSR (`lims[r] ..< lims[r + 1]` is query r); same candidates and distances as batchSearch.  One host synchronisation.
+    public func rangeSearch(_ q: [Float], nq: Int, radius: Float) throws -> (lims: [Int64], dist: [Float], ids: [Int64]) {
+        var res: OpaquePointer? = nil
+        try _vixCheck(vix_index_range_search(h, q, Int64(nq), radius, 0, nil, 0, Int32(VIX_FILTER_ALLOW.rawValue), &res),
+                      "vix_index_range_search")
+        defer { vix_range_result_destroy(res) }
+        let total = Int(vix_range_result_total(res))
+        var lims = [Int64](repeating: 0, count: nq + 1)
+        var dist = [Float](repeating: 0, count: total); var ids = [Int64](repeating: -1, count: total)
+        try _vixCheck(vix_range_result_get(res, &lims, &dist, &ids), "vix_range_result_get")
+        return (lims, dist, ids)
+    }
     // step 7 of the IVF-PQ query (docs/kernel-specs/DONE_22_adc_scan.md:873-878): ADC top-R, then Kernel #40 over the
     // original vectors (DenseArray reader: id = row of `vectors`); raw exact scores out (L2^2 / dot), best first
     public func batchSearchReranked(_ q: [Float], nq: Int, k: Int, rerankR: Int, vectors: UnsafePointer<Float>, count: Int)

@@ -90,7 +90,8 @@ _EXPORTS = [
     "vix_index_set_codebooks", "vix_index_get_coarse", "vix_index_get_codebooks", "vix_index_add", "vix_index_remove",
     "vix_index_import_lists", "vix_index_count", "vix_index_list_sizes", "vix_index_export_lists", "vix_index_clear",
     "vix_index_search", "vix_index_search_ex", "vix_index_search_rerank", "vix_index_trace", "vix_index_trace_get", "vix_index_probe_range", "vix_index_search_with_probes",
-    "vix_index_search_with_probes_ex", "vix_index_search_filtered",
+    "vix_index_search_with_probes_ex", "vix_index_search_filtered", "vix_index_range_search", "vix_range_result_nq",
+    "vix_range_result_total", "vix_range_result_get", "vix_range_result_destroy",
     "vix_comm_unique_id", "vix_comm_create", "vix_comm_destroy", "vix_comm_rank", "vix_comm_world",
     "vix_comm_uses_peer_memory", "vix_comm_trace", "vix_comm_trace_get", "vix_sharded_query_block", "vix_sharded_add", "vix_sharded_search",
     "vix_index_encode", "vix_index_add_encoded", "vix_debug_tc_scores_f32", "vix_debug_tc_codes", "vix_accel_rank_candidates_f32",
@@ -118,6 +119,9 @@ def lib() -> C.CDLL:
         L.vix_tc_shortlist_calls.restype = C.c_int64
         L.vix_tc_shortlist_exact_rows.restype = C.c_int64
         L.vix_index_count.restype = C.c_int64
+        L.vix_range_result_nq.restype = C.c_int64
+        L.vix_range_result_total.restype = C.c_int64
+        L.vix_range_result_destroy.restype = None
         L.vix_index_destroy.restype = None
         L.vix_index_params_default.restype = None
         L.vix_clear_error.restype = None

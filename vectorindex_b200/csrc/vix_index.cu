@@ -16,10 +16,13 @@
 #include "vix_exact.cuh"
 #include "vix_scan.cuh"
 #include "vix_index.cuh"
+#include "vix_range.cuh"
 
 #include <cub/cub.cuh>
 
 #include <new>
+#include <stdio.h>
+#include <stdlib.h>
 
 using namespace vix;
 
@@ -517,6 +520,52 @@ ivfflat_scan_kernel(const float* __restrict__ queries, int64_t nq, int d, const 
     }
 }
 
+// Range variant of the candidate scan: the same candidates and arithmetic, every candidate whose API distance is within the
+// radius appended to the range output (vix_range.cuh) with a per-query count.
+__global__ void __launch_bounds__(256)
+ivfflat_range_kernel(const float* __restrict__ queries, int64_t nq, int d, const int32_t* __restrict__ probes,
+                     int nprobe, const int64_t* __restrict__ list_off, const int32_t* __restrict__ list_len, int kc,
+                     const float* __restrict__ slot_vecs, const int64_t* __restrict__ slot_ids, int metric,
+                     const uint64_t* __restrict__ filter, int64_t filter_cap, int filter_deny, RangeOut out) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    float* s_q = reinterpret_cast<float*>(smem_raw);
+    __shared__ int s_cnt;
+    for (int64_t qi = blockIdx.x; qi < nq; qi += gridDim.x) {
+        __syncthreads();
+        for (int e = threadIdx.x; e < d; e += blockDim.x) s_q[e] = queries[qi * (int64_t)d + e];
+        if (threadIdx.x == 0) s_cnt = 0;
+        __syncthreads();
+        const float qmag2 = (metric == VIX_METRIC_COSINE) ? seq_sumsq(s_q, d) : 0.0f;
+        for (int p = 0; p < nprobe; ++p) {
+            const int l = probes[qi * (int64_t)nprobe + p];
+            if ((unsigned)l >= (unsigned)kc) continue;           // -1 padding, or an id no list has
+            const int64_t b = list_off[l];
+            const int len = list_len[l];
+            for (int base = 0; base < len; base += blockDim.x) {
+                const int i = base + threadIdx.x;
+                bool pass = false;
+                u64 key = 0;
+                if (i < len && (!filter || id_filter_pass(filter, filter_cap, filter_deny, slot_ids[b + i]))) {
+                    const float* v = slot_vecs + (b + i) * (int64_t)d;
+                    float dist;
+                    if (metric == VIX_METRIC_L2) dist = __fsqrt_rn(exact_pair<SpecDirect16L2>(s_q, v, d));
+                    else if (metric == VIX_METRIC_IP) dist = -exact_pair<SpecIp4>(s_q, v, d);
+                    else dist = cosine_distance(exact_pair<SpecIp4>(s_q, v, d), qmag2, seq_sumsq(v, d));
+                    pass = dist <= out.radius;
+                    key = make_key(dist, (uint32_t)slot_ids[b + i], 0);
+                }
+                const unsigned ball = __ballot_sync(0xFFFFFFFFu, pass);
+                if (ball) {
+                    range_append(out, ball, pass, key, (uint32_t)qi);
+                    if ((threadIdx.x & 31) == 0) atomicAdd(&s_cnt, __popc(ball));
+                }
+            }
+        }
+        __syncthreads();
+        if (threadIdx.x == 0) out.counts[qi] = (unsigned long long)s_cnt;
+    }
+}
+
 // ------------------------------------------------------------------------------------------------
 // host-side index logic
 // ------------------------------------------------------------------------------------------------
@@ -971,6 +1020,98 @@ int index_search_locked(vix_index* h, const float* queries, int64_t nq, int k, i
     return rc;
 }
 
+// One range search of an index whose mutex the caller holds: the candidates of index_search_locked (every row, or the probed
+// lists of the same probe selection), each kind through its range kernel, the output path of vix_range.cu.
+static int index_range_locked(vix_index* h, const float* queries, int64_t nq, float radius, int nprobe,
+                              const FilterArgs* filter, vix_range_result** out) {
+    const int d = h->p.d;
+    cudaStream_t s = ctx().stream;
+    const bool linear = h->p.kind == VIX_INDEX_FLAT || !h->has_coarse;
+    if (!linear) {
+        if (nprobe <= 0) nprobe = h->p.nprobe;
+        VIX_REQUIRE(nprobe > 0 && nprobe <= VIX_MAX_K, VIX_ERR_INVALID_K, "vix_index_range_search: nprobe = %d (1 .. %d)", nprobe,
+                    VIX_MAX_K);
+    }
+    if (nq == 0) return range_empty(0, out);
+    In<float> dq;
+    VIX_TRY(dq.stage(queries, (size_t)nq * d));
+    size_t cap = h->range_cap;
+    RangeInfo info;
+    char kernel[32] = "flat";
+    int rc;
+    if (linear) {
+        // a flat index, or an IVF-Flat index before optimize(): the flat engine over the stored rows (IVFIndex.swift:820-832)
+        Scratch<uint64_t> mask;
+        if (filter && h->n > 0) {
+            const int64_t words = (h->n + 63) / 64;
+            VIX_TRY(mask.alloc((size_t)words));
+            filter_row_mask_kernel<<<(unsigned)((words + 255) / 256), 256, 0, s>>>(h->ids.ptr, h->n, filter->words, filter->cap,
+                                                                                filter->deny, mask.ptr);
+            VIX_LAUNCH_CHECK();
+        }
+        rc = range_collect(nq, radius, cap, h->p.metric == VIX_METRIC_IP, [&](const RangeOut& o) {
+            return flat_range_device(dq.dev, nq, h->vecs.ptr, h->n, d, h->p.metric, h->ids.ptr, mask.ptr, o);
+        }, out, &info);
+    } else {
+        if (h->dirty) VIX_TRY(build_lists(h));
+        Scratch<int32_t> probes;
+        VIX_TRY(probes.alloc((size_t)nq * nprobe));
+        if (h->p.metric == VIX_METRIC_COSINE)
+            VIX_TRY(probe_select_cosine_device(dq.dev, nq, h->coarse.ptr, h->kc, d, h->coarse_norms.ptr, nprobe, probes.ptr));
+        else
+            VIX_TRY(probe_select_fast_device(dq.dev, nq, h->coarse.ptr, h->kc, d, h->p.metric, nprobe, h->coarse_norms.ptr,
+                                             probes.ptr, nullptr, h->coarse_norm_max.ptr));
+        if (h->p.kind == VIX_INDEX_IVF_PQ) {
+            ScanArgs a{};
+            a.queries = dq.dev; a.nq = nq; a.d = d; a.m = h->p.m; a.ks = h->p.ks; a.dsub = d / h->p.m;
+            a.probes = probes.ptr; a.nprobe = nprobe; a.coarse = h->coarse.ptr; a.kc = h->kc; a.codebooks = h->codebooks.ptr;
+            a.list_off = h->list_off.ptr; a.list_len = h->list_len.ptr;
+            a.slot_codes = h->slot_codes.ptr; a.slot_tx = h->slot_tx.ptr; a.slot_ids = h->slot_ids.ptr;
+            a.metric = h->p.metric; a.codebooks_t = h->codebooks_t.ptr;
+            if (filter) { a.filter = filter->words; a.filter_cap = filter->cap; a.filter_deny = filter->deny; }
+            Scratch<int> work_counter;
+            VIX_TRY(work_counter.alloc(2));
+            a.work_counter = work_counter.ptr;
+            const bool fast = scan_layout(a.m).fast && a.ks == 256;
+            Scratch<int32_t> order;
+            if (fast && nq > 2 * num_sms()) {
+                VIX_TRY(query_order(probes.ptr, nq, nprobe, h->list_len.ptr, h->kc, order));
+                a.order = order.ptr;
+            }
+            if (fast) snprintf(kernel, sizeof kernel, "fast G %d", a.m / 16);
+            else snprintf(kernel, sizeof kernel, "generic");
+            // never the list-major tensor-core scan: the query-major one with its range instantiations
+            rc = range_collect(nq, radius, cap, h->p.metric == VIX_METRIC_IP, [&](const RangeOut& o) {
+                ScanArgs b = a;
+                b.range = o;
+                return launch_ivfpq_scan_classic(b);
+            }, out, &info);
+        } else {
+            snprintf(kernel, sizeof kernel, "ivfflat");
+            const size_t smem = (size_t)d * 4;
+            VIX_CUDA(cudaFuncSetAttribute(ivfflat_range_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            int64_t grid = (int64_t)num_sms() * 4;
+            if (grid > nq) grid = nq;
+            // (the IVF-Flat scan keys the distance itself, so its zeros are +0 as in k-NN search)
+            rc = range_collect(nq, radius, cap, false, [&](const RangeOut& o) -> int {
+                ivfflat_range_kernel<<<(unsigned)grid, 256, smem, s>>>(dq.dev, nq, d, probes.ptr, nprobe, h->list_off.ptr,
+                                                                     h->list_len.ptr, h->kc, h->slot_vecs.ptr, h->slot_ids.ptr,
+                                                                     h->p.metric, filter ? filter->words : nullptr,
+                                                                     filter ? filter->cap : 0, filter ? filter->deny : 0, o);
+                VIX_LAUNCH_CHECK();
+                return VIX_OK;
+            }, out, &info);
+        }
+    }
+    VIX_TRY(rc);
+    h->range_cap = cap;
+    if (getenv("VIX_SCAN_DEBUG"))
+        fprintf(stderr, "[vix range] kind %s, kernel %s, filter %d, passes %d, total %lld, max_row %lld, sorted_long %lld\n",
+                h->p.kind == VIX_INDEX_FLAT ? "flat" : h->p.kind == VIX_INDEX_IVF_FLAT ? "ivfflat" : "ivfpq", kernel,
+                filter != nullptr, info.passes, (long long)info.total, (long long)info.max_row, (long long)info.sorted_long);
+    return VIX_OK;
+}
+
 // gather rows of the sorted list layout back to add order / CSR export
 __global__ void export_lists_kernel(const int32_t* __restrict__ slot_row, const int64_t* __restrict__ off,
                                     const int32_t* __restrict__ len, int kc, const uint8_t* __restrict__ codes,
@@ -1296,6 +1437,28 @@ int vix_index_search_filtered(vix_index_t* h, const float* queries, int64_t nq, 
     FilterArgs f;
     f.words = fw.dev; f.cap = filter_capacity; f.deny = filter_mode == VIX_FILTER_DENY;
     return index_search_locked(h, queries, nq, k, nprobe, out_dist, out_ids, nullptr, nullptr, nullptr, &f);
+}
+
+int vix_index_range_search(vix_index_t* h, const float* queries, int64_t nq, float radius, int nprobe,
+                           const uint64_t* filter_words, int64_t filter_capacity, int filter_mode, vix_range_result_t** out) {
+    VIX_TRY(ensure_device());
+    VIX_REQUIRE(h && out, VIX_ERR_NULL_PTR, "vix_index_range_search: null pointer");
+    *out = nullptr;
+    VIX_REQUIRE(queries || nq == 0, VIX_ERR_NULL_PTR, "vix_index_range_search: null queries");
+    VIX_REQUIRE(nq >= 0 && nq < 0x7FFFFFFFLL, VIX_ERR_INVALID_PARAM, "vix_index_range_search: nq must lie in [0, 2^31 - 1)");
+    VIX_REQUIRE(radius == radius, VIX_ERR_INVALID_PARAM, "vix_index_range_search: radius is NaN");
+    VIX_REQUIRE(filter_mode == VIX_FILTER_ALLOW || filter_mode == VIX_FILTER_DENY, VIX_ERR_INVALID_PARAM,
+                "vix_index_range_search: filter_mode must be VIX_FILTER_ALLOW or VIX_FILTER_DENY");
+    VIX_REQUIRE(filter_capacity >= 0, VIX_ERR_INVALID_PARAM, "vix_index_range_search: negative capacity");
+    std::lock_guard<std::mutex> lk(h->mu);
+    VIX_REQUIRE(h->p.kind != VIX_INDEX_IVF_PQ || (h->has_coarse && h->has_pq), VIX_ERR_NOT_TRAINED,
+                "vix_index_range_search: IVF-PQ index is not trained");
+    if (!filter_words) return index_range_locked(h, queries, nq, radius, nprobe, nullptr, out);
+    In<uint64_t> fw;
+    VIX_TRY(fw.stage(filter_words, (size_t)((filter_capacity + 63) / 64)));
+    FilterArgs f;
+    f.words = fw.dev; f.cap = filter_capacity; f.deny = filter_mode == VIX_FILTER_DENY;
+    return index_range_locked(h, queries, nq, radius, nprobe, &f, out);
 }
 
 int vix_index_search_with_probes_ex(vix_index_t* h, const float* queries, int64_t nq, int k, const int32_t* probes,

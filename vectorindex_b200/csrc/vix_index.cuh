@@ -127,6 +127,7 @@ struct vix_index {
     DevBuf<unsigned long long> trace_scanned;
     int trace_cap = 0, trace_n = 0;
     std::vector<int> trace_path;        // IVF-PQ scan path of each traced call
+    size_t range_cap = 0;               // range search: entries the last call returned (+1/8), the next call's first capacity
 };
 
 

@@ -402,8 +402,10 @@ __device__ __noinline__ uint32_t flush_queue(u64* wq, int Pw, int k, int cnt, bo
 }
 
 // m = 16 G; FILTER: an id filter is active; STATS: the phase counters of vix_search_stats are kept (separate
-// instantiations, so the production kernel pays neither in instructions nor in registers).
-template <int G, bool FILTER, bool STATS>
+// instantiations, so the production kernel pays neither in instructions nor in registers).  RANGE: range search -- the
+// acceptance test is the constant radius on the API distance instead of the running k-th bound, and accepted entries go to
+// a.range (vix_range.cuh) instead of the per-warp queues; s_ncand counts them per query.
+template <int G, bool FILTER, bool STATS, bool RANGE = false>
 __global__ void __launch_bounds__(kFastThreads, 1)
 ivfpq_scan_kernel(ScanArgs a) {
     constexpr int m = 16 * G;
@@ -509,7 +511,9 @@ ivfpq_scan_kernel(ScanArgs a) {
         // ---- warp 0 first selects the k best of the candidates published for the PREVIOUS query and warp 1 builds
         //      the NEXT query's probe table; the other warps are already scanning, and chunks are handed out
         //      dynamically, so nobody waits for either
-        if (warp == 0 && have_prev) {
+        if (RANGE && warp == 0 && have_prev) {
+            if (lane == 0) { a.range.counts[prev_qi] = (unsigned long long)s_ncand[buf ^ 1]; s_ncand[buf ^ 1] = 0; }
+        } else if (warp == 0 && have_prev) {
             const long long t0 = STATS ? clock64() : 0;
             if (STATS && a.phase_cycles && lane == 0) atomicAdd(a.phase_cycles + 6, (unsigned long long)s_ncand[buf ^ 1]);
             select_and_write(s_cand + (size_t)(buf ^ 1) * nwarps * a.Pw, s_ncand[buf ^ 1], a.k, order_max, prev_qi, a.out_dist,
@@ -610,6 +614,23 @@ ivfpq_scan_kernel(ScanArgs a) {
             const float sum = (bias + tx) + ((s0 + s1) + (s2 + s3));
             if (valid) ++scanned_local;
             const u64 key = make_key(sum, 0u, order_max);
+            if constexpr (RANGE) {
+                // the API distance k-NN search reports for this entry (L2: the score; IP: minus the score); with the id
+                // the key is the k-NN one, which orders as make_key(api distance, id, 0)
+                const float api = order_max ? -key_score(key, 1) : key_score(key, 0);
+                bool pass = valid && api <= a.range.radius;
+                uint32_t id = 0;
+                if (pass) {
+                    id = (uint32_t)a.slot_ids[g];
+                    if (FILTER) pass = id_filter_pass(a.filter, a.filter_cap, a.filter_deny, (int64_t)id);
+                }
+                const unsigned ball = __ballot_sync(0xFFFFFFFFu, pass);
+                if (ball) {
+                    range_append(a.range, ball, pass, key | (u64)id, (uint32_t)qi);
+                    if (lane == 0) atomicAdd(s_ncand + buf, __popc(ball));
+                }
+                return;
+            }
             uint32_t ku = valid ? (uint32_t)(key >> 32) : 0xFFFFFFFFu;
             thr_u = min(thr_u, cta_t);
             uint32_t fid = 0;
@@ -679,7 +700,7 @@ ivfpq_scan_kernel(ScanArgs a) {
         }
 #endif
         // ---- publish the entries that can still make the top k into the CTA candidate buffer ----
-        {
+        if constexpr (!RANGE) {
             const uint32_t t = *cta_thr;
             if (t < thr_u) thr_u = t;
             const int lo = sorted_valid ? 0 : a.k;
@@ -728,6 +749,8 @@ ivfpq_scan_kernel(ScanArgs a) {
 // ------------------------------------------------------------------------------------------------
 // generic m (not 32 F + {0, 8, 16}): plain AoS codes, [m][256] table, one stored vector per thread
 // ------------------------------------------------------------------------------------------------
+// RANGE: range search, as in the fast kernel (the per-query count sits where the selection queues would)
+template <bool RANGE = false>
 __global__ void __launch_bounds__(kScanThreads)
 ivfpq_scan_generic_kernel(ScanArgs a) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -784,6 +807,7 @@ ivfpq_scan_generic_kernel(ScanArgs a) {
             s_lut[e] = lut_scale * dot;
         }
         for (int i = lane; i < a.Pw; i += 32) wq[i] = kEmptyKey;
+        if (RANGE && tid == 0) *reinterpret_cast<int*>(s_wq) = 0;
         __syncthreads();
 
         const int nchunks = s_pref[a.nprobe];
@@ -809,6 +833,22 @@ ivfpq_scan_generic_kernel(ScanArgs a) {
             const float tx = valid ? a.slot_tx[g] : 0.0f;
             const float sum = (s_bias[p] + tx) + s0;
             if (valid) ++scanned_local;
+            if constexpr (RANGE) {
+                const u64 key = make_key(sum, 0u, order_max);
+                const float api = order_max ? -key_score(key, 1) : key_score(key, 0);
+                bool pass = valid && api <= a.range.radius;
+                uint32_t id = 0;
+                if (pass) {
+                    id = (uint32_t)a.slot_ids[g];
+                    if (a.filter) pass = id_filter_pass(a.filter, a.filter_cap, a.filter_deny, (int64_t)id);
+                }
+                const unsigned ball = __ballot_sync(0xFFFFFFFFu, pass);
+                if (ball) {
+                    range_append(a.range, ball, pass, key | (u64)id, (uint32_t)qi);
+                    if (lane == 0) atomicAdd(reinterpret_cast<int*>(s_wq), __popc(ball));
+                }
+                continue;
+            }
             bool pass = valid && (order_max ? !(sum < thr_s) : !(sum > thr_s));
             uint32_t id = 0;
             if (pass) {
@@ -829,6 +869,11 @@ ivfpq_scan_generic_kernel(ScanArgs a) {
                     if (t != kEmptyKey) thr_s = key_score(t, order_max);
                 }
             }
+        }
+        if constexpr (RANGE) {
+            __syncthreads();
+            if (tid == 0) a.range.counts[qi] = (unsigned long long)*reinterpret_cast<int*>(s_wq);
+            continue;
         }
         if (cnt > 0) {
             for (int i = a.k + cnt + lane; i < a.Pw; i += 32) wq[i] = kEmptyKey;
@@ -871,6 +916,7 @@ static size_t generic_smem_bytes(const ScanArgs& a) {
     size_t s = (size_t)a.m * a.ks * 4;
     s += (size_t)a.d * 4 + (size_t)a.nprobe * 12 + (size_t)(a.nprobe + 1) * 4 + 16;
     s += (size_t)kScanWarps * a.Pw * 8 + (size_t)a.P2 * 8;
+    if (a.range.keys) s += 16;                    // the per-query count of range search
     return s;
 }
 
@@ -903,7 +949,8 @@ static int launch_fast(ScanArgs& a, const FastPlan& f) {
     const bool stats = a.phase_cycles != nullptr;
     const size_t smem = f.smem;
     a.smem_bytes = (int)smem;
-    auto kern = stats ? ivfpq_scan_kernel<G, FILTER, true> : ivfpq_scan_kernel<G, FILTER, false>;
+    auto kern = a.range.keys ? ivfpq_scan_kernel<G, FILTER, false, true>
+              : stats ? ivfpq_scan_kernel<G, FILTER, true> : ivfpq_scan_kernel<G, FILTER, false>;
     VIX_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int64_t grid = num_sms();
     if (grid > a.nq) grid = a.nq;
@@ -985,9 +1032,10 @@ int launch_ivfpq_scan_classic(ScanArgs& a) {
     const ScanLayout L = scan_layout(a.m);
     const bool debug = getenv("VIX_SCAN_DEBUG") != nullptr;
     VIX_REQUIRE(a.nprobe > 0 && a.nprobe <= VIX_MAX_K, VIX_ERR_INVALID_K, "ivfpq scan: nprobe = %d (1 .. %d)", a.nprobe, VIX_MAX_K);
+    const bool range = a.range.keys != nullptr;   // range search: no selection queues, no merge
     if (!L.fast || a.ks != 256) {
-        a.Pw = next_pow2(a.k + 32);
-        a.P2 = next_pow2(kScanWarps * a.k);
+        a.Pw = range ? 0 : next_pow2(a.k + 32);
+        a.P2 = range ? 0 : next_pow2(kScanWarps * a.k);
         const size_t smem = generic_smem_bytes(a);
         VIX_REQUIRE(smem <= 227 * 1024, VIX_ERR_UNSUPPORTED,
                     "ivfpq scan: m = %d, k = %d, nprobe = %d need %zu bytes of shared memory", a.m, a.k, a.nprobe, smem);
@@ -995,18 +1043,19 @@ int launch_ivfpq_scan_classic(ScanArgs& a) {
             fprintf(stderr, "[vix scan] kernel generic, filter %d, stats %d, warps %d, Pw %d, P2 %d, table kernel, bias kernel, "
                     "order no, items %lld\n", a.filter != nullptr, a.phase_cycles != nullptr, kScanWarps, a.Pw, a.P2,
                     (long long)a.nq);
-        VIX_CUDA(cudaFuncSetAttribute(ivfpq_scan_generic_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        auto kern = range ? ivfpq_scan_generic_kernel<true> : ivfpq_scan_generic_kernel<false>;
+        VIX_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         int occ = 1;
-        VIX_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, ivfpq_scan_generic_kernel, kScanThreads, smem));
+        VIX_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, kScanThreads, smem));
         int64_t grid = (int64_t)num_sms() * (occ < 1 ? 1 : occ);
         if (grid > a.nq) grid = a.nq;
         if (a.ev_kernel[0]) VIX_CUDA(cudaEventRecord(a.ev_kernel[0], ctx().stream));
-        ivfpq_scan_generic_kernel<<<(unsigned)grid, kScanThreads, smem, ctx().stream>>>(a);
+        kern<<<(unsigned)grid, kScanThreads, smem, ctx().stream>>>(a);
         VIX_LAUNCH_CHECK();
         if (a.ev_kernel[1]) VIX_CUDA(cudaEventRecord(a.ev_kernel[1], ctx().stream));
         return VIX_OK;
     }
-    a.Pw = next_pow2(a.k + 64);
+    a.Pw = range ? 0 : next_pow2(a.k + 64);
     a.P2 = 0;
     const FastPlan plan = fast_plan(a);
     VIX_REQUIRE(plan.nwarps > 0, VIX_ERR_UNSUPPORTED,

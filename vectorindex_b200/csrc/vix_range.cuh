@@ -1,0 +1,72 @@
+// vix_range.cuh -- the output path of range search (vix_index_range_search): every candidate whose API distance is at most
+// the radius, per query, sorted by (distance, id).
+//
+// The scan kernels (flat pair tiles, the IVF-Flat candidate scan, the query-major IVF-PQ scan) append each passing candidate
+// as the library's 64-bit selection key (make_key over the API distance, ids < 2^32) together with its query index, into a
+// buffer the call owns: one atomicAdd on a shared cursor per warp (warp-aggregated), and a per-query count kept by the
+// kernel.  Entries past the capacity are counted but not written; the host reads the total once, and when it exceeds the
+// capacity the scan runs once more with the exact capacity.  vix_range.cu then groups the entries by query (exclusive scan
+// of the counts + counting-sort scatter) and sorts each query's keys: one CTA in shared memory up to kRangeSegment keys,
+// runs of that size merged pass by pass in global memory above it.  No CUB on this path.
+#pragma once
+
+#include "vix_common.cuh"
+
+#include <functional>
+
+namespace vix {
+
+// where a scan kernel writes what passes (device pointers)
+struct RangeOut {
+    u64* keys = nullptr;                       // [cap] make_key(api distance, id, 0)
+    uint32_t* qry = nullptr;                   // [cap] query of the entry
+    unsigned long long* cursor = nullptr;      // [1]   entries appended (may exceed cap)
+    unsigned long long* counts = nullptr;      // [nq]  entries per query (written or added by the scan kernels)
+    unsigned long long cap = 0;
+    float radius = 0.0f;
+};
+
+#ifdef __CUDACC__
+// warp-collective (all 32 lanes): append the entries of the lanes whose bit is set in `ball` (= ballot of `pass`)
+__device__ __forceinline__ void range_append(const RangeOut& o, unsigned ball, bool pass, u64 key, uint32_t q) {
+    const int lane = threadIdx.x & 31;
+    unsigned long long base = 0;
+    if (lane == 0) base = atomicAdd(o.cursor, (unsigned long long)__popc(ball));
+    base = __shfl_sync(0xFFFFFFFFu, base, 0);
+    if (pass) {
+        const unsigned long long pos = base + (unsigned long long)__popc(ball & ((1u << lane) - 1u));
+        if (pos < o.cap) { o.keys[pos] = key; o.qry[pos] = q; }
+    }
+}
+#endif
+
+}  // namespace vix
+
+// the result object of vix_index_range_search (device memory owned by it)
+struct vix_range_result {
+    int64_t nq = 0, total = 0;
+    int64_t* lims = nullptr;     // [nq + 1]
+    float* dist = nullptr;       // [total]
+    int64_t* ids = nullptr;      // [total]
+};
+
+namespace vix {
+
+// What one range call reports for the [vix range] line of VIX_SCAN_DEBUG.
+struct RangeInfo { int passes = 0; int64_t total = 0, max_row = 0, sorted_long = 0; };
+
+// Runs `scan` (which appends into the RangeOut it is handed and fills the per-query counts) once, or twice when the first
+// capacity (cap_hint, updated for the next call) is too small, then groups, sorts and decodes the entries into a new result
+// object.  neg_zero: the path reports a zero distance as -0 (inner product through the flat engine and the IVF-PQ scan,
+// whose API distance is the negated score); the key keeps +0.  The only host synchronisation is the read of the total.
+int range_collect(int64_t nq, float radius, size_t& cap_hint, bool neg_zero, const std::function<int(const RangeOut&)>& scan,
+                  vix_range_result** out, RangeInfo* info);
+
+// an empty result of nq rows (lims all 0)
+int range_empty(int64_t nq, vix_range_result** out);
+
+// flat range scan over xb (pair-tile engine, vix_scoring.cu); ids[r] is the id of row r; disabled_rows: bit r set => skipped
+int flat_range_device(const float* q, int64_t nq, const float* xb, int64_t n, int d, int metric, const int64_t* ids,
+                      const uint64_t* disabled_rows, const RangeOut& out);
+
+}  // namespace vix

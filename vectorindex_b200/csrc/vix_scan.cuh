@@ -3,6 +3,7 @@
 #pragma once
 
 #include "vix_common.cuh"
+#include "vix_range.cuh"
 
 namespace vix {
 
@@ -36,6 +37,8 @@ struct ScanArgs {
     cudaEvent_t ev_kernel[2];                     // optional: recorded around the dominant kernel of the launch
     int path;                                     // set by launch_ivfpq_scan: 0 query-major, 1 list-major (tensor cores)
     unsigned long long* phase_cycles;             // optional [3]: SM cycles in prologue / scan / tail wait, summed over CTAs
+    RangeOut range;                               // range search (range.keys set): entries within range.radius go here instead
+                                                  // of the top-k; launch_ivfpq_scan_classic only
 };
 
 // How the inverted lists are laid out for a given m.

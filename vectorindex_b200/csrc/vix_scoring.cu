@@ -8,19 +8,21 @@
 //   a16    vix_accel_rank_candidates_f32
 //
 // All of them are instances of one tiled kernel (PairTile, vix_exact.cuh) with three epilogues:
-// WRITE (materialise the tile), ARGMIN (running per-row minimum, tie -> lower index) and TOPK
+// WRITE (materialise the tile), ARGMIN (running per-row minimum, tie -> lower index), TOPK
 // (per-row shared-memory selection queues keyed by (score, id); partial results of the B-splits are
-// merged by merge_keys_kernel).  Distances come out bit-identical to the oracle's restatement of the
+// merged by merge_keys_kernel) and RANGE (every pair whose API distance is within a radius, appended to the
+// output path of range search, vix_range.cuh).  Distances come out bit-identical to the oracle's restatement of the
 // reference, so ids match even on ties.  The tensor-core path (vix_gemm.cu) uses these kernels to
 // rescore its shortlists.
 #include "vix_exact.cuh"
 #include "vix_topk.cuh"
+#include "vix_range.cuh"
 
 #include <math.h>
 
 namespace vix {
 
-enum Epilogue { EPI_WRITE = 0, EPI_ARGMIN = 1, EPI_TOPK = 2 };
+enum Epilogue { EPI_WRITE = 0, EPI_ARGMIN = 1, EPI_TOPK = 2, EPI_RANGE = 3 };
 enum Transform {
     TR_NONE = 0,      // raw score
     TR_CBS_L2 = 1,    // -2 * s + bnorm[b]        CentroidBatchScore L2 (CentroidBatchScore.swift:54-64)
@@ -44,6 +46,11 @@ struct PairArgs {
     // TOPK
     int k, P, order_max, nsplit; int64_t btiles_per_split;
     u64* keys_out;                 // [nA x nsplit x k]
+    // RANGE: the API distance of merge_keys_kernel's dist_mode (applied to the score as the selection key keeps it), the
+    // id of each B row (nullable: the row index), where passing pairs go
+    int dist_mode;
+    const int64_t* row_ids;
+    RangeOut range;
 };
 
 __device__ __forceinline__ float apply_transform(int tr, float s, const PairArgs& p, int64_t a, int64_t b) {
@@ -79,7 +86,7 @@ __global__ void __launch_bounds__(256) pair_kernel(PairArgs p) {
 
     const int64_t nbt = (p.nB + TB - 1) / TB;
     int64_t bt0 = 0, bt1 = nbt;
-    if (EPI == EPI_TOPK) {
+    if (EPI == EPI_TOPK || EPI == EPI_RANGE) {
         bt0 = (int64_t)blockIdx.y * p.btiles_per_split;
         bt1 = min(nbt, bt0 + p.btiles_per_split);
     }
@@ -99,6 +106,11 @@ __global__ void __launch_bounds__(256) pair_kernel(PairArgs p) {
         qcnt = reinterpret_cast<int*>(qthr + TA);              // [TA]
         for (int e = tid; e < TA * p.P; e += 256) qkeys[e] = kEmptyKey;
         for (int e = tid; e < TA; e += 256) { qthr[e] = kEmptyKey; qcnt[e] = 0; }
+    }
+    int* rcnt = nullptr;                                       // RANGE: entries per A row of this CTA
+    if (EPI == EPI_RANGE) {
+        rcnt = reinterpret_cast<int*>(extra);
+        for (int e = tid; e < TA; e += 256) rcnt[e] = 0;
     }
 
     for (int64_t bt = bt0; bt < bt1; ++bt) {
@@ -121,6 +133,32 @@ __global__ void __launch_bounds__(256) pair_kernel(PairArgs p) {
         float sc[TV][TC];
         Tile::compute(As, Bs, p.pitch, p.d, tx, ty, sc);
 
+        if constexpr (EPI == EPI_RANGE) {
+            // every thread reaches every append (warp-collective); out-of-range pairs simply do not pass
+#pragma unroll
+            for (int v = 0; v < TV; ++v) {
+                const int64_t a = a0 + tx + 16 * v;
+#pragma unroll
+                for (int c = 0; c < TC; ++c) {
+                    const int64_t b = b0 + ty + 16 * c;
+                    bool pass = false;
+                    u64 key = 0;
+                    if (a < p.nA && b < p.nB && !(p.disabled && ((p.disabled[b >> 6] >> (b & 63)) & 1ull))) {
+                        // the score as make_key keeps it (-0 -> +0), then merge_keys_kernel's API mapping
+                        const float f = fadd(apply_transform(p.transform, sc[v][c], p, a, b), 0.0f);
+                        const float api = p.dist_mode == 1 ? __fsqrt_rn(f) : p.dist_mode == 2 ? -f
+                                        : p.dist_mode == 3 ? fsub(1.0f, f) : f;
+                        pass = api <= p.range.radius;
+                        if (pass) key = make_key(api, (uint32_t)(p.row_ids ? p.row_ids[b] : b), 0);
+                    }
+                    const unsigned ball = __ballot_sync(0xFFFFFFFFu, pass);
+                    if (ball) {
+                        range_append(p.range, ball, pass, key, (uint32_t)a);
+                        if (pass) atomicAdd(rcnt + tx + 16 * v, 1);
+                    }
+                }
+            }
+        } else {
 #pragma unroll
         for (int v = 0; v < TV; ++v) {
             const int64_t a = a0 + tx + 16 * v;
@@ -146,6 +184,13 @@ __global__ void __launch_bounds__(256) pair_kernel(PairArgs p) {
                 }
             }
         }
+        }
+    }
+
+    if (EPI == EPI_RANGE) {
+        __syncthreads();
+        for (int r = tid; r < TA; r += 256)
+            if (a0 + r < p.nA && rcnt[r]) atomicAdd(p.range.counts + a0 + r, (unsigned long long)rcnt[r]);
     }
 
     if (EPI == EPI_ARGMIN) {
@@ -281,6 +326,7 @@ static size_t tile_smem(int tv, int d, int epi, int P) {
     size_t s = (size_t)(TA + TB) * pitch * 4 + 16;
     if (epi == EPI_TOPK) s += (size_t)TA * P * 8 + (size_t)TA * 12;
     if (epi == EPI_ARGMIN) s += (size_t)TA * 16 * 12 + (size_t)TA * 4;
+    if (epi == EPI_RANGE) s += (size_t)TA * 4;
     return s;
 }
 
@@ -385,6 +431,14 @@ static int launch_pair(PairArgs& p, int k_for_plan, int64_t* nsplit_out = nullpt
         p.nsplit = (int)nsplit;
         grid.y = (unsigned)nsplit;
         if (nsplit_out) { *nsplit_out = nsplit; return VIX_OK; }   // planning pass
+    }
+    if (EPI == EPI_RANGE) {
+        // the B tiles of an A tile are split over enough CTAs for ~4 waves of the SMs
+        int64_t nsplit = (4LL * num_sms() + atiles - 1) / atiles;
+        if (nsplit > btiles) nsplit = btiles;
+        if (nsplit < 1) nsplit = 1;
+        p.btiles_per_split = (btiles + nsplit - 1) / nsplit;
+        grid.y = (unsigned)((btiles + p.btiles_per_split - 1) / p.btiles_per_split);
     }
 #define VIX_LAUNCH_TV(TVV)                                                                                 \
     do {                                                                                                   \
@@ -531,6 +585,43 @@ static int flat_search_impl(const float* q, int64_t nq, const float* xb, int64_t
     }
     p.transform = TR_NONE;
     return pair_topk<SpecDirect16L2>(p, k, 0, raw_scores ? 0 : 1, out_dist, out_ids, nullptr);
+}
+
+// Range scan of a flat index: the pairs, transforms and API mapping of flat_search_impl (Direct16 below d = 256, Dot16 with
+// Norms.l2NormSquared norms from d = 256, Ip4, the two-pass cosine), every pair within out.radius appended
+int flat_range_device(const float* q, int64_t nq, const float* xb, int64_t n, int d, int metric, const int64_t* ids,
+                      const uint64_t* disabled_rows, const RangeOut& out) {
+    if (nq == 0 || n == 0) return VIX_OK;
+    PairArgs p{};
+    p.A = q; p.nA = nq; p.B = xb; p.nB = n; p.d = d; p.disabled = disabled_rows;
+    p.row_ids = ids; p.range = out;
+    if (metric == VIX_METRIC_IP) {
+        p.transform = TR_NONE; p.dist_mode = 2;
+        return launch_pair<SpecIp4, EPI_RANGE>(p, 0);
+    }
+    if (metric == VIX_METRIC_COSINE) {
+        Scratch<float> qi, xi;
+        VIX_TRY(qi.alloc((size_t)nq));
+        VIX_TRY(xi.alloc((size_t)n));
+        row_inv_norms_kernel<<<(unsigned)((nq + 127) / 128), 128, 0, ctx().stream>>>(q, nq, d, qi.ptr);
+        VIX_LAUNCH_CHECK();
+        row_inv_norms_kernel<<<(unsigned)((n + 127) / 128), 128, 0, ctx().stream>>>(xb, n, d, xi.ptr);
+        VIX_LAUNCH_CHECK();
+        p.transform = TR_COSINE; p.anorm = qi.ptr; p.bnorm = xi.ptr; p.dist_mode = 3;
+        return launch_pair<SpecIp4, EPI_RANGE>(p, 0);
+    }
+    p.dist_mode = 1;
+    if (d >= 256) {
+        Scratch<float> qn, xn;
+        VIX_TRY(qn.alloc((size_t)nq));
+        VIX_TRY(row_norms_device(q, nq, d, qn.ptr));
+        VIX_TRY(xn.alloc((size_t)n));
+        VIX_TRY(row_norms_device(xb, n, d, xn.ptr));
+        p.transform = TR_DOTFUSED; p.anorm = qn.ptr; p.bnorm = xn.ptr;
+        return launch_pair<SpecDot16, EPI_RANGE>(p, 0);
+    }
+    p.transform = TR_NONE;
+    return launch_pair<SpecDirect16L2, EPI_RANGE>(p, 0);
 }
 
 // CentroidBatchScore.swift:70-84, cosine: the block holds -<q, c>; 1 - dot qInv cInv = 1 + row qInv cInv, except where the

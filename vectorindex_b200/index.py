@@ -203,6 +203,38 @@ class _Index:
         valid = i[0] >= 0
         return [(int(a), float(b)) for a, b in zip(i[0][valid], d[0][valid])]
 
+    def range_search(self, queries, radius: float, nprobe: int = 0, filter=None):
+        """Every stored vector whose distance to a query is at most ``radius`` (the distance k-NN search returns: L2
+        sqrt(L2^2), or the ADC squared distance on an IVF-PQ index; IP -dot; cosine 1 - similarity), per query sorted by
+        (distance, id).  Candidates, ``nprobe`` and ``filter`` (an :class:`IDFilter`) are those of :meth:`batch_search`.
+        Returns CSR ``(lims int64 [nq + 1], distances f32 [total], ids int64 [total])``: row r is
+        ``[lims[r], lims[r + 1])``; numpy for host queries, torch tensors on the queries' device for CUDA tensors."""
+        q = as_input(queries, np.float32)
+        self._check_dim(q, "range_search")
+        nq = int(q.shape[0])
+        res = C.c_void_p(0)
+        try:
+            words = filter.words if filter is not None else None
+            check(lib().vix_index_range_search(self._h, ptr(q, np.float32), C.c_int64(nq), C.c_float(float(radius)),
+                                               C.c_int(nprobe), ptr(words, np.uint64),
+                                               C.c_int64(filter.capacity if filter is not None else 0),
+                                               C.c_int(filter.mode if filter is not None else 0), C.byref(res)))
+            total = int(lib().vix_range_result_total(res))
+            lims = empty_like_input(q, (nq + 1,), np.int64)
+            dist = empty_like_input(q, (total,), np.float32)
+            ids = empty_like_input(q, (total,), np.int64)
+            check(lib().vix_range_result_get(res, ptr(lims, np.int64), ptr(dist, np.float32) if total else None,
+                                             ptr(ids, np.int64) if total else None))
+            return lims, dist, ids
+        finally:
+            lib().vix_range_result_destroy(res)
+
+    def range_query(self, query, radius: float, nprobe: int = 0):
+        """:meth:`range_search` for one query: ``[(id, distance), ...]`` nearest first."""
+        q = np.ascontiguousarray(query, dtype=np.float32).reshape(1, -1)
+        _, d, i = self.range_search(q, radius, nprobe)
+        return [(int(a), float(b)) for a, b in zip(i, d)]
+
 
 class FlatIndex(_Index):
     kind = INDEX_FLAT
