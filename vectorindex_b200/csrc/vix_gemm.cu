@@ -40,6 +40,7 @@
 #include "vix_common.cuh"
 #include "vix_exact.cuh"
 #include "vix_tcgen05.cuh"
+#include "vix_group.cuh"
 #include "vix_topk.cuh"
 
 #include <stdlib.h>
@@ -725,12 +726,6 @@ __global__ void scatter_flat_rows_kernel(const float* __restrict__ sub_d, const 
     }
 }
 
-__global__ void gather_rows_f32_kernel(const float* __restrict__ x, int d, const int* __restrict__ rows, int n,
-                                       float* __restrict__ out) {
-    const int i = blockIdx.x;
-    if (i >= n) return;
-    for (int e = threadIdx.x; e < d; e += blockDim.x) out[(int64_t)i * d + e] = x[(int64_t)rows[i] * d + e];
-}
 __global__ void scatter_probe_rows_kernel(const int32_t* __restrict__ idx, const float* __restrict__ sc, int k,
                                           const int* __restrict__ rows, int n, int32_t* __restrict__ out_idx,
                                           float* __restrict__ out_sc) {
@@ -922,8 +917,7 @@ int flat_search_auto_device(const float* q, int64_t nq, const float* xb, int64_t
         VIX_TRY(sub.alloc((size_t)m * d));
         VIX_TRY(sub_d.alloc((size_t)m * k));
         VIX_TRY(sub_i.alloc((size_t)m * k));
-        tc::gather_rows_f32_kernel<<<m, 128, 0, s>>>(q, d, ovf_rows.ptr, m, sub.ptr);
-        VIX_LAUNCH_CHECK();
+        VIX_TRY(gather_rows(q, d, ovf_rows.ptr, m, sub.ptr));
         VIX_TRY(flat_search_device(sub.ptr, m, xb, n, d, metric, k, nullptr, sub_d.ptr, sub_i.ptr, raw_scores));
         tc::scatter_flat_rows_kernel<<<m, 128, 0, s>>>(sub_d.ptr, sub_i.ptr, k, ovf_rows.ptr, m, out_dist, out_ids);
         VIX_LAUNCH_CHECK();
@@ -986,8 +980,7 @@ int ivf_assign_auto_device(const float* x, int64_t n, int d, const float* c, int
         VIX_TRY(sub.alloc((size_t)m * d));
         VIX_TRY(sub_assign.alloc((size_t)m));
         VIX_TRY(sub_dist.alloc((size_t)m));
-        tc::gather_rows_f32_kernel<<<m, 128, 0, s>>>(x, d, ovf_rows.ptr, m, sub.ptr);
-        VIX_LAUNCH_CHECK();
+        VIX_TRY(gather_rows(x, d, ovf_rows.ptr, m, sub.ptr));
         VIX_TRY(ivf_assign_device(sub.ptr, m, d, c, kc, sub_assign.ptr, sub_dist.ptr));
         tc::scatter_assign_rows_kernel<<<(unsigned)((m + 255) / 256), 256, 0, s>>>(sub_assign.ptr, sub_dist.ptr, ovf_rows.ptr, m,
                                                                                 assign, dist);

@@ -17,8 +17,7 @@
 #include "vix_scan.cuh"
 #include "vix_index.cuh"
 #include "vix_range.cuh"
-
-#include <cub/cub.cuh>
+#include "vix_group.cuh"
 
 #include <new>
 #include <stdio.h>
@@ -31,46 +30,6 @@ namespace vix {
 // ------------------------------------------------------------------------------------------------
 // list building
 // ------------------------------------------------------------------------------------------------
-__global__ void iota_kernel(int32_t* a, int64_t n) {
-    int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) a[i] = (int32_t)i;
-}
-
-__global__ void hist_kernel(const int32_t* __restrict__ assign, int64_t n, int kc, int32_t* __restrict__ len) {
-    int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) {
-        int a = assign[i];
-        if (a >= 0 && a < kc) atomicAdd(len + a, 1);
-    }
-}
-
-// single CTA: off[l+1] = off[l] + roundup(len[l], align); also unpadded offsets (CSR of the sorted rows)
-__global__ void offsets_kernel(const int32_t* __restrict__ len, int kc, int align, int64_t* __restrict__ off,
-                               int64_t* __restrict__ off_raw) {
-    __shared__ int64_t s_pad[1024], s_raw[1024];
-    __shared__ int64_t carry_pad, carry_raw;
-    if (threadIdx.x == 0) { carry_pad = 0; carry_raw = 0; off[0] = 0; off_raw[0] = 0; }
-    __syncthreads();
-    for (int base = 0; base < kc; base += 1024) {
-        int l = base + threadIdx.x;
-        int64_t v = (l < kc) ? len[l] : 0;
-        int64_t vp = (v + align - 1) / align * align;
-        s_pad[threadIdx.x] = vp; s_raw[threadIdx.x] = v;
-        __syncthreads();
-        for (int o = 1; o < 1024; o <<= 1) {     // Hillis-Steele inclusive scan
-            int64_t a = 0, b = 0;
-            if ((int)threadIdx.x >= o) { a = s_pad[threadIdx.x - o]; b = s_raw[threadIdx.x - o]; }
-            __syncthreads();
-            s_pad[threadIdx.x] += a; s_raw[threadIdx.x] += b;
-            __syncthreads();
-        }
-        if (l < kc) { off[l + 1] = carry_pad + s_pad[threadIdx.x]; off_raw[l + 1] = carry_raw + s_raw[threadIdx.x]; }
-        __syncthreads();
-        if (threadIdx.x == 1023) { carry_pad += s_pad[1023]; carry_raw += s_raw[1023]; }
-        __syncthreads();
-    }
-}
-
 // slot_row[off[l] + r] = sorted_rows[off_raw[l] + r]
 // Rows without a list (assignment outside [0, kc): the -1 of an all-NaN / all-+inf score row, IVFIndex.swift:376-435
 // "guard best >= 0 else continue") carry the sort key kc, so they sort behind every list and are not placed.
@@ -207,16 +166,10 @@ int build_lists(vix_index* h) {
     cudaStream_t s = ctx().stream;
     VIX_TRY(h->list_len.resize((size_t)kc, false));
     VIX_TRY(h->list_off.resize((size_t)kc + 1, false));
-    VIX_CUDA(cudaMemsetAsync(h->list_len.ptr, 0, (size_t)kc * 4, s));
     Scratch<int64_t> off_raw;
     VIX_TRY(off_raw.alloc((size_t)kc + 1));
-    if (n > 0) {
-        hist_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(h->assign.ptr, n, kc, h->list_len.ptr);
-        VIX_LAUNCH_CHECK();
-    }
     h->align = (h->p.kind == VIX_INDEX_IVF_PQ) ? scan_layout(h->p.m).align : 32;
-    offsets_kernel<<<1, 1024, 0, s>>>(h->list_len.ptr, kc, h->align, h->list_off.ptr, off_raw.ptr);
-    VIX_LAUNCH_CHECK();
+    VIX_TRY(key_offsets(h->assign.ptr, n, kc, h->list_len.ptr, h->list_off.ptr, h->align, off_raw.ptr));
     int64_t nslots = 0;
     VIX_CUDA(cudaMemcpyAsync(&nslots, h->list_off.ptr + kc, 8, cudaMemcpyDeviceToHost, s));
     VIX_CUDA(cudaStreamSynchronize(s));
@@ -231,29 +184,17 @@ int build_lists(vix_index* h) {
         unsigned long long invalid = 0;
         VIX_TRY(count_invalid_assign(h->assign.ptr, n, kc, &invalid));
         Scratch<int32_t> keys;
-        const int32_t* sort_keys = h->assign.ptr;
+        const int32_t* list_keys = h->assign.ptr;
         if (invalid) {
             VIX_TRY(keys.alloc((size_t)n));
             sanitise_assign_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(h->assign.ptr, n, kc, keys.ptr);
             VIX_LAUNCH_CHECK();
-            sort_keys = keys.ptr;
+            list_keys = keys.ptr;
         }
-        Scratch<int32_t> rows_in, rows_out, lists_out;
-        VIX_TRY(rows_in.alloc((size_t)n));
+        Scratch<int32_t> rows_out, lists_out;
         VIX_TRY(rows_out.alloc((size_t)n));
         VIX_TRY(lists_out.alloc((size_t)n));
-        iota_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(rows_in.ptr, n);
-        VIX_LAUNCH_CHECK();
-        int bits = 1;
-        while ((1LL << bits) < (int64_t)kc + 1) ++bits;               // keys 0 .. kc
-        size_t tmp_bytes = 0;
-        VIX_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, sort_keys, lists_out.ptr, rows_in.ptr,
-                                                 rows_out.ptr, (int)n, 0, bits, s));
-        Scratch<unsigned char> tmp;
-        VIX_TRY(tmp.alloc(tmp_bytes + 16));
-        VIX_CUDA(cub::DeviceRadixSort::SortPairs(tmp.ptr, tmp_bytes, sort_keys, lists_out.ptr, rows_in.ptr,
-                                                 rows_out.ptr, (int)n, 0, bits, s));
-        ctx().launches += 1;
+        VIX_TRY(order_by_key(list_keys, n, kc + 1, rows_out.ptr, lists_out.ptr));   // keys 0 .. kc
         place_rows_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(rows_out.ptr, lists_out.ptr, n, kc, h->list_off.ptr,
                                                                      off_raw.ptr, h->slot_row.ptr);
         VIX_LAUNCH_CHECK();
@@ -588,15 +529,6 @@ __global__ void gather_ids_kernel(const int64_t* __restrict__ rows, const int64_
     if (i < n) out[i] = rows[i] >= 0 ? ids[rows[i]] : -1;
 }
 
-// PQTrain.swift:299-307: centroid norms as a strictly sequential sum of squares
-__global__ void seq_norms_kernel(const float* __restrict__ c, int64_t rows, int dsub, float* __restrict__ out) {
-    int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= rows) return;
-    float s = 0.0f;
-    for (int e = 0; e < dsub; ++e) s = __fadd_rn(s, __fmul_rn(c[i * dsub + e], c[i * dsub + e]));
-    out[i] = s;
-}
-
 // codebooks [m][ks][dsub] -> code-major copy [ks][m][dsub] (coalesced LUT build of the scan)
 __global__ void transpose_codebooks_kernel(const float* __restrict__ cb, int m, int ks, int dsub, float* __restrict__ out) {
     const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -651,11 +583,6 @@ static int check_ids_host(const int64_t* ids, int64_t n) {
     return VIX_OK;
 }
 
-__global__ void iota64_kernel(int64_t* a, int64_t n, int64_t start) {
-    int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) a[i] = start + i;
-}
-
 // An IVF-Flat index may hold vectors before it has a coarse quantiser (the reference's insert -> optimize() -> search,
 // IVFIndex.swift:279-451; until then searches are linear scans, :820-832): once centroids exist, every stored row gets
 // its list.
@@ -699,8 +626,7 @@ static int index_add_locked(vix_index* h, const float* x, const int64_t* ids, in
     if (ids) VIX_CUDA(cudaMemcpyAsync(h->ids.ptr + n0, ids, (size_t)n * 8, cudaMemcpyDefault, s));
     else {
         // (after a removal the count no longer names an unused id: automatic ids continue from the last one handed out)
-        iota64_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(h->ids.ptr + n0, n, h->next_auto_id);
-        VIX_LAUNCH_CHECK();
+        VIX_TRY(iota<int64_t>(h->ids.ptr + n0, n, h->next_auto_id));
     }
 
     if (h->p.kind == VIX_INDEX_FLAT || h->p.kind == VIX_INDEX_IVF_FLAT) {
@@ -828,21 +754,14 @@ static int index_remove_locked(vix_index* h, const int64_t* ids, int64_t n, int6
     VIX_TRY(keys.alloc((size_t)n));
     ids_to_keys_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(did.dev, n, keys_in.ptr);
     VIX_LAUNCH_CHECK();
-    size_t sort_bytes = 0, scan_bytes = 0;
-    VIX_CUDA(cub::DeviceRadixSort::SortKeys(nullptr, sort_bytes, keys_in.ptr, keys.ptr, (int)n, 0, 32, s));
+    VIX_TRY(sort_keys(keys_in.ptr, keys.ptr, n));
+    // 2. per stored row: keep flag; 3. new positions of the kept rows, and their number
     Scratch<int32_t> keep, pos;
     VIX_TRY(keep.alloc((size_t)rows + 1));
     VIX_TRY(pos.alloc((size_t)rows + 1));
-    VIX_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, keep.ptr, pos.ptr, (int)(rows + 1), s));
-    Scratch<unsigned char> tmp;
-    VIX_TRY(tmp.alloc((sort_bytes > scan_bytes ? sort_bytes : scan_bytes) + 16));
-    VIX_CUDA(cub::DeviceRadixSort::SortKeys(tmp.ptr, sort_bytes, keys_in.ptr, keys.ptr, (int)n, 0, 32, s));
-    ctx().launches += 1;
-    // 2. per stored row: keep flag; 3. new positions of the kept rows, and their number
     mark_removed_kernel<<<(unsigned)((rows + 1 + 255) / 256), 256, 0, s>>>(h->ids.ptr, rows, keys.ptr, n, keep.ptr);
     VIX_LAUNCH_CHECK();
-    VIX_CUDA(cub::DeviceScan::ExclusiveSum(tmp.ptr, scan_bytes, keep.ptr, pos.ptr, (int)(rows + 1), s));
-    ctx().launches += 1;
+    VIX_TRY(exclusive_sum(keep.ptr, pos.ptr, rows + 1));
     int32_t kept32 = 0;
     VIX_CUDA(cudaMemcpyAsync(&kept32, pos.ptr + rows, 4, cudaMemcpyDeviceToHost, s));
     VIX_CUDA(cudaStreamSynchronize(s));
@@ -1129,14 +1048,6 @@ __global__ void export_lists_kernel(const int32_t* __restrict__ slot_row, const 
     if (threadIdx.x == 0 && off_out) { off_out[l] = o; if (l == kc - 1) off_out[kc] = off_raw[kc]; }
 }
 
-__global__ void raw_offsets_kernel(const int32_t* __restrict__ len, int kc, int64_t* __restrict__ off_raw) {
-    if (threadIdx.x == 0 && blockIdx.x == 0) {
-        int64_t acc = 0;
-        for (int l = 0; l < kc; ++l) { off_raw[l] = acc; acc += len[l]; }
-        off_raw[kc] = acc;
-    }
-}
-
 __global__ void expand_assign_kernel(const int64_t* __restrict__ off, int kc, int32_t* __restrict__ assign) {
     const int l = blockIdx.x;
     if (l >= kc) return;
@@ -1213,9 +1124,7 @@ int vix_index_set_codebooks(vix_index_t* h, const float* codebooks, const float*
     else {
         // PQTrain.swift:299-307: sequential sum of squares per centroid
         VIX_TRY(h->cb_norms.resize((size_t)m * ks, false));
-        seq_norms_kernel<<<(unsigned)((m * ks + 127) / 128), 128, 0, ctx().stream>>>(h->codebooks.ptr, (int64_t)m * ks, dsub,
-                                                                                      h->cb_norms.ptr);
-        VIX_LAUNCH_CHECK();
+        VIX_TRY(seq_norms(h->codebooks.ptr, (int64_t)m * ks, dsub, h->cb_norms.ptr));
     }
     VIX_TRY(update_codebooks_t(h));
     h->has_pq = true;
@@ -1351,8 +1260,7 @@ int vix_index_export_lists(vix_index_t* h, int64_t* list_offsets, uint8_t* codes
     const int64_t n = h->n;
     Scratch<int64_t> off_raw;
     VIX_TRY(off_raw.alloc((size_t)kc + 1));
-    raw_offsets_kernel<<<1, 32, 0, ctx().stream>>>(h->list_len.ptr, kc, off_raw.ptr);
-    VIX_LAUNCH_CHECK();
+    VIX_TRY(offsets_from_counts(h->list_len.ptr, kc, 1, off_raw.ptr, nullptr));
     Out<int64_t> doff, dids;
     Out<uint8_t> dcodes;
     VIX_TRY(doff.stage(list_offsets, list_offsets ? (size_t)kc + 1 : 0));

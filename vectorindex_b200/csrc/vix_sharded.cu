@@ -19,8 +19,7 @@
 #include "vix_index.cuh"
 #include "vix_scan.cuh"
 #include "vix_topk.cuh"
-
-#include <cub/cub.cuh>
+#include "vix_group.cuh"
 
 #include <dlfcn.h>
 #include <nccl.h>
@@ -259,11 +258,6 @@ __global__ void peer_push_kernel(void* const* __restrict__ peer_base, int world,
     }
 }
 
-__global__ void fill_i32_kernel(int32_t* a, int64_t n, int32_t v) {
-    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) a[i] = v;
-}
-
 // local top-k -> packed keys (orderable API distance << 32 | id; ascending key order is mergeTopK's order for both
 // metrics, the API distance of the inner product being -dot) -> slot `rank` of [world][nq][k] in every destination
 __global__ void pack_result_keys_kernel(const float* __restrict__ dist, const int64_t* __restrict__ ids, int64_t total,
@@ -346,14 +340,13 @@ static int peer_barrier(vix_comm* c) {
 
 // owner rank of a list under block boundaries bounds[world + 1]
 __global__ void owner_kernel(const int32_t* __restrict__ assign, int64_t n, const int64_t* __restrict__ bounds, int world,
-                             int32_t* __restrict__ owner, int32_t* __restrict__ row, unsigned long long* __restrict__ counts) {
+                             int32_t* __restrict__ owner, unsigned long long* __restrict__ counts) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     const int64_t l = assign[i];
     int o = 0;
     while (o + 1 < world && l >= bounds[o + 1]) ++o;
     owner[i] = o;
-    row[i] = (int32_t)i;
     atomicAdd(counts + o, 1ull);
 }
 
@@ -501,11 +494,7 @@ int vix_sharded_search(vix_index_t* h, vix_comm_t* c, const float* queries, int6
         if (cnt > 0)
             VIX_TRY(probe_select_fast_device(qblock, cnt, h->coarse.ptr, h->kc, d, h->p.metric, nprobe, h->coarse_norms.ptr,
                                              pblock, nullptr, h->coarse_norm_max.ptr));
-        if (cnt < per) {
-            const int64_t pad = (per - cnt) * nprobe;
-            fill_i32_kernel<<<(unsigned)((pad + 255) / 256), 256, 0, s>>>(pblock + (size_t)cnt * nprobe, pad, -1);
-            VIX_LAUNCH_CHECK();
-        }
+        if (cnt < per) VIX_TRY(fill<int32_t>(pblock + (size_t)cnt * nprobe, (per - cnt) * nprobe, -1));
         // 3. the block travels to every peer (probes, and the queries when they came from the host), one barrier
         {
             const size_t offA = c->off_probes + (size_t)rank * per * nprobe * 4, nA = (size_t)per * nprobe * 4 / 16;
@@ -548,11 +537,7 @@ int vix_sharded_search(vix_index_t* h, vix_comm_t* c, const float* queries, int6
         if (cnt > 0)
             VIX_TRY(probe_select_fast_device(dq.dev + (size_t)lo * d, cnt, h->coarse.ptr, h->kc, d, h->p.metric, nprobe,
                                              h->coarse_norms.ptr, pblock, nullptr, h->coarse_norm_max.ptr));
-        if (cnt < per) {
-            const int64_t pad = (per - cnt) * nprobe;
-            fill_i32_kernel<<<(unsigned)((pad + 255) / 256), 256, 0, s>>>(pblock + (size_t)cnt * nprobe, pad, -1);
-            VIX_LAUNCH_CHECK();
-        }
+        if (cnt < per) VIX_TRY(fill<int32_t>(pblock + (size_t)cnt * nprobe, (per - cnt) * nprobe, -1));
         VIX_NCCL(g_nccl.AllGather(pblock, pall, (size_t)per * nprobe, ncclInt32, c->comm, s));   // in place
         mark(1);
         VIX_TRY(index_search_locked(h, dq.dev, nq, k, nprobe, ldist.ptr, lids.ptr, nullptr, nullptr, pall));
@@ -609,7 +594,7 @@ int vix_sharded_add(vix_index_t* h, vix_comm_t* c, const int64_t* list_bounds, c
     In<int64_t> dids;
     VIX_TRY(dx.stage(x, (size_t)n * d));
     VIX_TRY(dids.stage(ids, (size_t)n));
-    Scratch<int32_t> asg, owner, row, order, owner_sorted;
+    Scratch<int32_t> asg, owner, order;
     Scratch<uint8_t> codes;
     Scratch<unsigned long long> dcounts;
     Scratch<int64_t> dbounds;
@@ -630,20 +615,11 @@ int vix_sharded_add(vix_index_t* h, vix_comm_t* c, const int64_t* list_bounds, c
         VIX_TRY(encode_rows_device(h, dx.dev, n, asg.ptr, codes.ptr));
         // 2. rows ordered by owning rank (stable: rows keep their order inside a block)
         VIX_TRY(owner.alloc((size_t)n));
-        VIX_TRY(row.alloc((size_t)n));
         VIX_TRY(order.alloc((size_t)n));
-        VIX_TRY(owner_sorted.alloc((size_t)n));
-        owner_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(asg.ptr, n, dbounds.ptr, world, owner.ptr, row.ptr,
+        owner_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(asg.ptr, n, dbounds.ptr, world, owner.ptr,
                                                                dcounts.ptr + (size_t)world * world);
         VIX_LAUNCH_CHECK();
-        int bits = 1;
-        while ((1 << bits) < world) ++bits;
-        size_t tmp_bytes = 0;
-        VIX_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, owner.ptr, owner_sorted.ptr, row.ptr, order.ptr, (int)n, 0, bits, s));
-        Scratch<unsigned char> tmp;
-        VIX_TRY(tmp.alloc(tmp_bytes + 16));
-        VIX_CUDA(cub::DeviceRadixSort::SortPairs(tmp.ptr, tmp_bytes, owner.ptr, owner_sorted.ptr, row.ptr, order.ptr, (int)n, 0, bits, s));
-        ctx().launches += 1;
+        VIX_TRY(order_by_key(owner.ptr, n, world, order.ptr));
         VIX_TRY(s_asg.alloc((size_t)n));
         VIX_TRY(s_codes.alloc((size_t)n * m));
         VIX_TRY(s_ids.alloc((size_t)n));

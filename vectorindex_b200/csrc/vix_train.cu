@@ -8,15 +8,14 @@
 //                   the host with every distance pass, argmin and f64 accumulation on the GPU in the
 //                   reference's order (vix_train_parity.cu).
 //
-// Both modes share the building blocks here: bit-exact assignment kernels (vix_scoring.cu /
-// vix_pq_encode.cu) and a deterministic centroid update -- rows are stably sorted by assignment and
-// each (centroid, component) is summed sequentially in f64 in data order, which is exactly the
-// reference's accumulation order (KMeansMiniBatchKernel.swift:582, PQTrain.swift:1111), with no
-// atomics on the value path, so results are reproducible run to run and rank to rank.
+// Both modes build on the same blocks: bit-exact assignment kernels (vix_scoring.cu / vix_pq_encode.cu), the
+// stable grouping of rows by assignment (vix_group.cu), and a deterministic centroid update -- each (centroid,
+// component) is summed sequentially in f64 in the order of the stably sorted rows, which is exactly the
+// reference's accumulation order (KMeansMiniBatchKernel.swift:582, PQTrain.swift:1111), with no atomics on the
+// value path, so results are reproducible run to run and rank to rank.
 #include "vix_common.cuh"
 #include "vix_exact.cuh"
-
-#include <cub/cub.cuh>
+#include "vix_group.cuh"
 
 #include <vector>
 
@@ -27,50 +26,6 @@ int ivf_assign_auto_device(const float* x, int64_t n, int d, const float* c, int
 int pq_encode_device(const float* x, int64_t n, int d, int m, int ks, const float* cb, const float* csq,
                      const float* coarse, const int32_t* assign, uint8_t* codes, int use_dot, int layout,
                      int B, int g, int u4);
-
-// x_s[i] = x[(i * stride) % n ...]: deterministic strided sample of ns rows
-__global__ void gather_rows_kernel(const float* __restrict__ x, int d, const int64_t* __restrict__ rows, int64_t ns,
-                                   float* __restrict__ out) {
-    const int64_t i = blockIdx.x;
-    if (i >= ns) return;
-    const float* src = x + rows[i] * (int64_t)d;
-    for (int e = threadIdx.x; e < d; e += blockDim.x) out[i * (int64_t)d + e] = src[e];
-}
-
-__global__ void iota32_kernel(int32_t* a, int64_t n) {
-    int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) a[i] = (int32_t)i;
-}
-
-__global__ void count_kernel(const int32_t* __restrict__ assign, int64_t n, int kc, int32_t* __restrict__ cnt) {
-    int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) { int a = assign[i]; if (a >= 0 && a < kc) atomicAdd(cnt + a, 1); }
-}
-
-// exclusive scan of counts by one CTA (kc up to a few 100k)
-__global__ void excl_scan_kernel(const int32_t* __restrict__ cnt, int kc, int64_t* __restrict__ off) {
-    __shared__ int64_t s[1024];
-    __shared__ int64_t carry;
-    if (threadIdx.x == 0) carry = 0;
-    __syncthreads();
-    for (int base = 0; base < kc; base += 1024) {
-        int l = base + threadIdx.x;
-        int64_t v = l < kc ? cnt[l] : 0;
-        s[threadIdx.x] = v;
-        __syncthreads();
-        for (int o = 1; o < 1024; o <<= 1) {
-            int64_t a = (int)threadIdx.x >= o ? s[threadIdx.x - o] : 0;
-            __syncthreads();
-            s[threadIdx.x] += a;
-            __syncthreads();
-        }
-        if (l < kc) off[l] = carry + s[threadIdx.x] - v;
-        __syncthreads();
-        if (threadIdx.x == 1023) carry += s[1023];
-        __syncthreads();
-    }
-    if (threadIdx.x == 0) off[kc] = carry;
-}
 
 // centroid c := mean of its members, f64 sums in data order (rows sorted stably by assignment).
 // One CTA per centroid, threads over components.  Empty centroids are left untouched.
@@ -113,31 +68,11 @@ __global__ void repair_empty_kernel(const float* __restrict__ x, int d, int x_ld
 
 static int sort_by_assignment(const int32_t* assign, int64_t n, int kc, Scratch<int32_t>& rows_sorted,
                               Scratch<int32_t>& cnt, Scratch<int64_t>& off) {
-    cudaStream_t s = ctx().stream;
-    Scratch<int32_t> rows_in, keys_out;
-    VIX_TRY(rows_in.alloc((size_t)n));
-    VIX_TRY(keys_out.alloc((size_t)n));
     VIX_TRY(rows_sorted.alloc((size_t)n));
     VIX_TRY(cnt.alloc((size_t)kc));
     VIX_TRY(off.alloc((size_t)kc + 1));
-    iota32_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(rows_in.ptr, n);
-    VIX_LAUNCH_CHECK();
-    int bits = 1;
-    while ((1LL << bits) < kc) ++bits;
-    size_t tmp_bytes = 0;
-    VIX_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, assign, keys_out.ptr, rows_in.ptr, rows_sorted.ptr,
-                                             (int)n, 0, bits, s));
-    Scratch<unsigned char> tmp;
-    VIX_TRY(tmp.alloc(tmp_bytes + 16));
-    VIX_CUDA(cub::DeviceRadixSort::SortPairs(tmp.ptr, tmp_bytes, assign, keys_out.ptr, rows_in.ptr, rows_sorted.ptr,
-                                             (int)n, 0, bits, s));
-    ctx().launches += 1;
-    VIX_CUDA(cudaMemsetAsync(cnt.ptr, 0, (size_t)kc * 4, s));
-    count_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(assign, n, kc, cnt.ptr);
-    VIX_LAUNCH_CHECK();
-    excl_scan_kernel<<<1, 1024, 0, s>>>(cnt.ptr, kc, off.ptr);
-    VIX_LAUNCH_CHECK();
-    return VIX_OK;
+    VIX_TRY(order_by_key(assign, n, kc, rows_sorted.ptr));
+    return key_offsets(assign, n, kc, cnt.ptr, off.ptr);
 }
 
 // rows sorted by descending distance (ties: ascending row): keys = ~orderable(dist)
@@ -156,17 +91,8 @@ static int farthest_rows(const float* dist, int64_t n, Scratch<int32_t>& rows_so
     VIX_TRY(rows_sorted.alloc((size_t)n));
     dist_keys_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(dist, n, keys.ptr);
     VIX_LAUNCH_CHECK();
-    iota32_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(rows_in.ptr, n);
-    VIX_LAUNCH_CHECK();
-    size_t tmp_bytes = 0;
-    VIX_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, keys.ptr, keys_out.ptr, rows_in.ptr, rows_sorted.ptr,
-                                             (int)n, 0, 32, s));
-    Scratch<unsigned char> tmp;
-    VIX_TRY(tmp.alloc(tmp_bytes + 16));
-    VIX_CUDA(cub::DeviceRadixSort::SortPairs(tmp.ptr, tmp_bytes, keys.ptr, keys_out.ptr, rows_in.ptr, rows_sorted.ptr,
-                                             (int)n, 0, 32, s));
-    ctx().launches += 1;
-    return VIX_OK;
+    VIX_TRY(iota<int32_t>(rows_in.ptr, n, 0));
+    return sort_pairs<uint32_t>(keys.ptr, keys_out.ptr, rows_in.ptr, rows_sorted.ptr, n, 32);
 }
 
 // LCG of the reference (Utilities/RNG.swift:61-65) for the deterministic sample / init choices
@@ -231,8 +157,7 @@ int train_coarse_device(const float* x, int64_t n, int d, int kc, int metric, co
         VIX_TRY(drows.alloc((size_t)ns));
         VIX_CUDA(cudaMemcpyAsync(drows.ptr, rows.data(), (size_t)ns * 8, cudaMemcpyHostToDevice, s));
         VIX_TRY(xs.alloc((size_t)ns * d));
-        gather_rows_kernel<<<(unsigned)ns, 128, 0, s>>>(x, d, drows.ptr, ns, xs.ptr);
-        VIX_LAUNCH_CHECK();
+        VIX_TRY(gather_rows(x, d, drows.ptr, ns, xs.ptr));
         VIX_CUDA(cudaStreamSynchronize(s));
         xp = xs.ptr;
     }
@@ -243,8 +168,7 @@ int train_coarse_device(const float* x, int64_t n, int d, int kc, int metric, co
         Scratch<int64_t> dinit;
         VIX_TRY(dinit.alloc((size_t)kc));
         VIX_CUDA(cudaMemcpyAsync(dinit.ptr, init.data(), (size_t)kc * 8, cudaMemcpyHostToDevice, s));
-        gather_rows_kernel<<<(unsigned)kc, 128, 0, s>>>(xp, d, dinit.ptr, kc, centroids_out);
-        VIX_LAUNCH_CHECK();
+        VIX_TRY(gather_rows(xp, d, dinit.ptr, kc, centroids_out));
         VIX_CUDA(cudaStreamSynchronize(s));
     }
     Scratch<int32_t> assign;
@@ -288,14 +212,6 @@ __global__ void sub_dist_kernel(const float* __restrict__ xs, int64_t ns, int d,
     dist[i] = exact_pair<SpecKm11L2>(a, c, dsub);
 }
 
-__global__ void seq_norms_train_kernel(const float* __restrict__ c, int64_t rows, int dsub, float* __restrict__ out) {
-    int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= rows) return;
-    float s = 0.0f;
-    for (int e = 0; e < dsub; ++e) s = fadd(s, fmul(c[i * dsub + e], c[i * dsub + e]));
-    out[i] = s;
-}
-
 int train_pq_device(const float* x, int64_t n, int d, int m, int ks, const float* coarse, const int32_t* assign,
                     const vix_pq_train_cfg* cfg, float* codebooks_out, float* norms_out) {
     cudaStream_t s = ctx().stream;
@@ -330,8 +246,7 @@ int train_pq_device(const float* x, int64_t n, int d, int m, int ks, const float
         VIX_TRY(dinit.alloc((size_t)ks));
         VIX_TRY(tmp.alloc((size_t)ks * d));
         VIX_CUDA(cudaMemcpyAsync(dinit.ptr, full.data(), (size_t)ks * 8, cudaMemcpyHostToDevice, s));
-        gather_rows_kernel<<<(unsigned)ks, 128, 0, s>>>(xs.ptr, d, dinit.ptr, ks, tmp.ptr);
-        VIX_LAUNCH_CHECK();
+        VIX_TRY(gather_rows(xs.ptr, d, dinit.ptr, ks, tmp.ptr));
         // tmp[k][j*dsub + e] -> codebooks[j][k][e]
         for (int j = 0; j < m; ++j)
             VIX_CUDA(cudaMemcpy2DAsync(codebooks_out + (size_t)j * ks * dsub, (size_t)dsub * 4, tmp.ptr + (size_t)j * dsub,
@@ -368,10 +283,7 @@ int train_pq_device(const float* x, int64_t n, int d, int m, int ks, const float
             VIX_LAUNCH_CHECK();
         }
     }
-    if (norms_out) {
-        seq_norms_train_kernel<<<(unsigned)((m * ks + 127) / 128), 128, 0, s>>>(codebooks_out, (int64_t)m * ks, dsub, norms_out);
-        VIX_LAUNCH_CHECK();
-    }
+    if (norms_out) VIX_TRY(seq_norms(codebooks_out, (int64_t)m * ks, dsub, norms_out));
     return VIX_OK;
 }
 

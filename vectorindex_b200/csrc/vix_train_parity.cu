@@ -15,8 +15,7 @@
 // which is the reference's accumulation order (PQTrain.swift:1111).
 #include "vix_common.cuh"
 #include "vix_exact.cuh"
-
-#include <cub/cub.cuh>
+#include "vix_group.cuh"
 
 #include <algorithm>
 #include <vector>
@@ -178,15 +177,6 @@ __global__ void sub_centroid_update_kernel(SubSrc s, const int32_t* __restrict__
     }
 }
 
-__global__ void iota_i32_kernel(int32_t* a, int64_t n) {
-    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) a[i] = (int32_t)i;
-}
-__global__ void count_i32_kernel(const int32_t* __restrict__ a, int64_t n, int k, int32_t* __restrict__ cnt) {
-    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n && a[i] >= 0 && a[i] < k) atomicAdd(cnt + a[i], 1);
-}
-
 // km11 D^2 update of k-means++ (KMeansSeeding.swift:302-361): d2[i] = min(d2[i], safe(L2^2(x_i, c)))
 __global__ void km11_update_kernel(const float* __restrict__ x, int64_t n, int d, const float* __restrict__ c,
                                    float* __restrict__ d2) {
@@ -195,16 +185,6 @@ __global__ void km11_update_kernel(const float* __restrict__ x, int64_t n, int d
     const float ds = exact_pair<SpecKm11L2>(x + i * d, c, d);
     const float safe = (isfinite(ds) && ds >= 0.0f) ? ds : 0.0f;
     if (safe < d2[i]) d2[i] = safe;
-}
-__global__ void fill_f32_kernel(float* a, int64_t n, float v) {
-    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) a[i] = v;
-}
-__global__ void gather_rows_i64_kernel(const float* __restrict__ x, int d, const int64_t* __restrict__ rows, int64_t nr,
-                                       float* __restrict__ out) {
-    const int64_t i = blockIdx.x;
-    if (i >= nr) return;
-    for (int e = threadIdx.x; e < d; e += blockDim.x) out[i * d + e] = x[rows[i] * d + e];
 }
 // dist[i] = _vi_km12_l2sq_aos(rows[i], c)
 __global__ void km12_dist_to_row_kernel(const float* __restrict__ rows, int64_t n, int d, const float* __restrict__ c,
@@ -252,8 +232,7 @@ int kmeanspp_parity_device(const float* x, int64_t n, int d, int k, uint64_t see
     Lcg rng(seed, stream);
     Scratch<float> d2;
     VIX_TRY(d2.alloc((size_t)n));
-    fill_f32_kernel<<<blocks_for(n), 256, 0, s>>>(d2.ptr, n, INFINITY);
-    VIX_LAUNCH_CHECK();
+    VIX_TRY(fill<float>(d2.ptr, n, INFINITY));
     std::vector<float> w;
     int64_t sel = rng.next_int(n);                                               // KMeansSeeding.swift:223
     for (int t = 0; t < k; ++t) {
@@ -322,8 +301,7 @@ int kmeans_parity_device(const float* x, int64_t n, int d, int kc, const float* 
             for (int bi = 0; bi < bc; ++bi) bidx[(size_t)bi] = (int64_t)(rng.next() % (uint64_t)n);   // :524-528, with replacement
             current_tag += 1;
             VIX_TRY(to_device(d_bidx.ptr, bidx));
-            gather_rows_i64_kernel<<<(unsigned)bc, 128, 0, s>>>(x, d, d_bidx.ptr, bc, d_rows.ptr);
-            VIX_LAUNCH_CHECK();
+            VIX_TRY(gather_rows(x, d, d_bidx.ptr, bc, d_rows.ptr));
             // assignments use the centroids as of batch start
             VIX_TRY(ivf_assign_device(d_rows.ptr, bc, d, centroids_out, kc, d_bassign.ptr, nullptr));
             VIX_TRY(to_host(bassign, d_bassign.ptr, (size_t)bc));
@@ -381,8 +359,7 @@ int kmeans_parity_device(const float* x, int64_t n, int d, int kc, const float* 
             if (j < sm) res[(size_t)j] = i;
         }
         VIX_TRY(to_device(d_bidx.ptr, res));
-        gather_rows_i64_kernel<<<(unsigned)sm, 128, 0, s>>>(x, d, d_bidx.ptr, sm, d_rows.ptr);
-        VIX_LAUNCH_CHECK();
+        VIX_TRY(gather_rows(x, d, d_bidx.ptr, sm, d_rows.ptr));
         VIX_TRY(ivf_assign_device(d_rows.ptr, sm, d, centroids_out, kc, d_bassign.ptr, d_dist.ptr));
         VIX_TRY(to_host(dist, d_dist.ptr, (size_t)sm));
         double inertia = 0.0;
@@ -482,31 +459,13 @@ int seed_subspace(const SubSrc& src, int64_t npts, int ks, int use_residual, Xor
 // rows stably sorted by assignment + CSR offsets (device)
 int sort_rows_by_code(const int32_t* best_k, int64_t n, int ks, Scratch<int32_t>& rows_sorted, Scratch<int64_t>& off,
                       std::vector<int32_t>& counts_h) {
-    cudaStream_t s = ctx().stream;
-    Scratch<int32_t> rows_in, keys_out, cnt;
-    VIX_TRY(rows_in.alloc((size_t)n));
-    VIX_TRY(keys_out.alloc((size_t)n));
+    Scratch<int32_t> cnt;
     VIX_TRY(rows_sorted.alloc((size_t)n));
     VIX_TRY(cnt.alloc((size_t)ks));
     VIX_TRY(off.alloc((size_t)ks + 1));
-    iota_i32_kernel<<<blocks_for(n), 256, 0, s>>>(rows_in.ptr, n);
-    VIX_LAUNCH_CHECK();
-    int bits = 1;
-    while ((1LL << bits) < ks) ++bits;
-    size_t tmp_bytes = 0;
-    VIX_CUDA(cub::DeviceRadixSort::SortPairs(nullptr, tmp_bytes, best_k, keys_out.ptr, rows_in.ptr, rows_sorted.ptr, (int)n, 0, bits, s));
-    Scratch<unsigned char> tmp;
-    VIX_TRY(tmp.alloc(tmp_bytes + 16));
-    VIX_CUDA(cub::DeviceRadixSort::SortPairs(tmp.ptr, tmp_bytes, best_k, keys_out.ptr, rows_in.ptr, rows_sorted.ptr, (int)n, 0, bits, s));
-    ctx().launches += 1;
-    VIX_CUDA(cudaMemsetAsync(cnt.ptr, 0, (size_t)ks * 4, s));
-    count_i32_kernel<<<blocks_for(n), 256, 0, s>>>(best_k, n, ks, cnt.ptr);
-    VIX_LAUNCH_CHECK();
-    VIX_TRY(to_host(counts_h, cnt.ptr, (size_t)ks));
-    std::vector<int64_t> off_h((size_t)ks + 1, 0);
-    for (int k = 0; k < ks; ++k) off_h[(size_t)k + 1] = off_h[(size_t)k] + counts_h[(size_t)k];
-    VIX_TRY(to_device(off.ptr, off_h));
-    return VIX_OK;
+    VIX_TRY(order_by_key(best_k, n, ks, rows_sorted.ptr));
+    VIX_TRY(key_offsets(best_k, n, ks, cnt.ptr, off.ptr));
+    return to_host(counts_h, cnt.ptr, (size_t)ks);
 }
 
 // copy raw (non-residual) sub-vectors x[rows[t]] into C[ks_list[t]]
