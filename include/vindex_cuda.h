@@ -443,12 +443,18 @@ int vix_index_search_with_probes(vix_index_t* h, const float* queries, int64_t n
  *   vix_comm_create      collective; binds the calling thread's CUDA device
  *   vix_sharded_add      collective; x / ids: the rows THIS rank contributes (any rows; n may be 0).  Rows are assigned +
  *                        encoded here and appended on the rank owning their list: list l belongs to rank r iff
- *                        list_bounds[r] <= l < list_bounds[r + 1] (host array [world + 1], NULL = equal-count blocks)
+ *                        list_bounds[r] <= l < list_bounds[r + 1] (host array [world + 1], NULL = equal-count blocks).
+ *                        A row with no nearest list (NaN components) or an id outside [0, 2^32 - 1) on ANY rank makes
+ *                        every rank return VIX_ERR_INVALID_PARAM (naming that rank) before any row travels: no rank
+ *                        stores a row of the call
  *   vix_sharded_search   collective; every rank passes the SAME batch (host or device pointer; from a host pointer only
  *                        the rank's own 1/world block crosses PCIe) and receives the merged [nq x k] result.  Results
  *                        equal vix_index_search on one GPU holding all lists (same probe lists by construction; same
- *                        (distance, id) order: mergeTopK, TopKMerge.swift:11-61; a distance may differ in its last bit
- *                        when a row sits in another slot of its list, which changes the order its table entries are summed in).  Asynchronous mode: no host
+ *                        (distance, id) order: mergeTopK, TopKMerge.swift:11-61), bit for bit -- zero distances with
+ *                        their sign (IP -0, L2 +0) and NaN / -1 padding included -- when that GPU holds every row in the
+ *                        slot the shards do: rows inserted in the order the owners append them, i.e. rank 0's
+ *                        contributions first.  A row in another slot of its list may differ in the last bit of its
+ *                        distance (the slot decides the order its table entries are summed in).  Asynchronous mode: no host
  *                        synchronisation at all when the outputs are device pointers. */
 typedef struct vix_comm vix_comm_t;
 int vix_comm_unique_id(void* id_out, size_t capacity /* >= 128 */);
@@ -501,6 +507,12 @@ int vix_debug_tc_scores_f32(const float* queries, int64_t nq, const float* centr
  * layout (only L2 indexes with ks = 256, d = 2 m and m in {16, 32, 48, 64} do); out (host or device, nullable) receives
  * the bytes when cap holds them. */
 int vix_debug_tc_codes(vix_index_t* h, uint8_t* out, int64_t cap, int64_t* bytes_out);
+
+/* Test hook: the result merge of vix_sharded_search on one GPU.  dist_all / ids_all: [world x nq x k] per-rank top-k
+ * lists as the ranks' scans return them (API distances, ids; id -1 = none); they are packed into keys and merged by the
+ * kernels the exchange runs, into out [nq x k] (host or device pointers). */
+int vix_debug_shard_merge(const float* dist_all, const int64_t* ids_all, int world, int64_t nq, int k, int metric,
+                          float* out_dist, int64_t* out_ids);
 
 /* a16  AccelerableIndex-shaped convenience (AccelerableIndex.swift:15-127): candidates [c x d]
  * contiguous in, (indices into candidates, distances) out, per query. */

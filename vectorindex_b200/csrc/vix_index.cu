@@ -80,6 +80,17 @@ int count_invalid_assign(const int32_t* assign, int64_t n, int kc, unsigned long
     return VIX_OK;
 }
 
+int count_invalid_rows_device(const int32_t* assign, const int64_t* ids, int64_t n, int kc, unsigned long long* count_dev) {
+    if (n <= 0) return VIX_OK;
+    cudaStream_t s = ctx().stream;
+    const unsigned grid = (unsigned)((n + 255) / 256);
+    count_invalid_assign_kernel<<<grid, 256, 0, s>>>(assign, n, kc, count_dev);
+    VIX_LAUNCH_CHECK();
+    count_invalid_ids_kernel<<<grid, 256, 0, s>>>(ids, n, count_dev);
+    VIX_LAUNCH_CHECK();
+    return VIX_OK;
+}
+
 // Fill one slot: codes in the scan layout (vix_scan.cuh), id, t_x.  One warp per slot (lanes split the
 // sub-quantisers).  rotated != 0: byte b of slot g holds sub-quantiser (b & ~15) | ((b ^ g) & 15), chunk-blocked.
 __global__ void __launch_bounds__(256)

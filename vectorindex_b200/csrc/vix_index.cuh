@@ -143,6 +143,9 @@ int index_search_locked(vix_index* h, const float* queries, int64_t nq, int k, i
 int assign_lists_device(vix_index* h, const float* x, int64_t n, int32_t* assign);
 // number of assignments outside [0, kc) in a device array (synchronises the stream)
 int count_invalid_assign(const int32_t* assign, int64_t n, int kc, unsigned long long* out);
+// *count_dev += rows with an assignment outside [0, kc) + ids outside [0, 2^32 - 1) (device pointers; stream-ordered, no
+// synchronisation: a collective caller gathers the count with its peers' before any rank decides)
+int count_invalid_rows_device(const int32_t* assign, const int64_t* ids, int64_t n, int kc, unsigned long long* count_dev);
 // append already encoded rows (device or host pointers) to an IVF-PQ index whose mutex the caller holds
 int index_add_encoded_locked(vix_index* h, const int32_t* assign, const uint8_t* codes, const int64_t* ids, int64_t n);
 int build_lists(vix_index* h);

@@ -271,8 +271,9 @@ __global__ void pack_result_keys_kernel(const float* __restrict__ dist, const in
 }
 
 // keys_all: [world][nq][k] as gathered; one CTA per query selects the k smallest of its world x k keys (padding keys
-// come out as NaN / id -1)
-__global__ void merge_shard_keys_kernel(const u64* __restrict__ keys_all, int world, int64_t nq, int k, int P2,
+// come out as NaN / id -1).  The keys hold zero distances as +0 (make_key folds -0); one GPU returns a zero inner-product
+// distance as -0 (the API distance -score of a +0 score) and a zero L2 distance as +0, so the metric restores the sign.
+__global__ void merge_shard_keys_kernel(const u64* __restrict__ keys_all, int world, int64_t nq, int k, int P2, int metric,
                                         float* __restrict__ out_dist, int64_t* __restrict__ out_ids) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     u64* s = reinterpret_cast<u64*>(smem_raw);
@@ -292,19 +293,20 @@ __global__ void merge_shard_keys_kernel(const u64* __restrict__ keys_all, int wo
             out_dist[o] = __int_as_float(0x7fc00000);
             out_ids[o] = -1;
         } else {
-            out_dist[o] = key_score(key, 0);
+            const float v = key_score(key, 0);
+            out_dist[o] = (v == 0.0f && metric == VIX_METRIC_IP) ? -0.0f : v;
             out_ids[o] = (int64_t)key_id(key);
         }
     }
 }
 
-static int merge_shard_keys(const u64* keys_all, int world, int64_t nq, int k, float* out_dist, int64_t* out_ids) {
+static int merge_shard_keys(const u64* keys_all, int world, int64_t nq, int k, int metric, float* out_dist, int64_t* out_ids) {
     const int P2 = next_pow2(world * k < 2 ? 2 : world * k);
     const size_t smem = (size_t)P2 * 8;
     VIX_REQUIRE(smem <= 200 * 1024, VIX_ERR_UNSUPPORTED, "shard merge: %d keys per query exceed shared memory", world * k);
     VIX_CUDA(cudaFuncSetAttribute(merge_shard_keys_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const int threads = P2 / 2 < 32 ? 32 : (P2 / 2 > 256 ? 256 : P2 / 2);
-    merge_shard_keys_kernel<<<(unsigned)nq, threads, smem, ctx().stream>>>(keys_all, world, nq, k, P2, out_dist, out_ids);
+    merge_shard_keys_kernel<<<(unsigned)nq, threads, smem, ctx().stream>>>(keys_all, world, nq, k, P2, metric, out_dist, out_ids);
     VIX_LAUNCH_CHECK();
     return VIX_OK;
 }
@@ -516,7 +518,7 @@ int vix_sharded_search(vix_index_t* h, vix_comm_t* c, const float* queries, int6
                                                                               c->off_results + (size_t)rank * total * 8, nullptr);
         VIX_LAUNCH_CHECK();
         VIX_TRY(peer_barrier(c));
-        VIX_TRY(merge_shard_keys(rbuf, world, nq, k, dd.dev, di.dev));
+        VIX_TRY(merge_shard_keys(rbuf, world, nq, k, h->p.metric, dd.dev, di.dev));
     } else {
         // NCCL carries the two exchanges
         In<float> dq;
@@ -547,12 +549,39 @@ int vix_sharded_search(vix_index_t* h, vix_comm_t* c, const float* queries, int6
                                                                               kall + (size_t)rank * total);
         VIX_LAUNCH_CHECK();
         VIX_NCCL(g_nccl.AllGather(kall + (size_t)rank * total, kall, (size_t)total, ncclUint64, c->comm, s));
-        VIX_TRY(merge_shard_keys(kall, world, nq, k, dd.dev, di.dev));
+        VIX_TRY(merge_shard_keys(kall, world, nq, k, h->p.metric, dd.dev, di.dev));
     }
     mark(3);
     VIX_TRY(dd.commit());
     VIX_TRY(di.commit());
     return finish(dd.is_host() || di.is_host());
+}
+
+int vix_debug_shard_merge(const float* dist_all, const int64_t* ids_all, int world, int64_t nq, int k, int metric,
+                          float* out_dist, int64_t* out_ids) {
+    VIX_TRY(ensure_device());
+    VIX_REQUIRE(dist_all && ids_all && out_dist && out_ids, VIX_ERR_NULL_PTR, "vix_debug_shard_merge: null pointer");
+    VIX_REQUIRE(world > 0 && world <= 256 && nq >= 0 && k > 0 && k <= VIX_MAX_K, VIX_ERR_INVALID_PARAM,
+                "vix_debug_shard_merge: world / nq / k");
+    if (nq == 0) return VIX_OK;
+    const int64_t total = (int64_t)world * nq * k;
+    In<float> dd;
+    In<int64_t> di;
+    Out<float> od;
+    Out<int64_t> oi;
+    VIX_TRY(dd.stage(dist_all, (size_t)total));
+    VIX_TRY(di.stage(ids_all, (size_t)total));
+    VIX_TRY(od.stage(out_dist, (size_t)nq * k));
+    VIX_TRY(oi.stage(out_ids, (size_t)nq * k));
+    Scratch<u64> keys;
+    VIX_TRY(keys.alloc((size_t)total));
+    pack_result_keys_kernel<<<(unsigned)((total + 255) / 256), 256, 0, ctx().stream>>>(dd.dev, di.dev, total, nullptr, world, 0,
+                                                                                     keys.ptr);
+    VIX_LAUNCH_CHECK();
+    VIX_TRY(merge_shard_keys(keys.ptr, world, nq, k, metric, od.dev, oi.dev));
+    VIX_TRY(od.commit());
+    VIX_TRY(oi.commit());
+    return finish(od.is_host() || oi.is_host());
 }
 
 int vix_comm_trace(vix_comm_t* c, int enabled) {
@@ -589,7 +618,10 @@ int vix_sharded_add(vix_index_t* h, vix_comm_t* c, const int64_t* list_bounds, c
     VIX_REQUIRE(bounds[0] == 0 && bounds[world] == h->kc, VIX_ERR_INVALID_PARAM, "vix_sharded_add: bounds must run from 0 to %d", h->kc);
     for (int r = 0; r < world; ++r)
         VIX_REQUIRE(bounds[r + 1] >= bounds[r], VIX_ERR_INVALID_PARAM, "vix_sharded_add: bounds must ascend");
-    // 1. assign + encode what this rank was handed
+    // 1. assign what this rank was handed and count the rows no rank may store: no nearest list (NaN components) or an id
+    //    outside [0, 2^32 - 1).  The count rides in the all-gather of the send counts, so every rank sees every rank's count
+    //    before any row travels, and all of them refuse the call together (a rank that returned alone would leave its peers
+    //    waiting in the all-gather, or holding their share of the rows).
     In<float> dx;
     In<int64_t> dids;
     VIX_TRY(dx.stage(x, (size_t)n * d));
@@ -598,28 +630,39 @@ int vix_sharded_add(vix_index_t* h, vix_comm_t* c, const int64_t* list_bounds, c
     Scratch<uint8_t> codes;
     Scratch<unsigned long long> dcounts;
     Scratch<int64_t> dbounds;
-    VIX_TRY(dcounts.alloc((size_t)world * (world + 1)));
+    const size_t W = (size_t)world + 1;                                   // per rank: rows for each owner, then invalid rows
+    VIX_TRY(dcounts.alloc(W * (world + 1)));                              // [world][W] gathered, then this rank's [W]
     VIX_TRY(dbounds.alloc((size_t)world + 1));
-    VIX_CUDA(cudaMemsetAsync(dcounts.ptr, 0, sizeof(unsigned long long) * world * (world + 1), s));
+    VIX_CUDA(cudaMemsetAsync(dcounts.ptr, 0, sizeof(unsigned long long) * W * (world + 1), s));
     VIX_CUDA(cudaMemcpyAsync(dbounds.ptr, bounds.data(), sizeof(int64_t) * (world + 1), cudaMemcpyHostToDevice, s));
+    unsigned long long* mine = dcounts.ptr + W * world;
+    if (n > 0) {
+        VIX_TRY(asg.alloc((size_t)n));
+        VIX_TRY(assign_lists_device(h, dx.dev, n, asg.ptr));
+        VIX_TRY(count_invalid_rows_device(asg.ptr, dids.dev, n, h->kc, mine + world));
+        // rows ordered by owning rank (stable: rows keep their order inside a block)
+        VIX_TRY(owner.alloc((size_t)n));
+        VIX_TRY(order.alloc((size_t)n));
+        owner_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(asg.ptr, n, dbounds.ptr, world, owner.ptr, mine);
+        VIX_LAUNCH_CHECK();
+        VIX_TRY(order_by_key(owner.ptr, n, world, order.ptr));
+    }
+    // 2. everybody learns everybody's send counts and invalid rows
+    VIX_NCCL(g_nccl.AllGather(mine, dcounts.ptr, W, ncclUint64, c->comm, s));
+    std::vector<unsigned long long> counts(W * world);
+    VIX_CUDA(cudaMemcpyAsync(counts.data(), dcounts.ptr, sizeof(unsigned long long) * W * world, cudaMemcpyDeviceToHost, s));
+    VIX_CUDA(cudaStreamSynchronize(s));
+    for (int p = 0; p < world; ++p)
+        VIX_REQUIRE(counts[(size_t)p * W + world] == 0, VIX_ERR_INVALID_PARAM,
+                    "vix_sharded_add: rank %d was handed %llu rows with no nearest list (NaN components?) or an id outside "
+                    "[0, 2^32 - 1); no rank stored any row of this call", p, counts[(size_t)p * W + world]);
+    // 3. encode, in owner order
     Scratch<int32_t> s_asg;
     Scratch<uint8_t> s_codes;
     Scratch<int64_t> s_ids;
     if (n > 0) {
-        VIX_TRY(asg.alloc((size_t)n));
         VIX_TRY(codes.alloc((size_t)n * m));
-        VIX_TRY(assign_lists_device(h, dx.dev, n, asg.ptr));
-        unsigned long long invalid = 0;
-        VIX_TRY(count_invalid_assign(asg.ptr, n, h->kc, &invalid));
-        VIX_REQUIRE(invalid == 0, VIX_ERR_INVALID_PARAM, "vix_sharded_add: %llu rows have no nearest list (NaN components?)", invalid);
         VIX_TRY(encode_rows_device(h, dx.dev, n, asg.ptr, codes.ptr));
-        // 2. rows ordered by owning rank (stable: rows keep their order inside a block)
-        VIX_TRY(owner.alloc((size_t)n));
-        VIX_TRY(order.alloc((size_t)n));
-        owner_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(asg.ptr, n, dbounds.ptr, world, owner.ptr,
-                                                               dcounts.ptr + (size_t)world * world);
-        VIX_LAUNCH_CHECK();
-        VIX_TRY(order_by_key(owner.ptr, n, world, order.ptr));
         VIX_TRY(s_asg.alloc((size_t)n));
         VIX_TRY(s_codes.alloc((size_t)n * m));
         VIX_TRY(s_ids.alloc((size_t)n));
@@ -627,15 +670,10 @@ int vix_sharded_add(vix_index_t* h, vix_comm_t* c, const int64_t* list_bounds, c
                                                                      s_codes.ptr, s_ids.ptr);
         VIX_LAUNCH_CHECK();
     }
-    // 3. everybody learns everybody's send counts
-    VIX_NCCL(g_nccl.AllGather(dcounts.ptr + (size_t)world * world, dcounts.ptr, (size_t)world, ncclUint64, c->comm, s));
-    std::vector<unsigned long long> counts((size_t)world * world);
-    VIX_CUDA(cudaMemcpyAsync(counts.data(), dcounts.ptr, sizeof(unsigned long long) * world * world, cudaMemcpyDeviceToHost, s));
-    VIX_CUDA(cudaStreamSynchronize(s));
     std::vector<int64_t> send_off((size_t)world + 1, 0), recv_off((size_t)world + 1, 0);
     for (int p = 0; p < world; ++p) {
-        send_off[p + 1] = send_off[p] + (int64_t)counts[(size_t)rank * world + p];
-        recv_off[p + 1] = recv_off[p] + (int64_t)counts[(size_t)p * world + rank];
+        send_off[p + 1] = send_off[p] + (int64_t)counts[(size_t)rank * W + p];
+        recv_off[p + 1] = recv_off[p] + (int64_t)counts[(size_t)p * W + rank];
     }
     const int64_t nrecv = recv_off[world];
     // 4. rows travel to their owners
