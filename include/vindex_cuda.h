@@ -39,7 +39,10 @@
  *                            list-major scan), the locality order (yes / no) and the work items (query count, or device:
  *                            the queries the list-major scan hands back); and per vix_index_range_search call one line
  *                            "[vix range] kind K, kernel fast G n | generic | ivfflat | flat, filter 0|1, passes 1|2, total T,
- *                            max_row M, sorted_long L" (L: rows longer than the in-shared-memory sort, merged in global memory)
+ *                            max_row M, sorted_long L" (L: rows longer than the in-shared-memory sort, merged in global memory);
+ *                            and per vix_sharded_range_search call and rank (world > 1) one line "[vix sharded range] world W,
+ *                            peer 0|1, local T_r, total T, max_row M, grown 0|1" (T_r: this rank's entries, M: the longest
+ *                            merged row, grown: the range region of the communicator was (re)allocated by the call)
  *   VIX_DISABLE_TC, VIX_DISABLE_PQ_TC, VIX_DISABLE_LUT_IMAGE
  *                            exact CUDA-core kernels instead of the tensor-core shortlists / per-query tables built inside
  *                            the scan instead of batch-wide (the parity tests compare both ways)
@@ -391,7 +394,7 @@ int vix_index_search_ex(vix_index_t* h, const float* queries, int64_t nq, int k,
  *     are valid (an IP radius of -0.8 keeps dot >= 0.8);
  *   - filter_words (nullable): the id filter of vix_index_search_filtered, applied before the radius test;
  *   - a row stored twice, or a list probed twice, comes back twice; a dirty handle rebuilds its lists first, as search
- *     does; on a shard the result is what THIS rank holds (no cross-rank merge).
+ *     does; on a shard the result is what THIS rank holds (vix_sharded_range_search merges the ranks).
  * The call synchronises its stream once, even in asynchronous mode: the size of the answer depends on the data.  It
  * normally scans once; when the answer outgrows the capacity the handle remembers from its previous call, the scan runs a
  * second time with the exact capacity.  A result that does not fit in device memory returns VIX_ERR_OOM with nothing
@@ -463,8 +466,9 @@ int vix_comm_destroy(vix_comm_t* c);
 int vix_comm_rank(const vix_comm_t* c);
 int vix_comm_world(const vix_comm_t* c);
 int vix_comm_uses_peer_memory(const vix_comm_t* c);        /* 1 peer memory, 0 NCCL all-gathers, -1 not decided yet */
-/* measurement aid: CUDA events around the three phases of the LAST vix_sharded_search on this communicator --
- * probe selection + exchange | fused scan | result exchange + merge (ms; waits for that search to finish) */
+/* measurement aid: CUDA events around the three phases of the LAST vix_sharded_search, vix_sharded_search_filtered or
+ * vix_sharded_range_search on this communicator -- probe selection + exchange | fused scan (range: local scan and sort) |
+ * result exchange + merge (range: + decode) (ms; waits for that call to finish) */
 int vix_comm_trace(vix_comm_t* c, int enabled);
 int vix_comm_trace_get(vix_comm_t* c, float* phase_ms /* [3] */);
 /* rows [first, first + count) of a batch of nq queries are the block whose probe lists `rank` computes */
@@ -473,6 +477,34 @@ int vix_sharded_add(vix_index_t* h, vix_comm_t* c, const int64_t* list_bounds /*
                     const int64_t* ids, int64_t n);
 int vix_sharded_search(vix_index_t* h, vix_comm_t* c, const float* queries, int64_t nq, int k, int nprobe,
                        float* out_dist, int64_t* out_ids);
+
+/* Sharded range search and id filters: vix_index_range_search / vix_index_search_filtered over the list-sharded layout of
+ * vix_sharded_search.  Both are collective: every rank passes the same batch, radius (or k), nprobe and filter, host or
+ * device pointers (from a host pointer only the rank's own block of queries crosses PCIe), and every rank receives the
+ * whole merged answer.
+ *   - Parity: the answer equals the one-GPU call on an index holding every row in the slot the shards hold it in (rows
+ *     inserted in owner-append order, rank 0's contributions first), bit for bit: lims, ids, distance bits with the sign of
+ *     zero (IP -0, L2 +0), the (distance, id) order, rows stored twice and lists probed twice (each comes back twice).
+ *   - Refusals, on every rank alike and before any exchange: a NaN radius, a filter_mode other than VIX_FILTER_ALLOW /
+ *     VIX_FILTER_DENY or a negative filter_capacity (VIX_ERR_INVALID_PARAM); nprobe outside 1 .. VIX_MAX_K after the default
+ *     (VIX_ERR_INVALID_K); cosine (VIX_ERR_UNSUPPORTED); an index that is not a trained IVF-PQ index (VIX_ERR_NOT_TRAINED).
+ *   - Range: nq == 0 gives an empty result (lims = {0}) with no exchange; one rank is vix_index_range_search.  The probes
+ *     travel as in vix_sharded_search; each rank runs the query-major range scan over the probed lists it owns and sorts
+ *     its rows; the ranks exchange their row starts, then their sorted keys (a second peer-mapped region of the
+ *     communicator, grown collectively and geometrically, or NCCL: an all-gather of the row starts and grouped send /
+ *     receive of the keys); every rank merges the world sorted runs of each row on the device and decodes them.  Host
+ *     synchronisations: the local total, the global total and the collective verdict on the result's allocation.  A global
+ *     answer that does not fit in device memory on some rank makes every rank return VIX_ERR_OOM with nothing allocated and
+ *     the index unchanged; so does a failure of any rank's local scan (every rank returns that rank's code).  *out is
+ *     released with vix_range_result_destroy.
+ *   - Filtered k-NN: filter_words == NULL is vix_sharded_search; a filter sends each rank's scan down the query-major path,
+ *     as on one GPU. */
+int vix_sharded_range_search(vix_index_t* h, vix_comm_t* c, const float* queries, int64_t nq, float radius, int nprobe,
+                             const uint64_t* filter_words /* nullable */, int64_t filter_capacity, int filter_mode,
+                             vix_range_result_t** out);
+int vix_sharded_search_filtered(vix_index_t* h, vix_comm_t* c, const float* queries, int64_t nq, int k, int nprobe,
+                                const uint64_t* filter_words /* nullable */, int64_t filter_capacity, int filter_mode,
+                                float* out_dist, int64_t* out_ids);
 
 /* f-1  The IVF-PQ query with its optional last step (docs/kernel-specs/DONE_22_adc_scan.md:873-878, "7. Optional: exact
  * rerank (kernel #40)"; IVFIndex.swift:1380-1439): ADC search for the rerank_r best candidates per query (k <= rerank_r <=
@@ -513,6 +545,14 @@ int vix_debug_tc_codes(vix_index_t* h, uint8_t* out, int64_t cap, int64_t* bytes
  * kernels the exchange runs, into out [nq x k] (host or device pointers). */
 int vix_debug_shard_merge(const float* dist_all, const int64_t* ids_all, int world, int64_t nq, int k, int metric,
                           float* out_dist, int64_t* out_ids);
+
+/* Test hook: the merge of vix_sharded_range_search on one GPU.  lims_all: [world x (nq + 1)] the ranks' CSR row starts;
+ * dist_all / ids_all: their rows (API distances, ids), concatenated rank by rank, each row sorted by (distance, id) as
+ * vix_index_range_search returns it.  They are packed into keys and merged and decoded by the kernels the exchange runs
+ * (metric: the sign of zero distances), into a new result object (host or device pointers; world 1 .. 256). */
+int vix_debug_shard_range_merge(const int64_t* lims_all /* [world x (nq + 1)] */, const float* dist_all,
+                                const int64_t* ids_all /* concatenated rank by rank */, int world, int64_t nq, int metric,
+                                vix_range_result_t** out);
 
 /* a16  AccelerableIndex-shaped convenience (AccelerableIndex.swift:15-127): candidates [c x d]
  * contiguous in, (indices into candidates, distances) out, per query. */

@@ -127,5 +127,27 @@ public final class CUDAIVFPQIndex {
         try _vixCheck(vix_sharded_search(h, comm, q, Int64(nq), Int32(k), 0, &dist, &ids), "sharded_search")
         return (dist, ids)
     }
+    /// collective `filter:` search: the id bitset is applied before selection on every rank, as batchSearch(allow:)
+    public func shardedSearch(_ comm: OpaquePointer?, _ q: [Float], nq: Int, k: Int, filter allow: IDFilterBitset) throws
+        -> ([Float], [Int64]) {
+        var dist = [Float](repeating: .nan, count: nq * k); var ids = [Int64](repeating: -1, count: nq * k)
+        try _vixCheck(vix_sharded_search_filtered(h, comm, q, Int64(nq), Int32(k), 0, allow.readOnly, Int64(allow.capacity),
+                                                  Int32(VIX_FILTER_ALLOW.rawValue), &dist, &ids), "sharded_search_filtered")
+        return (dist, ids)
+    }
+    /// collective rangeSearch over the list shards: every rank receives the whole merged CSR, equal to rangeSearch on one GPU
+    /// holding every row
+    public func shardedRangeSearch(_ comm: OpaquePointer?, _ q: [Float], nq: Int, radius: Float) throws
+        -> (lims: [Int64], dist: [Float], ids: [Int64]) {
+        var res: OpaquePointer? = nil
+        try _vixCheck(vix_sharded_range_search(h, comm, q, Int64(nq), radius, 0, nil, 0, Int32(VIX_FILTER_ALLOW.rawValue), &res),
+                      "sharded_range_search")
+        defer { vix_range_result_destroy(res) }
+        let total = Int(vix_range_result_total(res))
+        var lims = [Int64](repeating: 0, count: nq + 1)
+        var dist = [Float](repeating: 0, count: total); var ids = [Int64](repeating: -1, count: total)
+        try _vixCheck(vix_range_result_get(res, &lims, &dist, &ids), "vix_range_result_get")
+        return (lims, dist, ids)
+    }
 }
 #endif

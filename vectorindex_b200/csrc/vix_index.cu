@@ -951,9 +951,10 @@ int index_search_locked(vix_index* h, const float* queries, int64_t nq, int k, i
 }
 
 // One range search of an index whose mutex the caller holds: the candidates of index_search_locked (every row, or the probed
-// lists of the same probe selection), each kind through its range kernel, the output path of vix_range.cu.
-static int index_range_locked(vix_index* h, const float* queries, int64_t nq, float radius, int nprobe,
-                              const FilterArgs* filter, vix_range_result** out) {
+// lists of the same probe selection, or the caller's given_probes), each kind through its range kernel, the output path of
+// vix_range.cu.  keys_out: stop before decoding and hand back the sorted keys and lims (out is not touched).
+int index_range_locked(vix_index* h, const float* queries, int64_t nq, float radius, int nprobe, const FilterArgs* filter,
+                       vix_range_result** out, const int32_t* given_probes, RangeKeys* keys_out) {
     const int d = h->p.d;
     cudaStream_t s = ctx().stream;
     const bool linear = h->p.kind == VIX_INDEX_FLAT || !h->has_coarse;
@@ -969,6 +970,10 @@ static int index_range_locked(vix_index* h, const float* queries, int64_t nq, fl
     RangeInfo info;
     char kernel[32] = "flat";
     int rc;
+    auto collect = [&](bool neg_zero, const std::function<int(const RangeOut&)>& scan) {
+        if (keys_out) return range_collect_keys(nq, radius, cap, scan, *keys_out, &info);
+        return range_collect(nq, radius, cap, neg_zero, scan, out, &info);
+    };
     if (linear) {
         // a flat index, or an IVF-Flat index before optimize(): the flat engine over the stored rows (IVFIndex.swift:820-832)
         Scratch<uint64_t> mask;
@@ -979,22 +984,31 @@ static int index_range_locked(vix_index* h, const float* queries, int64_t nq, fl
                                                                                 filter->deny, mask.ptr);
             VIX_LAUNCH_CHECK();
         }
-        rc = range_collect(nq, radius, cap, h->p.metric == VIX_METRIC_IP, [&](const RangeOut& o) {
+        rc = collect(h->p.metric == VIX_METRIC_IP, [&](const RangeOut& o) {
             return flat_range_device(dq.dev, nq, h->vecs.ptr, h->n, d, h->p.metric, h->ids.ptr, mask.ptr, o);
-        }, out, &info);
+        });
     } else {
         if (h->dirty) VIX_TRY(build_lists(h));
-        Scratch<int32_t> probes;
-        VIX_TRY(probes.alloc((size_t)nq * nprobe));
-        if (h->p.metric == VIX_METRIC_COSINE)
-            VIX_TRY(probe_select_cosine_device(dq.dev, nq, h->coarse.ptr, h->kc, d, h->coarse_norms.ptr, nprobe, probes.ptr));
-        else
-            VIX_TRY(probe_select_fast_device(dq.dev, nq, h->coarse.ptr, h->kc, d, h->p.metric, nprobe, h->coarse_norms.ptr,
-                                             probes.ptr, nullptr, h->coarse_norm_max.ptr));
+        Scratch<int32_t> probe_buf;
+        In<int32_t> gp;
+        const int32_t* probes = nullptr;
+        if (given_probes) {
+            // probe lists chosen by the caller (sharded range search: the lists of the whole batch, exchanged)
+            VIX_TRY(gp.stage(given_probes, (size_t)nq * nprobe));
+            probes = gp.dev;
+        } else {
+            VIX_TRY(probe_buf.alloc((size_t)nq * nprobe));
+            if (h->p.metric == VIX_METRIC_COSINE)
+                VIX_TRY(probe_select_cosine_device(dq.dev, nq, h->coarse.ptr, h->kc, d, h->coarse_norms.ptr, nprobe, probe_buf.ptr));
+            else
+                VIX_TRY(probe_select_fast_device(dq.dev, nq, h->coarse.ptr, h->kc, d, h->p.metric, nprobe, h->coarse_norms.ptr,
+                                                 probe_buf.ptr, nullptr, h->coarse_norm_max.ptr));
+            probes = probe_buf.ptr;
+        }
         if (h->p.kind == VIX_INDEX_IVF_PQ) {
             ScanArgs a{};
             a.queries = dq.dev; a.nq = nq; a.d = d; a.m = h->p.m; a.ks = h->p.ks; a.dsub = d / h->p.m;
-            a.probes = probes.ptr; a.nprobe = nprobe; a.coarse = h->coarse.ptr; a.kc = h->kc; a.codebooks = h->codebooks.ptr;
+            a.probes = probes; a.nprobe = nprobe; a.coarse = h->coarse.ptr; a.kc = h->kc; a.codebooks = h->codebooks.ptr;
             a.list_off = h->list_off.ptr; a.list_len = h->list_len.ptr;
             a.slot_codes = h->slot_codes.ptr; a.slot_tx = h->slot_tx.ptr; a.slot_ids = h->slot_ids.ptr;
             a.metric = h->p.metric; a.codebooks_t = h->codebooks_t.ptr;
@@ -1005,17 +1019,17 @@ static int index_range_locked(vix_index* h, const float* queries, int64_t nq, fl
             const bool fast = scan_layout(a.m).fast && a.ks == 256;
             Scratch<int32_t> order;
             if (fast && nq > 2 * num_sms()) {
-                VIX_TRY(query_order(probes.ptr, nq, nprobe, h->list_len.ptr, h->kc, order));
+                VIX_TRY(query_order(probes, nq, nprobe, h->list_len.ptr, h->kc, order));
                 a.order = order.ptr;
             }
             if (fast) snprintf(kernel, sizeof kernel, "fast G %d", a.m / 16);
             else snprintf(kernel, sizeof kernel, "generic");
             // never the list-major tensor-core scan: the query-major one with its range instantiations
-            rc = range_collect(nq, radius, cap, h->p.metric == VIX_METRIC_IP, [&](const RangeOut& o) {
+            rc = collect(h->p.metric == VIX_METRIC_IP, [&](const RangeOut& o) {
                 ScanArgs b = a;
                 b.range = o;
                 return launch_ivfpq_scan_classic(b);
-            }, out, &info);
+            });
         } else {
             snprintf(kernel, sizeof kernel, "ivfflat");
             const size_t smem = (size_t)d * 4;
@@ -1023,14 +1037,14 @@ static int index_range_locked(vix_index* h, const float* queries, int64_t nq, fl
             int64_t grid = (int64_t)num_sms() * 4;
             if (grid > nq) grid = nq;
             // (the IVF-Flat scan keys the distance itself, so its zeros are +0 as in k-NN search)
-            rc = range_collect(nq, radius, cap, false, [&](const RangeOut& o) -> int {
-                ivfflat_range_kernel<<<(unsigned)grid, 256, smem, s>>>(dq.dev, nq, d, probes.ptr, nprobe, h->list_off.ptr,
+            rc = collect(false, [&](const RangeOut& o) -> int {
+                ivfflat_range_kernel<<<(unsigned)grid, 256, smem, s>>>(dq.dev, nq, d, probes, nprobe, h->list_off.ptr,
                                                                      h->list_len.ptr, h->kc, h->slot_vecs.ptr, h->slot_ids.ptr,
                                                                      h->p.metric, filter ? filter->words : nullptr,
                                                                      filter ? filter->cap : 0, filter ? filter->deny : 0, o);
                 VIX_LAUNCH_CHECK();
                 return VIX_OK;
-            }, out, &info);
+            });
         }
     }
     VIX_TRY(rc);

@@ -139,6 +139,11 @@ struct FilterArgs { const uint64_t* words = nullptr; int64_t cap = 0; int deny =
 int index_search_locked(vix_index* h, const float* queries, int64_t nq, int k, int nprobe, float* out_dist,
                         int64_t* out_ids, int32_t* out_probes, vix_search_stats* stats,
                         const int32_t* given_probes = nullptr, const FilterArgs* filter = nullptr);
+// one range search of an index whose mutex the caller holds (vix_index.cu); given_probes: the caller's probe lists
+// [nq x nprobe]; keys_out: return the sorted keys and lims instead of a result object (no decode)
+struct RangeKeys;
+int index_range_locked(vix_index* h, const float* queries, int64_t nq, float radius, int nprobe, const FilterArgs* filter,
+                       vix_range_result** out, const int32_t* given_probes = nullptr, RangeKeys* keys_out = nullptr);
 // list assignment under the index's metric (device pointers)
 int assign_lists_device(vix_index* h, const float* x, int64_t n, int32_t* assign);
 // number of assignments outside [0, kc) in a device array (synchronises the stream)

@@ -116,14 +116,10 @@ __global__ void range_decode_kernel(const u64* __restrict__ keys, int64_t total,
                                     int64_t* __restrict__ ids) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= total) return;
-    const u64 key = keys[i];
-    float v = key_score(key, 0);
-    if (neg_zero && v == 0.0f) v = -0.0f;
-    dist[i] = v;
-    ids[i] = (int64_t)key_id(key);
+    range_decode_key(keys[i], neg_zero, dist + i, ids + i);
 }
 
-static void range_free(vix_range_result* r) {
+void range_free(vix_range_result* r) {
     if (!r) return;
     if (r->lims) cudaFree(r->lims);
     if (r->dist) cudaFree(r->dist);
@@ -131,8 +127,7 @@ static void range_free(vix_range_result* r) {
     delete r;
 }
 
-// the result object with its arrays allocated (freed again on failure)
-static int range_alloc(int64_t nq, int64_t total, vix_range_result** out) {
+int range_alloc(int64_t nq, int64_t total, vix_range_result** out) {
     vix_range_result* r = new (std::nothrow) vix_range_result();
     VIX_REQUIRE(r, VIX_ERR_OOM, "vix_index_range_search: out of host memory");
     r->nq = nq; r->total = total;
@@ -153,15 +148,14 @@ int range_empty(int64_t nq, vix_range_result** out) {
     return VIX_OK;
 }
 
-int range_collect(int64_t nq, float radius, size_t& cap_hint, bool neg_zero, const std::function<int(const RangeOut&)>& scan,
-                  vix_range_result** out, RangeInfo* info) {
+int range_collect_keys(int64_t nq, float radius, size_t& cap_hint, const std::function<int(const RangeOut&)>& scan,
+                       RangeKeys& rk, RangeInfo* info) {
     cudaStream_t s = ctx().stream;
     const size_t floor_cap = (size_t)(nq * 64 > 65536 ? nq * 64 : 65536);
     size_t cap = cap_hint > floor_cap ? cap_hint : floor_cap;
     Scratch<unsigned long long> ctr;                          // [cursor][counts nq][info 3]
     VIX_TRY(ctr.alloc((size_t)nq + 4));
-    Scratch<int64_t> lims;
-    VIX_TRY(lims.alloc((size_t)nq + 1));
+    VIX_TRY(rk.lims.alloc((size_t)nq + 1));
     Scratch<u64> keys;
     Scratch<uint32_t> qry;
     unsigned long long h_info[3] = {0, 0, 0};
@@ -174,7 +168,7 @@ int range_collect(int64_t nq, float radius, size_t& cap_hint, bool neg_zero, con
         o.keys = keys.ptr; o.qry = qry.ptr; o.cursor = ctr.ptr; o.counts = ctr.ptr + 1; o.cap = cap; o.radius = radius;
         VIX_TRY(scan(o));
         ++passes;
-        range_lims_kernel<<<1, 1024, 0, s>>>(o.counts, nq, lims.ptr, ctr.ptr + 1 + nq);
+        range_lims_kernel<<<1, 1024, 0, s>>>(o.counts, nq, rk.lims.ptr, ctr.ptr + 1 + nq);
         VIX_LAUNCH_CHECK();
         VIX_CUDA(cudaMemcpyAsync(h_info, ctr.ptr + 1 + nq, sizeof h_info, cudaMemcpyDeviceToHost, s));
         VIX_CUDA(cudaStreamSynchronize(s));                   // the one synchronisation: the size of the answer
@@ -187,39 +181,53 @@ int range_collect(int64_t nq, float radius, size_t& cap_hint, bool neg_zero, con
     const int64_t total = (int64_t)h_info[0];
     cap_hint = (size_t)(total + total / 8);
     if (info) { info->passes = passes; info->total = total; info->max_row = (int64_t)h_info[1]; info->sorted_long = (int64_t)h_info[2]; }
-
-    vix_range_result* r = nullptr;
-    VIX_TRY(range_alloc(nq, total, &r));
-    auto fail = [&](int rc) { range_free(r); return rc; };
-    cudaError_t ce = cudaMemcpyAsync(r->lims, lims.ptr, (size_t)(nq + 1) * 8, cudaMemcpyDeviceToDevice, s);
-    if (ce != cudaSuccess) return fail(cuda_fail(ce, "range lims copy", __FILE__, __LINE__));
+    rk.total = total;
+    rk.sorted = nullptr;
     if (total > 0) {
-        Scratch<u64> a, b;
-        int rc = a.alloc((size_t)total);
+        VIX_TRY(rk.a.alloc((size_t)total));
         const int64_t max_row = (int64_t)h_info[1];
-        if (rc == VIX_OK && max_row > kRangeSegment) rc = b.alloc((size_t)total);
-        if (rc != VIX_OK) return fail(rc);
-        ce = cudaMemsetAsync(ctr.ptr + 1, 0, (size_t)nq * 8, s);   // the counts become the scatter's fill cursors
-        if (ce != cudaSuccess) return fail(cuda_fail(ce, "range fill cursors", __FILE__, __LINE__));
+        if (max_row > kRangeSegment) VIX_TRY(rk.b.alloc((size_t)total));
+        VIX_CUDA(cudaMemsetAsync(ctr.ptr + 1, 0, (size_t)nq * 8, s));   // the counts become the scatter's fill cursors
         const unsigned grid = (unsigned)min((int64_t)num_sms() * 8, (total + 255) / 256);
-        range_scatter_kernel<<<grid, 256, 0, s>>>(keys.ptr, qry.ptr, total, lims.ptr, ctr.ptr + 1, a.ptr);
+        range_scatter_kernel<<<grid, 256, 0, s>>>(keys.ptr, qry.ptr, total, rk.lims.ptr, ctr.ptr + 1, rk.a.ptr);
         const unsigned rows_grid = (unsigned)min((int64_t)num_sms() * 4, nq);
-        range_sort_rows_kernel<<<rows_grid, 512, 0, s>>>(a.ptr, lims.ptr, nq);
+        range_sort_rows_kernel<<<rows_grid, 512, 0, s>>>(rk.a.ptr, rk.lims.ptr, nq);
         ctx().launches += 2;
-        u64* cur = a.ptr;
-        u64* oth = b.ptr;
+        u64* cur = rk.a.ptr;
+        u64* oth = rk.b.ptr;
         for (int64_t w = kRangeSegment; w < max_row; w *= 2) {
-            range_merge_pass_kernel<<<grid, 256, 0, s>>>(cur, oth, lims.ptr, nq, total, w);
+            range_merge_pass_kernel<<<grid, 256, 0, s>>>(cur, oth, rk.lims.ptr, nq, total, w);
             ctx().launches += 1;
             u64* t = cur; cur = oth; oth = t;
         }
-        range_decode_kernel<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(cur, total, neg_zero ? 1 : 0, r->dist, r->ids);
+        VIX_CUDA(cudaGetLastError());
+        rk.sorted = cur;
+    }
+    return VIX_OK;
+}
+
+int range_decode(int64_t nq, const int64_t* lims, const u64* sorted, int64_t total, bool neg_zero, vix_range_result** out) {
+    cudaStream_t s = ctx().stream;
+    vix_range_result* r = nullptr;
+    VIX_TRY(range_alloc(nq, total, &r));
+    auto fail = [&](int rc) { range_free(r); return rc; };
+    cudaError_t ce = cudaMemcpyAsync(r->lims, lims, (size_t)(nq + 1) * 8, cudaMemcpyDeviceToDevice, s);
+    if (ce != cudaSuccess) return fail(cuda_fail(ce, "range lims copy", __FILE__, __LINE__));
+    if (total > 0) {
+        range_decode_kernel<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(sorted, total, neg_zero ? 1 : 0, r->dist, r->ids);
         ctx().launches += 1;
         ce = cudaGetLastError();
-        if (ce != cudaSuccess) return fail(cuda_fail(ce, "range sort", __FILE__, __LINE__));
+        if (ce != cudaSuccess) return fail(cuda_fail(ce, "range decode", __FILE__, __LINE__));
     }
     *out = r;
     return VIX_OK;
+}
+
+int range_collect(int64_t nq, float radius, size_t& cap_hint, bool neg_zero, const std::function<int(const RangeOut&)>& scan,
+                  vix_range_result** out, RangeInfo* info) {
+    RangeKeys rk;
+    VIX_TRY(range_collect_keys(nq, radius, cap_hint, scan, rk, info));
+    return range_decode(nq, rk.lims.ptr, rk.sorted, rk.total, neg_zero, out);
 }
 
 }  // namespace vix

@@ -55,12 +55,43 @@ namespace vix {
 // What one range call reports for the [vix range] line of VIX_SCAN_DEBUG.
 struct RangeInfo { int passes = 0; int64_t total = 0, max_row = 0, sorted_long = 0; };
 
+// The grouped and sorted keys of one range call, before decoding (device buffers held by the caller): row q is
+// sorted[lims[q] .. lims[q + 1]), ascending.
+struct RangeKeys {
+    Scratch<int64_t> lims;                     // [nq + 1]
+    Scratch<u64> a, b;                         // sort buffers; `sorted` points into one of them
+    u64* sorted = nullptr;
+    int64_t total = 0;
+};
+
 // Runs `scan` (which appends into the RangeOut it is handed and fills the per-query counts) once, or twice when the first
-// capacity (cap_hint, updated for the next call) is too small, then groups, sorts and decodes the entries into a new result
-// object.  neg_zero: the path reports a zero distance as -0 (inner product through the flat engine and the IVF-PQ scan,
-// whose API distance is the negated score); the key keeps +0.  The only host synchronisation is the read of the total.
+// capacity (cap_hint, updated for the next call) is too small, then groups the entries by query and sorts each row.  The
+// only host synchronisation is the read of the total.
+int range_collect_keys(int64_t nq, float radius, size_t& cap_hint, const std::function<int(const RangeOut&)>& scan,
+                       RangeKeys& keys, RangeInfo* info);
+
+// sorted keys -> a new result object (lims copied from `lims`, device pointers).  neg_zero: the path reports a zero distance
+// as -0 (inner product through the flat engine and the IVF-PQ scan, whose API distance is the negated score); the key
+// keeps +0.
+int range_decode(int64_t nq, const int64_t* lims, const u64* sorted, int64_t total, bool neg_zero, vix_range_result** out);
+
+// range_collect_keys, then range_decode
 int range_collect(int64_t nq, float radius, size_t& cap_hint, bool neg_zero, const std::function<int(const RangeOut&)>& scan,
                   vix_range_result** out, RangeInfo* info);
+
+// the result object with its arrays allocated (freed again on failure), and its release
+int range_alloc(int64_t nq, int64_t total, vix_range_result** out);
+void range_free(vix_range_result* r);
+
+#ifdef __CUDACC__
+// one sorted key as the result reports it
+__device__ __forceinline__ void range_decode_key(u64 key, int neg_zero, float* dist, int64_t* id) {
+    float v = key_score(key, 0);
+    if (neg_zero && v == 0.0f) v = -0.0f;
+    *dist = v;
+    *id = (int64_t)key_id(key);
+}
+#endif
 
 // an empty result of nq rows (lims all 0)
 int range_empty(int64_t nq, vix_range_result** out);

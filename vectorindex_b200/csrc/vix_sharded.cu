@@ -20,6 +20,7 @@
 #include "vix_scan.cuh"
 #include "vix_topk.cuh"
 #include "vix_group.cuh"
+#include "vix_range.cuh"
 
 #include <dlfcn.h>
 #include <nccl.h>
@@ -115,6 +116,14 @@ struct vix_comm {
     // NCCL path: plain local buffers with the same roles
     void* gather_probes = nullptr; size_t gather_probes_bytes = 0;
     void* gather_keys = nullptr; size_t gather_keys_bytes = 0;
+    // range search: a second region, mapped like the first (peer memory only), grown collectively and geometrically:
+    //   [lims: world x (nq + 2) i64 -- each rank's local CSR row starts + its status][keys: the global answer's sorted keys,
+    //   rank by rank]
+    void* range_local = nullptr;
+    std::vector<void*> range_peer;
+    void** range_peer_dev = nullptr;
+    size_t range_off_keys = 0;
+    int64_t range_cap_nq = 0, range_cap_keys = 0;
     // optional phase events of the last search (vix_comm_trace): start | probes exchanged | scanned | merged
     bool trace = false;
     cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
@@ -363,6 +372,189 @@ __global__ void gather_rows_kernel(const int32_t* __restrict__ order, int64_t n,
     for (int j = 0; j < m; ++j) out_codes[i * (int64_t)m + j] = codes[r * (int64_t)m + j];
 }
 
+// ------------------------------------------------------------------------------------------------ sharded range search
+// n u64 words of src -> byte offset `off` of every rank's range region (this rank's included)
+__global__ void peer_store_kernel(const u64* __restrict__ src, int64_t n, void* const* __restrict__ peer_base, int world,
+                                  size_t off) {
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+        const u64 v = src[i];
+        for (int p = 0; p < world; ++p) reinterpret_cast<u64*>(static_cast<char*>(peer_base[p]) + off)[i] = v;
+    }
+}
+
+// lims_all: [world][nq + 2] every rank's local row starts (lims[nq] = its total) and its status.  glims[q] = the sum of the
+// ranks' row starts (q = 0 .. nq), the global row starts; meta = [base: world + 1 starts of the ranks' keys in the
+// concatenation][longest global row][status of every rank]
+__global__ void shard_range_lims_kernel(const int64_t* __restrict__ lims_all, int world, int64_t nq, int64_t* __restrict__ glims,
+                                        int64_t* __restrict__ meta) {
+    const int64_t L = nq + 2;
+    for (int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; q <= nq; q += (int64_t)gridDim.x * blockDim.x) {
+        int64_t g = 0, len = 0;
+        for (int r = 0; r < world; ++r) {
+            const int64_t* lr = lims_all + (size_t)r * L;
+            g += lr[q];
+            if (q < nq) len += lr[q + 1] - lr[q];
+        }
+        glims[q] = g;
+        if (q < nq && len > 0) atomicMax(reinterpret_cast<unsigned long long*>(meta + world + 1), (unsigned long long)len);
+    }
+    if (blockIdx.x == 0 && threadIdx.x == 0) {
+        int64_t acc = 0;
+        for (int r = 0; r < world; ++r) {
+            meta[r] = acc;
+            acc += lims_all[(size_t)r * L + nq];
+            meta[world + 2 + r] = lims_all[(size_t)r * L + nq + 1];
+        }
+        meta[world] = acc;
+    }
+}
+
+// The merge of the ranks' sorted runs into the global rows, decoded on the way (range_decode_key).  keys: every rank's local
+// answer, concatenated rank by rank (rank r's from base[r]); lims_all as above; glims: the global row starts.  Rank r's key
+// at place i of its row q goes to glims[q] + i + (keys of the lower ranks' rows q that are <= it) + (keys of the higher
+// ranks' rows q that are < it): one thread per key, a binary search in each other run.  Stable, and exact for equal keys
+// on different ranks (one id stored in lists two ranks own): they keep rank order, as one GPU's rows would hold them.
+__global__ void __launch_bounds__(256)
+shard_range_merge_kernel(const u64* __restrict__ keys, const int64_t* __restrict__ base, const int64_t* __restrict__ lims_all,
+                         int world, int64_t nq, const int64_t* __restrict__ glims, int64_t total, int neg_zero,
+                         float* __restrict__ out_dist, int64_t* __restrict__ out_ids) {
+    const int64_t L = nq + 2;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+        int ra = 0, rb = world;                               // rank of i: the last r with base[r] <= i
+        while (rb - ra > 1) { const int mid = (ra + rb) >> 1; if (base[mid] <= i) ra = mid; else rb = mid; }
+        const int r = ra;
+        const int64_t* lr = lims_all + (size_t)r * L;
+        const int64_t j = i - base[r];
+        int64_t qa = 0, qb = nq;                              // its row: the last q with lr[q] <= j
+        while (qb - qa > 1) { const int64_t mid = (qa + qb) >> 1; if (lr[mid] <= j) qa = mid; else qb = mid; }
+        const int64_t q = qa;
+        const u64 key = keys[i];
+        int64_t pos = glims[q] + (j - lr[q]);
+        for (int p = 0; p < world; ++p) {
+            if (p == r) continue;
+            const int64_t* lp = lims_all + (size_t)p * L;
+            const u64* run = keys + base[p] + lp[q];
+            int64_t x = 0, y = lp[q + 1] - lp[q];
+            if (p < r) {
+                while (x < y) { const int64_t mid = (x + y) >> 1; if (run[mid] <= key) x = mid + 1; else y = mid; }
+            } else {
+                while (x < y) { const int64_t mid = (x + y) >> 1; if (run[mid] < key) x = mid + 1; else y = mid; }
+            }
+            pos += x;
+        }
+        range_decode_key(key, neg_zero, out_dist + pos, out_ids + pos);
+    }
+}
+
+// lims_all [world][nq + 2] on the device -> glims [nq + 1] (device) and meta (host: base [world + 1], longest row, statuses
+// [world]).  Synchronises the stream: the size of the global answer.
+static int shard_range_lims(const int64_t* lims_all, int world, int64_t nq, int64_t* glims, std::vector<int64_t>& meta) {
+    cudaStream_t s = ctx().stream;
+    Scratch<int64_t> dmeta;
+    const size_t nm = 2 * (size_t)world + 2;
+    VIX_TRY(dmeta.alloc(nm));
+    VIX_CUDA(cudaMemsetAsync(dmeta.ptr, 0, nm * 8, s));
+    const int64_t want = (nq + 1 + 255) / 256;
+    const unsigned grid = (unsigned)(want < (int64_t)num_sms() * 4 ? want : (int64_t)num_sms() * 4);
+    shard_range_lims_kernel<<<grid, 256, 0, s>>>(lims_all, world, nq, glims, dmeta.ptr);
+    VIX_LAUNCH_CHECK();
+    meta.assign(nm, 0);
+    VIX_CUDA(cudaMemcpyAsync(meta.data(), dmeta.ptr, nm * 8, cudaMemcpyDeviceToHost, s));
+    VIX_CUDA(cudaStreamSynchronize(s));
+    return VIX_OK;
+}
+
+static int shard_range_merge(const u64* keys, const int64_t* base_dev, const int64_t* lims_all, int world, int64_t nq,
+                             const int64_t* glims, int64_t total, int metric, vix_range_result* r) {
+    cudaStream_t s = ctx().stream;
+    VIX_CUDA(cudaMemcpyAsync(r->lims, glims, (size_t)(nq + 1) * 8, cudaMemcpyDeviceToDevice, s));
+    if (total == 0) return VIX_OK;
+    const int64_t want = (total + 255) / 256;
+    const unsigned grid = (unsigned)(want < (int64_t)num_sms() * 8 ? want : (int64_t)num_sms() * 8);
+    shard_range_merge_kernel<<<grid, 256, 0, s>>>(keys, base_dev, lims_all, world, nq, glims, total,
+                                                  metric == VIX_METRIC_IP ? 1 : 0, r->dist, r->ids);
+    VIX_LAUNCH_CHECK();
+    return VIX_OK;
+}
+
+static void close_range_peers(vix_comm* c) {
+    for (int p = 0; p < (int)c->range_peer.size(); ++p)
+        if (p != c->rank && c->range_peer[p]) cudaIpcCloseMemHandle(c->range_peer[p]);
+    c->range_peer.clear();
+    if (c->range_local) cudaFree(c->range_local);
+    c->range_local = nullptr;
+    if (c->range_peer_dev) cudaFree(c->range_peer_dev);
+    c->range_peer_dev = nullptr;
+    c->range_cap_nq = c->range_cap_keys = 0;
+}
+
+// Collective (peer memory only): make every rank's range region hold nq rows of lims and `keys` keys, growing it
+// geometrically.  Every rank passes the same (nq, keys) -- the batch, and the global total all ranks computed -- so they
+// agree on whether to grow.  A rank that cannot allocate or map makes every rank return VIX_ERR_OOM with no region left.
+static int ensure_range_region(vix_comm* c, int64_t nq, int64_t keys, bool* grown) {
+    if (c->range_local && nq <= c->range_cap_nq && keys <= c->range_cap_keys) return VIX_OK;
+    cudaStream_t s = ctx().stream;
+    const int world = c->world;
+    int64_t cnq = c->range_cap_nq > 1024 ? c->range_cap_nq : 1024;
+    while (cnq < nq) cnq *= 2;
+    int64_t ck = c->range_cap_keys > 65536 ? c->range_cap_keys : 65536;
+    if (ck < keys) ck = keys + keys / 8 > 2 * ck ? keys + keys / 8 : 2 * ck;
+    const size_t off_k = ((size_t)world * (cnq + 2) * 8 + 255) & ~(size_t)255;
+    const size_t total = off_k + (size_t)ck * 8;
+    VIX_CUDA(cudaStreamSynchronize(s));                                   // nothing of mine still reads or writes the old one
+    void* fresh = nullptr;
+    int ok = 1;
+    cudaIpcMemHandle_t mine;
+    memset(&mine, 0, sizeof(mine));
+    if (cudaMalloc(&fresh, total) != cudaSuccess) { cudaGetLastError(); ok = 0; fresh = nullptr; }
+    if (ok && cudaIpcGetMemHandle(&mine, fresh) != cudaSuccess) { cudaGetLastError(); ok = 0; }
+    struct Msg { int ok; int pad; cudaIpcMemHandle_t h; };
+    Scratch<Msg> dmsg;
+    VIX_TRY(dmsg.alloc((size_t)world + 1));
+    Msg m;
+    memset(&m, 0, sizeof(m));
+    m.ok = ok; m.h = mine;
+    VIX_CUDA(cudaMemcpyAsync(dmsg.ptr + world, &m, sizeof(Msg), cudaMemcpyHostToDevice, s));
+    VIX_NCCL(g_nccl.AllGather(dmsg.ptr + world, dmsg.ptr, sizeof(Msg), ncclUint8, c->comm, s));
+    std::vector<Msg> all((size_t)world);
+    VIX_CUDA(cudaMemcpyAsync(all.data(), dmsg.ptr, sizeof(Msg) * world, cudaMemcpyDeviceToHost, s));
+    VIX_CUDA(cudaStreamSynchronize(s));
+    close_range_peers(c);                                                 // every rank has drained its stream
+    int all_ok = 1;
+    for (int p = 0; p < world; ++p) all_ok &= all[p].ok;
+    std::vector<void*> peer((size_t)world, nullptr);
+    for (int p = 0; p < world && all_ok; ++p) {
+        if (p == c->rank) { peer[p] = fresh; continue; }
+        if (cudaIpcOpenMemHandle(&peer[p], all[p].h, cudaIpcMemLazyEnablePeerAccess) != cudaSuccess) {
+            cudaGetLastError();
+            peer[p] = nullptr;
+            all_ok = 0;
+        }
+    }
+    void** pdev = nullptr;
+    if (all_ok && cudaMalloc(reinterpret_cast<void**>(&pdev), sizeof(void*) * world) != cudaSuccess) { cudaGetLastError(); all_ok = 0; }
+    Scratch<int> dflag;
+    VIX_TRY(dflag.alloc(1));
+    VIX_CUDA(cudaMemcpyAsync(dflag.ptr, &all_ok, 4, cudaMemcpyHostToDevice, s));
+    VIX_NCCL(g_nccl.AllReduce(dflag.ptr, dflag.ptr, 1, ncclInt32, ncclMin, c->comm, s));
+    VIX_CUDA(cudaMemcpyAsync(&all_ok, dflag.ptr, 4, cudaMemcpyDeviceToHost, s));
+    VIX_CUDA(cudaStreamSynchronize(s));
+    if (!all_ok) {
+        for (int p = 0; p < world; ++p)
+            if (p != c->rank && peer[p]) cudaIpcCloseMemHandle(peer[p]);
+        if (fresh) cudaFree(fresh);
+        if (pdev) cudaFree(pdev);
+        VIX_REQUIRE(false, VIX_ERR_OOM, "vix_sharded_range_search: a rank could not allocate or map a range region of %zu bytes "
+                    "(%lld rows, %lld keys)", total, (long long)cnq, (long long)ck);
+    }
+    VIX_CUDA(cudaMemcpyAsync(pdev, peer.data(), sizeof(void*) * world, cudaMemcpyHostToDevice, s));
+    VIX_CUDA(cudaStreamSynchronize(s));
+    c->range_local = fresh; c->range_peer = peer; c->range_peer_dev = pdev;
+    c->range_off_keys = off_k; c->range_cap_nq = cnq; c->range_cap_keys = ck;
+    *grown = true;
+    return VIX_OK;
+}
+
 }  // namespace vix
 
 extern "C" {
@@ -403,6 +595,7 @@ int vix_comm_destroy(vix_comm_t* c) {
     if (!c) return VIX_OK;
     cudaDeviceSynchronize();
     close_peers(c);
+    close_range_peers(c);
     if (c->gather_probes) cudaFree(c->gather_probes);
     if (c->gather_keys) cudaFree(c->gather_keys);
     for (auto& e : c->ev) if (e) cudaEventDestroy(e);
@@ -445,46 +638,31 @@ struct ThrHookScope {
     ~ThrHookScope() { set_scan_thr_hook(nullptr, nullptr); }
 };
 
-int vix_sharded_search(vix_index_t* h, vix_comm_t* c, const float* queries, int64_t nq, int k, int nprobe, float* out_dist,
-                       int64_t* out_ids) {
-    VIX_TRY(ensure_device());
-    VIX_REQUIRE(h && c, VIX_ERR_NULL_PTR, "vix_sharded_search: null handle");
-    if (nq <= 0 || k <= 0) return VIX_OK;                             // IVFIndex.swift:866 (every rank sees the same nq, k)
-    VIX_REQUIRE(queries && out_dist && out_ids, VIX_ERR_NULL_PTR, "vix_sharded_search: null pointer");
-    VIX_REQUIRE(k <= VIX_MAX_K, VIX_ERR_INVALID_K, "vix_sharded_search: k > %d", VIX_MAX_K);
-    std::lock_guard<std::mutex> lc(c->mu);
-    std::lock_guard<std::mutex> lk(h->mu);
-    VIX_REQUIRE(h->p.kind == VIX_INDEX_IVF_PQ && h->has_coarse && h->has_pq, VIX_ERR_NOT_TRAINED, "vix_sharded_search: needs a trained IVF-PQ index");
-    VIX_REQUIRE(h->p.metric != VIX_METRIC_COSINE, VIX_ERR_UNSUPPORTED, "vix_sharded_search: L2 / IP only");
-    if (nprobe <= 0) nprobe = h->p.nprobe;
-    VIX_REQUIRE(nprobe > 0 && nprobe <= VIX_MAX_K, VIX_ERR_INVALID_K, "vix_sharded_search: nprobe");
-    const int world = c->world, rank = c->rank, d = h->p.d;
-    if (world == 1) return index_search_locked(h, queries, nq, k, nprobe, out_dist, out_ids, nullptr, nullptr);
+}  // extern "C"
+
+namespace vix {
+
+// Steps 1-3 of a sharded call: this rank's block of the batch gets its probe lists against ALL centroids, and the block
+// (probes, plus the queries when they came from the host) reaches every rank -- stored into every peer's region with one
+// barrier, or an NCCL all-gather.  On return px.queries / px.probes are the whole batch's queries and probe lists on the
+// device.  The caller holds both mutexes and has called ensure_region.
+struct BatchProbes {
+    In<float> dq;
+    const float* queries = nullptr;
+    const int32_t* probes = nullptr;
+};
+
+static int exchange_probes(vix_index* h, vix_comm* c, const float* queries, int64_t nq, int nprobe, BatchProbes& px) {
     cudaStream_t s = ctx().stream;
-    if (h->dirty) VIX_TRY(build_lists(h));
-    VIX_TRY(ensure_region(c, nq, d, nprobe, k));
-    ThrHookScope thr_scope(c);                                        // (cleared again on every way out)
+    const int world = c->world, rank = c->rank, d = h->p.d;
     const bool host_q = !is_device_ptr(queries);
     const int64_t per = block_rows(nq, world);
     const int64_t lo = nq < (int64_t)rank * per ? nq : (int64_t)rank * per;
     const int64_t cnt = (nq < lo + per ? nq : lo + per) - lo;
-    const int64_t total = nq * (int64_t)k;
-    Out<float> dd;
-    Out<int64_t> di;
-    VIX_TRY(dd.stage(out_dist, (size_t)total));
-    VIX_TRY(di.stage(out_ids, (size_t)total));
-    Scratch<float> ldist;
-    Scratch<int64_t> lids;
-    VIX_TRY(ldist.alloc((size_t)total));
-    VIX_TRY(lids.alloc((size_t)total));
-    auto mark = [&](int i) { if (c->trace) cudaEventRecord(c->ev[i], s); };
-    mark(0);
-
     if (c->peer_state == 1) {
         char* base = static_cast<char*>(c->local);
         float* qbuf = reinterpret_cast<float*>(base + c->off_queries);          // [world * per][d] (this call's per)
         int32_t* pbuf = reinterpret_cast<int32_t*>(base + c->off_probes);       // [world * per][nprobe]
-        u64* rbuf = reinterpret_cast<u64*>(base + c->off_results);              // [world][nq][k]
         // 1. this rank's block of the batch: host queries cross PCIe once per rank, 1/world of the batch each
         const float* qblock = queries + (size_t)lo * d;
         if (host_q && cnt > 0) {
@@ -498,52 +676,97 @@ int vix_sharded_search(vix_index_t* h, vix_comm_t* c, const float* queries, int6
                                              pblock, nullptr, h->coarse_norm_max.ptr));
         if (cnt < per) VIX_TRY(fill<int32_t>(pblock + (size_t)cnt * nprobe, (per - cnt) * nprobe, -1));
         // 3. the block travels to every peer (probes, and the queries when they came from the host), one barrier
-        {
-            const size_t offA = c->off_probes + (size_t)rank * per * nprobe * 4, nA = (size_t)per * nprobe * 4 / 16;
-            const size_t offB = c->off_queries + (size_t)rank * per * d * 4, nB = host_q ? (size_t)per * d * 4 / 16 : 0;
-            const size_t n16 = nA + nB;
-            const size_t want = (n16 + 255) / 256;
-            const unsigned grid = (unsigned)(want < (size_t)(2 * num_sms()) ? (want ? want : 1) : (size_t)(2 * num_sms()));
-            peer_push_kernel<<<grid, 256, 0, s>>>(c->peer_dev, world, rank, offA, nA, offB, nB);
-            VIX_LAUNCH_CHECK();
-            VIX_TRY(peer_barrier(c));
-        }
-        mark(1);
-        // 4. fused scan over the probed lists this rank owns
-        const float* qall = host_q ? qbuf : queries;
-        VIX_TRY(index_search_locked(h, qall, nq, k, nprobe, ldist.ptr, lids.ptr, nullptr, nullptr, pbuf));
-        mark(2);
-        // 5. its top-k leaves as packed keys for slot `rank` of every rank's result buffer; barrier; merge
+        const size_t offA = c->off_probes + (size_t)rank * per * nprobe * 4, nA = (size_t)per * nprobe * 4 / 16;
+        const size_t offB = c->off_queries + (size_t)rank * per * d * 4, nB = host_q ? (size_t)per * d * 4 / 16 : 0;
+        const size_t n16 = nA + nB;
+        const size_t want = (n16 + 255) / 256;
+        const unsigned grid = (unsigned)(want < (size_t)(2 * num_sms()) ? (want ? want : 1) : (size_t)(2 * num_sms()));
+        peer_push_kernel<<<grid, 256, 0, s>>>(c->peer_dev, world, rank, offA, nA, offB, nB);
+        VIX_LAUNCH_CHECK();
+        VIX_TRY(peer_barrier(c));
+        px.queries = host_q ? qbuf : queries;
+        px.probes = pbuf;
+        return VIX_OK;
+    }
+    // NCCL carries the exchange
+    VIX_TRY(px.dq.stage(queries, (size_t)nq * d));
+    const size_t pbytes = (size_t)world * per * nprobe * 4;
+    if (pbytes > c->gather_probes_bytes) {
+        if (c->gather_probes) { VIX_CUDA(cudaStreamSynchronize(s)); cudaFree(c->gather_probes); c->gather_probes = nullptr; }
+        VIX_CUDA(cudaMalloc(&c->gather_probes, pbytes));
+        c->gather_probes_bytes = pbytes;
+    }
+    int32_t* pall = static_cast<int32_t*>(c->gather_probes);
+    int32_t* pblock = pall + (size_t)rank * per * nprobe;
+    if (cnt > 0)
+        VIX_TRY(probe_select_fast_device(px.dq.dev + (size_t)lo * d, cnt, h->coarse.ptr, h->kc, d, h->p.metric, nprobe,
+                                         h->coarse_norms.ptr, pblock, nullptr, h->coarse_norm_max.ptr));
+    if (cnt < per) VIX_TRY(fill<int32_t>(pblock + (size_t)cnt * nprobe, (per - cnt) * nprobe, -1));
+    VIX_NCCL(g_nccl.AllGather(pblock, pall, (size_t)per * nprobe, ncclInt32, c->comm, s));   // in place
+    px.queries = px.dq.dev;
+    px.probes = pall;
+    return VIX_OK;
+}
+
+// filter arguments of the C ABI -> FilterArgs over a staged copy of the words (f == nullptr when there is no filter)
+static int stage_filter(const uint64_t* words, int64_t capacity, int mode, In<uint64_t>& staged, FilterArgs& f,
+                        const FilterArgs*& fp) {
+    fp = nullptr;
+    if (!words) return VIX_OK;
+    VIX_TRY(staged.stage(words, (size_t)((capacity + 63) / 64)));
+    f.words = staged.dev; f.cap = capacity; f.deny = mode == VIX_FILTER_DENY;
+    fp = &f;
+    return VIX_OK;
+}
+
+// vix_sharded_search and vix_sharded_search_filtered (filter == nullptr: the unfiltered step, launch for launch)
+static int sharded_search(vix_index* h, vix_comm* c, const float* queries, int64_t nq, int k, int nprobe, const FilterArgs* filter,
+                          float* out_dist, int64_t* out_ids) {
+    std::lock_guard<std::mutex> lc(c->mu);
+    std::lock_guard<std::mutex> lk(h->mu);
+    VIX_REQUIRE(h->p.kind == VIX_INDEX_IVF_PQ && h->has_coarse && h->has_pq, VIX_ERR_NOT_TRAINED, "vix_sharded_search: needs a trained IVF-PQ index");
+    VIX_REQUIRE(h->p.metric != VIX_METRIC_COSINE, VIX_ERR_UNSUPPORTED, "vix_sharded_search: L2 / IP only");
+    if (nprobe <= 0) nprobe = h->p.nprobe;
+    VIX_REQUIRE(nprobe > 0 && nprobe <= VIX_MAX_K, VIX_ERR_INVALID_K, "vix_sharded_search: nprobe");
+    const int world = c->world, rank = c->rank, d = h->p.d;
+    if (world == 1) return index_search_locked(h, queries, nq, k, nprobe, out_dist, out_ids, nullptr, nullptr, nullptr, filter);
+    cudaStream_t s = ctx().stream;
+    if (h->dirty) VIX_TRY(build_lists(h));
+    VIX_TRY(ensure_region(c, nq, d, nprobe, k));
+    ThrHookScope thr_scope(c);                                        // (cleared again on every way out)
+    const int64_t total = nq * (int64_t)k;
+    Out<float> dd;
+    Out<int64_t> di;
+    VIX_TRY(dd.stage(out_dist, (size_t)total));
+    VIX_TRY(di.stage(out_ids, (size_t)total));
+    Scratch<float> ldist;
+    Scratch<int64_t> lids;
+    VIX_TRY(ldist.alloc((size_t)total));
+    VIX_TRY(lids.alloc((size_t)total));
+    auto mark = [&](int i) { if (c->trace) cudaEventRecord(c->ev[i], s); };
+    mark(0);
+    // 1-3. probes of this rank's block, exchanged
+    BatchProbes px;
+    VIX_TRY(exchange_probes(h, c, queries, nq, nprobe, px));
+    mark(1);
+    // 4. fused scan over the probed lists this rank owns (a filter sends it down the query-major path)
+    VIX_TRY(index_search_locked(h, px.queries, nq, k, nprobe, ldist.ptr, lids.ptr, nullptr, nullptr, px.probes, filter));
+    mark(2);
+    // 5. its top-k leaves as packed keys for slot `rank` of every rank's result buffer; barrier (or all-gather); merge
+    if (c->peer_state == 1) {
+        u64* rbuf = reinterpret_cast<u64*>(static_cast<char*>(c->local) + c->off_results);   // [world][nq][k]
         pack_result_keys_kernel<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(ldist.ptr, lids.ptr, total, c->peer_dev, world,
                                                                               c->off_results + (size_t)rank * total * 8, nullptr);
         VIX_LAUNCH_CHECK();
         VIX_TRY(peer_barrier(c));
         VIX_TRY(merge_shard_keys(rbuf, world, nq, k, h->p.metric, dd.dev, di.dev));
     } else {
-        // NCCL carries the two exchanges
-        In<float> dq;
-        VIX_TRY(dq.stage(queries, (size_t)nq * d));
-        const size_t pbytes = (size_t)world * per * nprobe * 4, kbytes = (size_t)world * total * 8;
-        if (pbytes > c->gather_probes_bytes) {
-            if (c->gather_probes) { VIX_CUDA(cudaStreamSynchronize(s)); cudaFree(c->gather_probes); c->gather_probes = nullptr; }
-            VIX_CUDA(cudaMalloc(&c->gather_probes, pbytes));
-            c->gather_probes_bytes = pbytes;
-        }
+        const size_t kbytes = (size_t)world * total * 8;
         if (kbytes > c->gather_keys_bytes) {
             if (c->gather_keys) { VIX_CUDA(cudaStreamSynchronize(s)); cudaFree(c->gather_keys); c->gather_keys = nullptr; }
             VIX_CUDA(cudaMalloc(&c->gather_keys, kbytes));
             c->gather_keys_bytes = kbytes;
         }
-        int32_t* pall = static_cast<int32_t*>(c->gather_probes);
-        int32_t* pblock = pall + (size_t)rank * per * nprobe;
-        if (cnt > 0)
-            VIX_TRY(probe_select_fast_device(dq.dev + (size_t)lo * d, cnt, h->coarse.ptr, h->kc, d, h->p.metric, nprobe,
-                                             h->coarse_norms.ptr, pblock, nullptr, h->coarse_norm_max.ptr));
-        if (cnt < per) VIX_TRY(fill<int32_t>(pblock + (size_t)cnt * nprobe, (per - cnt) * nprobe, -1));
-        VIX_NCCL(g_nccl.AllGather(pblock, pall, (size_t)per * nprobe, ncclInt32, c->comm, s));   // in place
-        mark(1);
-        VIX_TRY(index_search_locked(h, dq.dev, nq, k, nprobe, ldist.ptr, lids.ptr, nullptr, nullptr, pall));
-        mark(2);
         u64* kall = static_cast<u64*>(c->gather_keys);
         pack_result_keys_kernel<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(ldist.ptr, lids.ptr, total, nullptr, world, 0,
                                                                               kall + (size_t)rank * total);
@@ -555,6 +778,186 @@ int vix_sharded_search(vix_index_t* h, vix_comm_t* c, const float* queries, int6
     VIX_TRY(dd.commit());
     VIX_TRY(di.commit());
     return finish(dd.is_host() || di.is_host());
+}
+
+// The range step after the probe exchange: the local scan's sorted keys and lims (rc: its status) -> every rank's lims and
+// status (peer region + barrier, or all-gather) -> global row starts and total (synchronises) -> the keys of every rank
+// (peer region + barrier, or grouped send / receive) -> merge and decode into a new result object.
+static int sharded_range_exchange(vix_index* h, vix_comm* c, int64_t nq, int rc, RangeKeys& rk, bool grown,
+                                  vix_range_result** out) {
+    cudaStream_t s = ctx().stream;
+    const int world = c->world, rank = c->rank;
+    const int64_t L = nq + 2;
+    const bool peer = c->peer_state == 1;
+    Scratch<int64_t> mine, lims_all, glims, dbase;
+    VIX_TRY(mine.alloc((size_t)L));
+    VIX_TRY(lims_all.alloc((size_t)world * L));
+    VIX_TRY(glims.alloc((size_t)nq + 1));
+    VIX_TRY(dbase.alloc((size_t)world + 1));
+    // this rank's lims and status (a rank whose local pass failed sends empty rows and its code)
+    const int64_t status = rc;
+    if (rc == VIX_OK) VIX_CUDA(cudaMemcpyAsync(mine.ptr, rk.lims.ptr, (size_t)(nq + 1) * 8, cudaMemcpyDeviceToDevice, s));
+    else VIX_CUDA(cudaMemsetAsync(mine.ptr, 0, (size_t)(nq + 1) * 8, s));
+    VIX_CUDA(cudaMemcpyAsync(mine.ptr + nq + 1, &status, 8, cudaMemcpyHostToDevice, s));
+    if (peer) {
+        const int64_t want = (L + 255) / 256;
+        peer_store_kernel<<<(unsigned)(want < 64 ? want : 64), 256, 0, s>>>(reinterpret_cast<const u64*>(mine.ptr), L,
+                                                                           c->range_peer_dev, world, (size_t)rank * L * 8);
+        VIX_LAUNCH_CHECK();
+        VIX_TRY(peer_barrier(c));
+        VIX_CUDA(cudaMemcpyAsync(lims_all.ptr, c->range_local, (size_t)world * L * 8, cudaMemcpyDeviceToDevice, s));
+    } else {
+        VIX_NCCL(g_nccl.AllGather(mine.ptr, lims_all.ptr, (size_t)L, ncclInt64, c->comm, s));
+    }
+    std::vector<int64_t> meta;
+    VIX_TRY(shard_range_lims(lims_all.ptr, world, nq, glims.ptr, meta));    // the second synchronisation: the global total
+    if (rc != VIX_OK) return rc;                                          // (its own message stands)
+    for (int p = 0; p < world; ++p)
+        VIX_REQUIRE(meta[world + 2 + p] == VIX_OK, (int)meta[world + 2 + p], "vix_sharded_range_search: rank %d failed its local "
+                    "scan (status %lld); no rank returns a result", p, (long long)meta[world + 2 + p]);
+    const int64_t total = meta[world], max_row = meta[world + 1];
+    // room for the answer on every rank, decided together
+    if (peer) VIX_TRY(ensure_range_region(c, nq, total, &grown));
+    vix_range_result* r = nullptr;
+    Scratch<u64> kall;
+    int ok = range_alloc(nq, total, &r) == VIX_OK;
+    if (ok && !peer && kall.alloc((size_t)total) != VIX_OK) ok = 0;
+    {
+        Scratch<int> dflag;
+        int rc2 = dflag.alloc(1);
+        if (rc2 == VIX_OK) rc2 = cudaMemcpyAsync(dflag.ptr, &ok, 4, cudaMemcpyHostToDevice, s) == cudaSuccess ? VIX_OK : VIX_ERR_CUDA;
+        if (rc2 == VIX_OK) rc2 = g_nccl.AllReduce(dflag.ptr, dflag.ptr, 1, ncclInt32, ncclMin, c->comm, s) == ncclSuccess ? VIX_OK : VIX_ERR_CUDA;
+        if (rc2 == VIX_OK) rc2 = cudaMemcpyAsync(&ok, dflag.ptr, 4, cudaMemcpyDeviceToHost, s) == cudaSuccess ? VIX_OK : VIX_ERR_CUDA;
+        if (rc2 == VIX_OK) rc2 = cudaStreamSynchronize(s) == cudaSuccess ? VIX_OK : VIX_ERR_CUDA;
+        if (rc2 != VIX_OK || !ok) {
+            range_free(r);
+            VIX_REQUIRE(rc2 == VIX_OK, rc2, "vix_sharded_range_search: the allocation verdict failed");
+            VIX_REQUIRE(false, VIX_ERR_OOM, "vix_sharded_range_search: %lld results (%lld bytes) do not fit in device memory on "
+                        "every rank", (long long)total, (long long)total * 12);
+        }
+    }
+    auto fail = [&](int e) { range_free(r); return e; };
+    const int64_t mine_n = meta[rank + 1] - meta[rank];
+    const u64* keys = nullptr;
+    if (cudaMemcpyAsync(dbase.ptr, meta.data(), ((size_t)world + 1) * 8, cudaMemcpyHostToDevice, s) != cudaSuccess)
+        return fail(cuda_fail(cudaGetLastError(), "range base copy", __FILE__, __LINE__));
+    if (peer) {
+        // every store into a peer's region is behind this call's probe barrier, which the peer entered after its previous
+        // merge had read the region
+        if (mine_n > 0) {
+            const int64_t want = (mine_n + 255) / 256;
+            peer_store_kernel<<<(unsigned)(want < (int64_t)num_sms() * 4 ? want : (int64_t)num_sms() * 4), 256, 0, s>>>(
+                rk.sorted, mine_n, c->range_peer_dev, world, c->range_off_keys + (size_t)meta[rank] * 8);
+            ctx().launches += 1;
+        }
+        const int b = peer_barrier(c);
+        if (b != VIX_OK) return fail(b);
+        keys = reinterpret_cast<const u64*>(static_cast<char*>(c->range_local) + c->range_off_keys);
+    } else {
+        if (mine_n > 0 && cudaMemcpyAsync(kall.ptr + meta[rank], rk.sorted, (size_t)mine_n * 8, cudaMemcpyDeviceToDevice, s) != cudaSuccess)
+            return fail(cuda_fail(cudaGetLastError(), "range keys copy", __FILE__, __LINE__));
+        ncclResult_t nr = g_nccl.GroupStart();
+        for (int p = 0; p < world && nr == ncclSuccess; ++p) {
+            if (p == rank) continue;
+            const int64_t np_ = meta[p + 1] - meta[p];
+            if (mine_n > 0) nr = g_nccl.Send(rk.sorted, (size_t)mine_n, ncclUint64, p, c->comm, s);
+            if (nr == ncclSuccess && np_ > 0) nr = g_nccl.Recv(kall.ptr + meta[p], (size_t)np_, ncclUint64, p, c->comm, s);
+        }
+        const ncclResult_t ne = g_nccl.GroupEnd();
+        if (nr == ncclSuccess) nr = ne;
+        if (nr != ncclSuccess) {
+            set_error("NCCL error %d (%s): range keys exchange", (int)nr, g_nccl.GetErrorString(nr));
+            return fail(VIX_ERR_CUDA);
+        }
+        keys = kall.ptr;
+    }
+    const int mr = shard_range_merge(keys, dbase.ptr, lims_all.ptr, world, nq, glims.ptr, total, h->p.metric, r);
+    if (mr != VIX_OK) return fail(mr);
+    if (getenv("VIX_SCAN_DEBUG"))
+        fprintf(stderr, "[vix sharded range] world %d, peer %d, local %lld, total %lld, max_row %lld, grown %d\n", world,
+                peer ? 1 : 0, (long long)mine_n, (long long)total, (long long)max_row, grown ? 1 : 0);
+    *out = r;
+    return VIX_OK;
+}
+
+}  // namespace vix
+
+extern "C" {
+
+int vix_sharded_search(vix_index_t* h, vix_comm_t* c, const float* queries, int64_t nq, int k, int nprobe, float* out_dist,
+                       int64_t* out_ids) {
+    VIX_TRY(ensure_device());
+    VIX_REQUIRE(h && c, VIX_ERR_NULL_PTR, "vix_sharded_search: null handle");
+    if (nq <= 0 || k <= 0) return VIX_OK;                             // IVFIndex.swift:866 (every rank sees the same nq, k)
+    VIX_REQUIRE(queries && out_dist && out_ids, VIX_ERR_NULL_PTR, "vix_sharded_search: null pointer");
+    VIX_REQUIRE(k <= VIX_MAX_K, VIX_ERR_INVALID_K, "vix_sharded_search: k > %d", VIX_MAX_K);
+    return sharded_search(h, c, queries, nq, k, nprobe, nullptr, out_dist, out_ids);
+}
+
+int vix_sharded_search_filtered(vix_index_t* h, vix_comm_t* c, const float* queries, int64_t nq, int k, int nprobe,
+                                const uint64_t* filter_words, int64_t filter_capacity, int filter_mode, float* out_dist,
+                                int64_t* out_ids) {
+    VIX_TRY(ensure_device());
+    VIX_REQUIRE(h && c, VIX_ERR_NULL_PTR, "vix_sharded_search_filtered: null handle");
+    VIX_REQUIRE(filter_mode == VIX_FILTER_ALLOW || filter_mode == VIX_FILTER_DENY, VIX_ERR_INVALID_PARAM,
+                "vix_sharded_search_filtered: filter_mode must be VIX_FILTER_ALLOW or VIX_FILTER_DENY");
+    VIX_REQUIRE(filter_capacity >= 0, VIX_ERR_INVALID_PARAM, "vix_sharded_search_filtered: negative capacity");
+    if (nq <= 0 || k <= 0) return VIX_OK;
+    VIX_REQUIRE(queries && out_dist && out_ids, VIX_ERR_NULL_PTR, "vix_sharded_search_filtered: null pointer");
+    VIX_REQUIRE(k <= VIX_MAX_K, VIX_ERR_INVALID_K, "vix_sharded_search_filtered: k > %d", VIX_MAX_K);
+    In<uint64_t> fw;
+    FilterArgs f;
+    const FilterArgs* fp = nullptr;
+    VIX_TRY(stage_filter(filter_words, filter_capacity, filter_mode, fw, f, fp));
+    return sharded_search(h, c, queries, nq, k, nprobe, fp, out_dist, out_ids);
+}
+
+int vix_sharded_range_search(vix_index_t* h, vix_comm_t* c, const float* queries, int64_t nq, float radius, int nprobe,
+                             const uint64_t* filter_words, int64_t filter_capacity, int filter_mode, vix_range_result_t** out) {
+    VIX_TRY(ensure_device());
+    VIX_REQUIRE(h && c && out, VIX_ERR_NULL_PTR, "vix_sharded_range_search: null pointer");
+    *out = nullptr;
+    VIX_REQUIRE(queries || nq == 0, VIX_ERR_NULL_PTR, "vix_sharded_range_search: null queries");
+    VIX_REQUIRE(nq >= 0 && nq < 0x7FFFFFFFLL, VIX_ERR_INVALID_PARAM, "vix_sharded_range_search: nq must lie in [0, 2^31 - 1)");
+    VIX_REQUIRE(radius == radius, VIX_ERR_INVALID_PARAM, "vix_sharded_range_search: radius is NaN");
+    VIX_REQUIRE(filter_mode == VIX_FILTER_ALLOW || filter_mode == VIX_FILTER_DENY, VIX_ERR_INVALID_PARAM,
+                "vix_sharded_range_search: filter_mode must be VIX_FILTER_ALLOW or VIX_FILTER_DENY");
+    VIX_REQUIRE(filter_capacity >= 0, VIX_ERR_INVALID_PARAM, "vix_sharded_range_search: negative capacity");
+    std::lock_guard<std::mutex> lc(c->mu);
+    std::lock_guard<std::mutex> lk(h->mu);
+    VIX_REQUIRE(h->p.kind == VIX_INDEX_IVF_PQ && h->has_coarse && h->has_pq, VIX_ERR_NOT_TRAINED,
+                "vix_sharded_range_search: needs a trained IVF-PQ index");
+    VIX_REQUIRE(h->p.metric != VIX_METRIC_COSINE, VIX_ERR_UNSUPPORTED, "vix_sharded_range_search: L2 / IP only");
+    if (nprobe <= 0) nprobe = h->p.nprobe;
+    VIX_REQUIRE(nprobe > 0 && nprobe <= VIX_MAX_K, VIX_ERR_INVALID_K, "vix_sharded_range_search: nprobe = %d (1 .. %d)", nprobe,
+                VIX_MAX_K);
+    if (nq == 0) return range_empty(0, out);                          // (every rank sees the same nq: no exchange)
+    In<uint64_t> fw;
+    FilterArgs f;
+    const FilterArgs* fp = nullptr;
+    VIX_TRY(stage_filter(filter_words, filter_capacity, filter_mode, fw, f, fp));
+    const int world = c->world;
+    if (world == 1) return index_range_locked(h, queries, nq, radius, nprobe, fp, out);
+    cudaStream_t s = ctx().stream;
+    if (h->dirty) VIX_TRY(build_lists(h));
+    VIX_TRY(ensure_region(c, nq, h->p.d, nprobe, 1));
+    bool grown = false;
+    if (c->peer_state == 1) VIX_TRY(ensure_range_region(c, nq, 0, &grown));
+    auto mark = [&](int i) { if (c->trace) cudaEventRecord(c->ev[i], s); };
+    mark(0);
+    BatchProbes px;
+    VIX_TRY(exchange_probes(h, c, queries, nq, nprobe, px));
+    mark(1);
+    // the local scan and sort (its one synchronisation: the local total); a failure here travels with the lims, so that
+    // every rank returns it together
+    RangeKeys rk;
+    const int rc = index_range_locked(h, px.queries, nq, radius, nprobe, fp, nullptr, px.probes, &rk);
+    mark(2);
+    vix_range_result* r = nullptr;
+    VIX_TRY(sharded_range_exchange(h, c, nq, rc, rk, grown, &r));
+    mark(3);
+    *out = r;
+    return VIX_OK;
 }
 
 int vix_debug_shard_merge(const float* dist_all, const int64_t* ids_all, int world, int64_t nq, int k, int metric,
@@ -582,6 +985,58 @@ int vix_debug_shard_merge(const float* dist_all, const int64_t* ids_all, int wor
     VIX_TRY(od.commit());
     VIX_TRY(oi.commit());
     return finish(od.is_host() || oi.is_host());
+}
+
+int vix_debug_shard_range_merge(const int64_t* lims_all, const float* dist_all, const int64_t* ids_all, int world, int64_t nq,
+                                int metric, vix_range_result_t** out) {
+    VIX_TRY(ensure_device());
+    VIX_REQUIRE(lims_all && out, VIX_ERR_NULL_PTR, "vix_debug_shard_range_merge: null pointer");
+    *out = nullptr;
+    VIX_REQUIRE(world > 0 && world <= 256 && nq >= 0 && nq < 0x7FFFFFFFLL, VIX_ERR_INVALID_PARAM,
+                "vix_debug_shard_range_merge: world / nq");
+    cudaStream_t s = ctx().stream;
+    const int64_t L = nq + 2;
+    // the ranks' lims [world][nq + 1] -> the exchanged layout [world][nq + 2] (status 0)
+    std::vector<int64_t> h_lims((size_t)world * (nq + 1));
+    VIX_CUDA(cudaMemcpyAsync(h_lims.data(), lims_all, h_lims.size() * 8, cudaMemcpyDefault, s));
+    VIX_CUDA(cudaStreamSynchronize(s));
+    std::vector<int64_t> h_all((size_t)world * L, 0);
+    int64_t total = 0;
+    for (int r = 0; r < world; ++r) {
+        const int64_t* lr = h_lims.data() + (size_t)r * (nq + 1);
+        VIX_REQUIRE(lr[0] == 0, VIX_ERR_INVALID_PARAM, "vix_debug_shard_range_merge: rank %d: lims[0] != 0", r);
+        for (int64_t q = 0; q < nq; ++q)
+            VIX_REQUIRE(lr[q + 1] >= lr[q], VIX_ERR_INVALID_PARAM, "vix_debug_shard_range_merge: rank %d: lims descend", r);
+        for (int64_t q = 0; q <= nq; ++q) h_all[(size_t)r * L + q] = lr[q];
+        total += lr[nq];
+    }
+    VIX_REQUIRE(total == 0 || (dist_all && ids_all), VIX_ERR_NULL_PTR, "vix_debug_shard_range_merge: null rows");
+    Scratch<int64_t> dlims, glims, dbase;
+    VIX_TRY(dlims.alloc(h_all.size()));
+    VIX_TRY(glims.alloc((size_t)nq + 1));
+    VIX_TRY(dbase.alloc((size_t)world + 1));
+    VIX_CUDA(cudaMemcpyAsync(dlims.ptr, h_all.data(), h_all.size() * 8, cudaMemcpyHostToDevice, s));
+    In<float> dd;
+    In<int64_t> di;
+    VIX_TRY(dd.stage(dist_all, (size_t)total));
+    VIX_TRY(di.stage(ids_all, (size_t)total));
+    Scratch<u64> keys;
+    VIX_TRY(keys.alloc((size_t)total));
+    if (total > 0) {
+        pack_result_keys_kernel<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(dd.dev, di.dev, total, nullptr, world, 0, keys.ptr);
+        VIX_LAUNCH_CHECK();
+    }
+    std::vector<int64_t> meta;
+    VIX_TRY(shard_range_lims(dlims.ptr, world, nq, glims.ptr, meta));
+    VIX_CUDA(cudaMemcpyAsync(dbase.ptr, meta.data(), ((size_t)world + 1) * 8, cudaMemcpyHostToDevice, s));
+    vix_range_result* r = nullptr;
+    VIX_TRY(range_alloc(nq, total, &r));
+    const int rc = shard_range_merge(keys.ptr, dbase.ptr, dlims.ptr, world, nq, glims.ptr, total, metric, r);
+    if (rc != VIX_OK) { range_free(r); return rc; }
+    const cudaError_t e = cudaStreamSynchronize(s);                   // (meta, a host vector, is read by the copy above)
+    if (e != cudaSuccess) { range_free(r); VIX_CUDA(e); }
+    *out = r;
+    return VIX_OK;
 }
 
 int vix_comm_trace(vix_comm_t* c, int enabled) {

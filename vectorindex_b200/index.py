@@ -700,11 +700,14 @@ class ShardedIVFPQIndex:
                 buf[:cnt] = ids
         return self._all_gather(buf).view(self.world * per, nprobe)[:nq].contiguous()
 
-    def batch_search(self, queries, k, nprobe=0, out=None):
+    def batch_search(self, queries, k, nprobe=0, out=None, filter=None):
         """Replicated queries in, merged [nq x k] (distances, ids) out on every rank.  Host (numpy) queries are
         staged to the device once and only the merged result returns to the host.  ``out``: optional (distances f32,
-        ids int64) host arrays the result is written into (pinned ones make the copy back asynchronous)."""
+        ids int64) host arrays the result is written into (pinned ones make the copy back asynchronous).  ``filter``: an
+        :class:`IDFilter` (the same on every rank), applied before selection as in ``IVFPQIndex.batch_search``."""
         import torch
+        if filter is not None:
+            return self._filtered_search(queries, k, nprobe, filter, out)
         was_numpy = not _lib._is_torch(queries)
         if int(queries.shape[0]) == 0 or int(k) <= 0:                          # IVFIndex.swift:866: nothing to do
             kk = max(int(k), 0)
@@ -751,6 +754,61 @@ class ShardedIVFPQIndex:
         if was_numpy and _lib._is_torch(md):
             md, mi = md.cpu().numpy(), mi.cpu().numpy()
         return md, mi
+
+    def _filtered_search(self, queries, k, nprobe, filter, out):
+        """batch_search with an id filter: vix_sharded_search_filtered (one rank: the local index's filtered search)"""
+        nprobe = nprobe if nprobe > 0 else self.nprobe
+        comm = self._native()
+        if comm is None:
+            if self.world == 1 and hasattr(self.local, "_h"):
+                return self.local.batch_search(queries, k, nprobe=nprobe, filter=filter, out=out)
+            raise NotImplementedError("a filtered sharded search needs the library's exchange (NCCL ranks over IVFPQIndex "
+                                      "shards); the Python exchange path does not filter")
+        q = as_input(queries, np.float32)
+        nq, kk = int(q.shape[0]), max(int(k), 0)
+        if out is not None:
+            dist, ids = out
+        else:
+            dist, ids = empty_like_input(q, (nq, kk), np.float32), empty_like_input(q, (nq, kk), np.int64)
+        if nq == 0 or kk == 0:
+            return dist, ids
+        check(lib().vix_sharded_search_filtered(self.local._h, comm._c, ptr(q, np.float32), C.c_int64(nq), C.c_int(k),
+                                                C.c_int(nprobe), ptr(filter.words, np.uint64), C.c_int64(filter.capacity),
+                                                C.c_int(filter.mode), ptr(dist, np.float32), ptr(ids, np.int64)))
+        return dist, ids
+
+    def range_search(self, queries, radius: float, nprobe: int = 0, filter=None):
+        """Every stored vector within ``radius`` of each query, over all ranks' lists: ``IVFPQIndex.range_search`` on one
+        GPU holding every row (vix_sharded_range_search: the probes of the whole batch, each rank's range scan of the lists
+        it owns, the sorted rows exchanged and merged on the device).  Collective: every rank passes the same queries,
+        radius, nprobe and ``filter`` (an :class:`IDFilter`) and receives the whole CSR ``(lims int64 [nq + 1], distances
+        f32 [total], ids int64 [total])``: numpy for host queries, torch tensors on the queries' device for CUDA tensors."""
+        nprobe = nprobe if nprobe > 0 else self.nprobe
+        comm = self._native()
+        if comm is None:
+            if self.world == 1 and hasattr(self.local, "range_search"):
+                return self.local.range_search(queries, radius, nprobe=nprobe, filter=filter)
+            raise NotImplementedError("a sharded range search needs the library's exchange (NCCL ranks over IVFPQIndex "
+                                      "shards); the Python exchange path has none")
+        q = as_input(queries, np.float32)
+        self.local._check_dim(q, "range_search")
+        nq = int(q.shape[0])
+        res = C.c_void_p(0)
+        try:
+            words = filter.words if filter is not None else None
+            check(lib().vix_sharded_range_search(self.local._h, comm._c, ptr(q, np.float32), C.c_int64(nq),
+                                                 C.c_float(float(radius)), C.c_int(nprobe), ptr(words, np.uint64),
+                                                 C.c_int64(filter.capacity if filter is not None else 0),
+                                                 C.c_int(filter.mode if filter is not None else 0), C.byref(res)))
+            total = int(lib().vix_range_result_total(res))
+            lims = empty_like_input(q, (nq + 1,), np.int64)
+            dist = empty_like_input(q, (total,), np.float32)
+            ids = empty_like_input(q, (total,), np.int64)
+            check(lib().vix_range_result_get(res, ptr(lims, np.int64), ptr(dist, np.float32) if total else None,
+                                             ptr(ids, np.int64) if total else None))
+            return lims, dist, ids
+        finally:
+            lib().vix_range_result_destroy(res)
 
 
 class ReplicatedIVFPQIndex(ShardedIVFPQIndex):
@@ -806,10 +864,17 @@ class ReplicatedIVFPQIndex(ShardedIVFPQIndex):
                 a, co, i = a.numpy(), co.numpy(), i.numpy()
             self.local.add_encoded(a, co, i)
 
-    def batch_search(self, queries, k, nprobe=0, gather=True):
+    def range_search(self, queries, radius: float, nprobe: int = 0, filter=None):
+        """Not available: every replica holds every list, so the sharded merge would return each row ``world`` times."""
+        raise NotImplementedError("ReplicatedIVFPQIndex has no range search (ShardedIVFPQIndex.range_search merges list "
+                                  "shards; a replica holds all lists)")
+
+    def batch_search(self, queries, k, nprobe=0, gather=True, filter=None):
         """[nq x k] (distances, ids) of the whole batch on every rank (``gather=False``: this rank's block only, rows
-        ``query_block(nq)``)."""
+        ``query_block(nq)``).  ``filter`` is not available on replicas."""
         import torch
+        if filter is not None:
+            raise NotImplementedError("ReplicatedIVFPQIndex has no filtered search")
         was_numpy = not _lib._is_torch(queries)
         nprobe = nprobe if nprobe > 0 else self.nprobe
         nq = int(queries.shape[0])
