@@ -539,6 +539,10 @@ int vix_debug_tc_scores_f32(const float* queries, int64_t nq, const float* centr
  * layout (only L2 indexes with ks = 256, d = 2 m and m in {16, 32, 48, 64} do); out (host or device, nullable) receives
  * the bytes when cap holds them. */
 int vix_debug_tc_codes(vix_index_t* h, uint8_t* out, int64_t cap, int64_t* bytes_out);
+/* Test hook: the list-major scan's seed alone, thr[q] = the k-th smallest exact key (the query-major scan's distance) of the
+ * first 256 stored vectors of the query's first probed list that holds vectors, +inf when there are fewer than k;
+ * k <= 64, L2, ks = 256, dsub = 2, m in {16, 32, 48, 64} */
+int vix_debug_tc_seed(vix_index_t* h, const float* queries, int64_t nq, int k, const int32_t* probes, int nprobe, float* thr);
 
 /* Test hook: the result merge of vix_sharded_search on one GPU.  dist_all / ids_all: [world x nq x k] per-rank top-k
  * lists as the ranks' scans return them (API distances, ids; id -1 = none); they are packed into keys and merged by the

@@ -1318,6 +1318,34 @@ int vix_debug_tc_codes(vix_index_t* h, uint8_t* out, int64_t cap, int64_t* bytes
     return finish(true);
 }
 
+int vix_debug_tc_seed(vix_index_t* h, const float* queries, int64_t nq, int k, const int32_t* probes, int nprobe, float* thr) {
+    VIX_TRY(ensure_device());
+    VIX_REQUIRE(h && queries && probes && thr, VIX_ERR_NULL_PTR, "vix_debug_tc_seed: null pointer");
+    VIX_REQUIRE(nq > 0 && nq < 0x7FFFFFFFLL && nprobe > 0 && nprobe <= VIX_MAX_K, VIX_ERR_INVALID_PARAM,
+                "vix_debug_tc_seed: nq must lie in [1, 2^31 - 1), nprobe in [1, %d]", VIX_MAX_K);
+    VIX_REQUIRE(k >= 1 && k <= 64, VIX_ERR_INVALID_K, "vix_debug_tc_seed: k must lie in [1, 64]");
+    std::lock_guard<std::mutex> lk(h->mu);
+    VIX_REQUIRE(h->p.kind == VIX_INDEX_IVF_PQ && h->has_coarse && h->has_pq, VIX_ERR_NOT_TRAINED,
+                "vix_debug_tc_seed: not a trained IVF-PQ index");
+    VIX_REQUIRE(tc_codes_shape(h->p.metric, h->p.m, h->p.ks, h->p.d / h->p.m), VIX_ERR_INVALID_PARAM,
+                "vix_debug_tc_seed: the list-major scan does not take this shape");
+    if (h->dirty) VIX_TRY(build_lists(h));
+    In<float> dq;
+    In<int32_t> dp;
+    Out<float> dt;
+    VIX_TRY(dq.stage(queries, (size_t)nq * h->p.d));
+    VIX_TRY(dp.stage(probes, (size_t)nq * nprobe));
+    VIX_TRY(dt.stage(thr, (size_t)nq));
+    ScanArgs a{};
+    a.queries = dq.dev; a.nq = nq; a.d = h->p.d; a.m = h->p.m; a.ks = h->p.ks; a.dsub = h->p.d / h->p.m;
+    a.probes = const_cast<int32_t*>(dp.dev); a.nprobe = nprobe; a.coarse = h->coarse.ptr; a.kc = h->kc; a.k = k;
+    a.list_off = h->list_off.ptr; a.list_len = h->list_len.ptr; a.slot_codes = h->slot_codes.ptr; a.slot_tx = h->slot_tx.ptr;
+    a.codebooks_t = h->codebooks_t.ptr; a.metric = h->p.metric;
+    VIX_TRY(tc_seed_thresholds(a, dt.dev));
+    VIX_TRY(dt.commit());
+    return finish(dt.is_host());
+}
+
 int vix_index_clear(vix_index_t* h) {
     VIX_REQUIRE(h, VIX_ERR_NULL_PTR, "vix_index_clear: null handle");
     std::lock_guard<std::mutex> lk(h->mu);

@@ -563,31 +563,87 @@ table_kernel(const float* __restrict__ codebooks, int m, uint32_t* __restrict__ 
     }
 }
 
-// The seed: one CTA per query, one WARP per 32-vector chunk: the first kSeedChunks x 32 vectors of the query's first probed
-// list that holds vectors here get their exact keys -- the same table entries (lut_entry2 from the code-major codebooks,
-// L1-resident) in the same summation order as the look-up-table scan, but without building a 128 KB table -- and the CTA
-// sorts them.  The k-th of ANY k stored vectors is an upper bound of the query's k-th best distance: that is the threshold
-// of the filter (thr[q]; +inf when the sample holds fewer than k vectors).  (The whole list would give a tighter threshold
-// and fewer finalists, but costs more than the finalists it saves: C5 1.77 ms against 0.3 ms.  One warp walking the eight
-// chunks in sequence took 84 us for the 1250 queries a rank of eight seeds -- latency, not work.)  On the way the CTA
-// leaves ||q|| and the batch maximum of |q_e| (the fp16 scale) for query_prep_kernel.
+// ---- the seed's exact keys ----
+// The seed kernel is persistent: each CTA copies the code-major codebooks (codebooks_t, [256 codes][m] float2: 96 KB at
+// m = 48, 128 KB at m = 64) into shared memory once and then walks its share of the queries.  The look-ups are one LDS.64
+// per lane: the float2 of (code, j) sits in bank 2 j mod 32 (2 m is a multiple of 32), and the j of a warp instruction
+// spread over 16 values (the rotation of the rotated layout), so a warp's look-up costs the two wavefronts 256 bytes need.
+// From the read-only cache the same gathers touched up to 32 lines each.  (The finalists, log_key_kernel, keep the
+// read-only-cache gathers: the same shared-memory copy made that kernel slower at C5, 195 us against 122.)
+constexpr int kKeyThreads = 512;
+
+template <int G>
+__host__ __device__ constexpr int key_cb_bytes() { return 256 * 16 * G * 8; }
+
+template <int G>
+__device__ __forceinline__ void copy_codebooks(float2* s_cb, const float* __restrict__ codebooks_t) {
+    const float4* src = reinterpret_cast<const float4*>(codebooks_t);
+    float4* dst = reinterpret_cast<float4*>(s_cb);
+    for (int i = threadIdx.x; i < key_cb_bytes<G>() / 16; i += blockDim.x) dst[i] = __ldg(src + i);
+    __syncthreads();
+}
+
+// The look-up-table scan's key of one stored vector: its code bytes at src in the rotated layout (vix_scan.cuh) of slot sl,
+// the same table entries (lut_entry2 on the query pre-scaled by -2) summed into the same four partial sums in the same
+// order as log_key_kernel and the look-up-table scan, plus bias and t_x.  q = the query as float2 (q[2j], q[2j + 1]).
+template <int G>
+__device__ __forceinline__ float exact_key_sum(const float2* s_cb, const uint4* __restrict__ src, uint32_t sl, const float2* q,
+                                               float bias, float tx) {
+    constexpr int m = 16 * G;
+    float s[4] = {0.0f, 0.0f, 0.0f, 0.0f};
+#pragma unroll 1
+    for (int grp = 0; grp < G; ++grp) {                              // (unrolled, the gathers of all groups would be in
+        const uint4 w = __ldg(src + 32 * grp);                       // flight at once and spill)
+        const uint32_t x[4] = {w.x, w.y, w.z, w.w};
+#pragma unroll
+        for (int i4 = 0; i4 < 4; ++i4) {
+#pragma unroll
+            for (int t = 0; t < 4; ++t) {
+                const uint32_t b = 4 * i4 + t;
+                const uint32_t code = (x[i4] >> (8 * t)) & 255u;
+                const uint32_t j = 16u * grp + ((b ^ sl) & 15u);
+                const float2 v = s_cb[code * m + j];
+                const float2 qq = q[j];
+                s[t] = fadd(s[t], lut_entry2(qq.x * -2.0f, qq.y * -2.0f, v));     // the table build's pre-scaled query
+            }
+        }
+    }
+    return fadd(fadd(bias, tx), fadd(fadd(s[0], s[1]), fadd(s[2], s[3])));
+}
+
+// CTAs of a persistent key kernel: as many as fit on the device at once, no more than there is work for
+template <class K>
+static int key_grid(K kernel, int smem, int64_t want) {
+    int per_sm = 0;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kKeyThreads, smem) != cudaSuccess || per_sm < 1) per_sm = 1;
+    const int64_t cap = (int64_t)num_sms() * per_sm;
+    return (int)(want < 1 ? 1 : want < cap ? want : cap);
+}
+
+// The seed: one WARP per query, kSeedChunks rounds of 32 vectors: the first kSeedChunks x 32 vectors of the query's first
+// probed list that holds vectors here get their exact keys (exact_key_sum), and the warp selects the k-th smallest.  The
+// k-th of ANY k stored vectors is an upper bound of the query's k-th best distance: that is the threshold of the filter
+// (thr[q]; +inf when the sample holds fewer than k vectors or its k-th key is NaN).  (The whole list would give a tighter
+// threshold and fewer finalists, but costs more than the finalists it saves: C5 1.77 ms against 0.3 ms.)  On the way the
+// warp leaves ||q|| and the batch maximum of |q_e| (the fp16 scale) for query_prep_kernel.
 // A shard (only_first): only the rank that owns the query's FIRST probed list seeds it (the bounds are reduced over the
 // ranks; a seed from a farther list would be looser than the owner's and cost the same).
 template <int G>
-__global__ void __launch_bounds__(32 * kSeedChunks)
+__global__ void __launch_bounds__(kKeyThreads, 2)
 seed_scan_kernel(const float* __restrict__ queries, int64_t nq, const int32_t* __restrict__ probes, int nprobe, int kc,
                  int only_first, const float* __restrict__ coarse, const float* __restrict__ codebooks_t,
                  const int64_t* __restrict__ list_off, const int32_t* __restrict__ list_len, const uint8_t* __restrict__ slot_codes,
                  const float* __restrict__ slot_tx, int k, float* __restrict__ qnorm, unsigned int* __restrict__ maxabs,
                  float* __restrict__ thr) {
     constexpr int m = 16 * G, d = 2 * m;
-    __shared__ u64 s_keys[32 * kSeedChunks];
-    __shared__ float2 s_q[m];
-    __shared__ int s_list;
+    extern __shared__ float4 s_dyn[];
+    float2* const s_cb = reinterpret_cast<float2*>(s_dyn);
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int64_t q = blockIdx.x;
-    const float* qv = queries + q * d;
-    if (warp == 0) {
+    float2* const s_q = s_cb + 256 * m + warp * m;                   // this warp's query row
+    copy_codebooks<G>(s_cb, codebooks_t);
+    const int64_t nwarps = (int64_t)gridDim.x * (kKeyThreads / 32);
+    for (int64_t q = (int64_t)blockIdx.x * (kKeyThreads / 32) + warp; q < nq; q += nwarps) {
+        const float* qv = queries + q * d;
         // ||q|| and max |q_e|
         float s = 0.0f, mx = 0.0f;
         for (int e = lane; e < d; e += 32) { const float v = __ldg(qv + e); s = fmaf(v, v, s); mx = fmaxf(mx, fabsf(v)); }
@@ -606,59 +662,50 @@ seed_scan_kernel(const float* __restrict__ queries, int64_t nq, const int32_t* _
             if (ball) { const int src = __ffs(ball) - 1; l = __shfl_sync(0xFFFFFFFFu, lp, src); p0 = base + src; break; }
         }
         if (only_first && p0 != 0) l = -1;
-        if (lane == 0) s_list = l;
-    }
-    for (int j = threadIdx.x; j < m; j += blockDim.x) s_q[j] = make_float2(__ldg(qv + 2 * j) * -2.0f, __ldg(qv + 2 * j + 1) * -2.0f);
-    __syncthreads();
-    const int l = s_list;
-    if (l < 0) {
-        if (threadIdx.x == 0) thr[q] = __int_as_float(0x7f800000);
-        return;
-    }
-    // bias ||q - c_l||^2 in the order of probe_bias_kernel / build_probe_table (lane-strided partial sums, xor tree)
-    float bias = 0.0f;
-    {
-        const float* c = coarse + (int64_t)l * d;
-        for (int e = lane; e < d; e += 32) { const float df = __ldg(qv + e) - __ldg(c + e); bias = fmaf(df, df, bias); }
-        for (int o = 16; o > 0; o >>= 1) bias += __shfl_xor_sync(0xFFFFFFFFu, bias, o);
-    }
-    const int len = __ldg(list_len + l);
-    const uint32_t first = (uint32_t)(__ldg(list_off + l) >> 5);
-    const float2* cbt = reinterpret_cast<const float2*>(codebooks_t);
-    const uint32_t rot = (uint32_t)lane & 15u;
-    u64 key = kEmptyKey;
-    const int ch = warp;                                             // a SAMPLE of the list: any k vectors bound the k-th best
-    if (ch * 32 + lane < len) {
-        const uint32_t g = ((first + (uint32_t)ch) << 5) + (uint32_t)lane;
-        const uint4* src = reinterpret_cast<const uint4*>(slot_codes + (size_t)(first + ch) * (512u * G)) + lane;
-        float s[4] = {0.0f, 0.0f, 0.0f, 0.0f};
-#pragma unroll
-        for (int grp = 0; grp < G; ++grp) {
-            const uint4 w = __ldg(src + 32 * grp);
-            const uint32_t x[4] = {w.x, w.y, w.z, w.w};
-#pragma unroll
-            for (int i4 = 0; i4 < 4; ++i4) {
-#pragma unroll
-                for (int t = 0; t < 4; ++t) {
-                    const uint32_t b = 4 * i4 + t;
-                    const uint32_t code = (x[i4] >> (8 * t)) & 255u;
-                    const uint32_t j = 16u * grp + (b ^ rot);
-                    const float2 v = __ldg(cbt + code * m + j);
-                    const float2 qq = s_q[j];
-                    s[t] = fadd(s[t], lut_entry2(qq.x, qq.y, v));
-                }
-            }
+        if (l < 0) {
+            if (lane == 0) thr[q] = __int_as_float(0x7f800000);
+            continue;
         }
-        const float sum = fadd(fadd(bias, __ldg(slot_tx + g)), fadd(fadd(s[0], s[1]), fadd(s[2], s[3])));
-        key = make_key(sum, 0u, 0) | 0xFFFFFFFFull;                  // only the score matters: any id, the same for all
-    }
-    s_keys[threadIdx.x] = key;
-    __syncthreads();
-    bitonic_sort_keys<false>(s_keys, 32 * kSeedChunks, threadIdx.x, blockDim.x);
-    if (threadIdx.x == 0) {
-        const u64 kth = s_keys[k - 1];
-        const float t = key_score(kth, 0);
-        thr[q] = (kth != kEmptyKey && t == t) ? t : __int_as_float(0x7f800000);
+        __syncwarp();                                                // the previous query's reads of s_q are done
+        for (int j = lane; j < m; j += 32) s_q[j] = make_float2(__ldg(qv + 2 * j), __ldg(qv + 2 * j + 1));
+        __syncwarp();
+        // bias ||q - c_l||^2 in the order of probe_bias_kernel / build_probe_table (lane-strided partial sums, xor tree)
+        float bias = 0.0f;
+        {
+            const float* c = coarse + (int64_t)l * d;
+            for (int e = lane; e < d; e += 32) { const float df = __ldg(qv + e) - __ldg(c + e); bias = fmaf(df, df, bias); }
+            for (int o = 16; o > 0; o >>= 1) bias += __shfl_xor_sync(0xFFFFFFFFu, bias, o);
+        }
+        const int len = __ldg(list_len + l);
+        const uint32_t first = (uint32_t)(__ldg(list_off + l) >> 5);
+        // the orderable score bits of make_key (NaN and "no vector": 0xFFFFFFFF), one per chunk
+        uint32_t key[kSeedChunks];
+#pragma unroll
+        for (int ch = 0; ch < kSeedChunks; ++ch) key[ch] = 0xFFFFFFFFu;
+#pragma unroll 1
+        for (int ch = 0; ch < kSeedChunks && ch * 32 < len; ++ch) {   // a SAMPLE of the list: any k vectors bound the k-th best
+            uint32_t kv = 0xFFFFFFFFu;
+            if (ch * 32 + lane < len) {
+                const uint32_t g = ((first + (uint32_t)ch) << 5) + (uint32_t)lane;
+                const uint4* src = reinterpret_cast<const uint4*>(slot_codes + (size_t)(first + ch) * (512u * G)) + lane;
+                const float sum = exact_key_sum<G>(s_cb, src, (uint32_t)lane, s_q, bias,
+                                                   __ldg(slot_tx + g));
+                kv = (uint32_t)(make_key(sum, 0u, 0) >> 32);
+            }
+#pragma unroll
+            for (int c = 0; c < kSeedChunks; ++c) key[c] = c == ch ? kv : key[c];
+        }
+        // the k-th smallest of the 32 x kSeedChunks keys, one bit at a time from the top: bit b of the answer is 0 iff at
+        // least k keys are <= (the answer's bits above b, then all ones)
+        uint32_t kth = 0;
+        for (int b = 31; b >= 0; --b) {
+            const uint32_t t = kth | ((1u << b) - 1u);
+            int c = 0;
+#pragma unroll
+            for (int i = 0; i < kSeedChunks; ++i) c += key[i] <= t ? 1 : 0;
+            if ((int)__reduce_add_sync(0xFFFFFFFFu, (unsigned)c) < k) kth |= 1u << b;
+        }
+        if (lane == 0) thr[q] = kth != 0xFFFFFFFFu ? f32_from_orderable(kth) : __int_as_float(0x7f800000);
     }
 }
 
@@ -1064,6 +1111,39 @@ static StageTimes* stage_times() {
 }
 }  // namespace tcs
 
+// norms + seed (seed_scan_kernel): one warp per query
+static int launch_seed(const ScanArgs& a, int only_first, float* qnorm, unsigned int* maxabs, float* thr) {
+    using namespace tcs;
+    static_assert(32 * kSeedChunks >= 64, "k <= 64 keys out of the sample");
+    const int64_t want = (a.nq + kKeyThreads / 32 - 1) / (kKeyThreads / 32);
+#define VIX_SEED(GG)                                                                                                       \
+    do {                                                                                                                   \
+        const int sm = key_cb_bytes<GG>() + kKeyThreads / 32 * 16 * GG * 8;          /* + a query row per warp */        \
+        VIX_CUDA(cudaFuncSetAttribute(seed_scan_kernel<GG>, cudaFuncAttributeMaxDynamicSharedMemorySize, sm));              \
+        seed_scan_kernel<GG><<<key_grid(seed_scan_kernel<GG>, sm, want), kKeyThreads, sm, ctx().stream>>>(a.queries, a.nq,  \
+            a.probes, a.nprobe, a.kc, only_first, a.coarse, a.codebooks_t, a.list_off, a.list_len, a.slot_codes, a.slot_tx,  \
+            a.k, qnorm, maxabs, thr);                                                                                      \
+        VIX_LAUNCH_CHECK();                                                                                                \
+    } while (0)
+    switch (a.m / 16) {
+        case 1: VIX_SEED(1); break;
+        case 2: VIX_SEED(2); break;
+        case 3: VIX_SEED(3); break;
+        case 4: VIX_SEED(4); break;
+    }
+#undef VIX_SEED
+    return VIX_OK;
+}
+
+int tc_seed_thresholds(const ScanArgs& a, float* thr) {
+    Scratch<float> qnorm;
+    Scratch<unsigned int> maxabs;
+    VIX_TRY(qnorm.alloc((size_t)a.nq));
+    VIX_TRY(maxabs.alloc(1));
+    VIX_CUDA(cudaMemsetAsync(maxabs.ptr, 0, 4, ctx().stream));
+    return launch_seed(a, 0, qnorm.ptr, maxabs.ptr, thr);
+}
+
 bool tc_decode_table_shape(int m, int ks, int dsub) { return dsub == 2 && ks == 256 && (m == 16 || m == 32 || m == 48 || m == 64); }
 bool tc_codes_shape(int metric, int m, int ks, int dsub) { return metric == VIX_METRIC_L2 && tc_decode_table_shape(m, ks, dsub); }
 int tc_decode_table(const float* codebooks, int m, uint32_t* table, float* meta) {
@@ -1143,23 +1223,7 @@ int launch_ivfpq_scan_tc(ScanArgs& a) {
     mark();
     Scratch<float> thr;
     VIX_TRY(thr.alloc((size_t)nq));
-    {   // norms + seed: one CTA per query, one warp per sampled chunk
-        static_assert(32 * kSeedChunks >= 64, "k <= 64 keys out of the sample");
-#define VIX_SEED(GG)                                                                                                       \
-        do {                                                                                                               \
-            seed_scan_kernel<GG><<<(unsigned)nq, 32 * kSeedChunks, 0, s>>>(a.queries, nq, a.probes, a.nprobe, a.kc,          \
-                tls_thr_hook != nullptr, a.coarse, a.codebooks_t, a.list_off, a.list_len, a.slot_codes, a.slot_tx, k,       \
-                qnorm.ptr, maxabs.ptr, thr.ptr);                                                                           \
-            VIX_LAUNCH_CHECK();                                                                                            \
-        } while (0)
-        switch (G) {
-            case 1: VIX_SEED(1); break;
-            case 2: VIX_SEED(2); break;
-            case 3: VIX_SEED(3); break;
-            case 4: VIX_SEED(4); break;
-        }
-#undef VIX_SEED
-    }
+    VIX_TRY(launch_seed(a, tls_thr_hook != nullptr, qnorm.ptr, maxabs.ptr, thr.ptr));
     mark();
     if (tls_thr_hook) VIX_TRY(tls_thr_hook(tls_thr_ctx, thr.ptr, nq));         // sharded: the minimum over the ranks
     mark();

@@ -75,5 +75,8 @@ bool tc_decode_table_shape(int m, int ks, int dsub);
 // Built for L2 indexes of the decode table's shape (tc_codes_shape), which are the only ones the list-major path takes.
 bool tc_codes_shape(int metric, int m, int ks, int dsub);
 int tc_decode_table(const float* codebooks, int m, uint32_t* table, float* meta);
+// the list-major path's seed alone: thr[q] = the k-th smallest exact key of the first 256 vectors of the query's first
+// probed list that holds vectors (+inf: fewer than k of them); k <= 64, the shapes of tc_codes_shape
+int tc_seed_thresholds(const ScanArgs& a, float* thr);
 
 }  // namespace vix
