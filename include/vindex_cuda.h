@@ -93,6 +93,8 @@ typedef enum { VIX_METRIC_L2 = 0, VIX_METRIC_IP = 1, VIX_METRIC_COSINE = 2 } vix
 typedef enum { VIX_ORDER_MIN = 0, VIX_ORDER_MAX = 1 } vix_ordering;
 
 #define VIX_MAX_K 512      /* largest k / nprobe served by the fused selection kernels */
+#define VIX_MAX_K_LARGE 16384  /* largest k of index / flat k-NN search: VIX_MAX_K < k <= VIX_MAX_K_LARGE takes the exact
+                                  two-pass route over the range-search scans (and the largest rerank_r) */
 
 /* ------------------------------------------------------------------------------------------------ */
 /* Library / context                                                                                */
@@ -134,7 +136,8 @@ int vix_row_norms_f32(const float* x, int64_t n, int d, float* out);
 /* a1-a4  Batched exact search = ScoreBlock.run + selectTopK + API distance mapping
  * (FlatIndexOptimized.swift:390-477) for nq queries at once, top-k fused into the scan (no [nq x n]
  * matrix is written).  ids are base row indices.  out_dist: L2 => sqrt(L2^2), IP => -dot.
- * Rows with fewer than k results are padded with id -1 / NaN.  k <= VIX_MAX_K. */
+ * Rows with fewer than k results are padded with id -1 / NaN.  k <= VIX_MAX_K_LARGE: above VIX_MAX_K the exact two-pass
+ * route of vix_index_search (same results, ties to the smaller row), which synchronises the stream. */
 int vix_flat_search_f32(const float* queries, int64_t nq, const float* xb, int64_t n, int d,
                         int metric, int k, float* out_dist, int64_t* out_ids);
 
@@ -359,7 +362,18 @@ int     vix_index_clear(vix_index_t* h);
  * NaN (the row is the k smallest probed ids); an infinite one can give NaN where the oracle gives +-inf, because the scan
  * adds the per-probe and per-code terms of its decomposition (+inf + -inf); a query whose L2 distances overflow gets +inf.
  * With sharding the result is this shard's local top-k (merge with
- * vix_merge_topk_f32 after an all-gather). */
+ * vix_merge_topk_f32 after an all-gather).
+ * k <= VIX_MAX_K_LARGE (above: VIX_ERR_INVALID_K).  VIX_MAX_K < k <= VIX_MAX_K_LARGE takes an exact two-pass route over the
+ * range-search scans (every kind, metric and filter; the same outputs, padding, tie and NaN rules, and search(k)[:, :k2]
+ * == search(k2) bit for bit): a seed pass bounds each query's k-th distance from a subset of its candidates (IVF: the
+ * probes, in order, that hold about 2 k vectors; flat: the fused top-512 of 2 k / 512 row blocks), a collect pass keeps
+ * every candidate within that bound, and the rows are sorted by (distance, id) and cut at k.  IVF-PQ takes the query-major
+ * scan on this route.  The route synchronises its stream, even in asynchronous mode (the size of the collect depends on
+ * the data); a collect that does not fit in device memory returns VIX_ERR_OOM with the handle unchanged; it is not
+ * recorded by vix_index_trace; vix_search_stats reports scan_path = 2, merge_candidates = the entries collected (the
+ * row lengths before the cut), the three ms_* times, cycle counters 0.  VIX_SCAN_DEBUG=1 prints one line per call:
+ * "[vix knn] kind K, kernel fast G n | generic | ivfflat | flat, filter 0|1, k K, seed S, total T, passes P, max_row M"
+ * (S seed entries, T collected entries, P scans of the collect: 2 when it outgrew the capacity the handle remembers). */
 int vix_index_search(vix_index_t* h, const float* queries, int64_t nq, int k, int nprobe,
                      float* out_dist, int64_t* out_ids);
 
@@ -376,7 +390,8 @@ typedef struct {
     int64_t cycles_select, cycles_probe_table, cycles_lut;   /* the three concurrent pieces of the prologue */
     int64_t merge_candidates;                                 /* entries handed to the per-query top-k merge */
     float   ms_scan_kernel;       /* CUDA-event time of the stage's dominant kernel alone (the scan proper)              */
-    int32_t scan_path;            /* IVF-PQ: 0 = query-major look-up-table scan, 1 = list-major tensor-core scan           */
+    int32_t scan_path;            /* IVF-PQ: 0 = query-major look-up-table scan, 1 = list-major tensor-core scan;
+                                     2 = the two-pass route of k > VIX_MAX_K (every kind)                                  */
 } vix_search_stats;
 int vix_index_search_ex(vix_index_t* h, const float* queries, int64_t nq, int k, int nprobe,
                         float* out_dist, int64_t* out_ids, int32_t* out_probes /* [nq x nprobe] nullable */,
@@ -417,7 +432,8 @@ void    vix_range_result_destroy(vix_range_result_t* r);   /* NULL is a no-op */
  * VIX_FILTER_DENY keeps ids whose bit is 0.  The filter is applied BEFORE selection (the pre-filter of
  * IVFIndex.search / FlatIndex.search, IVFIndex.swift:813, 1034; FlatIndex.swift:61): the result is the k best of the
  * vectors that pass, possibly fewer than k (padding id -1 / NaN).  filter_words == NULL => unfiltered search.
- * Closure filters over metadata are host-side objects in the reference; evaluate them on the host into a bitset. */
+ * Closure filters over metadata are host-side objects in the reference; evaluate them on the host into a bitset.
+ * k as vix_index_search: up to VIX_MAX_K_LARGE, the two-pass route above VIX_MAX_K with the filter on both passes. */
 enum { VIX_FILTER_ALLOW = 0, VIX_FILTER_DENY = 1 };
 int vix_index_search_filtered(vix_index_t* h, const float* queries, int64_t nq, int k, int nprobe,
                               const uint64_t* filter_words /* [ceil(capacity / 64)] */, int64_t filter_capacity,
@@ -432,6 +448,7 @@ int vix_index_search_filtered(vix_index_t* h, const float* queries, int64_t nq, 
  * list and appended there with vix_index_add_encoded. */
 int vix_index_probe_range(vix_index_t* h, const float* queries, int64_t nq, int nprobe, int list_begin, int list_count,
                           int32_t* list_ids_out /* [nq x nprobe] */, float* list_scores_out /* nullable */);
+/* (k as vix_index_search: up to VIX_MAX_K_LARGE; both passes of the two-pass route use the given probes) */
 int vix_index_search_with_probes(vix_index_t* h, const float* queries, int64_t nq, int k, const int32_t* probes,
                                  int nprobe, float* out_dist, int64_t* out_ids);
 
@@ -508,7 +525,8 @@ int vix_sharded_search_filtered(vix_index_t* h, vix_comm_t* c, const float* quer
 
 /* f-1  The IVF-PQ query with its optional last step (docs/kernel-specs/DONE_22_adc_scan.md:873-878, "7. Optional: exact
  * rerank (kernel #40)"; IVFIndex.swift:1380-1439): ADC search for the rerank_r best candidates per query (k <= rerank_r <=
- * VIX_MAX_K), then rerank_exact_topk over the ORIGINAL vectors with the DenseArray reader: id -> row of xb [N x d] (ids
+ * VIX_MAX_K_LARGE; above VIX_MAX_K through the two-pass route of vix_index_search, which synchronises; the re-rank's own
+ * limits -- C <= 16384 candidates and its shared memory -- return VIX_ERR_UNSUPPORTED), then rerank_exact_topk over the ORIGINAL vectors with the DenseArray reader: id -> row of xb [N x d] (ids
  * outside [0, N) are missing and skipped).  Outputs as vix_rerank_exact_topk_f32: raw exact scores (L2^2 / dot), best
  * first by (score under the metric's ordering, smaller id), padded with +-inf / id -1.  xb may live on the device (it is
  * staged per call otherwise). */

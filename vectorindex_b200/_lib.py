@@ -20,6 +20,7 @@ METRIC_L2, METRIC_IP = 0, 1
 ORDER_MIN, ORDER_MAX = 0, 1
 INDEX_FLAT, INDEX_IVF_FLAT, INDEX_IVF_PQ = 0, 1, 2
 MAX_K = 512
+MAX_K_LARGE = 16384          # k-NN search beyond MAX_K: the exact two-pass route over the range-search scans
 
 STATUS_NAMES = {
     0: "ok", -1: "invalidDim", -2: "invalidK", -3: "nullPtr", -4: "invalidLayout", -5: "invalidParameter",

@@ -19,6 +19,7 @@
 #include "vix_range.cuh"
 #include "vix_group.cuh"
 
+#include <algorithm>
 #include <new>
 #include <stdio.h>
 #include <stdlib.h>
@@ -488,6 +489,7 @@ ivfflat_range_kernel(const float* __restrict__ queries, int64_t nq, int d, const
         if (threadIdx.x == 0) s_cnt = 0;
         __syncthreads();
         const float qmag2 = (metric == VIX_METRIC_COSINE) ? seq_sumsq(s_q, d) : 0.0f;
+        const uint32_t qbound = out.bound ? out.bound[qi] : 0xFFFFFFFFu;
         for (int p = 0; p < nprobe; ++p) {
             const int l = probes[qi * (int64_t)nprobe + p];
             if ((unsigned)l >= (unsigned)kc) continue;           // -1 padding, or an id no list has
@@ -503,8 +505,8 @@ ivfflat_range_kernel(const float* __restrict__ queries, int64_t nq, int d, const
                     if (metric == VIX_METRIC_L2) dist = __fsqrt_rn(exact_pair<SpecDirect16L2>(s_q, v, d));
                     else if (metric == VIX_METRIC_IP) dist = -exact_pair<SpecIp4>(s_q, v, d);
                     else dist = cosine_distance(exact_pair<SpecIp4>(s_q, v, d), qmag2, seq_sumsq(v, d));
-                    pass = dist <= out.radius;
                     key = make_key(dist, (uint32_t)slot_ids[b + i], 0);
+                    pass = out.bound ? (uint32_t)(key >> 32) <= qbound : dist <= out.radius;
                 }
                 const unsigned ball = __ballot_sync(0xFFFFFFFFu, pass);
                 if (ball) {
@@ -804,6 +806,148 @@ static int index_remove_locked(vix_index* h, const int64_t* ids, int64_t n, int6
     return VIX_OK;
 }
 
+// k-NN search for VIX_MAX_K < k <= VIX_MAX_K_LARGE (vix_knn_large.cu): the candidates of index_search_locked (every row,
+// or the probed lists of the same probe selection / the caller's given_probes), a seed pass and a collect pass through the
+// kind's range kernel, the sorted rows cut at k.  Synchronises the stream (the collect's size depends on the data); not
+// traced.  The handle keeps only the collect's capacity hint, written once the call has succeeded.
+static int index_knn_large_locked(vix_index* h, const float* queries, int64_t nq, int k, int nprobe, float* out_dist,
+                                  int64_t* out_ids, int32_t* out_probes, vix_search_stats* stats,
+                                  const int32_t* given_probes, const FilterArgs* filter) {
+    const int d = h->p.d;
+    cudaStream_t s = ctx().stream;
+    const bool linear = h->p.kind == VIX_INDEX_FLAT || !h->has_coarse;
+    VIX_REQUIRE(!linear || h->p.kind != VIX_INDEX_IVF_PQ, VIX_ERR_NOT_TRAINED, "index_search: IVF-PQ index is not trained");
+    VIX_REQUIRE(nq < 0x7FFFFFFFLL, VIX_ERR_INVALID_PARAM, "index_search: k > %d needs nq < 2^31 - 1", VIX_MAX_K);
+    if (!linear) {
+        if (nprobe <= 0) nprobe = h->p.nprobe;
+        VIX_REQUIRE(nprobe > 0 && nprobe <= VIX_MAX_K, VIX_ERR_INVALID_K, "index_search: nprobe = %d (1 .. %d)", nprobe,
+                    VIX_MAX_K);
+    }
+    In<float> dq;
+    Out<float> dd;
+    Out<int64_t> di;
+    Out<int32_t> dp;
+    VIX_TRY(dq.stage(queries, (size_t)nq * d));
+    VIX_TRY(dd.stage(out_dist, (size_t)nq * k));
+    VIX_TRY(di.stage(out_ids, (size_t)nq * k));
+    cudaEvent_t* ev = h->ev;
+    if (stats && !ev[0]) for (int e = 0; e < 5; ++e) VIX_CUDA(cudaEventCreate(&ev[e]));
+    if (stats) VIX_CUDA(cudaEventRecord(ev[0], s));
+    size_t cap = h->knn_cap;
+    KnnInfo info;
+    char kernel[32] = "flat";
+    if (linear) {
+        // a flat index, or an IVF-Flat index before optimize(): the flat engine over the stored rows, row indices as ids
+        Scratch<uint64_t> mask;
+        if (filter && h->n > 0) {
+            const int64_t words = (h->n + 63) / 64;
+            VIX_TRY(mask.alloc((size_t)words));
+            filter_row_mask_kernel<<<(unsigned)((words + 255) / 256), 256, 0, s>>>(h->ids.ptr, h->n, filter->words, filter->cap,
+                                                                                filter->deny, mask.ptr);
+            VIX_LAUNCH_CHECK();
+        }
+        if (stats) VIX_CUDA(cudaEventRecord(ev[1], s));
+        Scratch<int64_t> rows;
+        VIX_TRY(rows.alloc((size_t)nq * k));
+        VIX_TRY(flat_knn_large_device(dq.dev, nq, h->vecs.ptr, h->n, d, h->p.metric, k, mask.ptr, cap, dd.dev, rows.ptr, &info));
+        gather_ids_kernel<<<(unsigned)((nq * k + 255) / 256), 256, 0, s>>>(rows.ptr, h->ids.ptr, di.dev, nq * (int64_t)k);
+        VIX_LAUNCH_CHECK();
+    } else {
+        if (h->dirty) VIX_TRY(build_lists(h));
+        VIX_TRY(dp.stage(out_probes, out_probes ? (size_t)nq * nprobe : 0));
+        Scratch<int32_t> probe_buf;
+        In<int32_t> gp;
+        const int32_t* probes = nullptr;
+        if (given_probes) {
+            VIX_TRY(gp.stage(given_probes, (size_t)nq * nprobe));
+            if (dp.dev) VIX_CUDA(cudaMemcpyAsync(dp.dev, gp.dev, (size_t)nq * nprobe * 4, cudaMemcpyDeviceToDevice, s));
+            probes = gp.dev;
+        } else {
+            int32_t* pp = dp.dev;
+            if (!pp) { VIX_TRY(probe_buf.alloc((size_t)nq * nprobe)); pp = probe_buf.ptr; }
+            if (h->p.metric == VIX_METRIC_COSINE)
+                VIX_TRY(probe_select_cosine_device(dq.dev, nq, h->coarse.ptr, h->kc, d, h->coarse_norms.ptr, nprobe, pp));
+            else
+                VIX_TRY(probe_select_fast_device(dq.dev, nq, h->coarse.ptr, h->kc, d, h->p.metric, nprobe, h->coarse_norms.ptr, pp,
+                                                 nullptr, h->coarse_norm_max.ptr));
+            probes = pp;
+        }
+        if (stats) VIX_CUDA(cudaEventRecord(ev[1], s));
+        Scratch<int32_t> prefix;
+        VIX_TRY(prefix.alloc((size_t)nq * nprobe));
+        size_t seed_cap = 0, max_entries = 0;
+        VIX_TRY(knn_probe_prefix(probes, nq, nprobe, h->list_len.ptr, h->kc, k, prefix.ptr, &seed_cap, &max_entries));
+        // the kind's range kernel over a probe list [nq x nprobe] (never the list-major tensor-core scan)
+        std::function<int(const int32_t*, const RangeOut&)> scan;
+        ScanArgs a{};
+        Scratch<int> work_counter;
+        Scratch<int32_t> order;
+        if (h->p.kind == VIX_INDEX_IVF_PQ) {
+            a.queries = dq.dev; a.nq = nq; a.d = d; a.m = h->p.m; a.ks = h->p.ks; a.dsub = d / h->p.m;
+            a.nprobe = nprobe; a.coarse = h->coarse.ptr; a.kc = h->kc; a.codebooks = h->codebooks.ptr;
+            a.list_off = h->list_off.ptr; a.list_len = h->list_len.ptr;
+            a.slot_codes = h->slot_codes.ptr; a.slot_tx = h->slot_tx.ptr; a.slot_ids = h->slot_ids.ptr;
+            a.metric = h->p.metric; a.codebooks_t = h->codebooks_t.ptr;
+            if (filter) { a.filter = filter->words; a.filter_cap = filter->cap; a.filter_deny = filter->deny; }
+            VIX_TRY(work_counter.alloc(2));
+            a.work_counter = work_counter.ptr;
+            const bool fast = scan_layout(a.m).fast && a.ks == 256;
+            if (fast && nq > 2 * num_sms()) {
+                VIX_TRY(query_order(probes, nq, nprobe, h->list_len.ptr, h->kc, order));
+                a.order = order.ptr;
+            }
+            if (fast) snprintf(kernel, sizeof kernel, "fast G %d", a.m / 16);
+            else snprintf(kernel, sizeof kernel, "generic");
+            scan = [&](const int32_t* pr, const RangeOut& o) {
+                ScanArgs b = a;
+                b.probes = pr;
+                b.range = o;
+                return launch_ivfpq_scan_classic(b);
+            };
+        } else {
+            snprintf(kernel, sizeof kernel, "ivfflat");
+            const size_t smem = (size_t)d * 4;
+            VIX_CUDA(cudaFuncSetAttribute(ivfflat_range_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            const int64_t grid = std::min<int64_t>((int64_t)num_sms() * 4, nq);
+            scan = [&, smem, grid](const int32_t* pr, const RangeOut& o) -> int {
+                ivfflat_range_kernel<<<(unsigned)grid, 256, smem, s>>>(dq.dev, nq, d, pr, nprobe, h->list_off.ptr, h->list_len.ptr,
+                                                                     h->kc, h->slot_vecs.ptr, h->slot_ids.ptr, h->p.metric,
+                                                                     filter ? filter->words : nullptr, filter ? filter->cap : 0,
+                                                                     filter ? filter->deny : 0, o);
+                VIX_LAUNCH_CHECK();
+                return VIX_OK;
+            };
+        }
+        const std::function<int(const RangeOut&)> seed = [&](const RangeOut& o) { return scan(prefix.ptr, o); };
+        const std::function<int(const RangeOut&)> collect = [&](const RangeOut& o) { return scan(probes, o); };
+        // (IVF-PQ reports a zero inner-product distance as -0, IVF-Flat keys the distance itself: +0)
+        KnnDecode dec;
+        dec.neg_zero = h->p.kind == VIX_INDEX_IVF_PQ && h->p.metric == VIX_METRIC_IP;
+        VIX_TRY(knn_large_run(nq, k, dec, seed_cap, &seed, collect, max_entries, cap, dd.dev, di.dev, &info));
+        VIX_TRY(dp.commit());
+    }
+    if (stats) VIX_CUDA(cudaEventRecord(ev[2], s));
+    VIX_TRY(dd.commit());
+    VIX_TRY(di.commit());
+    const int rc = finish(true);
+    if (rc != VIX_OK) return rc;
+    h->knn_cap = cap;
+    if (stats) {
+        VIX_CUDA(cudaEventSynchronize(ev[2]));
+        cudaEventElapsedTime(&stats->ms_coarse, ev[0], ev[1]);
+        cudaEventElapsedTime(&stats->ms_scan, ev[1], ev[2]);
+        cudaEventElapsedTime(&stats->ms_total, ev[0], ev[2]);
+        stats->scan_path = 2;
+        stats->merge_candidates = info.collect.total;
+    }
+    if (getenv("VIX_SCAN_DEBUG"))
+        fprintf(stderr, "[vix knn] kind %s, kernel %s, filter %d, k %d, seed %lld, total %lld, passes %d, max_row %lld\n",
+                h->p.kind == VIX_INDEX_FLAT ? "flat" : h->p.kind == VIX_INDEX_IVF_FLAT ? "ivfflat" : "ivfpq", kernel,
+                filter != nullptr, k, (long long)info.seed, (long long)info.collect.total, info.collect.passes,
+                (long long)info.collect.max_row);
+    return VIX_OK;
+}
+
 int index_search_locked(vix_index* h, const float* queries, int64_t nq, int k, int nprobe, float* out_dist,
                         int64_t* out_ids, int32_t* out_probes, vix_search_stats* stats,
                         const int32_t* given_probes, const FilterArgs* filter) {
@@ -812,7 +956,9 @@ int index_search_locked(vix_index* h, const float* queries, int64_t nq, int k, i
     if (stats) memset(stats, 0, sizeof(*stats));
     if (k <= 0 || nq <= 0) return VIX_OK;                      // IVFIndex.swift:866
     VIX_REQUIRE(queries && out_dist && out_ids, VIX_ERR_NULL_PTR, "index_search: null pointer");
-    VIX_REQUIRE(k <= VIX_MAX_K, VIX_ERR_INVALID_K, "index_search: k > %d", VIX_MAX_K);
+    VIX_REQUIRE(k <= VIX_MAX_K_LARGE, VIX_ERR_INVALID_K, "index_search: k > %d", VIX_MAX_K_LARGE);
+    if (k > VIX_MAX_K)
+        return index_knn_large_locked(h, queries, nq, k, nprobe, out_dist, out_ids, out_probes, stats, given_probes, filter);
     In<float> dq;
     Out<float> dd;
     Out<int64_t> di;
@@ -1577,7 +1723,7 @@ int vix_index_search_rerank(vix_index_t* h, const float* queries, int64_t nq, in
     if (k <= 0 || nq <= 0) return VIX_OK;
     VIX_REQUIRE(queries && xb && out_scores && out_ids, VIX_ERR_NULL_PTR, "vix_index_search_rerank: null pointer");
     VIX_REQUIRE(rerank_r >= k, VIX_ERR_INVALID_K, "vix_index_search_rerank: rerank_r (%d) must be >= k (%d) (ExactRerank.swift:730)", rerank_r, k);
-    VIX_REQUIRE(rerank_r <= VIX_MAX_K, VIX_ERR_INVALID_K, "vix_index_search_rerank: rerank_r > %d", VIX_MAX_K);
+    VIX_REQUIRE(rerank_r <= VIX_MAX_K_LARGE, VIX_ERR_INVALID_K, "vix_index_search_rerank: rerank_r > %d", VIX_MAX_K_LARGE);
     VIX_REQUIRE(h->p.metric != VIX_METRIC_COSINE, VIX_ERR_UNSUPPORTED, "vix_index_search_rerank: L2 / IP (Kernel #40's metrics on this path)");
     In<float> dq;
     VIX_TRY(dq.stage(queries, (size_t)nq * h->p.d));

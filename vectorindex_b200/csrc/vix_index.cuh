@@ -16,7 +16,7 @@ int pq_encode_device(const float* x, int64_t n, int d, int m, int ks, const floa
 int flat_search_device(const float* q, int64_t nq, const float* xb, int64_t n, int d, int metric, int k,
                        const float* xb_norm, float* out_dist, int64_t* out_ids, bool raw_scores);
 int flat_search_masked_device(const float* q, int64_t nq, const float* xb, int64_t n, int d, int metric, int k,
-                              const uint64_t* disabled_rows, float* out_dist, int64_t* out_ids);
+                              const uint64_t* disabled_rows, float* out_dist, int64_t* out_ids, bool raw_scores = false);
 int flat_search_auto_device(const float* q, int64_t nq, const float* xb, int64_t n, int d, int metric, int k,
                             const float* xb_norm, float* out_dist, int64_t* out_ids, bool raw_scores);
 int probe_select_device(const float* q, int64_t nq, const float* c, int kc, int d, int metric, int nprobe,
@@ -128,6 +128,7 @@ struct vix_index {
     int trace_cap = 0, trace_n = 0;
     std::vector<int> trace_path;        // IVF-PQ scan path of each traced call
     size_t range_cap = 0;               // range search: entries the last call returned (+1/8), the next call's first capacity
+    size_t knn_cap = 0;                 // k-NN search beyond VIX_MAX_K: the same for its collect pass (vix_knn_large.cu)
 };
 
 

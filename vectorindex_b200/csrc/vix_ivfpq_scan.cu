@@ -403,8 +403,9 @@ __device__ __noinline__ uint32_t flush_queue(u64* wq, int Pw, int k, int cnt, bo
 
 // m = 16 G; FILTER: an id filter is active; STATS: the phase counters of vix_search_stats are kept (separate
 // instantiations, so the production kernel pays neither in instructions nor in registers).  RANGE: range search -- the
-// acceptance test is the constant radius on the API distance instead of the running k-th bound, and accepted entries go to
-// a.range (vix_range.cuh) instead of the per-warp queues; s_ncand counts them per query.
+// acceptance test is the constant radius on the API distance (or, k-NN search beyond VIX_MAX_K, the query's key bound,
+// kept with its buffer in s_bnd) instead of the running k-th bound, and accepted entries go to a.range (vix_range.cuh)
+// instead of the per-warp queues; s_ncand counts them per query.
 template <int G, bool FILTER, bool STATS, bool RANGE = false>
 __global__ void __launch_bounds__(kFastThreads, 1)
 ivfpq_scan_kernel(ScanArgs a) {
@@ -426,7 +427,8 @@ ivfpq_scan_kernel(ScanArgs a) {
     int* s_thr = s_item + 2;                                              // [1] CTA acceptance threshold
     int* s_ncand = s_thr + 1;                                             // [2] candidates published for the merge
     int* s_next = s_ncand + 2;                                            // [1] next chunk to hand out
-    u64* s_wq = reinterpret_cast<u64*>((reinterpret_cast<uintptr_t>(s_next + 1) + 15) & ~(uintptr_t)15);
+    uint32_t* s_bnd = reinterpret_cast<uint32_t*>(s_next + 1);            // RANGE: [2] key bound of the query of a buffer
+    u64* s_wq = reinterpret_cast<u64*>((reinterpret_cast<uintptr_t>(s_bnd + (RANGE ? 2 : 0)) + 15) & ~(uintptr_t)15);
     u64* s_cand = s_wq + (size_t)nwarps * a.Pw;                           // [2][nwarps * Pw] published candidates
     unsigned char* misc_end = reinterpret_cast<unsigned char*>(s_cand + 2 * (size_t)nwarps * a.Pw);
     const uint32_t dyn_abs = (uint32_t)__cvta_generic_to_shared(smem_raw);
@@ -471,6 +473,7 @@ ivfpq_scan_kernel(ScanArgs a) {
                           a.bias ? a.bias + qn * (int64_t)a.nprobe : nullptr, a.nprobe, a.list_off, a.list_len, a.kc,
                           pt + a.nprobe, pt + 2 * a.nprobe, pt + 3 * a.nprobe, reinterpret_cast<float*>(pt), s_np + b,
                           s_qv + b * a.d);
+        if (RANGE && a.range.bound && lane == 0) s_bnd[b] = a.range.bound[qn];
     };
 
     if (tid == 32) { s_item[0] = atomicAdd(a.work_counter, 1); s_ncand[0] = 0; s_ncand[1] = 0; }
@@ -617,8 +620,14 @@ ivfpq_scan_kernel(ScanArgs a) {
             if constexpr (RANGE) {
                 // the API distance k-NN search reports for this entry (L2: the score; IP: minus the score); with the id
                 // the key is the k-NN one, which orders as make_key(api distance, id, 0)
-                const float api = order_max ? -key_score(key, 1) : key_score(key, 0);
-                bool pass = valid && api <= a.range.radius;
+                // (a per-query key bound compares the key's high word, which orders as the API distance)
+                bool pass;
+                if (a.range.bound) {
+                    pass = valid && (uint32_t)(key >> 32) <= s_bnd[buf];
+                } else {
+                    const float api = order_max ? -key_score(key, 1) : key_score(key, 0);
+                    pass = valid && api <= a.range.radius;
+                }
                 uint32_t id = 0;
                 if (pass) {
                     id = (uint32_t)a.slot_ids[g];
@@ -811,6 +820,7 @@ ivfpq_scan_generic_kernel(ScanArgs a) {
         __syncthreads();
 
         const int nchunks = s_pref[a.nprobe];
+        const uint32_t qbound = RANGE && a.range.bound ? a.range.bound[qi] : 0xFFFFFFFFu;
         int cnt = 0;
         float thr_s = order_max ? -INFINITY : INFINITY;
         int p = 0;
@@ -835,8 +845,13 @@ ivfpq_scan_generic_kernel(ScanArgs a) {
             if (valid) ++scanned_local;
             if constexpr (RANGE) {
                 const u64 key = make_key(sum, 0u, order_max);
-                const float api = order_max ? -key_score(key, 1) : key_score(key, 0);
-                bool pass = valid && api <= a.range.radius;
+                bool pass;
+                if (a.range.bound) {
+                    pass = valid && (uint32_t)(key >> 32) <= qbound;
+                } else {
+                    const float api = order_max ? -key_score(key, 1) : key_score(key, 0);
+                    pass = valid && api <= a.range.radius;
+                }
                 uint32_t id = 0;
                 if (pass) {
                     id = (uint32_t)a.slot_ids[g];

@@ -149,7 +149,8 @@ int range_empty(int64_t nq, vix_range_result** out) {
 }
 
 int range_collect_keys(int64_t nq, float radius, size_t& cap_hint, const std::function<int(const RangeOut&)>& scan,
-                       RangeKeys& rk, RangeInfo* info) {
+                       RangeKeys& rk, RangeInfo* info, const uint32_t* bound, const unsigned long long* flag_dev,
+                       unsigned long long* flag_host) {
     cudaStream_t s = ctx().stream;
     const size_t floor_cap = (size_t)(nq * 64 > 65536 ? nq * 64 : 65536);
     size_t cap = cap_hint > floor_cap ? cap_hint : floor_cap;
@@ -166,11 +167,13 @@ int range_collect_keys(int64_t nq, float radius, size_t& cap_hint, const std::fu
         VIX_CUDA(cudaMemsetAsync(ctr.ptr, 0, ((size_t)nq + 1) * 8, s));
         RangeOut o;
         o.keys = keys.ptr; o.qry = qry.ptr; o.cursor = ctr.ptr; o.counts = ctr.ptr + 1; o.cap = cap; o.radius = radius;
+        o.bound = bound;
         VIX_TRY(scan(o));
         ++passes;
         range_lims_kernel<<<1, 1024, 0, s>>>(o.counts, nq, rk.lims.ptr, ctr.ptr + 1 + nq);
         VIX_LAUNCH_CHECK();
         VIX_CUDA(cudaMemcpyAsync(h_info, ctr.ptr + 1 + nq, sizeof h_info, cudaMemcpyDeviceToHost, s));
+        if (flag_dev) VIX_CUDA(cudaMemcpyAsync(flag_host, flag_dev, sizeof *flag_host, cudaMemcpyDeviceToHost, s));
         VIX_CUDA(cudaStreamSynchronize(s));                   // the one synchronisation: the size of the answer
         if (h_info[0] <= cap) break;
         VIX_REQUIRE(passes == 1, VIX_ERR_CONTRACT, "range search: the second pass found %llu entries after a first count of %zu",

@@ -24,6 +24,11 @@ struct RangeOut {
     unsigned long long* counts = nullptr;      // [nq]  entries per query (written or added by the scan kernels)
     unsigned long long cap = 0;
     float radius = 0.0f;
+    // k-NN search beyond VIX_MAX_K (vix_knn_large.cu): when set, an entry passes when the high word of its key is at most
+    // bound[query] (the key space of make_key, so NaN distances pass a bound of 0xFFFFFFFF); radius is then not read.  The
+    // key is then the one the kind's k-NN search selects on: the IVF scans' as in range search, the flat engine's the
+    // score in the order of its metric (KnnDecode)
+    const uint32_t* bound = nullptr;           // [nq]
 };
 
 #ifdef __CUDACC__
@@ -66,9 +71,11 @@ struct RangeKeys {
 
 // Runs `scan` (which appends into the RangeOut it is handed and fills the per-query counts) once, or twice when the first
 // capacity (cap_hint, updated for the next call) is too small, then groups the entries by query and sorts each row.  The
-// only host synchronisation is the read of the total.
+// only host synchronisation is the read of the total.  bound: handed to the scan in RangeOut::bound.  flag_dev / flag_host:
+// a device word the scan writes, read in the same synchronisation as the total (the value after the last pass).
 int range_collect_keys(int64_t nq, float radius, size_t& cap_hint, const std::function<int(const RangeOut&)>& scan,
-                       RangeKeys& keys, RangeInfo* info);
+                       RangeKeys& keys, RangeInfo* info, const uint32_t* bound = nullptr,
+                       const unsigned long long* flag_dev = nullptr, unsigned long long* flag_host = nullptr);
 
 // sorted keys -> a new result object (lims copied from `lims`, device pointers).  neg_zero: the path reports a zero distance
 // as -0 (inner product through the flat engine and the IVF-PQ scan, whose API distance is the negated score); the key
@@ -92,6 +99,31 @@ __device__ __forceinline__ void range_decode_key(u64 key, int neg_zero, float* d
     *id = (int64_t)key_id(key);
 }
 #endif
+
+// ---- k-NN search for VIX_MAX_K < k <= VIX_MAX_K_LARGE (vix_knn_large.cu) ----
+constexpr int kKnnBeta = 2;                    // the seed covers about kKnnBeta * k candidates per query
+
+// what one call reports for the [vix knn] line of VIX_SCAN_DEBUG and vix_search_stats
+struct KnnInfo { int64_t seed = 0; RangeInfo collect; };
+
+// the seed's probe prefix of every query (device [nq x nprobe]); seed_cap: the stored vectors of all prefixes,
+// max_entries: those of all probes (synchronises the stream)
+int knn_probe_prefix(const int32_t* probes, int64_t nq, int nprobe, const int32_t* list_len, int kc, int k, int32_t* prefix,
+                     size_t* seed_cap, size_t* max_entries);
+
+// how a collected key becomes the reported distance: key_score(key, order_max), then dist_mode as the fused flat search
+// maps it (0 itself, 1 sqrt, 2 negated, 3 1 - score), and neg_zero as range_decode_key
+struct KnnDecode { int order_max = 0, dist_mode = 0, neg_zero = 0; };
+
+// seed (nullable: every candidate passes), collect with the per-query bound, cut -> out [nq x k] (device).  seed_cap: the
+// seed's capacity; max_entries: an upper bound of the candidates; cap_hint: the collect's first capacity, updated on success.
+int knn_large_run(int64_t nq, int k, KnnDecode dec, size_t seed_cap, const std::function<int(const RangeOut&)>* seed,
+                  const std::function<int(const RangeOut&)>& collect, size_t max_entries, size_t& cap_hint, float* out_dist,
+                  int64_t* out_ids, KnnInfo* info);
+
+// the flat engine's route (ids = row indices; disabled_rows: bit r set => row r skipped)
+int flat_knn_large_device(const float* q, int64_t nq, const float* xb, int64_t n, int d, int metric, int k,
+                          const uint64_t* disabled_rows, size_t& cap_hint, float* out_dist, int64_t* out_rows, KnnInfo* info);
 
 // an empty result of nq rows (lims all 0)
 int range_empty(int64_t nq, vix_range_result** out);

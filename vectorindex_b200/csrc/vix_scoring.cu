@@ -19,6 +19,8 @@
 #include "vix_range.cuh"
 
 #include <math.h>
+#include <stdio.h>
+#include <stdlib.h>
 
 namespace vix {
 
@@ -108,9 +110,15 @@ __global__ void __launch_bounds__(256) pair_kernel(PairArgs p) {
         for (int e = tid; e < TA; e += 256) { qthr[e] = kEmptyKey; qcnt[e] = 0; }
     }
     int* rcnt = nullptr;                                       // RANGE: entries per A row of this CTA
+    uint32_t bnd[TV];                                          // RANGE with a per-query key bound: the bound of each A row
     if (EPI == EPI_RANGE) {
         rcnt = reinterpret_cast<int*>(extra);
         for (int e = tid; e < TA; e += 256) rcnt[e] = 0;
+#pragma unroll
+        for (int v = 0; v < TV; ++v) {
+            const int64_t a = a0 + tx + 16 * v;
+            bnd[v] = p.range.bound && a < p.nA ? p.range.bound[a] : 0xFFFFFFFFu;
+        }
     }
 
     for (int64_t bt = bt0; bt < bt1; ++bt) {
@@ -148,8 +156,15 @@ __global__ void __launch_bounds__(256) pair_kernel(PairArgs p) {
                         const float f = fadd(apply_transform(p.transform, sc[v][c], p, a, b), 0.0f);
                         const float api = p.dist_mode == 1 ? __fsqrt_rn(f) : p.dist_mode == 2 ? -f
                                         : p.dist_mode == 3 ? fsub(1.0f, f) : f;
-                        pass = api <= p.range.radius;
-                        if (pass) key = make_key(api, (uint32_t)(p.row_ids ? p.row_ids[b] : b), 0);
+                        if (p.range.bound) {
+                            // k-NN beyond VIX_MAX_K: the selection key of the fused flat search (the score, in the order
+                            // of its metric), so that pairs whose API distances round together keep the fused order
+                            key = make_key(f, (uint32_t)(p.row_ids ? p.row_ids[b] : b), p.dist_mode >= 2);
+                            pass = (uint32_t)(key >> 32) <= bnd[v];
+                        } else {
+                            pass = api <= p.range.radius;
+                            if (pass) key = make_key(api, (uint32_t)(p.row_ids ? p.row_ids[b] : b), 0);
+                        }
                     }
                     const unsigned ball = __ballot_sync(0xFFFFFFFFu, pass);
                     if (ball) {
@@ -536,8 +551,8 @@ int flat_search_device(const float* q, int64_t nq, const float* xb, int64_t n, i
 
 // same scan with a row mask (bit b set => base row b is skipped): the pre-filter of FlatIndex.search (FlatIndex.swift:61)
 int flat_search_masked_device(const float* q, int64_t nq, const float* xb, int64_t n, int d, int metric, int k,
-                              const uint64_t* disabled_rows, float* out_dist, int64_t* out_ids) {
-    return flat_search_impl(q, nq, xb, n, d, metric, k, nullptr, out_dist, out_ids, false, disabled_rows);
+                              const uint64_t* disabled_rows, float* out_dist, int64_t* out_ids, bool raw_scores) {
+    return flat_search_impl(q, nq, xb, n, d, metric, k, nullptr, out_dist, out_ids, raw_scores, disabled_rows);
 }
 
 static int flat_search_impl(const float* q, int64_t nq, const float* xb, int64_t n, int d, int metric, int k,
@@ -938,8 +953,10 @@ int vix_flat_search_f32(const float* queries, int64_t nq, const float* xb, int64
     VIX_REQUIRE(d > 0 && n >= 0 && nq >= 0, VIX_ERR_INVALID_DIM, "vix_flat_search_f32: bad shape");
     VIX_REQUIRE(metric == VIX_METRIC_L2 || metric == VIX_METRIC_IP || metric == VIX_METRIC_COSINE, VIX_ERR_INVALID_PARAM,
                 "vix_flat_search_f32: metric");
-    VIX_REQUIRE(k <= VIX_MAX_K, VIX_ERR_INVALID_K, "vix_flat_search_f32: k > %d", VIX_MAX_K);
+    VIX_REQUIRE(k <= VIX_MAX_K_LARGE, VIX_ERR_INVALID_K, "vix_flat_search_f32: k > %d", VIX_MAX_K_LARGE);
     VIX_REQUIRE(n < (1LL << 32) - 1, VIX_ERR_INVALID_PARAM, "vix_flat_search_f32: n must be < 2^32 - 1");
+    VIX_REQUIRE(k <= VIX_MAX_K || nq < 0x7FFFFFFFLL, VIX_ERR_INVALID_PARAM, "vix_flat_search_f32: k > %d needs nq < 2^31 - 1",
+                VIX_MAX_K);
     In<float> dq, dx;
     Out<float> dd;
     Out<int64_t> di;
@@ -947,6 +964,15 @@ int vix_flat_search_f32(const float* queries, int64_t nq, const float* xb, int64
     VIX_TRY(dx.stage(xb, (size_t)n * d));
     VIX_TRY(dd.stage(out_dist, (size_t)nq * k));
     VIX_TRY(di.stage(out_ids, (size_t)nq * k));
+    if (k > VIX_MAX_K) {
+        // the two-pass route of vix_knn_large.cu (synchronises); the capacity hint lives for this call only
+        size_t cap = 0;
+        KnnInfo info;
+        VIX_TRY(flat_knn_large_device(dq.dev, nq, dx.dev, n, d, metric, k, nullptr, cap, dd.dev, di.dev, &info));
+        if (getenv("VIX_SCAN_DEBUG"))
+            fprintf(stderr, "[vix knn] kind flat, kernel flat, filter 0, k %d, seed %lld, total %lld, passes %d, max_row %lld\n", k,
+                    (long long)info.seed, (long long)info.collect.total, info.collect.passes, (long long)info.collect.max_row);
+    } else
     VIX_TRY(flat_search_auto_device(dq.dev, nq, dx.dev, n, d, metric, k, nullptr, dd.dev, di.dev, false));   // tensor-core shortlist + exact rescoring
     VIX_TRY(dd.commit());
     VIX_TRY(di.commit());
