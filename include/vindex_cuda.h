@@ -42,7 +42,11 @@
  *                            max_row M, sorted_long L" (L: rows longer than the in-shared-memory sort, merged in global memory);
  *                            and per vix_sharded_range_search call and rank (world > 1) one line "[vix sharded range] world W,
  *                            peer 0|1, local T_r, total T, max_row M, grown 0|1" (T_r: this rank's entries, M: the longest
- *                            merged row, grown: the range region of the communicator was (re)allocated by the call)
+ *                            merged row, grown: the range region of the communicator was (re)allocated by the call); and
+ *                            per vix_sharded_search / _filtered call with k > VIX_MAX_K and rank (world > 1) one line
+ *                            "[vix sharded knn] world W, peer 0|1, k K, seed S_r, local T_r, sent X_r, total T, max_row M,
+ *                            grown 0|1" (S_r: this rank's seed entries, T_r: its collected entries, X_r: those left after
+ *                            each row is cut at k, T: the merged entries before the cut at k)
  *   VIX_DISABLE_TC, VIX_DISABLE_PQ_TC, VIX_DISABLE_LUT_IMAGE
  *                            exact CUDA-core kernels instead of the tensor-core shortlists / per-query tables built inside
  *                            the scan instead of batch-wide (the parity tests compare both ways)
@@ -475,7 +479,20 @@ int vix_index_search_with_probes(vix_index_t* h, const float* queries, int64_t n
  *                        slot the shards do: rows inserted in the order the owners append them, i.e. rank 0's
  *                        contributions first.  A row in another slot of its list may differ in the last bit of its
  *                        distance (the slot decides the order its table entries are summed in).  Asynchronous mode: no host
- *                        synchronisation at all when the outputs are device pointers. */
+ *                        synchronisation at all when the outputs are device pointers (k <= VIX_MAX_K).
+ *                        k <= VIX_MAX_K_LARGE (above: VIX_ERR_INVALID_K; k > VIX_MAX_K with nq >= 2^31 - 1:
+ *                        VIX_ERR_INVALID_PARAM; both on every rank before any exchange), with the same parity, and
+ *                        search(k)[:, :k2] == search(k2) for every k2 <= k.  Above VIX_MAX_K (world > 1) the call takes
+ *                        the two-pass route of vix_index_search with one bound per query shared by all ranks: each rank
+ *                        seeds over the probes of the lists it owns that hold about 2 k vectors, the ranks take the
+ *                        minimum of their k-th seed distances (peer memory or an NCCL all-reduce), each rank collects
+ *                        the candidates within it from its probed lists and cuts every sorted row at k, and the cut rows
+ *                        are exchanged, merged and cut at k as sharded range search exchanges its rows (at most world x k
+ *                        keys per query travel).  That route synchronises the stream even in asynchronous mode.  A rank
+ *                        whose local pass fails makes every rank return its code; a merged answer that does not fit
+ *                        makes every rank return VIX_ERR_OOM; a merged row shorter than k within a finite bound (the two
+ *                        passes disagreed on a distance) makes every rank return VIX_ERR_CONTRACT.  One rank is
+ *                        vix_index_search. */
 typedef struct vix_comm vix_comm_t;
 int vix_comm_unique_id(void* id_out, size_t capacity /* >= 128 */);
 int vix_comm_create(const void* id, size_t id_bytes, int rank, int world, vix_comm_t** out);
@@ -484,8 +501,9 @@ int vix_comm_rank(const vix_comm_t* c);
 int vix_comm_world(const vix_comm_t* c);
 int vix_comm_uses_peer_memory(const vix_comm_t* c);        /* 1 peer memory, 0 NCCL all-gathers, -1 not decided yet */
 /* measurement aid: CUDA events around the three phases of the LAST vix_sharded_search, vix_sharded_search_filtered or
- * vix_sharded_range_search on this communicator -- probe selection + exchange | fused scan (range: local scan and sort) |
- * result exchange + merge (range: + decode) (ms; waits for that call to finish) */
+ * vix_sharded_range_search on this communicator -- probe selection + exchange | fused scan (range: local scan and sort;
+ * k > VIX_MAX_K: seed, bound exchange, collect and cut at k) | result exchange + merge (range: + decode; k > VIX_MAX_K:
+ * + cut at k) (ms; waits for that call to finish) */
 int vix_comm_trace(vix_comm_t* c, int enabled);
 int vix_comm_trace_get(vix_comm_t* c, float* phase_ms /* [3] */);
 /* rows [first, first + count) of a batch of nq queries are the block whose probe lists `rank` computes */
@@ -515,7 +533,7 @@ int vix_sharded_search(vix_index_t* h, vix_comm_t* c, const float* queries, int6
  *     the index unchanged; so does a failure of any rank's local scan (every rank returns that rank's code).  *out is
  *     released with vix_range_result_destroy.
  *   - Filtered k-NN: filter_words == NULL is vix_sharded_search; a filter sends each rank's scan down the query-major path,
- *     as on one GPU. */
+ *     as on one GPU.  k as vix_sharded_search: up to VIX_MAX_K_LARGE, the filter applied on both passes on every rank. */
 int vix_sharded_range_search(vix_index_t* h, vix_comm_t* c, const float* queries, int64_t nq, float radius, int nprobe,
                              const uint64_t* filter_words /* nullable */, int64_t filter_capacity, int filter_mode,
                              vix_range_result_t** out);
@@ -575,6 +593,13 @@ int vix_debug_shard_merge(const float* dist_all, const int64_t* ids_all, int wor
 int vix_debug_shard_range_merge(const int64_t* lims_all /* [world x (nq + 1)] */, const float* dist_all,
                                 const int64_t* ids_all /* concatenated rank by rank */, int world, int64_t nq, int metric,
                                 vix_range_result_t** out);
+
+/* Test hook: the merge and cut of vix_sharded_search with k > VIX_MAX_K on one GPU.  Input as vix_debug_shard_range_merge
+ * (each rank's rows sorted by (distance, id), of any length); the merged rows are cut at k into out [nq x k], padded with
+ * id -1 / NaN (host or device pointers; world 1 .. 256, 1 <= k <= VIX_MAX_K_LARGE). */
+int vix_debug_shard_knn_merge(const int64_t* lims_all /* [world x (nq + 1)] */, const float* dist_all,
+                              const int64_t* ids_all /* concatenated rank by rank */, int world, int64_t nq, int k, int metric,
+                              float* out_dist, int64_t* out_ids);
 
 /* a16  AccelerableIndex-shaped convenience (AccelerableIndex.swift:15-127): candidates [c x d]
  * contiguous in, (indices into candidates, distances) out, per query. */

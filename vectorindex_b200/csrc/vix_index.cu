@@ -806,6 +806,50 @@ static int index_remove_locked(vix_index* h, const int64_t* ids, int64_t n, int6
     return VIX_OK;
 }
 
+int ivf_range_scan(vix_index* h, const float* dq, int64_t nq, int nprobe, const int32_t* probes, const FilterArgs* filter,
+                   IvfRangeScan& out) {
+    const int d = h->p.d;
+    cudaStream_t s = ctx().stream;
+    if (h->p.kind == VIX_INDEX_IVF_PQ) {
+        ScanArgs a{};
+        a.queries = dq; a.nq = nq; a.d = d; a.m = h->p.m; a.ks = h->p.ks; a.dsub = d / h->p.m;
+        a.nprobe = nprobe; a.coarse = h->coarse.ptr; a.kc = h->kc; a.codebooks = h->codebooks.ptr;
+        a.list_off = h->list_off.ptr; a.list_len = h->list_len.ptr;
+        a.slot_codes = h->slot_codes.ptr; a.slot_tx = h->slot_tx.ptr; a.slot_ids = h->slot_ids.ptr;
+        a.metric = h->p.metric; a.codebooks_t = h->codebooks_t.ptr;
+        if (filter) { a.filter = filter->words; a.filter_cap = filter->cap; a.filter_deny = filter->deny; }
+        VIX_TRY(out.work_counter.alloc(2));
+        a.work_counter = out.work_counter.ptr;
+        const bool fast = scan_layout(a.m).fast && a.ks == 256;
+        if (fast && nq > 2 * num_sms()) {
+            VIX_TRY(query_order(probes, nq, nprobe, h->list_len.ptr, h->kc, out.order));
+            a.order = out.order.ptr;
+        }
+        if (fast) snprintf(out.kernel, sizeof out.kernel, "fast G %d", a.m / 16);
+        else snprintf(out.kernel, sizeof out.kernel, "generic");
+        out.run = [a](const int32_t* pr, const RangeOut& o) {
+            ScanArgs b = a;
+            b.probes = pr;
+            b.range = o;
+            return launch_ivfpq_scan_classic(b);
+        };
+        return VIX_OK;
+    }
+    snprintf(out.kernel, sizeof out.kernel, "ivfflat");
+    const size_t smem = (size_t)d * 4;
+    VIX_CUDA(cudaFuncSetAttribute(ivfflat_range_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const int64_t grid = std::min<int64_t>((int64_t)num_sms() * 4, nq);
+    const FilterArgs f = filter ? *filter : FilterArgs{};
+    out.run = [=](const int32_t* pr, const RangeOut& o) -> int {
+        ivfflat_range_kernel<<<(unsigned)grid, 256, smem, s>>>(dq, nq, d, pr, nprobe, h->list_off.ptr, h->list_len.ptr, h->kc,
+                                                             h->slot_vecs.ptr, h->slot_ids.ptr, h->p.metric, f.words, f.cap,
+                                                             f.deny, o);
+        VIX_LAUNCH_CHECK();
+        return VIX_OK;
+    };
+    return VIX_OK;
+}
+
 // k-NN search for VIX_MAX_K < k <= VIX_MAX_K_LARGE (vix_knn_large.cu): the candidates of index_search_locked (every row,
 // or the probed lists of the same probe selection / the caller's given_probes), a seed pass and a collect pass through the
 // kind's range kernel, the sorted rows cut at k.  Synchronises the stream (the collect's size depends on the data); not
@@ -877,49 +921,11 @@ static int index_knn_large_locked(vix_index* h, const float* queries, int64_t nq
         VIX_TRY(prefix.alloc((size_t)nq * nprobe));
         size_t seed_cap = 0, max_entries = 0;
         VIX_TRY(knn_probe_prefix(probes, nq, nprobe, h->list_len.ptr, h->kc, k, prefix.ptr, &seed_cap, &max_entries));
-        // the kind's range kernel over a probe list [nq x nprobe] (never the list-major tensor-core scan)
-        std::function<int(const int32_t*, const RangeOut&)> scan;
-        ScanArgs a{};
-        Scratch<int> work_counter;
-        Scratch<int32_t> order;
-        if (h->p.kind == VIX_INDEX_IVF_PQ) {
-            a.queries = dq.dev; a.nq = nq; a.d = d; a.m = h->p.m; a.ks = h->p.ks; a.dsub = d / h->p.m;
-            a.nprobe = nprobe; a.coarse = h->coarse.ptr; a.kc = h->kc; a.codebooks = h->codebooks.ptr;
-            a.list_off = h->list_off.ptr; a.list_len = h->list_len.ptr;
-            a.slot_codes = h->slot_codes.ptr; a.slot_tx = h->slot_tx.ptr; a.slot_ids = h->slot_ids.ptr;
-            a.metric = h->p.metric; a.codebooks_t = h->codebooks_t.ptr;
-            if (filter) { a.filter = filter->words; a.filter_cap = filter->cap; a.filter_deny = filter->deny; }
-            VIX_TRY(work_counter.alloc(2));
-            a.work_counter = work_counter.ptr;
-            const bool fast = scan_layout(a.m).fast && a.ks == 256;
-            if (fast && nq > 2 * num_sms()) {
-                VIX_TRY(query_order(probes, nq, nprobe, h->list_len.ptr, h->kc, order));
-                a.order = order.ptr;
-            }
-            if (fast) snprintf(kernel, sizeof kernel, "fast G %d", a.m / 16);
-            else snprintf(kernel, sizeof kernel, "generic");
-            scan = [&](const int32_t* pr, const RangeOut& o) {
-                ScanArgs b = a;
-                b.probes = pr;
-                b.range = o;
-                return launch_ivfpq_scan_classic(b);
-            };
-        } else {
-            snprintf(kernel, sizeof kernel, "ivfflat");
-            const size_t smem = (size_t)d * 4;
-            VIX_CUDA(cudaFuncSetAttribute(ivfflat_range_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            const int64_t grid = std::min<int64_t>((int64_t)num_sms() * 4, nq);
-            scan = [&, smem, grid](const int32_t* pr, const RangeOut& o) -> int {
-                ivfflat_range_kernel<<<(unsigned)grid, 256, smem, s>>>(dq.dev, nq, d, pr, nprobe, h->list_off.ptr, h->list_len.ptr,
-                                                                     h->kc, h->slot_vecs.ptr, h->slot_ids.ptr, h->p.metric,
-                                                                     filter ? filter->words : nullptr, filter ? filter->cap : 0,
-                                                                     filter ? filter->deny : 0, o);
-                VIX_LAUNCH_CHECK();
-                return VIX_OK;
-            };
-        }
-        const std::function<int(const RangeOut&)> seed = [&](const RangeOut& o) { return scan(prefix.ptr, o); };
-        const std::function<int(const RangeOut&)> collect = [&](const RangeOut& o) { return scan(probes, o); };
+        IvfRangeScan scan;
+        VIX_TRY(ivf_range_scan(h, dq.dev, nq, nprobe, probes, filter, scan));
+        snprintf(kernel, sizeof kernel, "%s", scan.kernel);
+        const std::function<int(const RangeOut&)> seed = [&](const RangeOut& o) { return scan.run(prefix.ptr, o); };
+        const std::function<int(const RangeOut&)> collect = [&](const RangeOut& o) { return scan.run(probes, o); };
         // (IVF-PQ reports a zero inner-product distance as -0, IVF-Flat keys the distance itself: +0)
         KnnDecode dec;
         dec.neg_zero = h->p.kind == VIX_INDEX_IVF_PQ && h->p.metric == VIX_METRIC_IP;

@@ -4,6 +4,7 @@
 
 #include "vix_common.cuh"
 
+#include <functional>
 #include <mutex>
 #include <vector>
 
@@ -145,6 +146,20 @@ int index_search_locked(vix_index* h, const float* queries, int64_t nq, int k, i
 struct RangeKeys;
 int index_range_locked(vix_index* h, const float* queries, int64_t nq, float radius, int nprobe, const FilterArgs* filter,
                        vix_range_result** out, const int32_t* given_probes = nullptr, RangeKeys* keys_out = nullptr);
+// The kind's range kernel over a probe list [nq x nprobe] of an IVF index with built lists (IVF-PQ: the query-major scan,
+// fast or generic, never the list-major one; IVF-Flat: ivfflat_range_kernel), with the id filter: what both passes of k-NN
+// search beyond VIX_MAX_K run, on one GPU and on every rank of a sharded call.  probes: the list the work order is computed
+// from (the fast kernel's locality order for nq > 2 x SMs); run() takes that list or a prefix of it.  dq: device queries
+// that outlive the object.
+struct RangeOut;
+struct IvfRangeScan {
+    Scratch<int> work_counter;
+    Scratch<int32_t> order;
+    std::function<int(const int32_t*, const RangeOut&)> run;
+    char kernel[32] = "";               // the [vix knn] line's kernel name
+};
+int ivf_range_scan(vix_index* h, const float* dq, int64_t nq, int nprobe, const int32_t* probes, const FilterArgs* filter,
+                   IvfRangeScan& out);
 // list assignment under the index's metric (device pointers)
 int assign_lists_device(vix_index* h, const float* x, int64_t n, int32_t* assign);
 // number of assignments outside [0, kc) in a device array (synchronises the stream)

@@ -16,6 +16,9 @@
 //
 // The two passes must agree on every distance (they run the same kernels on the same data): a row shorter than k whose
 // bound is not 0xFFFFFFFF means they did not, and the call fails with VIX_ERR_CONTRACT.
+//
+// The halves are separate (knn_seed_bound, knn_collect) because sharded search (vix_sharded.cu) runs the seed on every rank,
+// takes the minimum of the ranks' bounds between them, and exchanges each rank's collected rows cut at k (knn_trim).
 #include "vix_common.cuh"
 #include "vix_index.cuh"
 #include "vix_range.cuh"
@@ -110,6 +113,25 @@ __global__ void knn_cut_kernel(const u64* __restrict__ sorted, const int64_t* __
     } else { out_dist[e] = __int_as_float(0x7fc00000); out_ids[e] = -1; }
 }
 
+// counts[q] = min(k, row length): the keys of row q that can still belong to a top k
+__global__ void knn_trim_counts_kernel(const int64_t* __restrict__ lims, int64_t nq, int k,
+                                       unsigned long long* __restrict__ counts) {
+    const int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= nq) return;
+    const int64_t len = lims[q + 1] - lims[q];
+    counts[q] = (unsigned long long)(len < k ? len : k);
+}
+
+// the first min(k, row length) keys of every sorted row, compacted at the new row starts out_lims (one CTA per row)
+__global__ void __launch_bounds__(256)
+knn_trim_kernel(const u64* __restrict__ sorted, const int64_t* __restrict__ lims, int64_t nq, int k,
+                const int64_t* __restrict__ out_lims, u64* __restrict__ out) {
+    for (int64_t q = blockIdx.x; q < nq; q += gridDim.x) {
+        const int64_t lo = lims[q], olo = out_lims[q], n = out_lims[q + 1] - olo;
+        for (int64_t i = threadIdx.x; i < n; i += blockDim.x) out[olo + i] = sorted[lo + i];
+    }
+}
+
 int knn_probe_prefix(const int32_t* probes, int64_t nq, int nprobe, const int32_t* list_len, int kc, int k,
                      int32_t* prefix, size_t* seed_cap, size_t* max_entries) {
     cudaStream_t s = ctx().stream;
@@ -127,39 +149,74 @@ int knn_probe_prefix(const int32_t* probes, int64_t nq, int nprobe, const int32_
     return VIX_OK;
 }
 
+int knn_seed_bound(int64_t nq, int k, size_t seed_cap, const std::function<int(const RangeOut&)>* seed, uint32_t* bound,
+                   int64_t* seed_total) {
+    cudaStream_t s = ctx().stream;
+    VIX_CUDA(cudaMemsetAsync(bound, 0xFF, (size_t)nq * 4, s));           // every candidate passes (the seed's own bound)
+    *seed_total = 0;
+    if (!seed) return VIX_OK;
+    RangeKeys srk;
+    RangeInfo si;
+    VIX_TRY(range_collect_keys(nq, INFINITY, seed_cap, *seed, srk, &si, bound));
+    *seed_total = srk.total;
+    if (srk.total > 0) {
+        knn_bound_kernel<<<(unsigned)((nq + 255) / 256), 256, 0, s>>>(srk.sorted, srk.lims.ptr, nq, k, bound);
+        VIX_LAUNCH_CHECK();
+    }
+    return VIX_OK;
+}
+
+int knn_collect(int64_t nq, int k, const uint32_t* bound, const std::function<int(const RangeOut&)>& collect,
+                size_t max_entries, size_t& cap, RangeKeys& rk, RangeInfo* info, unsigned long long* short_rows) {
+    cudaStream_t s = ctx().stream;
+    // first capacity: the hint of the last call, at least kKnnBeta k per query, never more than the candidates
+    const size_t floor_cap = std::min((size_t)kKnnBeta * (size_t)k * (size_t)nq, max_entries);
+    if (cap < floor_cap) cap = floor_cap;
+    if (!short_rows) return range_collect_keys(nq, INFINITY, cap, collect, rk, info, bound);
+    Scratch<unsigned long long> flag;
+    VIX_TRY(flag.alloc(1));
+    auto checked = [&](const RangeOut& o) -> int {
+        VIX_CUDA(cudaMemsetAsync(flag.ptr, 0, 8, s));
+        VIX_TRY(collect(o));
+        knn_short_kernel<<<(unsigned)((nq + 255) / 256), 256, 0, s>>>(o.counts, o.bound, nq, k, flag.ptr);
+        VIX_LAUNCH_CHECK();
+        return VIX_OK;
+    };
+    *short_rows = 0;
+    return range_collect_keys(nq, INFINITY, cap, checked, rk, info, bound, flag.ptr, short_rows);
+}
+
+int knn_trim(int64_t nq, int k, const RangeKeys& rk, RangeKeys& out) {
+    cudaStream_t s = ctx().stream;
+    VIX_TRY(out.lims.alloc((size_t)nq + 1));
+    Scratch<unsigned long long> cnt;                                     // [counts nq][scan info 3]
+    VIX_TRY(cnt.alloc((size_t)nq + 3));
+    knn_trim_counts_kernel<<<(unsigned)((nq + 255) / 256), 256, 0, s>>>(rk.lims.ptr, nq, k, cnt.ptr);
+    VIX_LAUNCH_CHECK();
+    VIX_TRY(range_lims(cnt.ptr, nq, out.lims.ptr, cnt.ptr + nq));
+    // (the trimmed total stays on the device: the exchange of the row starts carries it)
+    out.total = std::min<int64_t>(rk.total, nq * (int64_t)k);
+    out.sorted = nullptr;
+    if (out.total == 0) return VIX_OK;
+    VIX_TRY(out.a.alloc((size_t)out.total));
+    out.sorted = out.a.ptr;
+    const unsigned grid = (unsigned)std::min<int64_t>((int64_t)num_sms() * 8, nq);
+    knn_trim_kernel<<<grid, 256, 0, s>>>(rk.sorted, rk.lims.ptr, nq, k, out.lims.ptr, out.a.ptr);
+    VIX_LAUNCH_CHECK();
+    return VIX_OK;
+}
+
 int knn_large_run(int64_t nq, int k, KnnDecode dec, size_t seed_cap, const std::function<int(const RangeOut&)>* seed,
                   const std::function<int(const RangeOut&)>& collect, size_t max_entries, size_t& cap_hint, float* out_dist,
                   int64_t* out_ids, KnnInfo* info) {
     cudaStream_t s = ctx().stream;
-    const unsigned grid_q = (unsigned)((nq + 255) / 256);
     Scratch<uint32_t> bound;
     VIX_TRY(bound.alloc((size_t)nq));
-    VIX_CUDA(cudaMemsetAsync(bound.ptr, 0xFF, (size_t)nq * 4, s));       // every candidate passes (the seed's own bound)
-    if (seed) {
-        RangeKeys srk;
-        RangeInfo si;
-        VIX_TRY(range_collect_keys(nq, INFINITY, seed_cap, *seed, srk, &si, bound.ptr));
-        info->seed = srk.total;
-        if (srk.total > 0) {
-            knn_bound_kernel<<<grid_q, 256, 0, s>>>(srk.sorted, srk.lims.ptr, nq, k, bound.ptr);
-            VIX_LAUNCH_CHECK();
-        }
-    }
-    Scratch<unsigned long long> flag;
-    VIX_TRY(flag.alloc(1));
+    VIX_TRY(knn_seed_bound(nq, k, seed_cap, seed, bound.ptr, &info->seed));
+    size_t cap = cap_hint;
     unsigned long long short_rows = 0;
-    auto checked = [&](const RangeOut& o) -> int {
-        VIX_CUDA(cudaMemsetAsync(flag.ptr, 0, 8, s));
-        VIX_TRY(collect(o));
-        knn_short_kernel<<<grid_q, 256, 0, s>>>(o.counts, o.bound, nq, k, flag.ptr);
-        VIX_LAUNCH_CHECK();
-        return VIX_OK;
-    };
-    // first capacity: the hint of the last call, at least kKnnBeta k per query, never more than the candidates
-    const size_t floor_cap = std::min((size_t)kKnnBeta * (size_t)k * (size_t)nq, max_entries);
-    size_t cap = cap_hint > floor_cap ? cap_hint : floor_cap;
     RangeKeys rk;
-    VIX_TRY(range_collect_keys(nq, INFINITY, cap, checked, rk, &info->collect, bound.ptr, flag.ptr, &short_rows));
+    VIX_TRY(knn_collect(nq, k, bound.ptr, collect, max_entries, cap, rk, &info->collect, &short_rows));
     VIX_REQUIRE(short_rows == 0, VIX_ERR_CONTRACT,
                 "k-NN search (k = %d): %llu queries collected fewer than k entries within the bound their seed pass found",
                 k, short_rows);

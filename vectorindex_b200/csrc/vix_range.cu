@@ -119,6 +119,12 @@ __global__ void range_decode_kernel(const u64* __restrict__ keys, int64_t total,
     range_decode_key(keys[i], neg_zero, dist + i, ids + i);
 }
 
+int range_lims(const unsigned long long* counts, int64_t nq, int64_t* lims, unsigned long long* info) {
+    range_lims_kernel<<<1, 1024, 0, ctx().stream>>>(counts, nq, lims, info);
+    VIX_LAUNCH_CHECK();
+    return VIX_OK;
+}
+
 void range_free(vix_range_result* r) {
     if (!r) return;
     if (r->lims) cudaFree(r->lims);

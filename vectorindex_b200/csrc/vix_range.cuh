@@ -121,6 +121,22 @@ int knn_large_run(int64_t nq, int k, KnnDecode dec, size_t seed_cap, const std::
                   const std::function<int(const RangeOut&)>& collect, size_t max_entries, size_t& cap_hint, float* out_dist,
                   int64_t* out_ids, KnnInfo* info);
 
+// The halves of knn_large_run.  knn_seed_bound: bound [nq] (device) <- the word of each row's k-th sorted seed key,
+// 0xFFFFFFFF where the seed holds fewer than k or there is no seed (seed nullable); *seed_total: the seed's entries.
+int knn_seed_bound(int64_t nq, int k, size_t seed_cap, const std::function<int(const RangeOut&)>* seed, uint32_t* bound,
+                   int64_t* seed_total);
+// knn_collect: the candidates within the bound, grouped and sorted (rk).  cap: in, the hint of the last call; out, the
+// next call's.  short_rows (nullable): the queries whose row is shorter than k although their bound is finite.
+int knn_collect(int64_t nq, int k, const uint32_t* bound, const std::function<int(const RangeOut&)>& collect,
+                size_t max_entries, size_t& cap, RangeKeys& rk, RangeInfo* info, unsigned long long* short_rows);
+// the first min(k, row length) keys of every sorted row of rk, compacted with new row starts (out.lims, device).  out.total
+// is an upper bound (min(rk.total, nq k)); the exact total is out.lims[nq] on the device.
+int knn_trim(int64_t nq, int k, const RangeKeys& rk, RangeKeys& out);
+
+// lims = exclusive scan of counts [nq] (lims[nq] = total), info [3] = {total, longest row, rows longer than the in-shared-
+// memory sort} (device pointers, one launch)
+int range_lims(const unsigned long long* counts, int64_t nq, int64_t* lims, unsigned long long* info);
+
 // the flat engine's route (ids = row indices; disabled_rows: bit r set => row r skipped)
 int flat_knn_large_device(const float* q, int64_t nq, const float* xb, int64_t n, int d, int metric, int k,
                           const uint64_t* disabled_rows, size_t& cap_hint, float* out_dist, int64_t* out_rows, KnnInfo* info);

@@ -27,6 +27,8 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <algorithm>
+#include <functional>
 #include <new>
 #include <vector>
 
@@ -116,13 +118,16 @@ struct vix_comm {
     // NCCL path: plain local buffers with the same roles
     void* gather_probes = nullptr; size_t gather_probes_bytes = 0;
     void* gather_keys = nullptr; size_t gather_keys_bytes = 0;
-    // range search: a second region, mapped like the first (peer memory only), grown collectively and geometrically:
-    //   [lims: world x (nq + 2) i64 -- each rank's local CSR row starts + its status][keys: the global answer's sorted keys,
-    //   rank by rank]
+    // range search (and k-NN search beyond VIX_MAX_K): a second region, mapped like the first (peer memory only), grown
+    // collectively and geometrically:
+    //   [lims: world x (nq + 2) i64 -- each rank's local CSR row starts + its status]
+    //   [bounds: world x nq u32 -- each rank's k-NN seed bounds; apart from the lims, which a fast peer may already store
+    //    while this rank still reads the bounds]
+    //   [keys: the global answer's sorted keys, rank by rank]
     void* range_local = nullptr;
     std::vector<void*> range_peer;
     void** range_peer_dev = nullptr;
-    size_t range_off_keys = 0;
+    size_t range_off_bounds = 0, range_off_keys = 0;
     int64_t range_cap_nq = 0, range_cap_keys = 0;
     // optional phase events of the last search (vix_comm_trace): start | probes exchanged | scanned | merged
     bool trace = false;
@@ -409,41 +414,109 @@ __global__ void shard_range_lims_kernel(const int64_t* __restrict__ lims_all, in
     }
 }
 
-// The merge of the ranks' sorted runs into the global rows, decoded on the way (range_decode_key).  keys: every rank's local
-// answer, concatenated rank by rank (rank r's from base[r]); lims_all as above; glims: the global row starts.  Rank r's key
-// at place i of its row q goes to glims[q] + i + (keys of the lower ranks' rows q that are <= it) + (keys of the higher
-// ranks' rows q that are < it): one thread per key, a binary search in each other run.  Stable, and exact for equal keys
-// on different ranks (one id stored in lists two ranks own): they keep rank order, as one GPU's rows would hold them.
+// The merge of the ranks' sorted runs of every row.  keys: every rank's rows, concatenated rank by rank (rank r's from
+// base[r]); lims_all as above.  Key i, at place j of rank r's run of row q, has place j + (keys of the lower ranks' runs of
+// row q that are <= it) + (keys of the higher ranks' runs of row q that are < it) in the merged row q: one binary search in
+// each other run.  Stable, and exact for equal keys on different ranks (one id stored in lists two ranks own): they keep
+// rank order, as one GPU's rows would hold them.  Returns that place, *row = q.
+__device__ __forceinline__ int64_t shard_merge_place(const u64* __restrict__ keys, const int64_t* __restrict__ base,
+                                                     const int64_t* __restrict__ lims_all, int world, int64_t nq, int64_t i,
+                                                     int64_t* row) {
+    const int64_t L = nq + 2;
+    int ra = 0, rb = world;                                   // rank of i: the last r with base[r] <= i
+    while (rb - ra > 1) { const int mid = (ra + rb) >> 1; if (base[mid] <= i) ra = mid; else rb = mid; }
+    const int r = ra;
+    const int64_t* lr = lims_all + (size_t)r * L;
+    const int64_t j = i - base[r];
+    int64_t qa = 0, qb = nq;                                  // its row: the last q with lr[q] <= j
+    while (qb - qa > 1) { const int64_t mid = (qa + qb) >> 1; if (lr[mid] <= j) qa = mid; else qb = mid; }
+    const int64_t q = qa;
+    const u64 key = keys[i];
+    int64_t pos = j - lr[q];
+    for (int p = 0; p < world; ++p) {
+        if (p == r) continue;
+        const int64_t* lp = lims_all + (size_t)p * L;
+        const u64* run = keys + base[p] + lp[q];
+        int64_t x = 0, y = lp[q + 1] - lp[q];
+        if (p < r) {
+            while (x < y) { const int64_t mid = (x + y) >> 1; if (run[mid] <= key) x = mid + 1; else y = mid; }
+        } else {
+            while (x < y) { const int64_t mid = (x + y) >> 1; if (run[mid] < key) x = mid + 1; else y = mid; }
+        }
+        pos += x;
+    }
+    *row = q;
+    return pos;
+}
+
+// range search: every key to its place in the global rows (glims: their starts), decoded on the way (range_decode_key)
 __global__ void __launch_bounds__(256)
 shard_range_merge_kernel(const u64* __restrict__ keys, const int64_t* __restrict__ base, const int64_t* __restrict__ lims_all,
                          int world, int64_t nq, const int64_t* __restrict__ glims, int64_t total, int neg_zero,
                          float* __restrict__ out_dist, int64_t* __restrict__ out_ids) {
-    const int64_t L = nq + 2;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
-        int ra = 0, rb = world;                               // rank of i: the last r with base[r] <= i
-        while (rb - ra > 1) { const int mid = (ra + rb) >> 1; if (base[mid] <= i) ra = mid; else rb = mid; }
-        const int r = ra;
-        const int64_t* lr = lims_all + (size_t)r * L;
-        const int64_t j = i - base[r];
-        int64_t qa = 0, qb = nq;                              // its row: the last q with lr[q] <= j
-        while (qb - qa > 1) { const int64_t mid = (qa + qb) >> 1; if (lr[mid] <= j) qa = mid; else qb = mid; }
-        const int64_t q = qa;
-        const u64 key = keys[i];
-        int64_t pos = glims[q] + (j - lr[q]);
-        for (int p = 0; p < world; ++p) {
-            if (p == r) continue;
-            const int64_t* lp = lims_all + (size_t)p * L;
-            const u64* run = keys + base[p] + lp[q];
-            int64_t x = 0, y = lp[q + 1] - lp[q];
-            if (p < r) {
-                while (x < y) { const int64_t mid = (x + y) >> 1; if (run[mid] <= key) x = mid + 1; else y = mid; }
-            } else {
-                while (x < y) { const int64_t mid = (x + y) >> 1; if (run[mid] < key) x = mid + 1; else y = mid; }
-            }
-            pos += x;
-        }
-        range_decode_key(key, neg_zero, out_dist + pos, out_ids + pos);
+        int64_t q;
+        const int64_t place = shard_merge_place(keys, base, lims_all, world, nq, i, &q);
+        const int64_t pos = glims[q] + place;
+        range_decode_key(keys[i], neg_zero, out_dist + pos, out_ids + pos);
     }
+}
+
+// k-NN search beyond VIX_MAX_K: the merged rows cut at k, straight into out [nq x k]: a key is written only when its place
+// is < k; the places of a row from its length (glims) to k are padded with id -1 / NaN.
+//
+// Exactness of the sharded route (sharded_knn_large).  Let C be a query's global candidate multiset, C = the union over
+// the ranks of C_r (the probed lists rank r owns).  Each rank's seed S_r, a subset of C_r with |S_r| >= k, gives tau_r >=
+// the k-th word of C; so does tau = min_r tau_r (tau_r = 0xFFFFFFFF when |S_r| < k).  The keys of C with word <= tau hold
+// the true top k and every tie at the k-th distance.  The global top k restricted to C_r is a prefix of rank r's sorted
+// collected row of length at most k, so cutting each row at k before the exchange loses nothing, and the merged rows cut at
+// k are the one-GPU answer.  If tau != 0xFFFFFFFF, the rank that attained it holds at least k keys within it, so the merged
+// row holds at least k; a shorter one means the two passes disagreed on a distance (shard_knn_short_kernel).  At most
+// world x k keys per query travel, and that many only when no rank's seed reaches k.
+__global__ void __launch_bounds__(256)
+shard_knn_merge_kernel(const u64* __restrict__ keys, const int64_t* __restrict__ base, const int64_t* __restrict__ lims_all,
+                       int world, int64_t nq, const int64_t* __restrict__ glims, int64_t total, int k, int neg_zero,
+                       float* __restrict__ out_dist, int64_t* __restrict__ out_ids) {
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += stride) {
+        int64_t q;
+        const int64_t place = shard_merge_place(keys, base, lims_all, world, nq, i, &q);
+        if (place < k) range_decode_key(keys[i], neg_zero, out_dist + q * k + place, out_ids + q * k + place);
+    }
+    for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < nq * (int64_t)k; e += stride) {
+        const int64_t q = e / k, j = e - q * k;
+        if (j >= glims[q + 1] - glims[q]) { out_dist[e] = __int_as_float(0x7fc00000); out_ids[e] = -1; }
+    }
+}
+
+// flag += queries whose merged row (the sum of the ranks' trimmed rows, lims_all as above) is shorter than k although their
+// bound is finite
+__global__ void shard_knn_short_kernel(const int64_t* __restrict__ lims_all, int world, int64_t nq, int k,
+                                       const uint32_t* __restrict__ bound, unsigned long long* __restrict__ flag) {
+    const int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= nq) return;
+    int64_t len = 0;
+    for (int r = 0; r < world; ++r) len += lims_all[(size_t)r * (nq + 2) + q + 1] - lims_all[(size_t)r * (nq + 2) + q];
+    if (len < k && bound[q] != 0xFFFFFFFFu) atomicAdd(flag, 1ull);
+}
+
+// The ranks' k-NN seed bounds over peer memory: tau [nq] -> slot `rank` of the bound slice [world][stride] of every rank's
+// range region (this rank's included); after a barrier, tau = the minimum of the slots here.  The minimum is unsigned: the
+// key words order like the distances (make_key), NaN's word being the largest.
+__global__ void push_knn_bounds_kernel(const uint32_t* __restrict__ tau, int64_t nq, void* const* __restrict__ peer_base,
+                                       int world, size_t off) {
+    for (int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; q < nq; q += (int64_t)gridDim.x * blockDim.x) {
+        const uint32_t v = tau[q];
+        for (int p = 0; p < world; ++p) reinterpret_cast<uint32_t*>(static_cast<char*>(peer_base[p]) + off)[q] = v;
+    }
+}
+__global__ void min_knn_bounds_kernel(const uint32_t* __restrict__ slots, int world, int64_t stride, int64_t nq,
+                                      uint32_t* __restrict__ tau) {
+    const int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= nq) return;
+    uint32_t v = 0xFFFFFFFFu;
+    for (int r = 0; r < world; ++r) v = min(v, slots[(size_t)r * stride + q]);
+    tau[q] = v;
 }
 
 // lims_all [world][nq + 2] on the device -> glims [nq + 1] (device) and meta (host: base [world + 1], longest row, statuses
@@ -477,6 +550,16 @@ static int shard_range_merge(const u64* keys, const int64_t* base_dev, const int
     return VIX_OK;
 }
 
+static int shard_knn_merge(const u64* keys, const int64_t* base_dev, const int64_t* lims_all, int world, int64_t nq,
+                           const int64_t* glims, int64_t total, int k, int metric, float* out_dist, int64_t* out_ids) {
+    const int64_t want = (std::max<int64_t>(total, nq * (int64_t)k) + 255) / 256;
+    const unsigned grid = (unsigned)(want < (int64_t)num_sms() * 8 ? want : (int64_t)num_sms() * 8);
+    shard_knn_merge_kernel<<<grid, 256, 0, ctx().stream>>>(keys, base_dev, lims_all, world, nq, glims, total, k,
+                                                           metric == VIX_METRIC_IP ? 1 : 0, out_dist, out_ids);
+    VIX_LAUNCH_CHECK();
+    return VIX_OK;
+}
+
 static void close_range_peers(vix_comm* c) {
     for (int p = 0; p < (int)c->range_peer.size(); ++p)
         if (p != c->rank && c->range_peer[p]) cudaIpcCloseMemHandle(c->range_peer[p]);
@@ -499,7 +582,8 @@ static int ensure_range_region(vix_comm* c, int64_t nq, int64_t keys, bool* grow
     while (cnq < nq) cnq *= 2;
     int64_t ck = c->range_cap_keys > 65536 ? c->range_cap_keys : 65536;
     if (ck < keys) ck = keys + keys / 8 > 2 * ck ? keys + keys / 8 : 2 * ck;
-    const size_t off_k = ((size_t)world * (cnq + 2) * 8 + 255) & ~(size_t)255;
+    const size_t off_b = ((size_t)world * (cnq + 2) * 8 + 255) & ~(size_t)255;
+    const size_t off_k = (off_b + (size_t)world * cnq * 4 + 255) & ~(size_t)255;
     const size_t total = off_k + (size_t)ck * 8;
     VIX_CUDA(cudaStreamSynchronize(s));                                   // nothing of mine still reads or writes the old one
     void* fresh = nullptr;
@@ -550,7 +634,7 @@ static int ensure_range_region(vix_comm* c, int64_t nq, int64_t keys, bool* grow
     VIX_CUDA(cudaMemcpyAsync(pdev, peer.data(), sizeof(void*) * world, cudaMemcpyHostToDevice, s));
     VIX_CUDA(cudaStreamSynchronize(s));
     c->range_local = fresh; c->range_peer = peer; c->range_peer_dev = pdev;
-    c->range_off_keys = off_k; c->range_cap_nq = cnq; c->range_cap_keys = ck;
+    c->range_off_bounds = off_b; c->range_off_keys = off_k; c->range_cap_nq = cnq; c->range_cap_keys = ck;
     *grown = true;
     return VIX_OK;
 }
@@ -719,7 +803,12 @@ static int stage_filter(const uint64_t* words, int64_t capacity, int mode, In<ui
     return VIX_OK;
 }
 
-// vix_sharded_search and vix_sharded_search_filtered (filter == nullptr: the unfiltered step, launch for launch)
+// forward: k > VIX_MAX_K at world > 1 (below)
+static int sharded_knn_large(vix_index* h, vix_comm* c, const float* queries, int64_t nq, int k, int nprobe,
+                             const FilterArgs* filter, float* out_dist, int64_t* out_ids);
+
+// vix_sharded_search and vix_sharded_search_filtered (filter == nullptr: the unfiltered step, launch for launch; k above
+// VIX_MAX_K at world > 1: sharded_knn_large)
 static int sharded_search(vix_index* h, vix_comm* c, const float* queries, int64_t nq, int k, int nprobe, const FilterArgs* filter,
                           float* out_dist, int64_t* out_ids) {
     std::lock_guard<std::mutex> lc(c->mu);
@@ -730,8 +819,9 @@ static int sharded_search(vix_index* h, vix_comm* c, const float* queries, int64
     VIX_REQUIRE(nprobe > 0 && nprobe <= VIX_MAX_K, VIX_ERR_INVALID_K, "vix_sharded_search: nprobe");
     const int world = c->world, rank = c->rank, d = h->p.d;
     if (world == 1) return index_search_locked(h, queries, nq, k, nprobe, out_dist, out_ids, nullptr, nullptr, nullptr, filter);
-    cudaStream_t s = ctx().stream;
     if (h->dirty) VIX_TRY(build_lists(h));
+    if (k > VIX_MAX_K) return sharded_knn_large(h, c, queries, nq, k, nprobe, filter, out_dist, out_ids);
+    cudaStream_t s = ctx().stream;
     VIX_TRY(ensure_region(c, nq, d, nprobe, k));
     ThrHookScope thr_scope(c);                                        // (cleared again on every way out)
     const int64_t total = nq * (int64_t)k;
@@ -780,15 +870,30 @@ static int sharded_search(vix_index* h, vix_comm* c, const float* queries, int64
     return finish(dd.is_host() || di.is_host());
 }
 
-// The range step after the probe exchange: the local scan's sorted keys and lims (rc: its status) -> every rank's lims and
-// status (peer region + barrier, or all-gather) -> global row starts and total (synchronises) -> the keys of every rank
-// (peer region + barrier, or grouped send / receive) -> merge and decode into a new result object.
-static int sharded_range_exchange(vix_index* h, vix_comm* c, int64_t nq, int rc, RangeKeys& rk, bool grown,
-                                  vix_range_result** out) {
+// The last step of sharded_range_exchange: range search decodes the merged rows into a new result object (*out); k-NN
+// search beyond VIX_MAX_K (out == nullptr) cuts them at k into [nq x k] (dist, ids: device), after checking on the exchanged
+// row starts that no row whose bound is finite came out shorter than k.
+struct ShardTail {
+    vix_range_result** out = nullptr;
+    int k = 0;
+    const uint32_t* bound = nullptr;
+    float* dist = nullptr;
+    int64_t* ids = nullptr;
+};
+// what the exchange reports for the VIX_SCAN_DEBUG lines: this rank's entries, the merged entries, the longest merged row
+struct ShardTotals { int64_t mine = 0, total = 0, max_row = 0; bool grown = false; };
+
+// The step after each rank's local pass: its sorted keys and lims (rc: its status) -> every rank's lims and status (peer
+// region + barrier, or all-gather) -> global row starts and total (synchronises) -> the keys of every rank (peer region +
+// barrier, or grouped send / receive) -> merge, then the tail's last step.
+static int sharded_range_exchange(vix_index* h, vix_comm* c, int64_t nq, int rc, RangeKeys& rk, bool grown, const ShardTail& t,
+                                  ShardTotals* st) {
     cudaStream_t s = ctx().stream;
     const int world = c->world, rank = c->rank;
     const int64_t L = nq + 2;
     const bool peer = c->peer_state == 1;
+    const bool knn = t.out == nullptr;
+    const char* who = knn ? "vix_sharded_search" : "vix_sharded_range_search";
     Scratch<int64_t> mine, lims_all, glims, dbase;
     VIX_TRY(mine.alloc((size_t)L));
     VIX_TRY(lims_all.alloc((size_t)world * L));
@@ -809,18 +914,32 @@ static int sharded_range_exchange(vix_index* h, vix_comm* c, int64_t nq, int rc,
     } else {
         VIX_NCCL(g_nccl.AllGather(mine.ptr, lims_all.ptr, (size_t)L, ncclInt64, c->comm, s));
     }
+    // k-NN: rows shorter than k within a finite bound, counted from the row starts every rank now holds (read in the
+    // synchronisation of shard_range_lims)
+    Scratch<unsigned long long> dshort;
+    unsigned long long short_rows = 0;
+    if (knn) {
+        VIX_TRY(dshort.alloc(1));
+        VIX_CUDA(cudaMemsetAsync(dshort.ptr, 0, 8, s));
+        shard_knn_short_kernel<<<(unsigned)((nq + 255) / 256), 256, 0, s>>>(lims_all.ptr, world, nq, t.k, t.bound, dshort.ptr);
+        VIX_LAUNCH_CHECK();
+        VIX_CUDA(cudaMemcpyAsync(&short_rows, dshort.ptr, 8, cudaMemcpyDeviceToHost, s));
+    }
     std::vector<int64_t> meta;
     VIX_TRY(shard_range_lims(lims_all.ptr, world, nq, glims.ptr, meta));    // the second synchronisation: the global total
     if (rc != VIX_OK) return rc;                                          // (its own message stands)
     for (int p = 0; p < world; ++p)
-        VIX_REQUIRE(meta[world + 2 + p] == VIX_OK, (int)meta[world + 2 + p], "vix_sharded_range_search: rank %d failed its local "
-                    "scan (status %lld); no rank returns a result", p, (long long)meta[world + 2 + p]);
+        VIX_REQUIRE(meta[world + 2 + p] == VIX_OK, (int)meta[world + 2 + p], "%s: rank %d failed its local "
+                    "scan (status %lld); no rank returns a result", who, p, (long long)meta[world + 2 + p]);
+    // (every rank holds the same row starts and bounds, so every rank refuses here together)
+    VIX_REQUIRE(short_rows == 0, VIX_ERR_CONTRACT, "%s (k = %d): %llu queries merged fewer than k entries within the bound "
+                "the ranks' seed passes found", who, t.k, short_rows);
     const int64_t total = meta[world], max_row = meta[world + 1];
     // room for the answer on every rank, decided together
     if (peer) VIX_TRY(ensure_range_region(c, nq, total, &grown));
     vix_range_result* r = nullptr;
     Scratch<u64> kall;
-    int ok = range_alloc(nq, total, &r) == VIX_OK;
+    int ok = knn ? 1 : range_alloc(nq, total, &r) == VIX_OK;
     if (ok && !peer && kall.alloc((size_t)total) != VIX_OK) ok = 0;
     {
         Scratch<int> dflag;
@@ -831,9 +950,9 @@ static int sharded_range_exchange(vix_index* h, vix_comm* c, int64_t nq, int rc,
         if (rc2 == VIX_OK) rc2 = cudaStreamSynchronize(s) == cudaSuccess ? VIX_OK : VIX_ERR_CUDA;
         if (rc2 != VIX_OK || !ok) {
             range_free(r);
-            VIX_REQUIRE(rc2 == VIX_OK, rc2, "vix_sharded_range_search: the allocation verdict failed");
-            VIX_REQUIRE(false, VIX_ERR_OOM, "vix_sharded_range_search: %lld results (%lld bytes) do not fit in device memory on "
-                        "every rank", (long long)total, (long long)total * 12);
+            VIX_REQUIRE(rc2 == VIX_OK, rc2, "%s: the allocation verdict failed", who);
+            VIX_REQUIRE(false, VIX_ERR_OOM, "%s: %lld results (%lld bytes) do not fit in device memory on "
+                        "every rank", who, (long long)total, (long long)total * (knn ? 8 : 12));
         }
     }
     auto fail = [&](int e) { range_free(r); return e; };
@@ -871,12 +990,148 @@ static int sharded_range_exchange(vix_index* h, vix_comm* c, int64_t nq, int rc,
         }
         keys = kall.ptr;
     }
-    const int mr = shard_range_merge(keys, dbase.ptr, lims_all.ptr, world, nq, glims.ptr, total, h->p.metric, r);
+    const int mr = knn ? shard_knn_merge(keys, dbase.ptr, lims_all.ptr, world, nq, glims.ptr, total, t.k, h->p.metric, t.dist, t.ids)
+                       : shard_range_merge(keys, dbase.ptr, lims_all.ptr, world, nq, glims.ptr, total, h->p.metric, r);
     if (mr != VIX_OK) return fail(mr);
-    if (getenv("VIX_SCAN_DEBUG"))
+    if (getenv("VIX_SCAN_DEBUG") && !knn)
         fprintf(stderr, "[vix sharded range] world %d, peer %d, local %lld, total %lld, max_row %lld, grown %d\n", world,
                 peer ? 1 : 0, (long long)mine_n, (long long)total, (long long)max_row, grown ? 1 : 0);
-    *out = r;
+    st->mine = mine_n; st->total = total; st->max_row = max_row; st->grown = grown;
+    if (!knn) *t.out = r;
+    return VIX_OK;
+}
+
+// the ranks' k-NN seed bounds [nq] (device) -> their unsigned minimum, on every rank: peer memory (the bound slice of the
+// range region, one barrier) or an NCCL all-reduce
+static int bound_min_over_ranks(vix_comm* c, uint32_t* tau, int64_t nq) {
+    cudaStream_t s = ctx().stream;
+    if (c->peer_state != 1) {
+        VIX_NCCL(g_nccl.AllReduce(tau, tau, (size_t)nq, ncclUint32, ncclMin, c->comm, s));
+        return VIX_OK;
+    }
+    const int64_t stride = c->range_cap_nq;
+    const int64_t want = (nq + 255) / 256;
+    push_knn_bounds_kernel<<<(unsigned)(want < 64 ? want : 64), 256, 0, s>>>(tau, nq, c->range_peer_dev, c->world,
+                                                                            c->range_off_bounds + (size_t)c->rank * stride * 4);
+    VIX_LAUNCH_CHECK();
+    VIX_TRY(peer_barrier(c));
+    const uint32_t* slots = reinterpret_cast<const uint32_t*>(static_cast<char*>(c->range_local) + c->range_off_bounds);
+    min_knn_bounds_kernel<<<(unsigned)want, 256, 0, s>>>(slots, c->world, stride, nq, tau);
+    VIX_LAUNCH_CHECK();
+    return VIX_OK;
+}
+
+// vix_sharded_search / vix_sharded_search_filtered with VIX_MAX_K < k <= VIX_MAX_K_LARGE and world > 1: the one-GPU two-pass
+// route (vix_knn_large.cu) with one bound per query shared by all ranks (see shard_knn_merge_kernel for why it is exact):
+//   1. the probes of the batch, exchanged as for every sharded call;
+//   2. each rank's seed over the probe prefix of the lists it owns (those it does not own have length 0) -> tau_r;
+//   3. tau = the minimum of the tau_r over the ranks;
+//   4. each rank's collect within tau over every probed list it owns, each sorted row cut at k (knn_trim);
+//   5. the cut rows exchanged as range search exchanges its rows, merged, and cut at k into [nq x k].
+// A rank whose seed or collect fails still enters every exchange (all-ones bounds, empty rows and its status), so every
+// rank returns its code.  Synchronises the stream; the handle's knn_cap is written once the call has succeeded.
+static int sharded_knn_large(vix_index* h, vix_comm* c, const float* queries, int64_t nq, int k, int nprobe,
+                             const FilterArgs* filter, float* out_dist, int64_t* out_ids) {
+    cudaStream_t s = ctx().stream;
+    VIX_TRY(ensure_region(c, nq, h->p.d, nprobe, 1));                 // (no [world x nq x k] result slab: k is large)
+    bool grown = false;
+    if (c->peer_state == 1) VIX_TRY(ensure_range_region(c, nq, 0, &grown));
+    Out<float> dd;
+    Out<int64_t> di;
+    VIX_TRY(dd.stage(out_dist, (size_t)nq * k));
+    VIX_TRY(di.stage(out_ids, (size_t)nq * k));
+    Scratch<uint32_t> tau;
+    VIX_TRY(tau.alloc((size_t)nq));
+    auto mark = [&](int i) { if (c->trace) cudaEventRecord(c->ev[i], s); };
+    mark(0);
+    BatchProbes px;
+    VIX_TRY(exchange_probes(h, c, queries, nq, nprobe, px));
+    mark(1);
+    // 2. the local seed -> tau_r
+    IvfRangeScan scan;
+    Scratch<int32_t> prefix;
+    size_t seed_cap = 0, max_entries = 0;
+    int64_t seed_n = 0;
+    int rc = ivf_range_scan(h, px.queries, nq, nprobe, px.probes, filter, scan);
+    if (rc == VIX_OK) rc = prefix.alloc((size_t)nq * nprobe);
+    if (rc == VIX_OK)
+        rc = knn_probe_prefix(px.probes, nq, nprobe, h->list_len.ptr, h->kc, k, prefix.ptr, &seed_cap, &max_entries);
+    const std::function<int(const RangeOut&)> seed = [&](const RangeOut& o) { return scan.run(prefix.ptr, o); };
+    const std::function<int(const RangeOut&)> collect = [&](const RangeOut& o) { return scan.run(px.probes, o); };
+    if (rc == VIX_OK) rc = knn_seed_bound(nq, k, seed_cap, &seed, tau.ptr, &seed_n);
+    if (rc != VIX_OK) VIX_CUDA(cudaMemsetAsync(tau.ptr, 0xFF, (size_t)nq * 4, s));
+    // 3. tau = min over the ranks
+    VIX_TRY(bound_min_over_ranks(c, tau.ptr, nq));
+    // 4. the local collect within tau, each row cut at k
+    RangeKeys rk, cut;
+    RangeInfo ci;
+    size_t cap = h->knn_cap;
+    if (rc == VIX_OK) rc = knn_collect(nq, k, tau.ptr, collect, max_entries, cap, rk, &ci, nullptr);
+    if (rc == VIX_OK) rc = knn_trim(nq, k, rk, cut);
+    mark(2);
+    // 5. exchange, merge, cut
+    ShardTail tail;
+    tail.k = k; tail.bound = tau.ptr; tail.dist = dd.dev; tail.ids = di.dev;
+    ShardTotals st;
+    VIX_TRY(sharded_range_exchange(h, c, nq, rc, cut, grown, tail, &st));
+    mark(3);
+    if (getenv("VIX_SCAN_DEBUG"))
+        fprintf(stderr, "[vix sharded knn] world %d, peer %d, k %d, seed %lld, local %lld, sent %lld, total %lld, max_row %lld, "
+                "grown %d\n", c->world, c->peer_state == 1 ? 1 : 0, k, (long long)seed_n, (long long)ci.total,
+                (long long)st.mine, (long long)st.total, (long long)st.max_row, st.grown ? 1 : 0);
+    VIX_TRY(dd.commit());
+    VIX_TRY(di.commit());
+    VIX_TRY(finish(true));
+    h->knn_cap = cap;
+    return VIX_OK;
+}
+
+// The test hooks' input: the ranks' lims [world][nq + 1] and rows (API distances, ids, concatenated rank by rank) -> the
+// exchanged layout (lims [world][nq + 2], status 0), the packed keys, the global row starts and the ranks' key bases, as
+// the exchange holds them.
+struct DebugShardRuns {
+    Scratch<int64_t> dlims, glims, dbase;
+    Scratch<u64> keys;
+    In<float> dd;
+    In<int64_t> di;
+    std::vector<int64_t> meta;
+    int64_t total = 0;
+};
+
+static int debug_shard_runs(const char* who, const int64_t* lims_all, const float* dist_all, const int64_t* ids_all, int world,
+                            int64_t nq, DebugShardRuns& in) {
+    cudaStream_t s = ctx().stream;
+    const int64_t L = nq + 2;
+    // the ranks' lims [world][nq + 1] -> the exchanged layout [world][nq + 2] (status 0)
+    std::vector<int64_t> h_lims((size_t)world * (nq + 1));
+    VIX_CUDA(cudaMemcpyAsync(h_lims.data(), lims_all, h_lims.size() * 8, cudaMemcpyDefault, s));
+    VIX_CUDA(cudaStreamSynchronize(s));
+    std::vector<int64_t> h_all((size_t)world * L, 0);
+    int64_t total = 0;
+    for (int r = 0; r < world; ++r) {
+        const int64_t* lr = h_lims.data() + (size_t)r * (nq + 1);
+        VIX_REQUIRE(lr[0] == 0, VIX_ERR_INVALID_PARAM, "%s: rank %d: lims[0] != 0", who, r);
+        for (int64_t q = 0; q < nq; ++q)
+            VIX_REQUIRE(lr[q + 1] >= lr[q], VIX_ERR_INVALID_PARAM, "%s: rank %d: lims descend", who, r);
+        for (int64_t q = 0; q <= nq; ++q) h_all[(size_t)r * L + q] = lr[q];
+        total += lr[nq];
+    }
+    VIX_REQUIRE(total == 0 || (dist_all && ids_all), VIX_ERR_NULL_PTR, "%s: null rows", who);
+    VIX_TRY(in.dlims.alloc(h_all.size()));
+    VIX_TRY(in.glims.alloc((size_t)nq + 1));
+    VIX_TRY(in.dbase.alloc((size_t)world + 1));
+    VIX_CUDA(cudaMemcpyAsync(in.dlims.ptr, h_all.data(), h_all.size() * 8, cudaMemcpyHostToDevice, s));
+    VIX_TRY(in.dd.stage(dist_all, (size_t)total));
+    VIX_TRY(in.di.stage(ids_all, (size_t)total));
+    VIX_TRY(in.keys.alloc((size_t)total));
+    if (total > 0) {
+        pack_result_keys_kernel<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(in.dd.dev, in.di.dev, total, nullptr, world, 0,
+                                                                              in.keys.ptr);
+        VIX_LAUNCH_CHECK();
+    }
+    VIX_TRY(shard_range_lims(in.dlims.ptr, world, nq, in.glims.ptr, in.meta));
+    VIX_CUDA(cudaMemcpyAsync(in.dbase.ptr, in.meta.data(), ((size_t)world + 1) * 8, cudaMemcpyHostToDevice, s));
+    in.total = total;
     return VIX_OK;
 }
 
@@ -890,7 +1145,9 @@ int vix_sharded_search(vix_index_t* h, vix_comm_t* c, const float* queries, int6
     VIX_REQUIRE(h && c, VIX_ERR_NULL_PTR, "vix_sharded_search: null handle");
     if (nq <= 0 || k <= 0) return VIX_OK;                             // IVFIndex.swift:866 (every rank sees the same nq, k)
     VIX_REQUIRE(queries && out_dist && out_ids, VIX_ERR_NULL_PTR, "vix_sharded_search: null pointer");
-    VIX_REQUIRE(k <= VIX_MAX_K, VIX_ERR_INVALID_K, "vix_sharded_search: k > %d", VIX_MAX_K);
+    VIX_REQUIRE(k <= VIX_MAX_K_LARGE, VIX_ERR_INVALID_K, "vix_sharded_search: k > %d", VIX_MAX_K_LARGE);
+    VIX_REQUIRE(k <= VIX_MAX_K || nq < 0x7FFFFFFFLL, VIX_ERR_INVALID_PARAM, "vix_sharded_search: k > %d needs nq < 2^31 - 1",
+                VIX_MAX_K);
     return sharded_search(h, c, queries, nq, k, nprobe, nullptr, out_dist, out_ids);
 }
 
@@ -904,7 +1161,9 @@ int vix_sharded_search_filtered(vix_index_t* h, vix_comm_t* c, const float* quer
     VIX_REQUIRE(filter_capacity >= 0, VIX_ERR_INVALID_PARAM, "vix_sharded_search_filtered: negative capacity");
     if (nq <= 0 || k <= 0) return VIX_OK;
     VIX_REQUIRE(queries && out_dist && out_ids, VIX_ERR_NULL_PTR, "vix_sharded_search_filtered: null pointer");
-    VIX_REQUIRE(k <= VIX_MAX_K, VIX_ERR_INVALID_K, "vix_sharded_search_filtered: k > %d", VIX_MAX_K);
+    VIX_REQUIRE(k <= VIX_MAX_K_LARGE, VIX_ERR_INVALID_K, "vix_sharded_search_filtered: k > %d", VIX_MAX_K_LARGE);
+    VIX_REQUIRE(k <= VIX_MAX_K || nq < 0x7FFFFFFFLL, VIX_ERR_INVALID_PARAM,
+                "vix_sharded_search_filtered: k > %d needs nq < 2^31 - 1", VIX_MAX_K);
     In<uint64_t> fw;
     FilterArgs f;
     const FilterArgs* fp = nullptr;
@@ -954,7 +1213,10 @@ int vix_sharded_range_search(vix_index_t* h, vix_comm_t* c, const float* queries
     const int rc = index_range_locked(h, px.queries, nq, radius, nprobe, fp, nullptr, px.probes, &rk);
     mark(2);
     vix_range_result* r = nullptr;
-    VIX_TRY(sharded_range_exchange(h, c, nq, rc, rk, grown, &r));
+    ShardTail tail;
+    tail.out = &r;
+    ShardTotals st;
+    VIX_TRY(sharded_range_exchange(h, c, nq, rc, rk, grown, tail, &st));
     mark(3);
     *out = r;
     return VIX_OK;
@@ -995,48 +1257,36 @@ int vix_debug_shard_range_merge(const int64_t* lims_all, const float* dist_all, 
     VIX_REQUIRE(world > 0 && world <= 256 && nq >= 0 && nq < 0x7FFFFFFFLL, VIX_ERR_INVALID_PARAM,
                 "vix_debug_shard_range_merge: world / nq");
     cudaStream_t s = ctx().stream;
-    const int64_t L = nq + 2;
-    // the ranks' lims [world][nq + 1] -> the exchanged layout [world][nq + 2] (status 0)
-    std::vector<int64_t> h_lims((size_t)world * (nq + 1));
-    VIX_CUDA(cudaMemcpyAsync(h_lims.data(), lims_all, h_lims.size() * 8, cudaMemcpyDefault, s));
-    VIX_CUDA(cudaStreamSynchronize(s));
-    std::vector<int64_t> h_all((size_t)world * L, 0);
-    int64_t total = 0;
-    for (int r = 0; r < world; ++r) {
-        const int64_t* lr = h_lims.data() + (size_t)r * (nq + 1);
-        VIX_REQUIRE(lr[0] == 0, VIX_ERR_INVALID_PARAM, "vix_debug_shard_range_merge: rank %d: lims[0] != 0", r);
-        for (int64_t q = 0; q < nq; ++q)
-            VIX_REQUIRE(lr[q + 1] >= lr[q], VIX_ERR_INVALID_PARAM, "vix_debug_shard_range_merge: rank %d: lims descend", r);
-        for (int64_t q = 0; q <= nq; ++q) h_all[(size_t)r * L + q] = lr[q];
-        total += lr[nq];
-    }
-    VIX_REQUIRE(total == 0 || (dist_all && ids_all), VIX_ERR_NULL_PTR, "vix_debug_shard_range_merge: null rows");
-    Scratch<int64_t> dlims, glims, dbase;
-    VIX_TRY(dlims.alloc(h_all.size()));
-    VIX_TRY(glims.alloc((size_t)nq + 1));
-    VIX_TRY(dbase.alloc((size_t)world + 1));
-    VIX_CUDA(cudaMemcpyAsync(dlims.ptr, h_all.data(), h_all.size() * 8, cudaMemcpyHostToDevice, s));
-    In<float> dd;
-    In<int64_t> di;
-    VIX_TRY(dd.stage(dist_all, (size_t)total));
-    VIX_TRY(di.stage(ids_all, (size_t)total));
-    Scratch<u64> keys;
-    VIX_TRY(keys.alloc((size_t)total));
-    if (total > 0) {
-        pack_result_keys_kernel<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(dd.dev, di.dev, total, nullptr, world, 0, keys.ptr);
-        VIX_LAUNCH_CHECK();
-    }
-    std::vector<int64_t> meta;
-    VIX_TRY(shard_range_lims(dlims.ptr, world, nq, glims.ptr, meta));
-    VIX_CUDA(cudaMemcpyAsync(dbase.ptr, meta.data(), ((size_t)world + 1) * 8, cudaMemcpyHostToDevice, s));
+    DebugShardRuns in;
+    VIX_TRY(debug_shard_runs("vix_debug_shard_range_merge", lims_all, dist_all, ids_all, world, nq, in));
     vix_range_result* r = nullptr;
-    VIX_TRY(range_alloc(nq, total, &r));
-    const int rc = shard_range_merge(keys.ptr, dbase.ptr, dlims.ptr, world, nq, glims.ptr, total, metric, r);
+    VIX_TRY(range_alloc(nq, in.total, &r));
+    const int rc = shard_range_merge(in.keys.ptr, in.dbase.ptr, in.dlims.ptr, world, nq, in.glims.ptr, in.total, metric, r);
     if (rc != VIX_OK) { range_free(r); return rc; }
     const cudaError_t e = cudaStreamSynchronize(s);                   // (meta, a host vector, is read by the copy above)
     if (e != cudaSuccess) { range_free(r); VIX_CUDA(e); }
     *out = r;
     return VIX_OK;
+}
+
+int vix_debug_shard_knn_merge(const int64_t* lims_all, const float* dist_all, const int64_t* ids_all, int world, int64_t nq,
+                              int k, int metric, float* out_dist, int64_t* out_ids) {
+    VIX_TRY(ensure_device());
+    VIX_REQUIRE(lims_all && out_dist && out_ids, VIX_ERR_NULL_PTR, "vix_debug_shard_knn_merge: null pointer");
+    VIX_REQUIRE(world > 0 && world <= 256 && nq >= 0 && nq < 0x7FFFFFFFLL && k > 0 && k <= VIX_MAX_K_LARGE,
+                VIX_ERR_INVALID_PARAM, "vix_debug_shard_knn_merge: world / nq / k");
+    DebugShardRuns in;
+    VIX_TRY(debug_shard_runs("vix_debug_shard_knn_merge", lims_all, dist_all, ids_all, world, nq, in));
+    Out<float> od;
+    Out<int64_t> oi;
+    VIX_TRY(od.stage(out_dist, (size_t)nq * k));
+    VIX_TRY(oi.stage(out_ids, (size_t)nq * k));
+    if (nq > 0)
+        VIX_TRY(shard_knn_merge(in.keys.ptr, in.dbase.ptr, in.dlims.ptr, world, nq, in.glims.ptr, in.total, k, metric, od.dev,
+                                oi.dev));
+    VIX_TRY(od.commit());
+    VIX_TRY(oi.commit());
+    return finish(true);                                              // (meta, a host vector, is read by a copy)
 }
 
 int vix_comm_trace(vix_comm_t* c, int enabled) {

@@ -704,7 +704,10 @@ class ShardedIVFPQIndex:
         """Replicated queries in, merged [nq x k] (distances, ids) out on every rank.  Host (numpy) queries are
         staged to the device once and only the merged result returns to the host.  ``out``: optional (distances f32,
         ids int64) host arrays the result is written into (pinned ones make the copy back asynchronous).  ``filter``: an
-        :class:`IDFilter` (the same on every rank), applied before selection as in ``IVFPQIndex.batch_search``."""
+        :class:`IDFilter` (the same on every rank), applied before selection as in ``IVFPQIndex.batch_search``.  ``k`` goes
+        up to ``VIX_MAX_K_LARGE`` (16384) through the library's exchange, as on one GPU: above 512 each rank runs the
+        exact two-pass route with one bound per query shared by all ranks, the rows cut at k are exchanged and merged on
+        the device, and the call synchronises.  (The Python exchange path of CPU / gloo ranks is not covered by this.)"""
         import torch
         if filter is not None:
             return self._filtered_search(queries, k, nprobe, filter, out)
@@ -756,7 +759,8 @@ class ShardedIVFPQIndex:
         return md, mi
 
     def _filtered_search(self, queries, k, nprobe, filter, out):
-        """batch_search with an id filter: vix_sharded_search_filtered (one rank: the local index's filtered search)"""
+        """batch_search with an id filter: vix_sharded_search_filtered (one rank: the local index's filtered search); k up to
+        ``VIX_MAX_K_LARGE``, the filter applied on both passes of the large-k route on every rank"""
         nprobe = nprobe if nprobe > 0 else self.nprobe
         comm = self._native()
         if comm is None:
