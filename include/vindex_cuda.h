@@ -465,12 +465,15 @@ int vix_index_search_with_probes(vix_index_t* h, const float* queries, int64_t n
  * (decided once, collectively; VIX_NO_P2P=1 forces the fallback).
  *   vix_comm_unique_id   rank 0: the NCCL id (128 bytes) the host hands to every rank by its own means
  *   vix_comm_create      collective; binds the calling thread's CUDA device
- *   vix_sharded_add      collective; x / ids: the rows THIS rank contributes (any rows; n may be 0).  Rows are assigned +
- *                        encoded here and appended on the rank owning their list: list l belongs to rank r iff
- *                        list_bounds[r] <= l < list_bounds[r + 1] (host array [world + 1], NULL = equal-count blocks).
- *                        A row with no nearest list (NaN components) or an id outside [0, 2^32 - 1) on ANY rank makes
- *                        every rank return VIX_ERR_INVALID_PARAM (naming that rank) before any row travels: no rank
- *                        stores a row of the call
+ *   vix_sharded_add      collective; x / ids: the rows THIS rank contributes (any rows; n may be 0).  IVF-PQ and IVF-Flat:
+ *                        rows are assigned (+ encoded) here and appended on the rank owning their list: list l belongs to
+ *                        rank r iff list_bounds[r] <= l < list_bounds[r + 1] (host array [world + 1], NULL = equal-count
+ *                        blocks); IVF-Flat rows travel as vectors with their assignment, which the owner keeps.  Flat: rows
+ *                        stay on the rank that passes them (list_bounds must be NULL, else VIX_ERR_INVALID_PARAM).
+ *                        A row with no nearest list (NaN components; IVF kinds) or an id outside [0, 2^32 - 1) on ANY rank
+ *                        makes every rank return VIX_ERR_INVALID_PARAM (naming that rank) before any row is stored or
+ *                        travels: no rank stores a row of the call.  An IVF-Flat index needs its centroids first
+ *                        (VIX_ERR_NOT_TRAINED): the sharded layout files every row into its list
  *   vix_sharded_search   collective; every rank passes the SAME batch (host or device pointer; from a host pointer only
  *                        the rank's own 1/world block crosses PCIe) and receives the merged [nq x k] result.  Results
  *                        equal vix_index_search on one GPU holding all lists (same probe lists by construction; same
@@ -492,7 +495,15 @@ int vix_index_search_with_probes(vix_index_t* h, const float* queries, int64_t n
  *                        whose local pass fails makes every rank return its code; a merged answer that does not fit
  *                        makes every rank return VIX_ERR_OOM; a merged row shorter than k within a finite bound (the two
  *                        passes disagreed on a distance) makes every rank return VIX_ERR_CONTRACT.  One rank is
- *                        vix_index_search. */
+ *                        vix_index_search.
+ *                        Every index kind: flat, IVF-Flat (L2, IP, cosine) and IVF-PQ (L2, IP).  Flat: no probes; each rank
+ *                        runs the fused flat search over its rows (k > VIX_MAX_K: the flat two-pass route with the shared
+ *                        bound) and the ranks' results merge by raw score and then rank, so the answer equals one GPU
+ *                        holding rank 0's rows first, then rank 1's, ..., each rank's in add order (flat search breaks ties
+ *                        at one score by row, and maps scores to distances only after selecting).  IVF-Flat: as IVF-PQ
+ *                        (probes exchanged, each rank scans the lists it owns); its distances are exact per pair and its
+ *                        ties fall to the id, so the answer does not depend on the slots.  Zero distances keep one GPU's
+ *                        sign per kind: IP -0 from flat and IVF-PQ, +0 from IVF-Flat. */
 typedef struct vix_comm vix_comm_t;
 int vix_comm_unique_id(void* id_out, size_t capacity /* >= 128 */);
 int vix_comm_create(const void* id, size_t id_bytes, int rank, int world, vix_comm_t** out);
@@ -519,10 +530,13 @@ int vix_sharded_search(vix_index_t* h, vix_comm_t* c, const float* queries, int6
  * whole merged answer.
  *   - Parity: the answer equals the one-GPU call on an index holding every row in the slot the shards hold it in (rows
  *     inserted in owner-append order, rank 0's contributions first), bit for bit: lims, ids, distance bits with the sign of
- *     zero (IP -0, L2 +0), the (distance, id) order, rows stored twice and lists probed twice (each comes back twice).
+ *     zero (IP -0, L2 +0; IVF-Flat +0), the (distance, id) order, rows stored twice and lists probed twice (each comes back
+ *     twice).  A flat index has no probes: each rank runs the flat range scan over its rows.
  *   - Refusals, on every rank alike and before any exchange: a NaN radius, a filter_mode other than VIX_FILTER_ALLOW /
  *     VIX_FILTER_DENY or a negative filter_capacity (VIX_ERR_INVALID_PARAM); nprobe outside 1 .. VIX_MAX_K after the default
- *     (VIX_ERR_INVALID_K); cosine (VIX_ERR_UNSUPPORTED); an index that is not a trained IVF-PQ index (VIX_ERR_NOT_TRAINED).
+ *     (VIX_ERR_INVALID_K; not read for a flat index); an IVF-PQ index that is not trained (VIX_ERR_NOT_TRAINED) or uses
+ *     cosine (VIX_ERR_UNSUPPORTED); an IVF-Flat index without coarse centroids (VIX_ERR_NOT_TRAINED).  Flat and IVF-Flat
+ *     indexes follow the parity of vix_sharded_search for their kind (flat: rows in rank order; IVF-Flat: any slots).
  *   - Range: nq == 0 gives an empty result (lims = {0}) with no exchange; one rank is vix_index_range_search.  The probes
  *     travel as in vix_sharded_search; each rank runs the query-major range scan over the probed lists it owns and sorts
  *     its rows; the ranks exchange their row starts, then their sorted keys (a second peer-mapped region of the
@@ -600,6 +614,28 @@ int vix_debug_shard_range_merge(const int64_t* lims_all /* [world x (nq + 1)] */
 int vix_debug_shard_knn_merge(const int64_t* lims_all /* [world x (nq + 1)] */, const float* dist_all,
                               const int64_t* ids_all /* concatenated rank by rank */, int world, int64_t nq, int k, int metric,
                               float* out_dist, int64_t* out_ids);
+
+/* Test hook: the merge of the flat kind's sharded k-NN search on one GPU.  lims_all: [world x (nq + 1)] the ranks' CSR row
+ * starts; score_all / ids_all: their rows as the flat engine selects them -- RAW scores (L2^2, dot, cosine similarity) and
+ * ids, concatenated rank by rank, each row in the flat search's order (score in the metric's order, then row).  They are
+ * keyed (score word, id) and merged by the score word and then the rank, as one GPU holding the ranks' rows rank by rank
+ * orders them, then mapped to API distances (sqrt, -s, 1 - s).  k > 0: the merged rows cut at k into out [nq x k], padded
+ * with id -1 / NaN; k == 0: the whole merged rows into out [total] and their starts into out_lims [nq + 1] (nullable)
+ * (host or device pointers; world 1 .. 256, 0 <= k <= VIX_MAX_K_LARGE). */
+int vix_debug_shard_flat_merge(const int64_t* lims_all /* [world x (nq + 1)] */, const float* score_all,
+                               const int64_t* ids_all /* concatenated rank by rank */, int world, int64_t nq, int k, int metric,
+                               int64_t* out_lims /* nullable */, float* out_dist, int64_t* out_ids);
+
+/* Test hook: a sharded call with every rank on one GPU.  shards: the world ranks' handles (distinct, one kind, metric and
+ * dimension; each holds what that rank would hold after vix_sharded_add).  Every rank's local pass runs as in
+ * vix_sharded_search / vix_sharded_search_filtered / vix_sharded_range_search (the probes of the whole batch selected once;
+ * for k > VIX_MAX_K each rank's seed, the minimum of the ranks' bounds, each rank's collect cut at k) and the answer is merged
+ * by the kernels the exchange runs; only the transport between the ranks is left out.  out_range == NULL: k-NN into out_dist
+ * / out_ids [nq x k] (k <= 0 or nq == 0: nothing); otherwise range search with `radius` into a new result object.  Filter
+ * arguments as vix_sharded_search_filtered (filter_words NULL: none). */
+int vix_debug_sharded_emulate(vix_index_t* const* shards, int world, const float* queries, int64_t nq, int k, int nprobe,
+                              float radius, const uint64_t* filter_words /* nullable */, int64_t filter_capacity,
+                              int filter_mode, float* out_dist, int64_t* out_ids, vix_range_result_t** out_range /* nullable */);
 
 /* a16  AccelerableIndex-shaped convenience (AccelerableIndex.swift:15-127): candidates [c x d]
  * contiguous in, (indices into candidates, distances) out, per query. */

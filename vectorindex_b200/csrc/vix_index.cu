@@ -1670,6 +1670,64 @@ int index_add_encoded_locked(vix_index* h, const int32_t* assign, const uint8_t*
     h->dirty = true;
     return finish(true);
 }
+
+// The IVF-Flat sibling: rows whose lists are known, filed as index_add_locked files them (vectors, ids and assignments
+// appended in order; the lists are rebuilt at the next search).  The assignment is taken as given, not recomputed.
+int index_add_assigned_locked(vix_index* h, const int32_t* assign, const float* x, const int64_t* ids, int64_t n) {
+    VIX_REQUIRE(h->p.kind == VIX_INDEX_IVF_FLAT && h->has_coarse, VIX_ERR_NOT_TRAINED,
+                "index_add_assigned: needs an IVF-Flat index with coarse centroids");
+    if (n <= 0) return VIX_OK;
+    VIX_REQUIRE(h->n + n < 0x7FFFFFFFLL, VIX_ERR_INVALID_PARAM, "index shard limited to 2^31 - 1 rows");
+    VIX_TRY(is_device_ptr(ids) ? check_ids_device(ids, n) : check_ids_host(ids, n));
+    cudaStream_t s = ctx().stream;
+    {
+        In<int32_t> da;
+        VIX_TRY(da.stage(assign, (size_t)n));
+        unsigned long long invalid = 0;
+        VIX_TRY(count_invalid_assign(da.dev, n, h->kc, &invalid));
+        VIX_REQUIRE(invalid == 0, VIX_ERR_INVALID_PARAM, "index_add_assigned: %llu of %lld list assignments lie outside [0, %d)",
+                    invalid, (long long)n, h->kc);
+    }
+    const int64_t n0 = h->n, d = h->p.d;
+    VIX_TRY(h->ids.resize((size_t)(n0 + n)));
+    VIX_TRY(h->assign.resize((size_t)(n0 + n)));
+    VIX_TRY(h->vecs.resize((size_t)(n0 + n) * d));
+    VIX_CUDA(cudaMemcpyAsync(h->ids.ptr + n0, ids, (size_t)n * 8, cudaMemcpyDefault, s));
+    VIX_CUDA(cudaMemcpyAsync(h->assign.ptr + n0, assign, (size_t)n * 4, cudaMemcpyDefault, s));
+    VIX_CUDA(cudaMemcpyAsync(h->vecs.ptr + (size_t)n0 * d, x, (size_t)n * d * 4, cudaMemcpyDefault, s));
+    h->n = n0 + n;
+    h->next_auto_id += n;
+    h->dirty = true;
+    return finish(true);
+}
+
+int index_add_rows_locked(vix_index* h, const float* x, const int64_t* ids, int64_t n) {
+    return index_add_locked(h, x, ids, n);
+}
+
+int count_invalid_ids_device(const int64_t* ids, int64_t n, unsigned long long* count_dev) {
+    if (n <= 0) return VIX_OK;
+    count_invalid_ids_kernel<<<(unsigned)((n + 255) / 256), 256, 0, ctx().stream>>>(ids, n, count_dev);
+    VIX_LAUNCH_CHECK();
+    return VIX_OK;
+}
+
+int select_probes_device(vix_index* h, const float* q, int64_t nq, int nprobe, int32_t* out) {
+    if (h->p.metric == VIX_METRIC_COSINE)
+        return probe_select_cosine_device(q, nq, h->coarse.ptr, h->kc, h->p.d, h->coarse_norms.ptr, nprobe, out);
+    return probe_select_fast_device(q, nq, h->coarse.ptr, h->kc, h->p.d, h->p.metric, nprobe, h->coarse_norms.ptr, out, nullptr,
+                                    h->coarse_norm_max.ptr);
+}
+
+int filter_row_mask(vix_index* h, const FilterArgs* filter, Scratch<uint64_t>& mask) {
+    if (!filter || h->n == 0) return VIX_OK;
+    const int64_t words = (h->n + 63) / 64;
+    VIX_TRY(mask.alloc((size_t)words));
+    filter_row_mask_kernel<<<(unsigned)((words + 255) / 256), 256, 0, ctx().stream>>>(h->ids.ptr, h->n, filter->words, filter->cap,
+                                                                                    filter->deny, mask.ptr);
+    VIX_LAUNCH_CHECK();
+    return VIX_OK;
+}
 }  // namespace vix
 extern "C" {
 

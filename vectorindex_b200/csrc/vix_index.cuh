@@ -169,6 +169,18 @@ int count_invalid_assign(const int32_t* assign, int64_t n, int kc, unsigned long
 int count_invalid_rows_device(const int32_t* assign, const int64_t* ids, int64_t n, int kc, unsigned long long* count_dev);
 // append already encoded rows (device or host pointers) to an IVF-PQ index whose mutex the caller holds
 int index_add_encoded_locked(vix_index* h, const int32_t* assign, const uint8_t* codes, const int64_t* ids, int64_t n);
+// append rows of an IVF-Flat index with centroids whose list assignments are known (the sharded add's owner side; files
+// them exactly as vix_index_add would, without recomputing the assignment)
+int index_add_assigned_locked(vix_index* h, const int32_t* assign, const float* x, const int64_t* ids, int64_t n);
+// vix_index_add of an index whose mutex the caller holds (host or device pointers; ids nullable)
+int index_add_rows_locked(vix_index* h, const float* x, const int64_t* ids, int64_t n);
+// *count_dev += ids outside [0, 2^32 - 1) (device pointers; stream-ordered, no synchronisation)
+int count_invalid_ids_device(const int64_t* ids, int64_t n, unsigned long long* count_dev);
+// the probe lists of index_search_locked: the cosine selection or the fast one, by the index's metric (device pointers)
+int select_probes_device(vix_index* h, const float* q, int64_t nq, int nprobe, int32_t* out);
+// the flat engine's row mask of an id filter over the stored rows (bit r set => row r fails); mask stays empty without a
+// filter or rows
+int filter_row_mask(vix_index* h, const FilterArgs* filter, Scratch<uint64_t>& mask);
 int build_lists(vix_index* h);
 // residual PQ codes (u8, or packed u4 when ks = 16) of rows whose list assignments are known (device pointers)
 int encode_rows_device(vix_index* h, const float* x, int64_t n, const int32_t* assign, uint8_t* codes);

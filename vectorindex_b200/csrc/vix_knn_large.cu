@@ -227,46 +227,52 @@ int knn_large_run(int64_t nq, int k, KnnDecode dec, size_t seed_cap, const std::
     return VIX_OK;
 }
 
-int flat_knn_large_device(const float* q, int64_t nq, const float* xb, int64_t n, int d, int metric, int k,
-                          const uint64_t* disabled_rows, size_t& cap_hint, float* out_dist, int64_t* out_rows, KnnInfo* info) {
+int flat_knn_pass(const float* q, int64_t nq, const float* xb, int64_t n, int d, int metric, int k,
+                  const uint64_t* disabled_rows, FlatKnnPass& p) {
     // seed blocks: T = ceil(kKnnBeta k / VIX_MAX_K) contiguous blocks whose boundaries are multiples of 64 rows (the
     // filter's row mask is then offset by whole words); none when every row fits the seed's budget anyway
     // the fused flat search's selection: the score, largest first for inner product and cosine, then its API mapping
-    KnnDecode dec;
-    dec.order_max = metric != VIX_METRIC_L2;
-    dec.dist_mode = metric == VIX_METRIC_L2 ? 1 : metric == VIX_METRIC_IP ? 2 : 3;
-    std::function<int(const RangeOut&)> seed;
-    size_t seed_cap = 0;
-    Scratch<float> bd;
-    Scratch<int64_t> bi;
+    p.dec = flat_knn_decode(metric);
+    p.seed = nullptr;
+    p.seed_cap = 0;
+    p.max_entries = (size_t)(nq * n);
     if (n > (int64_t)kKnnBeta * k) {
         const int64_t T = ((int64_t)kKnnBeta * k + VIX_MAX_K - 1) / VIX_MAX_K;
         const int64_t nb = ((n + T - 1) / T + 63) / 64 * 64;
-        for (int64_t base = 0; base < n; base += nb) seed_cap += (size_t)nq * (size_t)std::min<int64_t>(VIX_MAX_K, std::min(nb, n - base));
+        for (int64_t base = 0; base < n; base += nb) p.seed_cap += (size_t)nq * (size_t)std::min<int64_t>(VIX_MAX_K, std::min(nb, n - base));
         const int64_t kb_max = std::min<int64_t>(VIX_MAX_K, nb);
-        VIX_TRY(bd.alloc((size_t)(nq * kb_max)));
-        VIX_TRY(bi.alloc((size_t)(nq * kb_max)));
-        seed = [&, nb](const RangeOut& o) -> int {
+        VIX_TRY(p.bd.alloc((size_t)(nq * kb_max)));
+        VIX_TRY(p.bi.alloc((size_t)(nq * kb_max)));
+        float* bd = p.bd.ptr;
+        int64_t* bi = p.bi.ptr;
+        const int order_max = p.dec.order_max;
+        p.seed = [=](const RangeOut& o) -> int {
             for (int64_t base = 0; base < n; base += nb) {
                 const int64_t rows = std::min(nb, n - base);
                 const int kb = (int)std::min<int64_t>(VIX_MAX_K, rows);
                 if (disabled_rows)
                     VIX_TRY(flat_search_masked_device(q, nq, xb + (size_t)base * d, rows, d, metric, kb, disabled_rows + base / 64,
-                                                      bd.ptr, bi.ptr, true));
+                                                      bd, bi, true));
                 else
-                    VIX_TRY(flat_search_auto_device(q, nq, xb + (size_t)base * d, rows, d, metric, kb, nullptr, bd.ptr, bi.ptr,
-                                                    true));
+                    VIX_TRY(flat_search_auto_device(q, nq, xb + (size_t)base * d, rows, d, metric, kb, nullptr, bd, bi, true));
                 const unsigned grid = (unsigned)std::min<int64_t>((int64_t)num_sms() * 8, nq);
-                knn_flat_seed_kernel<<<grid, 256, 0, ctx().stream>>>(bd.ptr, bi.ptr, nq, kb, base, dec.order_max, o);
+                knn_flat_seed_kernel<<<grid, 256, 0, ctx().stream>>>(bd, bi, nq, kb, base, order_max, o);
                 VIX_LAUNCH_CHECK();
             }
             return VIX_OK;
         };
     }
     // (row indices as ids and the raw score as the key: the order of the fused flat search, ties to the smaller row)
-    auto collect = [&](const RangeOut& o) { return flat_range_device(q, nq, xb, n, d, metric, nullptr, disabled_rows, o); };
-    return knn_large_run(nq, k, dec, seed_cap, seed ? &seed : nullptr, collect, (size_t)(nq * n), cap_hint, out_dist, out_rows,
-                         info);
+    p.collect = [=](const RangeOut& o) { return flat_range_device(q, nq, xb, n, d, metric, nullptr, disabled_rows, o); };
+    return VIX_OK;
+}
+
+int flat_knn_large_device(const float* q, int64_t nq, const float* xb, int64_t n, int d, int metric, int k,
+                          const uint64_t* disabled_rows, size_t& cap_hint, float* out_dist, int64_t* out_rows, KnnInfo* info) {
+    FlatKnnPass p;
+    VIX_TRY(flat_knn_pass(q, nq, xb, n, d, metric, k, disabled_rows, p));
+    return knn_large_run(nq, k, p.dec, p.seed_cap, p.seed ? &p.seed : nullptr, p.collect, p.max_entries, cap_hint, out_dist,
+                         out_rows, info);
 }
 
 }  // namespace vix

@@ -137,6 +137,29 @@ int knn_trim(int64_t nq, int k, const RangeKeys& rk, RangeKeys& out);
 // memory sort} (device pointers, one launch)
 int range_lims(const unsigned long long* counts, int64_t nq, int64_t* lims, unsigned long long* info);
 
+// the fused flat search's selection key and API mapping: the raw score, largest first for inner product and cosine, then
+// sqrt (L2), -s (IP) or 1 - s (cosine); the zero of an IP distance is -0 by that mapping
+inline KnnDecode flat_knn_decode(int metric) {
+    KnnDecode dec;
+    dec.order_max = metric != VIX_METRIC_L2;
+    dec.dist_mode = metric == VIX_METRIC_L2 ? 1 : metric == VIX_METRIC_IP ? 2 : 3;
+    return dec;
+}
+
+// The flat engine's two passes, apart (flat_knn_large_device runs them as knn_large_run; sharded search runs the seed on
+// every rank, takes the minimum of the ranks' bounds, then the collect): seed over T row blocks (empty when every row fits
+// the seed's budget), collect = the flat range kernel within the bound; both key (raw score word, row index).  The
+// functions capture q, xb and the mask by value and the seed's buffers of the object, which must outlive them.
+struct FlatKnnPass {
+    KnnDecode dec;
+    size_t seed_cap = 0, max_entries = 0;
+    std::function<int(const RangeOut&)> seed, collect;
+    Scratch<float> bd;
+    Scratch<int64_t> bi;
+};
+int flat_knn_pass(const float* q, int64_t nq, const float* xb, int64_t n, int d, int metric, int k,
+                  const uint64_t* disabled_rows, FlatKnnPass& p);
+
 // the flat engine's route (ids = row indices; disabled_rows: bit r set => row r skipped)
 int flat_knn_large_device(const float* q, int64_t nq, const float* xb, int64_t n, int d, int metric, int k,
                           const uint64_t* disabled_rows, size_t& cap_hint, float* out_dist, int64_t* out_rows, KnnInfo* info);

@@ -29,7 +29,9 @@
 
 #include <algorithm>
 #include <functional>
+#include <memory>
 #include <new>
+#include <optional>
 #include <vector>
 
 namespace vix {
@@ -285,9 +287,10 @@ __global__ void pack_result_keys_kernel(const float* __restrict__ dist, const in
 }
 
 // keys_all: [world][nq][k] as gathered; one CTA per query selects the k smallest of its world x k keys (padding keys
-// come out as NaN / id -1).  The keys hold zero distances as +0 (make_key folds -0); one GPU returns a zero inner-product
-// distance as -0 (the API distance -score of a +0 score) and a zero L2 distance as +0, so the metric restores the sign.
-__global__ void merge_shard_keys_kernel(const u64* __restrict__ keys_all, int world, int64_t nq, int k, int P2, int metric,
+// come out as NaN / id -1).  The keys hold zero distances as +0 (make_key folds -0); one GPU's IVF-PQ scan returns a zero
+// inner-product distance as -0 (the API distance -score of a +0 score), its IVF-Flat scan and every L2 distance +0, so
+// neg_zero (the kind's, as KnnDecode's) restores the sign.
+__global__ void merge_shard_keys_kernel(const u64* __restrict__ keys_all, int world, int64_t nq, int k, int P2, int neg_zero,
                                         float* __restrict__ out_dist, int64_t* __restrict__ out_ids) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     u64* s = reinterpret_cast<u64*>(smem_raw);
@@ -308,19 +311,19 @@ __global__ void merge_shard_keys_kernel(const u64* __restrict__ keys_all, int wo
             out_ids[o] = -1;
         } else {
             const float v = key_score(key, 0);
-            out_dist[o] = (v == 0.0f && metric == VIX_METRIC_IP) ? -0.0f : v;
+            out_dist[o] = (v == 0.0f && neg_zero) ? -0.0f : v;
             out_ids[o] = (int64_t)key_id(key);
         }
     }
 }
 
-static int merge_shard_keys(const u64* keys_all, int world, int64_t nq, int k, int metric, float* out_dist, int64_t* out_ids) {
+static int merge_shard_keys(const u64* keys_all, int world, int64_t nq, int k, int neg_zero, float* out_dist, int64_t* out_ids) {
     const int P2 = next_pow2(world * k < 2 ? 2 : world * k);
     const size_t smem = (size_t)P2 * 8;
     VIX_REQUIRE(smem <= 200 * 1024, VIX_ERR_UNSUPPORTED, "shard merge: %d keys per query exceed shared memory", world * k);
     VIX_CUDA(cudaFuncSetAttribute(merge_shard_keys_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     const int threads = P2 / 2 < 32 ? 32 : (P2 / 2 > 256 ? 256 : P2 / 2);
-    merge_shard_keys_kernel<<<(unsigned)nq, threads, smem, ctx().stream>>>(keys_all, world, nq, k, P2, metric, out_dist, out_ids);
+    merge_shard_keys_kernel<<<(unsigned)nq, threads, smem, ctx().stream>>>(keys_all, world, nq, k, P2, neg_zero, out_dist, out_ids);
     VIX_LAUNCH_CHECK();
     return VIX_OK;
 }
@@ -377,6 +380,18 @@ __global__ void gather_rows_kernel(const int32_t* __restrict__ order, int64_t n,
     for (int j = 0; j < m; ++j) out_codes[i * (int64_t)m + j] = codes[r * (int64_t)m + j];
 }
 
+// the IVF-Flat sibling of gather_rows_kernel: float rows of d components
+__global__ void gather_vec_rows_kernel(const int32_t* __restrict__ order, int64_t n, int d, const int32_t* __restrict__ assign,
+                                       const float* __restrict__ x, const int64_t* __restrict__ ids, int32_t* __restrict__ out_assign,
+                                       float* __restrict__ out_x, int64_t* __restrict__ out_ids) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const int64_t r = order[i];
+    out_assign[i] = assign[r];
+    out_ids[i] = ids[r];
+    for (int j = 0; j < d; ++j) out_x[i * (int64_t)d + j] = x[r * (int64_t)d + j];
+}
+
 // ------------------------------------------------------------------------------------------------ sharded range search
 // n u64 words of src -> byte offset `off` of every rank's range region (this rank's included)
 __global__ void peer_store_kernel(const u64* __restrict__ src, int64_t n, void* const* __restrict__ peer_base, int world,
@@ -419,6 +434,10 @@ __global__ void shard_range_lims_kernel(const int64_t* __restrict__ lims_all, in
 // row q that are <= it) + (keys of the higher ranks' runs of row q that are < it) in the merged row q: one binary search in
 // each other run.  Stable, and exact for equal keys on different ranks (one id stored in lists two ranks own): they keep
 // rank order, as one GPU's rows would hold them.  Returns that place, *row = q.
+// kWord: compare the high words only (the flat engine's keys, whose order within a run is (score word, row) and whose low
+// word then carries the user id): ties at one word keep rank order, and inside a rank the run's own order -- together the
+// global row order of one GPU holding the ranks' rows rank by rank.
+template <bool kWord = false>
 __device__ __forceinline__ int64_t shard_merge_place(const u64* __restrict__ keys, const int64_t* __restrict__ base,
                                                      const int64_t* __restrict__ lims_all, int world, int64_t nq, int64_t i,
                                                      int64_t* row) {
@@ -438,7 +457,14 @@ __device__ __forceinline__ int64_t shard_merge_place(const u64* __restrict__ key
         const int64_t* lp = lims_all + (size_t)p * L;
         const u64* run = keys + base[p] + lp[q];
         int64_t x = 0, y = lp[q + 1] - lp[q];
-        if (p < r) {
+        if (kWord) {
+            const uint32_t w = (uint32_t)(key >> 32);
+            if (p < r) {
+                while (x < y) { const int64_t mid = (x + y) >> 1; if ((uint32_t)(run[mid] >> 32) <= w) x = mid + 1; else y = mid; }
+            } else {
+                while (x < y) { const int64_t mid = (x + y) >> 1; if ((uint32_t)(run[mid] >> 32) < w) x = mid + 1; else y = mid; }
+            }
+        } else if (p < r) {
             while (x < y) { const int64_t mid = (x + y) >> 1; if (run[mid] <= key) x = mid + 1; else y = mid; }
         } else {
             while (x < y) { const int64_t mid = (x + y) >> 1; if (run[mid] < key) x = mid + 1; else y = mid; }
@@ -487,6 +513,105 @@ shard_knn_merge_kernel(const u64* __restrict__ keys, const int64_t* __restrict__
         const int64_t q = e / k, j = e - q * k;
         if (j >= glims[q + 1] - glims[q]) { out_dist[e] = __int_as_float(0x7fc00000); out_ids[e] = -1; }
     }
+}
+
+// ---- the flat kind: keys (raw score word in the metric's order, user id), merged by word and rank (trap: one GPU orders
+// flat results by (raw score, row) and maps to API distances only then -- sqrt and 1 - s can round two scores to one
+// distance, and equal scores fall to the smaller ROW, i.e. the lower rank, not the smaller id)
+__device__ __forceinline__ void flat_decode_key(u64 key, int order_max, int dist_mode, float* dist, int64_t* id) {
+    float v = key_score(key, order_max);
+    if (dist_mode == 1) v = __fsqrt_rn(v);
+    else if (dist_mode == 2) v = -v;
+    else if (dist_mode == 3) v = __fsub_rn(1.0f, v);
+    *dist = v;
+    *id = (int64_t)key_id(key);
+}
+
+// the per-rank CSR runs of the flat kind merged by (word, rank, place in the run), decoded with the flat API mapping: k > 0
+// cuts every merged row at k into out [nq x k] (padding id -1 / NaN past the row's length), k == 0 writes the whole rows at
+// glims
+__global__ void __launch_bounds__(256)
+shard_flat_merge_kernel(const u64* __restrict__ keys, const int64_t* __restrict__ base, const int64_t* __restrict__ lims_all,
+                        int world, int64_t nq, const int64_t* __restrict__ glims, int64_t total, int k, int order_max,
+                        int dist_mode, float* __restrict__ out_dist, int64_t* __restrict__ out_ids) {
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += stride) {
+        int64_t q;
+        const int64_t place = shard_merge_place<true>(keys, base, lims_all, world, nq, i, &q);
+        if (k == 0) flat_decode_key(keys[i], order_max, dist_mode, out_dist + glims[q] + place, out_ids + glims[q] + place);
+        else if (place < k) flat_decode_key(keys[i], order_max, dist_mode, out_dist + q * k + place, out_ids + q * k + place);
+    }
+    if (k == 0) return;
+    for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < nq * (int64_t)k; e += stride) {
+        const int64_t q = e / k, j = e - q * k;
+        if (j >= glims[q + 1] - glims[q]) { out_dist[e] = __int_as_float(0x7fc00000); out_ids[e] = -1; }
+    }
+}
+
+// k <= VIX_MAX_K: keys_all [world][nq][k], each rank's row its fused top-k (word, user id) in the flat search's order with
+// its padding (kEmptyKey: no real key is, ids being < 2^32 - 1) at the end.  One CTA per query: the length of every run
+// (its real keys, so that a NaN score -- word 0xFFFFFFFF -- is never confused with padding), then every real key to its
+// place by shard_merge_place's word rule, the places from the merged length to k padded.
+__global__ void __launch_bounds__(256)
+merge_flat_keys_kernel(const u64* __restrict__ keys_all, int world, int64_t nq, int k, int order_max, int dist_mode,
+                       float* __restrict__ out_dist, int64_t* __restrict__ out_ids) {
+    extern __shared__ int s_len[];                               // [world]
+    const int64_t q = blockIdx.x;
+    for (int r = threadIdx.x; r < world; r += blockDim.x) {
+        const u64* run = keys_all + ((size_t)r * nq + q) * k;
+        int x = 0, y = k;
+        while (x < y) { const int mid = (x + y) >> 1; if (run[mid] != kEmptyKey) x = mid + 1; else y = mid; }
+        s_len[r] = x;
+    }
+    __syncthreads();
+    int merged = 0;
+    for (int r = 0; r < world; ++r) merged += s_len[r];
+    for (int i = threadIdx.x; i < world * k; i += blockDim.x) {
+        const int r = i / k, j = i - r * k;
+        if (j >= s_len[r]) continue;
+        const u64 key = keys_all[((size_t)r * nq + q) * k + j];
+        const uint32_t w = (uint32_t)(key >> 32);
+        int pos = j;
+        for (int p = 0; p < world && pos < k; ++p) {
+            if (p == r) continue;
+            const u64* run = keys_all + ((size_t)p * nq + q) * k;
+            int x = 0, y = s_len[p];
+            if (p < r) {
+                while (x < y) { const int mid = (x + y) >> 1; if ((uint32_t)(run[mid] >> 32) <= w) x = mid + 1; else y = mid; }
+            } else {
+                while (x < y) { const int mid = (x + y) >> 1; if ((uint32_t)(run[mid] >> 32) < w) x = mid + 1; else y = mid; }
+            }
+            pos += x;
+        }
+        if (pos < k) flat_decode_key(key, order_max, dist_mode, out_dist + q * k + pos, out_ids + q * k + pos);
+    }
+    for (int j = merged + threadIdx.x; j < k; j += blockDim.x) {
+        out_dist[q * k + j] = __int_as_float(0x7fc00000);
+        out_ids[q * k + j] = -1;
+    }
+}
+
+// a rank's fused flat top-k (raw scores, local rows, -1 padding) -> keys (score word, user id of the row; row_ids == nullptr:
+// the row itself) for slot `rank` of every destination, as pack_result_keys_kernel
+__global__ void pack_flat_keys_kernel(const float* __restrict__ score, const int64_t* __restrict__ rows,
+                                      const int64_t* __restrict__ row_ids, int64_t total, int order_max,
+                                      void* const* __restrict__ peer_base, int world, size_t off, u64* __restrict__ local_only) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= total) return;
+    const int64_t r = rows[i];
+    const u64 key = r < 0 ? kEmptyKey : make_key(score[i], (uint32_t)(row_ids ? row_ids[r] : r), order_max);
+    if (local_only) { local_only[i] = key; return; }
+    for (int p = 0; p < world; ++p) reinterpret_cast<u64*>(static_cast<char*>(peer_base[p]) + off)[i] = key;
+}
+
+// the low word of every key of the sorted rows (lims [nq + 1]) from local row to user id; the order stays (one CTA per row)
+__global__ void __launch_bounds__(256)
+relabel_rows_kernel(u64* __restrict__ keys, const int64_t* __restrict__ lims, int64_t nq, const int64_t* __restrict__ row_ids) {
+    for (int64_t q = blockIdx.x; q < nq; q += gridDim.x)
+        for (int64_t i = lims[q] + threadIdx.x; i < lims[q + 1]; i += blockDim.x) {
+            const u64 key = keys[i];
+            keys[i] = (key & 0xFFFFFFFF00000000ull) | (uint32_t)row_ids[(uint32_t)key];
+        }
 }
 
 // flag += queries whose merged row (the sum of the ranks' trimmed rows, lims_all as above) is shorter than k although their
@@ -538,25 +663,71 @@ static int shard_range_lims(const int64_t* lims_all, int world, int64_t nq, int6
 }
 
 static int shard_range_merge(const u64* keys, const int64_t* base_dev, const int64_t* lims_all, int world, int64_t nq,
-                             const int64_t* glims, int64_t total, int metric, vix_range_result* r) {
+                             const int64_t* glims, int64_t total, int neg_zero, vix_range_result* r) {
     cudaStream_t s = ctx().stream;
     VIX_CUDA(cudaMemcpyAsync(r->lims, glims, (size_t)(nq + 1) * 8, cudaMemcpyDeviceToDevice, s));
     if (total == 0) return VIX_OK;
     const int64_t want = (total + 255) / 256;
     const unsigned grid = (unsigned)(want < (int64_t)num_sms() * 8 ? want : (int64_t)num_sms() * 8);
-    shard_range_merge_kernel<<<grid, 256, 0, s>>>(keys, base_dev, lims_all, world, nq, glims, total,
-                                                  metric == VIX_METRIC_IP ? 1 : 0, r->dist, r->ids);
+    shard_range_merge_kernel<<<grid, 256, 0, s>>>(keys, base_dev, lims_all, world, nq, glims, total, neg_zero, r->dist, r->ids);
     VIX_LAUNCH_CHECK();
     return VIX_OK;
 }
 
 static int shard_knn_merge(const u64* keys, const int64_t* base_dev, const int64_t* lims_all, int world, int64_t nq,
-                           const int64_t* glims, int64_t total, int k, int metric, float* out_dist, int64_t* out_ids) {
+                           const int64_t* glims, int64_t total, int k, int neg_zero, float* out_dist, int64_t* out_ids) {
     const int64_t want = (std::max<int64_t>(total, nq * (int64_t)k) + 255) / 256;
     const unsigned grid = (unsigned)(want < (int64_t)num_sms() * 8 ? want : (int64_t)num_sms() * 8);
-    shard_knn_merge_kernel<<<grid, 256, 0, ctx().stream>>>(keys, base_dev, lims_all, world, nq, glims, total, k,
-                                                           metric == VIX_METRIC_IP ? 1 : 0, out_dist, out_ids);
+    shard_knn_merge_kernel<<<grid, 256, 0, ctx().stream>>>(keys, base_dev, lims_all, world, nq, glims, total, k, neg_zero,
+                                                           out_dist, out_ids);
     VIX_LAUNCH_CHECK();
+    return VIX_OK;
+}
+
+// the flat kind's merge of the ranks' CSR runs (shard_flat_merge_kernel; k == 0: whole rows at glims)
+static int shard_flat_merge(const u64* keys, const int64_t* base_dev, const int64_t* lims_all, int world, int64_t nq,
+                            const int64_t* glims, int64_t total, int k, int metric, float* out_dist, int64_t* out_ids) {
+    const KnnDecode dec = flat_knn_decode(metric);
+    const int64_t want = (std::max<int64_t>(total, nq * (int64_t)k) + 255) / 256;
+    if (want == 0) return VIX_OK;
+    const unsigned grid = (unsigned)(want < (int64_t)num_sms() * 8 ? want : (int64_t)num_sms() * 8);
+    shard_flat_merge_kernel<<<grid, 256, 0, ctx().stream>>>(keys, base_dev, lims_all, world, nq, glims, total, k, dec.order_max,
+                                                            dec.dist_mode, out_dist, out_ids);
+    VIX_LAUNCH_CHECK();
+    return VIX_OK;
+}
+
+// the flat kind's merge of k <= VIX_MAX_K: keys_all [world][nq][k] -> out [nq x k]
+static int merge_flat_keys(const u64* keys_all, int world, int64_t nq, int k, int metric, float* out_dist, int64_t* out_ids) {
+    if (nq == 0) return VIX_OK;
+    const KnnDecode dec = flat_knn_decode(metric);
+    merge_flat_keys_kernel<<<(unsigned)nq, 256, (size_t)world * 4, ctx().stream>>>(keys_all, world, nq, k, dec.order_max,
+                                                                                  dec.dist_mode, out_dist, out_ids);
+    VIX_LAUNCH_CHECK();
+    return VIX_OK;
+}
+
+// The sign one GPU gives a zero distance (the keys hold +0): k-NN of the IVF-PQ scan with inner product -0, of the IVF-Flat
+// scan +0 (it keys the distance itself); the flat engine's mapping (flat_knn_decode) restores its own.  Range search: the
+// flat engine's and the IVF-PQ scan's inner product -0, IVF-Flat +0.
+static int knn_neg_zero(const vix_index* h) { return h->p.kind == VIX_INDEX_IVF_PQ && h->p.metric == VIX_METRIC_IP; }
+static int range_neg_zero(const vix_index* h) { return h->p.kind != VIX_INDEX_IVF_FLAT && h->p.metric == VIX_METRIC_IP; }
+
+static const char* kind_name(const vix_index* h) {
+    return h->p.kind == VIX_INDEX_FLAT ? "flat" : h->p.kind == VIX_INDEX_IVF_FLAT ? "ivfflat" : "ivfpq";
+}
+
+// What a sharded call needs of the handle, checked on every rank before any exchange: an IVF-PQ index trained, with L2 / IP
+// (the messages and codes of the IVF-PQ-only layout); an IVF-Flat index with coarse centroids (the sharded layout files
+// every row into its list: there is no "rows wait for optimize()" state); a flat index as it is.
+static int sharded_kind_check(const vix_index* h, const char* who) {
+    if (h->p.kind == VIX_INDEX_IVF_PQ) {
+        VIX_REQUIRE(h->has_coarse && h->has_pq, VIX_ERR_NOT_TRAINED, "%s: needs a trained IVF-PQ index", who);
+        VIX_REQUIRE(h->p.metric != VIX_METRIC_COSINE, VIX_ERR_UNSUPPORTED, "%s: L2 / IP only", who);
+    } else if (h->p.kind == VIX_INDEX_IVF_FLAT) {
+        VIX_REQUIRE(h->has_coarse, VIX_ERR_NOT_TRAINED, "%s: an IVF-Flat index needs its coarse centroids (set or trained) "
+                    "before it is sharded", who);
+    }
     return VIX_OK;
 }
 
@@ -730,6 +901,9 @@ namespace vix {
 // (probes, plus the queries when they came from the host) reaches every rank -- stored into every peer's region with one
 // barrier, or an NCCL all-gather.  On return px.queries / px.probes are the whole batch's queries and probe lists on the
 // device.  The caller holds both mutexes and has called ensure_region.
+// A flat index has no probes (px.probes stays null): only the queries travel, and over peer memory the barrier still
+// comes first -- it is what orders this call's stores into the peers' regions (the result slab, the range region) after
+// every peer's reads of them in the previous call.
 struct BatchProbes {
     In<float> dq;
     const float* queries = nullptr;
@@ -743,6 +917,8 @@ static int exchange_probes(vix_index* h, vix_comm* c, const float* queries, int6
     const int64_t per = block_rows(nq, world);
     const int64_t lo = nq < (int64_t)rank * per ? nq : (int64_t)rank * per;
     const int64_t cnt = (nq < lo + per ? nq : lo + per) - lo;
+    const bool flat = h->p.kind == VIX_INDEX_FLAT;
+    if (flat) nprobe = 0;
     if (c->peer_state == 1) {
         char* base = static_cast<char*>(c->local);
         float* qbuf = reinterpret_cast<float*>(base + c->off_queries);          // [world * per][d] (this call's per)
@@ -753,12 +929,11 @@ static int exchange_probes(vix_index* h, vix_comm* c, const float* queries, int6
             VIX_CUDA(cudaMemcpyAsync(qbuf + (size_t)lo * d, qblock, (size_t)cnt * d * 4, cudaMemcpyHostToDevice, s));
             qblock = qbuf + (size_t)lo * d;
         }
-        // 2. its probe lists against ALL centroids, straight into slot `rank` of the local probe buffer
+        // 2. its probe lists against ALL centroids (the selection of index_search_locked: cosine or fast, by the metric),
+        //    straight into slot `rank` of the local probe buffer
         int32_t* pblock = pbuf + (size_t)rank * per * nprobe;
-        if (cnt > 0)
-            VIX_TRY(probe_select_fast_device(qblock, cnt, h->coarse.ptr, h->kc, d, h->p.metric, nprobe, h->coarse_norms.ptr,
-                                             pblock, nullptr, h->coarse_norm_max.ptr));
-        if (cnt < per) VIX_TRY(fill<int32_t>(pblock + (size_t)cnt * nprobe, (per - cnt) * nprobe, -1));
+        if (!flat && cnt > 0) VIX_TRY(select_probes_device(h, qblock, cnt, nprobe, pblock));
+        if (!flat && cnt < per) VIX_TRY(fill<int32_t>(pblock + (size_t)cnt * nprobe, (per - cnt) * nprobe, -1));
         // 3. the block travels to every peer (probes, and the queries when they came from the host), one barrier
         const size_t offA = c->off_probes + (size_t)rank * per * nprobe * 4, nA = (size_t)per * nprobe * 4 / 16;
         const size_t offB = c->off_queries + (size_t)rank * per * d * 4, nB = host_q ? (size_t)per * d * 4 / 16 : 0;
@@ -769,11 +944,13 @@ static int exchange_probes(vix_index* h, vix_comm* c, const float* queries, int6
         VIX_LAUNCH_CHECK();
         VIX_TRY(peer_barrier(c));
         px.queries = host_q ? qbuf : queries;
-        px.probes = pbuf;
+        px.probes = flat ? nullptr : pbuf;
         return VIX_OK;
     }
     // NCCL carries the exchange
     VIX_TRY(px.dq.stage(queries, (size_t)nq * d));
+    px.queries = px.dq.dev;
+    if (flat) return VIX_OK;
     const size_t pbytes = (size_t)world * per * nprobe * 4;
     if (pbytes > c->gather_probes_bytes) {
         if (c->gather_probes) { VIX_CUDA(cudaStreamSynchronize(s)); cudaFree(c->gather_probes); c->gather_probes = nullptr; }
@@ -782,9 +959,7 @@ static int exchange_probes(vix_index* h, vix_comm* c, const float* queries, int6
     }
     int32_t* pall = static_cast<int32_t*>(c->gather_probes);
     int32_t* pblock = pall + (size_t)rank * per * nprobe;
-    if (cnt > 0)
-        VIX_TRY(probe_select_fast_device(px.dq.dev + (size_t)lo * d, cnt, h->coarse.ptr, h->kc, d, h->p.metric, nprobe,
-                                         h->coarse_norms.ptr, pblock, nullptr, h->coarse_norm_max.ptr));
+    if (cnt > 0) VIX_TRY(select_probes_device(h, px.dq.dev + (size_t)lo * d, cnt, nprobe, pblock));
     if (cnt < per) VIX_TRY(fill<int32_t>(pblock + (size_t)cnt * nprobe, (per - cnt) * nprobe, -1));
     VIX_NCCL(g_nccl.AllGather(pblock, pall, (size_t)per * nprobe, ncclInt32, c->comm, s));   // in place
     px.queries = px.dq.dev;
@@ -803,53 +978,142 @@ static int stage_filter(const uint64_t* words, int64_t capacity, int mode, In<ui
     return VIX_OK;
 }
 
+// A rank's pass of k <= VIX_MAX_K over what it holds, packed as keys for slot `rank` of every destination (peer_base, off)
+// or into local_only [nq x k].  IVF kinds: the fused scan over the probed lists the rank owns (a filter sends it down the
+// query-major path), keys (API distance, id).  Flat: the fused flat search over the rank's rows with raw scores, keys
+// (score word in the metric's order, user id of the row) -- merged by merge_flat_keys_kernel, never on the full key.
+// scanned (nullable): an event recorded between the scan and the pack (the trace's phase boundary).
+static int local_knn_keys(vix_index* h, const float* dq, int64_t nq, int k, int nprobe, const int32_t* probes,
+                          const FilterArgs* filter, void* const* peer_base, int world, size_t off, u64* local_only,
+                          cudaEvent_t scanned = nullptr) {
+    cudaStream_t s = ctx().stream;
+    const int64_t total = nq * (int64_t)k;
+    Scratch<float> ldist;
+    Scratch<int64_t> lids;
+    VIX_TRY(ldist.alloc((size_t)total));
+    VIX_TRY(lids.alloc((size_t)total));
+    const unsigned grid = (unsigned)((total + 255) / 256);
+    if (h->p.kind == VIX_INDEX_FLAT) {
+        const int d = h->p.d, metric = h->p.metric;
+        Scratch<uint64_t> mask;
+        VIX_TRY(filter_row_mask(h, filter, mask));
+        if (mask.ptr) VIX_TRY(flat_search_masked_device(dq, nq, h->vecs.ptr, h->n, d, metric, k, mask.ptr, ldist.ptr, lids.ptr, true));
+        else VIX_TRY(flat_search_auto_device(dq, nq, h->vecs.ptr, h->n, d, metric, k, nullptr, ldist.ptr, lids.ptr, true));
+        if (scanned) VIX_CUDA(cudaEventRecord(scanned, s));
+        pack_flat_keys_kernel<<<grid, 256, 0, s>>>(ldist.ptr, lids.ptr, h->ids.ptr, total, metric != VIX_METRIC_L2, peer_base, world,
+                                                   off, local_only);
+    } else {
+        VIX_TRY(index_search_locked(h, dq, nq, k, nprobe, ldist.ptr, lids.ptr, nullptr, nullptr, probes, filter));
+        if (scanned) VIX_CUDA(cudaEventRecord(scanned, s));
+        pack_result_keys_kernel<<<grid, 256, 0, s>>>(ldist.ptr, lids.ptr, total, peer_base, world, off, local_only);
+    }
+    VIX_LAUNCH_CHECK();
+    return VIX_OK;
+}
+
+// the merge of k <= VIX_MAX_K over the gathered keys [world][nq][k], by kind
+static int merge_knn_keys(const vix_index* h, const u64* keys_all, int world, int64_t nq, int k, float* out_dist, int64_t* out_ids) {
+    if (h->p.kind == VIX_INDEX_FLAT) return merge_flat_keys(keys_all, world, nq, k, h->p.metric, out_dist, out_ids);
+    return merge_shard_keys(keys_all, world, nq, k, knn_neg_zero(h), out_dist, out_ids);
+}
+
+// The rank-local halves of k > VIX_MAX_K (sharded_knn_large, and the one-GPU emulation of the ranks): the seed -> tau_r;
+// then, with the ranks' minimum, the collect within it and every sorted row cut at k.  IVF kinds: the kind's range scan
+// over the probe prefix of the lists the rank owns / over every probed list, keys (API distance, id).  Flat: the flat
+// engine's seed blocks and range kernel over the rank's rows, keys (score word, row), the cut rows relabelled to user ids
+// in place (their order stays: the word, then the row).
+struct LocalKnnLarge {
+    IvfRangeScan scan;
+    Scratch<int32_t> prefix;
+    Scratch<uint64_t> mask;
+    FlatKnnPass flat;
+    std::function<int(const RangeOut&)> seed, collect;
+    size_t seed_cap = 0, max_entries = 0;
+};
+
+static int local_knn_prepare(vix_index* h, const float* dq, int64_t nq, int k, int nprobe, const int32_t* probes,
+                             const FilterArgs* filter, LocalKnnLarge& L) {
+    if (h->p.kind == VIX_INDEX_FLAT) {
+        VIX_TRY(filter_row_mask(h, filter, L.mask));
+        VIX_TRY(flat_knn_pass(dq, nq, h->vecs.ptr, h->n, h->p.d, h->p.metric, k, L.mask.ptr, L.flat));
+        L.seed = L.flat.seed;
+        L.collect = L.flat.collect;
+        L.seed_cap = L.flat.seed_cap;
+        L.max_entries = L.flat.max_entries;
+        return VIX_OK;
+    }
+    VIX_TRY(ivf_range_scan(h, dq, nq, nprobe, probes, filter, L.scan));
+    VIX_TRY(L.prefix.alloc((size_t)nq * nprobe));
+    VIX_TRY(knn_probe_prefix(probes, nq, nprobe, h->list_len.ptr, h->kc, k, L.prefix.ptr, &L.seed_cap, &L.max_entries));
+    IvfRangeScan* sc = &L.scan;
+    const int32_t* pre = L.prefix.ptr;
+    L.seed = [sc, pre](const RangeOut& o) { return sc->run(pre, o); };
+    L.collect = [sc, probes](const RangeOut& o) { return sc->run(probes, o); };
+    return VIX_OK;
+}
+
+static int local_knn_seed(LocalKnnLarge& L, int64_t nq, int k, uint32_t* tau, int64_t* seed_n) {
+    return knn_seed_bound(nq, k, L.seed_cap, L.seed ? &L.seed : nullptr, tau, seed_n);
+}
+
+static int local_knn_cut(vix_index* h, LocalKnnLarge& L, int64_t nq, int k, const uint32_t* tau, size_t& cap, RangeKeys& rk,
+                         RangeKeys& cut, RangeInfo* ci) {
+    VIX_TRY(knn_collect(nq, k, tau, L.collect, L.max_entries, cap, rk, ci, nullptr));
+    VIX_TRY(knn_trim(nq, k, rk, cut));
+    if (h->p.kind == VIX_INDEX_FLAT && cut.sorted) {
+        const unsigned grid = (unsigned)std::min<int64_t>((int64_t)num_sms() * 8, nq);
+        relabel_rows_kernel<<<grid, 256, 0, ctx().stream>>>(cut.sorted, cut.lims.ptr, nq, h->ids.ptr);
+        VIX_LAUNCH_CHECK();
+    }
+    return VIX_OK;
+}
+
 // forward: k > VIX_MAX_K at world > 1 (below)
 static int sharded_knn_large(vix_index* h, vix_comm* c, const float* queries, int64_t nq, int k, int nprobe,
                              const FilterArgs* filter, float* out_dist, int64_t* out_ids);
 
 // vix_sharded_search and vix_sharded_search_filtered (filter == nullptr: the unfiltered step, launch for launch; k above
-// VIX_MAX_K at world > 1: sharded_knn_large)
+// VIX_MAX_K at world > 1: sharded_knn_large).  A flat index has no probes: phase 1 is empty and every rank searches its rows.
 static int sharded_search(vix_index* h, vix_comm* c, const float* queries, int64_t nq, int k, int nprobe, const FilterArgs* filter,
                           float* out_dist, int64_t* out_ids) {
     std::lock_guard<std::mutex> lc(c->mu);
     std::lock_guard<std::mutex> lk(h->mu);
-    VIX_REQUIRE(h->p.kind == VIX_INDEX_IVF_PQ && h->has_coarse && h->has_pq, VIX_ERR_NOT_TRAINED, "vix_sharded_search: needs a trained IVF-PQ index");
-    VIX_REQUIRE(h->p.metric != VIX_METRIC_COSINE, VIX_ERR_UNSUPPORTED, "vix_sharded_search: L2 / IP only");
-    if (nprobe <= 0) nprobe = h->p.nprobe;
-    VIX_REQUIRE(nprobe > 0 && nprobe <= VIX_MAX_K, VIX_ERR_INVALID_K, "vix_sharded_search: nprobe");
+    VIX_TRY(sharded_kind_check(h, "vix_sharded_search"));
+    const bool flat = h->p.kind == VIX_INDEX_FLAT;
+    if (!flat) {
+        if (nprobe <= 0) nprobe = h->p.nprobe;
+        VIX_REQUIRE(nprobe > 0 && nprobe <= VIX_MAX_K, VIX_ERR_INVALID_K, "vix_sharded_search: nprobe");
+    }
     const int world = c->world, rank = c->rank, d = h->p.d;
     if (world == 1) return index_search_locked(h, queries, nq, k, nprobe, out_dist, out_ids, nullptr, nullptr, nullptr, filter);
-    if (h->dirty) VIX_TRY(build_lists(h));
+    if (!flat && h->dirty) VIX_TRY(build_lists(h));
     if (k > VIX_MAX_K) return sharded_knn_large(h, c, queries, nq, k, nprobe, filter, out_dist, out_ids);
     cudaStream_t s = ctx().stream;
-    VIX_TRY(ensure_region(c, nq, d, nprobe, k));
-    ThrHookScope thr_scope(c);                                        // (cleared again on every way out)
+    VIX_TRY(ensure_region(c, nq, d, flat ? 1 : nprobe, k));
+    // the list-major scan's bounds over the ranks (only an IVF-PQ index can take that scan; cleared again on every way out)
+    std::optional<ThrHookScope> thr_scope;
+    if (h->p.kind == VIX_INDEX_IVF_PQ) thr_scope.emplace(c);
     const int64_t total = nq * (int64_t)k;
     Out<float> dd;
     Out<int64_t> di;
     VIX_TRY(dd.stage(out_dist, (size_t)total));
     VIX_TRY(di.stage(out_ids, (size_t)total));
-    Scratch<float> ldist;
-    Scratch<int64_t> lids;
-    VIX_TRY(ldist.alloc((size_t)total));
-    VIX_TRY(lids.alloc((size_t)total));
     auto mark = [&](int i) { if (c->trace) cudaEventRecord(c->ev[i], s); };
     mark(0);
-    // 1-3. probes of this rank's block, exchanged
+    // 1-3. probes of this rank's block, exchanged (flat: the queries only)
     BatchProbes px;
     VIX_TRY(exchange_probes(h, c, queries, nq, nprobe, px));
+    const float* dq = px.queries;
+    const int32_t* probes = px.probes;
     mark(1);
-    // 4. fused scan over the probed lists this rank owns (a filter sends it down the query-major path)
-    VIX_TRY(index_search_locked(h, px.queries, nq, k, nprobe, ldist.ptr, lids.ptr, nullptr, nullptr, px.probes, filter));
-    mark(2);
-    // 5. its top-k leaves as packed keys for slot `rank` of every rank's result buffer; barrier (or all-gather); merge
+    // 4-5. the local pass; its top-k leaves as packed keys for slot `rank` of every rank's result buffer; barrier (or
+    //      all-gather); merge
     if (c->peer_state == 1) {
         u64* rbuf = reinterpret_cast<u64*>(static_cast<char*>(c->local) + c->off_results);   // [world][nq][k]
-        pack_result_keys_kernel<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(ldist.ptr, lids.ptr, total, c->peer_dev, world,
-                                                                              c->off_results + (size_t)rank * total * 8, nullptr);
-        VIX_LAUNCH_CHECK();
+        VIX_TRY(local_knn_keys(h, dq, nq, k, nprobe, probes, filter, c->peer_dev, world, c->off_results + (size_t)rank * total * 8,
+                               nullptr, c->trace ? c->ev[2] : nullptr));
         VIX_TRY(peer_barrier(c));
-        VIX_TRY(merge_shard_keys(rbuf, world, nq, k, h->p.metric, dd.dev, di.dev));
+        VIX_TRY(merge_knn_keys(h, rbuf, world, nq, k, dd.dev, di.dev));
     } else {
         const size_t kbytes = (size_t)world * total * 8;
         if (kbytes > c->gather_keys_bytes) {
@@ -858,11 +1122,10 @@ static int sharded_search(vix_index* h, vix_comm* c, const float* queries, int64
             c->gather_keys_bytes = kbytes;
         }
         u64* kall = static_cast<u64*>(c->gather_keys);
-        pack_result_keys_kernel<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(ldist.ptr, lids.ptr, total, nullptr, world, 0,
-                                                                              kall + (size_t)rank * total);
-        VIX_LAUNCH_CHECK();
+        VIX_TRY(local_knn_keys(h, dq, nq, k, nprobe, probes, filter, nullptr, world, 0, kall + (size_t)rank * total,
+                               c->trace ? c->ev[2] : nullptr));
         VIX_NCCL(g_nccl.AllGather(kall + (size_t)rank * total, kall, (size_t)total, ncclUint64, c->comm, s));
-        VIX_TRY(merge_shard_keys(kall, world, nq, k, h->p.metric, dd.dev, di.dev));
+        VIX_TRY(merge_knn_keys(h, kall, world, nq, k, dd.dev, di.dev));
     }
     mark(3);
     VIX_TRY(dd.commit());
@@ -873,12 +1136,16 @@ static int sharded_search(vix_index* h, vix_comm* c, const float* queries, int64
 // The last step of sharded_range_exchange: range search decodes the merged rows into a new result object (*out); k-NN
 // search beyond VIX_MAX_K (out == nullptr) cuts them at k into [nq x k] (dist, ids: device), after checking on the exchanged
 // row starts that no row whose bound is finite came out shorter than k.
+// neg_zero: the kind's zero sign (knn_neg_zero / range_neg_zero); flat_metric >= 0: the flat kind's k-NN keys (score word,
+// user id), merged by shard_flat_merge with that metric's mapping.
 struct ShardTail {
     vix_range_result** out = nullptr;
     int k = 0;
     const uint32_t* bound = nullptr;
     float* dist = nullptr;
     int64_t* ids = nullptr;
+    int neg_zero = 0;
+    int flat_metric = -1;
 };
 // what the exchange reports for the VIX_SCAN_DEBUG lines: this rank's entries, the merged entries, the longest merged row
 struct ShardTotals { int64_t mine = 0, total = 0, max_row = 0; bool grown = false; };
@@ -990,12 +1257,14 @@ static int sharded_range_exchange(vix_index* h, vix_comm* c, int64_t nq, int rc,
         }
         keys = kall.ptr;
     }
-    const int mr = knn ? shard_knn_merge(keys, dbase.ptr, lims_all.ptr, world, nq, glims.ptr, total, t.k, h->p.metric, t.dist, t.ids)
-                       : shard_range_merge(keys, dbase.ptr, lims_all.ptr, world, nq, glims.ptr, total, h->p.metric, r);
+    const int mr = !knn ? shard_range_merge(keys, dbase.ptr, lims_all.ptr, world, nq, glims.ptr, total, t.neg_zero, r)
+                 : t.flat_metric >= 0 ? shard_flat_merge(keys, dbase.ptr, lims_all.ptr, world, nq, glims.ptr, total, t.k, t.flat_metric,
+                                                          t.dist, t.ids)
+                 : shard_knn_merge(keys, dbase.ptr, lims_all.ptr, world, nq, glims.ptr, total, t.k, t.neg_zero, t.dist, t.ids);
     if (mr != VIX_OK) return fail(mr);
     if (getenv("VIX_SCAN_DEBUG") && !knn)
-        fprintf(stderr, "[vix sharded range] world %d, peer %d, local %lld, total %lld, max_row %lld, grown %d\n", world,
-                peer ? 1 : 0, (long long)mine_n, (long long)total, (long long)max_row, grown ? 1 : 0);
+        fprintf(stderr, "[vix sharded range] world %d, peer %d, local %lld, total %lld, max_row %lld, grown %d, kind %s\n", world,
+                peer ? 1 : 0, (long long)mine_n, (long long)total, (long long)max_row, grown ? 1 : 0, kind_name(h));
     st->mine = mine_n; st->total = total; st->max_row = max_row; st->grown = grown;
     if (!knn) *t.out = r;
     return VIX_OK;
@@ -1023,17 +1292,19 @@ static int bound_min_over_ranks(vix_comm* c, uint32_t* tau, int64_t nq) {
 
 // vix_sharded_search / vix_sharded_search_filtered with VIX_MAX_K < k <= VIX_MAX_K_LARGE and world > 1: the one-GPU two-pass
 // route (vix_knn_large.cu) with one bound per query shared by all ranks (see shard_knn_merge_kernel for why it is exact):
-//   1. the probes of the batch, exchanged as for every sharded call;
-//   2. each rank's seed over the probe prefix of the lists it owns (those it does not own have length 0) -> tau_r;
+//   1. the probes of the batch, exchanged as for every sharded call (flat: none);
+//   2. each rank's seed over the probe prefix of the lists it owns (those it does not own have length 0; flat: the flat
+//      engine's seed blocks over its rows) -> tau_r;
 //   3. tau = the minimum of the tau_r over the ranks;
-//   4. each rank's collect within tau over every probed list it owns, each sorted row cut at k (knn_trim);
-//   5. the cut rows exchanged as range search exchanges its rows, merged, and cut at k into [nq x k].
+//   4. each rank's collect within tau over every probed list it owns (flat: its rows), each sorted row cut at k (knn_trim);
+//   5. the cut rows exchanged as range search exchanges its rows, merged (flat: by score word and rank), and cut at k.
 // A rank whose seed or collect fails still enters every exchange (all-ones bounds, empty rows and its status), so every
 // rank returns its code.  Synchronises the stream; the handle's knn_cap is written once the call has succeeded.
 static int sharded_knn_large(vix_index* h, vix_comm* c, const float* queries, int64_t nq, int k, int nprobe,
                              const FilterArgs* filter, float* out_dist, int64_t* out_ids) {
     cudaStream_t s = ctx().stream;
-    VIX_TRY(ensure_region(c, nq, h->p.d, nprobe, 1));                 // (no [world x nq x k] result slab: k is large)
+    const bool flat = h->p.kind == VIX_INDEX_FLAT;
+    VIX_TRY(ensure_region(c, nq, h->p.d, flat ? 1 : nprobe, 1));     // (no [world x nq x k] result slab: k is large)
     bool grown = false;
     if (c->peer_state == 1) VIX_TRY(ensure_range_region(c, nq, 0, &grown));
     Out<float> dd;
@@ -1046,19 +1317,14 @@ static int sharded_knn_large(vix_index* h, vix_comm* c, const float* queries, in
     mark(0);
     BatchProbes px;
     VIX_TRY(exchange_probes(h, c, queries, nq, nprobe, px));
+    const float* dq = px.queries;
+    const int32_t* probes = px.probes;
     mark(1);
     // 2. the local seed -> tau_r
-    IvfRangeScan scan;
-    Scratch<int32_t> prefix;
-    size_t seed_cap = 0, max_entries = 0;
+    LocalKnnLarge L;
     int64_t seed_n = 0;
-    int rc = ivf_range_scan(h, px.queries, nq, nprobe, px.probes, filter, scan);
-    if (rc == VIX_OK) rc = prefix.alloc((size_t)nq * nprobe);
-    if (rc == VIX_OK)
-        rc = knn_probe_prefix(px.probes, nq, nprobe, h->list_len.ptr, h->kc, k, prefix.ptr, &seed_cap, &max_entries);
-    const std::function<int(const RangeOut&)> seed = [&](const RangeOut& o) { return scan.run(prefix.ptr, o); };
-    const std::function<int(const RangeOut&)> collect = [&](const RangeOut& o) { return scan.run(px.probes, o); };
-    if (rc == VIX_OK) rc = knn_seed_bound(nq, k, seed_cap, &seed, tau.ptr, &seed_n);
+    int rc = local_knn_prepare(h, dq, nq, k, nprobe, probes, filter, L);
+    if (rc == VIX_OK) rc = local_knn_seed(L, nq, k, tau.ptr, &seed_n);
     if (rc != VIX_OK) VIX_CUDA(cudaMemsetAsync(tau.ptr, 0xFF, (size_t)nq * 4, s));
     // 3. tau = min over the ranks
     VIX_TRY(bound_min_over_ranks(c, tau.ptr, nq));
@@ -1066,19 +1332,20 @@ static int sharded_knn_large(vix_index* h, vix_comm* c, const float* queries, in
     RangeKeys rk, cut;
     RangeInfo ci;
     size_t cap = h->knn_cap;
-    if (rc == VIX_OK) rc = knn_collect(nq, k, tau.ptr, collect, max_entries, cap, rk, &ci, nullptr);
-    if (rc == VIX_OK) rc = knn_trim(nq, k, rk, cut);
+    if (rc == VIX_OK) rc = local_knn_cut(h, L, nq, k, tau.ptr, cap, rk, cut, &ci);
     mark(2);
     // 5. exchange, merge, cut
     ShardTail tail;
     tail.k = k; tail.bound = tau.ptr; tail.dist = dd.dev; tail.ids = di.dev;
+    tail.neg_zero = knn_neg_zero(h);
+    tail.flat_metric = flat ? h->p.metric : -1;
     ShardTotals st;
     VIX_TRY(sharded_range_exchange(h, c, nq, rc, cut, grown, tail, &st));
     mark(3);
     if (getenv("VIX_SCAN_DEBUG"))
         fprintf(stderr, "[vix sharded knn] world %d, peer %d, k %d, seed %lld, local %lld, sent %lld, total %lld, max_row %lld, "
-                "grown %d\n", c->world, c->peer_state == 1 ? 1 : 0, k, (long long)seed_n, (long long)ci.total,
-                (long long)st.mine, (long long)st.total, (long long)st.max_row, st.grown ? 1 : 0);
+                "grown %d, kind %s\n", c->world, c->peer_state == 1 ? 1 : 0, k, (long long)seed_n, (long long)ci.total,
+                (long long)st.mine, (long long)st.total, (long long)st.max_row, st.grown ? 1 : 0, kind_name(h));
     VIX_TRY(dd.commit());
     VIX_TRY(di.commit());
     VIX_TRY(finish(true));
@@ -1099,7 +1366,7 @@ struct DebugShardRuns {
 };
 
 static int debug_shard_runs(const char* who, const int64_t* lims_all, const float* dist_all, const int64_t* ids_all, int world,
-                            int64_t nq, DebugShardRuns& in) {
+                            int64_t nq, DebugShardRuns& in, int flat_order_max = -1) {
     cudaStream_t s = ctx().stream;
     const int64_t L = nq + 2;
     // the ranks' lims [world][nq + 1] -> the exchanged layout [world][nq + 2] (status 0)
@@ -1125,8 +1392,12 @@ static int debug_shard_runs(const char* who, const int64_t* lims_all, const floa
     VIX_TRY(in.di.stage(ids_all, (size_t)total));
     VIX_TRY(in.keys.alloc((size_t)total));
     if (total > 0) {
-        pack_result_keys_kernel<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(in.dd.dev, in.di.dev, total, nullptr, world, 0,
-                                                                              in.keys.ptr);
+        if (flat_order_max >= 0)                                          // (raw scores: the flat kind's keys)
+            pack_flat_keys_kernel<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(in.dd.dev, in.di.dev, nullptr, total,
+                                                                                flat_order_max, nullptr, world, 0, in.keys.ptr);
+        else
+            pack_result_keys_kernel<<<(unsigned)((total + 255) / 256), 256, 0, s>>>(in.dd.dev, in.di.dev, total, nullptr, world,
+                                                                                  0, in.keys.ptr);
         VIX_LAUNCH_CHECK();
     }
     VIX_TRY(shard_range_lims(in.dlims.ptr, world, nq, in.glims.ptr, in.meta));
@@ -1184,12 +1455,13 @@ int vix_sharded_range_search(vix_index_t* h, vix_comm_t* c, const float* queries
     VIX_REQUIRE(filter_capacity >= 0, VIX_ERR_INVALID_PARAM, "vix_sharded_range_search: negative capacity");
     std::lock_guard<std::mutex> lc(c->mu);
     std::lock_guard<std::mutex> lk(h->mu);
-    VIX_REQUIRE(h->p.kind == VIX_INDEX_IVF_PQ && h->has_coarse && h->has_pq, VIX_ERR_NOT_TRAINED,
-                "vix_sharded_range_search: needs a trained IVF-PQ index");
-    VIX_REQUIRE(h->p.metric != VIX_METRIC_COSINE, VIX_ERR_UNSUPPORTED, "vix_sharded_range_search: L2 / IP only");
-    if (nprobe <= 0) nprobe = h->p.nprobe;
-    VIX_REQUIRE(nprobe > 0 && nprobe <= VIX_MAX_K, VIX_ERR_INVALID_K, "vix_sharded_range_search: nprobe = %d (1 .. %d)", nprobe,
-                VIX_MAX_K);
+    VIX_TRY(sharded_kind_check(h, "vix_sharded_range_search"));
+    const bool flat = h->p.kind == VIX_INDEX_FLAT;                    // (no probes: nprobe is not read, as on one GPU)
+    if (!flat) {
+        if (nprobe <= 0) nprobe = h->p.nprobe;
+        VIX_REQUIRE(nprobe > 0 && nprobe <= VIX_MAX_K, VIX_ERR_INVALID_K, "vix_sharded_range_search: nprobe = %d (1 .. %d)", nprobe,
+                    VIX_MAX_K);
+    }
     if (nq == 0) return range_empty(0, out);                          // (every rank sees the same nq: no exchange)
     In<uint64_t> fw;
     FilterArgs f;
@@ -1198,23 +1470,26 @@ int vix_sharded_range_search(vix_index_t* h, vix_comm_t* c, const float* queries
     const int world = c->world;
     if (world == 1) return index_range_locked(h, queries, nq, radius, nprobe, fp, out);
     cudaStream_t s = ctx().stream;
-    if (h->dirty) VIX_TRY(build_lists(h));
-    VIX_TRY(ensure_region(c, nq, h->p.d, nprobe, 1));
+    if (!flat && h->dirty) VIX_TRY(build_lists(h));
+    VIX_TRY(ensure_region(c, nq, h->p.d, flat ? 1 : nprobe, 1));
     bool grown = false;
     if (c->peer_state == 1) VIX_TRY(ensure_range_region(c, nq, 0, &grown));
     auto mark = [&](int i) { if (c->trace) cudaEventRecord(c->ev[i], s); };
     mark(0);
     BatchProbes px;
     VIX_TRY(exchange_probes(h, c, queries, nq, nprobe, px));
+    const float* dq = px.queries;
+    const int32_t* probes = px.probes;
     mark(1);
     // the local scan and sort (its one synchronisation: the local total); a failure here travels with the lims, so that
-    // every rank returns it together
+    // every rank returns it together.  Every kind's keys are (API distance, user id): the merge is the same for all.
     RangeKeys rk;
-    const int rc = index_range_locked(h, px.queries, nq, radius, nprobe, fp, nullptr, px.probes, &rk);
+    const int rc = index_range_locked(h, dq, nq, radius, nprobe, fp, nullptr, probes, &rk);
     mark(2);
     vix_range_result* r = nullptr;
     ShardTail tail;
     tail.out = &r;
+    tail.neg_zero = range_neg_zero(h);
     ShardTotals st;
     VIX_TRY(sharded_range_exchange(h, c, nq, rc, rk, grown, tail, &st));
     mark(3);
@@ -1243,7 +1518,7 @@ int vix_debug_shard_merge(const float* dist_all, const int64_t* ids_all, int wor
     pack_result_keys_kernel<<<(unsigned)((total + 255) / 256), 256, 0, ctx().stream>>>(dd.dev, di.dev, total, nullptr, world, 0,
                                                                                      keys.ptr);
     VIX_LAUNCH_CHECK();
-    VIX_TRY(merge_shard_keys(keys.ptr, world, nq, k, metric, od.dev, oi.dev));
+    VIX_TRY(merge_shard_keys(keys.ptr, world, nq, k, metric == VIX_METRIC_IP, od.dev, oi.dev));
     VIX_TRY(od.commit());
     VIX_TRY(oi.commit());
     return finish(od.is_host() || oi.is_host());
@@ -1261,7 +1536,8 @@ int vix_debug_shard_range_merge(const int64_t* lims_all, const float* dist_all, 
     VIX_TRY(debug_shard_runs("vix_debug_shard_range_merge", lims_all, dist_all, ids_all, world, nq, in));
     vix_range_result* r = nullptr;
     VIX_TRY(range_alloc(nq, in.total, &r));
-    const int rc = shard_range_merge(in.keys.ptr, in.dbase.ptr, in.dlims.ptr, world, nq, in.glims.ptr, in.total, metric, r);
+    const int rc = shard_range_merge(in.keys.ptr, in.dbase.ptr, in.dlims.ptr, world, nq, in.glims.ptr, in.total,
+                                     metric == VIX_METRIC_IP, r);
     if (rc != VIX_OK) { range_free(r); return rc; }
     const cudaError_t e = cudaStreamSynchronize(s);                   // (meta, a host vector, is read by the copy above)
     if (e != cudaSuccess) { range_free(r); VIX_CUDA(e); }
@@ -1282,11 +1558,175 @@ int vix_debug_shard_knn_merge(const int64_t* lims_all, const float* dist_all, co
     VIX_TRY(od.stage(out_dist, (size_t)nq * k));
     VIX_TRY(oi.stage(out_ids, (size_t)nq * k));
     if (nq > 0)
-        VIX_TRY(shard_knn_merge(in.keys.ptr, in.dbase.ptr, in.dlims.ptr, world, nq, in.glims.ptr, in.total, k, metric, od.dev,
-                                oi.dev));
+        VIX_TRY(shard_knn_merge(in.keys.ptr, in.dbase.ptr, in.dlims.ptr, world, nq, in.glims.ptr, in.total, k,
+                                metric == VIX_METRIC_IP, od.dev, oi.dev));
     VIX_TRY(od.commit());
     VIX_TRY(oi.commit());
     return finish(true);                                              // (meta, a host vector, is read by a copy)
+}
+
+int vix_debug_shard_flat_merge(const int64_t* lims_all, const float* score_all, const int64_t* ids_all, int world, int64_t nq,
+                               int k, int metric, int64_t* out_lims, float* out_dist, int64_t* out_ids) {
+    VIX_TRY(ensure_device());
+    VIX_REQUIRE(lims_all && out_dist && out_ids, VIX_ERR_NULL_PTR, "vix_debug_shard_flat_merge: null pointer");
+    VIX_REQUIRE(world > 0 && world <= 256 && nq >= 0 && nq < 0x7FFFFFFFLL && k >= 0 && k <= VIX_MAX_K_LARGE,
+                VIX_ERR_INVALID_PARAM, "vix_debug_shard_flat_merge: world / nq / k");
+    VIX_REQUIRE(metric == VIX_METRIC_L2 || metric == VIX_METRIC_IP || metric == VIX_METRIC_COSINE, VIX_ERR_INVALID_PARAM,
+                "vix_debug_shard_flat_merge: metric");
+    DebugShardRuns in;
+    VIX_TRY(debug_shard_runs("vix_debug_shard_flat_merge", lims_all, score_all, ids_all, world, nq, in,
+                             metric != VIX_METRIC_L2 ? 1 : 0));
+    const size_t n_out = k > 0 ? (size_t)nq * k : (size_t)in.total;
+    Out<float> od;
+    Out<int64_t> oi;
+    Out<int64_t> ol;
+    VIX_TRY(od.stage(out_dist, n_out));
+    VIX_TRY(oi.stage(out_ids, n_out));
+    VIX_TRY(ol.stage(out_lims, out_lims ? (size_t)nq + 1 : 0));
+    if (nq > 0)
+        VIX_TRY(shard_flat_merge(in.keys.ptr, in.dbase.ptr, in.dlims.ptr, world, nq, in.glims.ptr, in.total, k, metric, od.dev,
+                                 oi.dev));
+    if (ol.dev) VIX_CUDA(cudaMemcpyAsync(ol.dev, in.glims.ptr, ((size_t)nq + 1) * 8, cudaMemcpyDeviceToDevice, ctx().stream));
+    VIX_TRY(od.commit());
+    VIX_TRY(oi.commit());
+    VIX_TRY(ol.commit());
+    return finish(true);
+}
+
+int vix_debug_sharded_emulate(vix_index_t* const* shards, int world, const float* queries, int64_t nq, int k, int nprobe,
+                              float radius, const uint64_t* filter_words, int64_t filter_capacity, int filter_mode,
+                              float* out_dist, int64_t* out_ids, vix_range_result_t** out_range) {
+    const char* who = "vix_debug_sharded_emulate";
+    VIX_TRY(ensure_device());
+    VIX_REQUIRE(shards && world > 0 && world <= 256, VIX_ERR_INVALID_PARAM, "%s: shards / world", who);
+    const bool range = out_range != nullptr;
+    if (range) *out_range = nullptr;
+    for (int r = 0; r < world; ++r) {
+        VIX_REQUIRE(shards[r], VIX_ERR_NULL_PTR, "%s: null shard %d", who, r);
+        for (int p = 0; p < r; ++p) VIX_REQUIRE(shards[p] != shards[r], VIX_ERR_INVALID_PARAM, "%s: shard %d repeats shard %d", who, r, p);
+        VIX_REQUIRE(shards[r]->p.kind == shards[0]->p.kind && shards[r]->p.metric == shards[0]->p.metric &&
+                    shards[r]->p.d == shards[0]->p.d, VIX_ERR_INVALID_PARAM, "%s: shard %d differs in kind, metric or dimension", who, r);
+    }
+    VIX_REQUIRE(filter_mode == VIX_FILTER_ALLOW || filter_mode == VIX_FILTER_DENY, VIX_ERR_INVALID_PARAM,
+                "%s: filter_mode must be VIX_FILTER_ALLOW or VIX_FILTER_DENY", who);
+    VIX_REQUIRE(filter_capacity >= 0, VIX_ERR_INVALID_PARAM, "%s: negative capacity", who);
+    VIX_REQUIRE(nq >= 0 && nq < 0x7FFFFFFFLL, VIX_ERR_INVALID_PARAM, "%s: nq must lie in [0, 2^31 - 1)", who);
+    VIX_REQUIRE(!range || radius == radius, VIX_ERR_INVALID_PARAM, "%s: radius is NaN", who);
+    std::vector<std::unique_lock<std::mutex>> locks;
+    for (int r = 0; r < world; ++r) locks.emplace_back(shards[r]->mu);
+    for (int r = 0; r < world; ++r) VIX_TRY(sharded_kind_check(shards[r], who));
+    vix_index* h0 = shards[0];
+    const bool flat = h0->p.kind == VIX_INDEX_FLAT;
+    const int d = h0->p.d;
+    if (!flat) {
+        if (nprobe <= 0) nprobe = h0->p.nprobe;
+        VIX_REQUIRE(nprobe > 0 && nprobe <= VIX_MAX_K, VIX_ERR_INVALID_K, "%s: nprobe = %d (1 .. %d)", who, nprobe, VIX_MAX_K);
+    }
+    if (range && nq == 0) return range_empty(0, out_range);
+    if (!range) {
+        if (nq == 0 || k <= 0) return VIX_OK;
+        VIX_REQUIRE(out_dist && out_ids, VIX_ERR_NULL_PTR, "%s: null outputs", who);
+        VIX_REQUIRE(k <= VIX_MAX_K_LARGE, VIX_ERR_INVALID_K, "%s: k > %d", who, VIX_MAX_K_LARGE);
+    }
+    VIX_REQUIRE(queries, VIX_ERR_NULL_PTR, "%s: null queries", who);
+    cudaStream_t s = ctx().stream;
+    In<uint64_t> fw;
+    FilterArgs f;
+    const FilterArgs* fp = nullptr;
+    VIX_TRY(stage_filter(filter_words, filter_capacity, filter_mode, fw, f, fp));
+    In<float> dq;
+    VIX_TRY(dq.stage(queries, (size_t)nq * d));
+    // the probes of the whole batch (every rank selects them against the same centroids)
+    Scratch<int32_t> pr;
+    const int32_t* probes = nullptr;
+    if (!flat) {
+        for (int r = 0; r < world; ++r)
+            if (shards[r]->dirty) VIX_TRY(build_lists(shards[r]));
+        VIX_TRY(pr.alloc((size_t)nq * nprobe));
+        VIX_TRY(select_probes_device(h0, dq.dev, nq, nprobe, pr.ptr));
+        probes = pr.ptr;
+    }
+    if (!range && k <= VIX_MAX_K) {
+        const int64_t total = nq * (int64_t)k;
+        Out<float> dd;
+        Out<int64_t> di;
+        VIX_TRY(dd.stage(out_dist, (size_t)total));
+        VIX_TRY(di.stage(out_ids, (size_t)total));
+        Scratch<u64> keys_all;
+        VIX_TRY(keys_all.alloc((size_t)world * total));
+        for (int r = 0; r < world; ++r)
+            VIX_TRY(local_knn_keys(shards[r], dq.dev, nq, k, nprobe, probes, fp, nullptr, world, 0, keys_all.ptr + (size_t)r * total));
+        VIX_TRY(merge_knn_keys(h0, keys_all.ptr, world, nq, k, dd.dev, di.dev));
+        VIX_TRY(dd.commit());
+        VIX_TRY(di.commit());
+        return finish(true);
+    }
+    // every rank's sorted rows: its range rows, or its k-NN rows within the shared bound cut at k
+    std::vector<std::unique_ptr<RangeKeys>> runs;
+    for (int r = 0; r < world; ++r) runs.emplace_back(new RangeKeys());
+    if (range) {
+        for (int r = 0; r < world; ++r)
+            VIX_TRY(index_range_locked(shards[r], dq.dev, nq, radius, nprobe, fp, nullptr, probes, runs[r].get()));
+    } else {
+        std::vector<std::unique_ptr<LocalKnnLarge>> L;
+        Scratch<uint32_t> slots, tau;
+        VIX_TRY(slots.alloc((size_t)world * nq));
+        VIX_TRY(tau.alloc((size_t)nq));
+        for (int r = 0; r < world; ++r) {
+            L.emplace_back(new LocalKnnLarge());
+            int64_t seed_n = 0;
+            VIX_TRY(local_knn_prepare(shards[r], dq.dev, nq, k, nprobe, probes, fp, *L[r]));
+            VIX_TRY(local_knn_seed(*L[r], nq, k, slots.ptr + (size_t)r * nq, &seed_n));
+        }
+        min_knn_bounds_kernel<<<(unsigned)((nq + 255) / 256), 256, 0, s>>>(slots.ptr, world, nq, nq, tau.ptr);
+        VIX_LAUNCH_CHECK();
+        for (int r = 0; r < world; ++r) {
+            RangeKeys rk;
+            RangeInfo ci;
+            size_t cap = shards[r]->knn_cap;
+            VIX_TRY(local_knn_cut(shards[r], *L[r], nq, k, tau.ptr, cap, rk, *runs[r], &ci));
+        }
+    }
+    // the exchanged layout, as sharded_range_exchange holds it: lims [world][nq + 2] (status 0), keys rank by rank
+    const int64_t L2 = nq + 2;
+    Scratch<int64_t> lims_all, glims, dbase;
+    VIX_TRY(lims_all.alloc((size_t)world * L2));
+    VIX_TRY(glims.alloc((size_t)nq + 1));
+    VIX_TRY(dbase.alloc((size_t)world + 1));
+    VIX_CUDA(cudaMemsetAsync(lims_all.ptr, 0, (size_t)world * L2 * 8, s));
+    std::vector<int64_t> tot((size_t)world, 0);
+    for (int r = 0; r < world; ++r) {
+        VIX_CUDA(cudaMemcpyAsync(lims_all.ptr + (size_t)r * L2, runs[r]->lims.ptr, (size_t)(nq + 1) * 8, cudaMemcpyDeviceToDevice, s));
+        VIX_CUDA(cudaMemcpyAsync(&tot[r], runs[r]->lims.ptr + nq, 8, cudaMemcpyDeviceToHost, s));
+    }
+    VIX_CUDA(cudaStreamSynchronize(s));
+    int64_t total = 0;
+    for (int r = 0; r < world; ++r) total += tot[r];
+    Scratch<u64> keys;
+    VIX_TRY(keys.alloc((size_t)total));
+    for (int64_t r = 0, at = 0; r < world; at += tot[r], ++r)
+        if (tot[r] > 0) VIX_CUDA(cudaMemcpyAsync(keys.ptr + at, runs[r]->sorted, (size_t)tot[r] * 8, cudaMemcpyDeviceToDevice, s));
+    std::vector<int64_t> meta;
+    VIX_TRY(shard_range_lims(lims_all.ptr, world, nq, glims.ptr, meta));
+    VIX_CUDA(cudaMemcpyAsync(dbase.ptr, meta.data(), ((size_t)world + 1) * 8, cudaMemcpyHostToDevice, s));
+    if (range) {
+        vix_range_result* res = nullptr;
+        VIX_TRY(range_alloc(nq, total, &res));
+        int rc = shard_range_merge(keys.ptr, dbase.ptr, lims_all.ptr, world, nq, glims.ptr, total, range_neg_zero(h0), res);
+        if (rc == VIX_OK) rc = finish(true);
+        if (rc != VIX_OK) { range_free(res); return rc; }
+        *out_range = res;
+        return VIX_OK;
+    }
+    Out<float> dd;
+    Out<int64_t> di;
+    VIX_TRY(dd.stage(out_dist, (size_t)nq * k));
+    VIX_TRY(di.stage(out_ids, (size_t)nq * k));
+    if (flat) VIX_TRY(shard_flat_merge(keys.ptr, dbase.ptr, lims_all.ptr, world, nq, glims.ptr, total, k, h0->p.metric, dd.dev, di.dev));
+    else VIX_TRY(shard_knn_merge(keys.ptr, dbase.ptr, lims_all.ptr, world, nq, glims.ptr, total, k, knn_neg_zero(h0), dd.dev, di.dev));
+    VIX_TRY(dd.commit());
+    VIX_TRY(di.commit());
+    return finish(true);
 }
 
 int vix_comm_trace(vix_comm_t* c, int enabled) {
@@ -1314,9 +1754,31 @@ int vix_sharded_add(vix_index_t* h, vix_comm_t* c, const int64_t* list_bounds, c
     VIX_REQUIRE(n >= 0 && (n == 0 || (x && ids)), VIX_ERR_NULL_PTR, "vix_sharded_add: null pointer (explicit ids are required)");
     std::lock_guard<std::mutex> lc(c->mu);
     std::lock_guard<std::mutex> lk(h->mu);
-    VIX_REQUIRE(h->p.kind == VIX_INDEX_IVF_PQ && h->has_coarse && h->has_pq, VIX_ERR_NOT_TRAINED, "vix_sharded_add: needs a trained IVF-PQ index");
-    const int world = c->world, rank = c->rank, d = h->p.d, m = h->code_bytes();   // m: bytes per stored code
+    VIX_TRY(sharded_kind_check(h, "vix_sharded_add"));
+    const int world = c->world, rank = c->rank, d = h->p.d;
     cudaStream_t s = ctx().stream;
+    if (h->p.kind == VIX_INDEX_FLAT) {
+        // rows stay on the rank that passes them: no list partition, no row exchange.  The call stays collective: the count
+        // of ids outside [0, 2^32 - 1) is all-gathered before any rank stores a row, so all ranks refuse together.
+        VIX_REQUIRE(!list_bounds, VIX_ERR_INVALID_PARAM, "vix_sharded_add: a flat index has no list partition (list_bounds must "
+                    "be NULL)");
+        In<int64_t> dids;
+        VIX_TRY(dids.stage(ids, (size_t)n));
+        Scratch<unsigned long long> dcounts;
+        VIX_TRY(dcounts.alloc((size_t)world + 1));
+        VIX_CUDA(cudaMemsetAsync(dcounts.ptr, 0, sizeof(unsigned long long) * (world + 1), s));
+        VIX_TRY(count_invalid_ids_device(dids.dev, n, dcounts.ptr + world));
+        VIX_NCCL(g_nccl.AllGather(dcounts.ptr + world, dcounts.ptr, 1, ncclUint64, c->comm, s));
+        std::vector<unsigned long long> counts((size_t)world);
+        VIX_CUDA(cudaMemcpyAsync(counts.data(), dcounts.ptr, sizeof(unsigned long long) * world, cudaMemcpyDeviceToHost, s));
+        VIX_CUDA(cudaStreamSynchronize(s));
+        for (int p = 0; p < world; ++p)
+            VIX_REQUIRE(counts[p] == 0, VIX_ERR_INVALID_PARAM, "vix_sharded_add: rank %d was handed %llu ids outside [0, 2^32 - 1); "
+                        "no rank stored any row of this call", p, counts[p]);
+        return index_add_rows_locked(h, x, dids.dev, n);
+    }
+    const bool ivfflat = h->p.kind == VIX_INDEX_IVF_FLAT;
+    const int m = ivfflat ? 0 : h->code_bytes();                          // m: bytes per stored code (IVF-PQ)
     // block boundaries of the list partition: given, or equal-count blocks
     std::vector<int64_t> bounds((size_t)world + 1);
     for (int r = 0; r <= world; ++r) bounds[r] = list_bounds ? list_bounds[r] : (int64_t)h->kc * r / world;
@@ -1361,18 +1823,25 @@ int vix_sharded_add(vix_index_t* h, vix_comm_t* c, const int64_t* list_bounds, c
         VIX_REQUIRE(counts[(size_t)p * W + world] == 0, VIX_ERR_INVALID_PARAM,
                     "vix_sharded_add: rank %d was handed %llu rows with no nearest list (NaN components?) or an id outside "
                     "[0, 2^32 - 1); no rank stored any row of this call", p, counts[(size_t)p * W + world]);
-    // 3. encode, in owner order
+    // 3. encode (IVF-PQ), in owner order; IVF-Flat rows travel as they are (4 d + 12 bytes each instead of m + 12)
     Scratch<int32_t> s_asg;
     Scratch<uint8_t> s_codes;
+    Scratch<float> s_x;
     Scratch<int64_t> s_ids;
     if (n > 0) {
-        VIX_TRY(codes.alloc((size_t)n * m));
-        VIX_TRY(encode_rows_device(h, dx.dev, n, asg.ptr, codes.ptr));
         VIX_TRY(s_asg.alloc((size_t)n));
-        VIX_TRY(s_codes.alloc((size_t)n * m));
         VIX_TRY(s_ids.alloc((size_t)n));
-        gather_rows_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(order.ptr, n, m, asg.ptr, codes.ptr, dids.dev, s_asg.ptr,
-                                                                     s_codes.ptr, s_ids.ptr);
+        if (ivfflat) {
+            VIX_TRY(s_x.alloc((size_t)n * d));
+            gather_vec_rows_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(order.ptr, n, d, asg.ptr, dx.dev, dids.dev, s_asg.ptr,
+                                                                             s_x.ptr, s_ids.ptr);
+        } else {
+            VIX_TRY(codes.alloc((size_t)n * m));
+            VIX_TRY(encode_rows_device(h, dx.dev, n, asg.ptr, codes.ptr));
+            VIX_TRY(s_codes.alloc((size_t)n * m));
+            gather_rows_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(order.ptr, n, m, asg.ptr, codes.ptr, dids.dev, s_asg.ptr,
+                                                                         s_codes.ptr, s_ids.ptr);
+        }
         VIX_LAUNCH_CHECK();
     }
     std::vector<int64_t> send_off((size_t)world + 1, 0), recv_off((size_t)world + 1, 0);
@@ -1384,27 +1853,34 @@ int vix_sharded_add(vix_index_t* h, vix_comm_t* c, const int64_t* list_bounds, c
     // 4. rows travel to their owners
     Scratch<int32_t> r_asg;
     Scratch<uint8_t> r_codes;
+    Scratch<float> r_x;
     Scratch<int64_t> r_ids;
     VIX_TRY(r_asg.alloc((size_t)nrecv));
-    VIX_TRY(r_codes.alloc((size_t)nrecv * m));
+    if (ivfflat) VIX_TRY(r_x.alloc((size_t)nrecv * d));
+    else VIX_TRY(r_codes.alloc((size_t)nrecv * m));
     VIX_TRY(r_ids.alloc((size_t)nrecv));
     VIX_NCCL(g_nccl.GroupStart());
     for (int p = 0; p < world; ++p) {
         const int64_t sc = send_off[p + 1] - send_off[p], rc = recv_off[p + 1] - recv_off[p];
         if (sc > 0) {
             VIX_NCCL(g_nccl.Send(s_asg.ptr + send_off[p], (size_t)sc, ncclInt32, p, c->comm, s));
-            VIX_NCCL(g_nccl.Send(s_codes.ptr + (size_t)send_off[p] * m, (size_t)sc * m, ncclUint8, p, c->comm, s));
+            if (ivfflat) VIX_NCCL(g_nccl.Send(s_x.ptr + (size_t)send_off[p] * d, (size_t)sc * d, ncclFloat, p, c->comm, s));
+            else VIX_NCCL(g_nccl.Send(s_codes.ptr + (size_t)send_off[p] * m, (size_t)sc * m, ncclUint8, p, c->comm, s));
             VIX_NCCL(g_nccl.Send(s_ids.ptr + send_off[p], (size_t)sc, ncclInt64, p, c->comm, s));
         }
         if (rc > 0) {
             VIX_NCCL(g_nccl.Recv(r_asg.ptr + recv_off[p], (size_t)rc, ncclInt32, p, c->comm, s));
-            VIX_NCCL(g_nccl.Recv(r_codes.ptr + (size_t)recv_off[p] * m, (size_t)rc * m, ncclUint8, p, c->comm, s));
+            if (ivfflat) VIX_NCCL(g_nccl.Recv(r_x.ptr + (size_t)recv_off[p] * d, (size_t)rc * d, ncclFloat, p, c->comm, s));
+            else VIX_NCCL(g_nccl.Recv(r_codes.ptr + (size_t)recv_off[p] * m, (size_t)rc * m, ncclUint8, p, c->comm, s));
             VIX_NCCL(g_nccl.Recv(r_ids.ptr + recv_off[p], (size_t)rc, ncclInt64, p, c->comm, s));
         }
     }
     VIX_NCCL(g_nccl.GroupEnd());
-    // 5. append (already encoded)
-    if (nrecv > 0) VIX_TRY(index_add_encoded_locked(h, r_asg.ptr, r_codes.ptr, r_ids.ptr, nrecv));
+    // 5. append with the given assignments (IVF-PQ: already encoded)
+    if (nrecv > 0) {
+        if (ivfflat) VIX_TRY(index_add_assigned_locked(h, r_asg.ptr, r_x.ptr, r_ids.ptr, nrecv));
+        else VIX_TRY(index_add_encoded_locked(h, r_asg.ptr, r_codes.ptr, r_ids.ptr, nrecv));
+    }
     return finish(true);
 }
 

@@ -905,3 +905,164 @@ class ReplicatedIVFPQIndex(ShardedIVFPQIndex):
                 return self._to_host(md.contiguous()), self._to_host(mi.contiguous())
             return md.numpy().copy(), mi.numpy().copy()
         return md.contiguous(), mi.contiguous()
+
+
+class _ShardedExactIndex:
+    """The sharded layout of the exact kinds (flat, IVF-Flat) over the ranks of a ``torch.distributed`` NCCL group: every
+    call is one library call over a ``vix_comm_t`` (vix_sharded_add / vix_sharded_search_filtered /
+    vix_sharded_range_search), bit for bit the one-GPU answer on an index holding every row in the slot the shards hold
+    it in.  One rank is the local index.  There is no Python exchange for these kinds: a group whose backend is not NCCL
+    raises ``NotImplementedError``."""
+
+    def _setup(self, local, group):
+        import torch.distributed as dist
+        self.group = group
+        self.rank = dist.get_rank(group) if dist.is_initialized() else 0
+        self.world = dist.get_world_size(group) if dist.is_initialized() else 1
+        self.local = local
+        self.bounds = None
+
+    def _native(self):
+        if self.world <= 1:
+            return None
+        import torch.distributed as dist
+        if dist.get_backend(self.group) != "nccl":
+            raise NotImplementedError(f"{type(self).__name__} needs the library's exchange (one NCCL rank per GPU); there "
+                                      "is no Python exchange for the exact kinds")
+        if self.__dict__.get("comm") is None:
+            self.comm = Comm.from_torch(self.group)
+        return self.comm
+
+    def _pinned(self, tag, shape, dtype):
+        return ShardedIVFPQIndex._pinned(self, tag, shape, dtype)
+
+    @property
+    def count(self) -> int:
+        """rows THIS rank holds"""
+        return self.local.count
+
+    def add(self, vectors, ids):
+        """Collective: the rows THIS rank contributes (any rows; n may be 0; explicit ids)."""
+        comm = self._native()
+        if comm is None:
+            self.local.batch_insert(vectors, ids)
+            return
+        x = as_input(vectors, np.float32)
+        self.local._check_dim(x, "add")
+        i = as_input(ids, np.int64)
+        b = None if self.bounds is None else np.ascontiguousarray(self.bounds, dtype=np.int64)
+        check(lib().vix_sharded_add(self.local._h, comm._c, ptr(b), ptr(x, np.float32), ptr(i, np.int64),
+                                    C.c_int64(int(x.shape[0]))))
+
+    def remove(self, ids) -> int:
+        """Collective: every rank passes the SAME ids and removes the rows of them it holds; returns the rows removed on all
+        ranks together."""
+        n = self.local.batch_remove(ids)
+        if self.world == 1:
+            return n
+        import torch
+        import torch.distributed as dist
+        t = torch.tensor([n], dtype=torch.int64, device=torch.device("cuda", torch.cuda.current_device()))
+        dist.all_reduce(t, group=self.group)
+        return int(t.item())
+
+    def batch_search(self, queries, k, nprobe=0, out=None, filter=None):
+        """Collective: every rank passes the same queries, k (up to ``VIX_MAX_K_LARGE``), nprobe and ``filter`` (an
+        :class:`IDFilter`) and receives the merged [nq x k] (distances, ids).  Host queries: over peer memory only this rank's
+        block crosses PCIe (the library moves it to the peers), and the result lands in pinned memory; ``out``: optional
+        (distances f32, ids int64) arrays to write into."""
+        import torch
+        comm = self._native()
+        if comm is None:
+            return self.local.batch_search(queries, k, nprobe, filter=filter, out=out)
+        q = as_input(queries, np.float32)
+        self.local._check_dim(q, "batch_search")
+        nq, kk = int(q.shape[0]), max(int(k), 0)
+        host = not _lib._is_torch(queries)
+        if out is not None:
+            dist_, ids = out
+        elif host and nq and kk:
+            dist_, ids = self._pinned("d", (nq, kk), torch.float32), self._pinned("i", (nq, kk), torch.int64)
+        else:
+            dist_, ids = empty_like_input(q, (nq, kk), np.float32), empty_like_input(q, (nq, kk), np.int64)
+        if nq and kk:
+            words = filter.words if filter is not None else None
+            check(lib().vix_sharded_search_filtered(self.local._h, comm._c, ptr(q, np.float32), C.c_int64(nq), C.c_int(k),
+                                                    C.c_int(nprobe), ptr(words, np.uint64),
+                                                    C.c_int64(filter.capacity if filter is not None else 0),
+                                                    C.c_int(filter.mode if filter is not None else 0),
+                                                    ptr(dist_, np.float32), ptr(ids, np.int64)))
+        if out is None and host and nq and kk:
+            return dist_.numpy().copy(), ids.numpy().copy()
+        return dist_, ids
+
+    def range_search(self, queries, radius: float, nprobe: int = 0, filter=None):
+        """Collective: every stored vector within ``radius`` of each query over all ranks, as the local index's
+        ``range_search`` on one GPU holding every row: CSR ``(lims int64 [nq + 1], distances f32 [total], ids int64
+        [total])``, numpy for host queries, torch tensors on the queries' device for CUDA tensors."""
+        comm = self._native()
+        if comm is None:
+            return self.local.range_search(queries, radius, nprobe=nprobe, filter=filter)
+        q = as_input(queries, np.float32)
+        self.local._check_dim(q, "range_search")
+        nq = int(q.shape[0])
+        res = C.c_void_p(0)
+        try:
+            words = filter.words if filter is not None else None
+            check(lib().vix_sharded_range_search(self.local._h, comm._c, ptr(q, np.float32), C.c_int64(nq),
+                                                 C.c_float(float(radius)), C.c_int(nprobe), ptr(words, np.uint64),
+                                                 C.c_int64(filter.capacity if filter is not None else 0),
+                                                 C.c_int(filter.mode if filter is not None else 0), C.byref(res)))
+            total = int(lib().vix_range_result_total(res))
+            lims = empty_like_input(q, (nq + 1,), np.int64)
+            dist_ = empty_like_input(q, (total,), np.float32)
+            ids = empty_like_input(q, (total,), np.int64)
+            check(lib().vix_range_result_get(res, ptr(lims, np.int64), ptr(dist_, np.float32) if total else None,
+                                             ptr(ids, np.int64) if total else None))
+            return lims, dist_, ids
+        finally:
+            lib().vix_range_result_destroy(res)
+
+
+class ShardedFlatIndex(_ShardedExactIndex):
+    """Flat index partitioned by rows: a row stays on the rank that adds it (no exchange at build time), every rank scans
+    its rows and the per-rank results are merged on the device.  The answer equals ``FlatIndex`` on one GPU holding rank
+    0's rows first, then rank 1's, and so on, each in add order: flat search breaks ties at an equal score by row."""
+
+    def __init__(self, dimension, metric="euclidean", group=None):
+        self._setup(FlatIndex(dimension, metric), group)
+
+
+class ShardedIVFFlatIndex(_ShardedExactIndex):
+    """IVF-Flat index partitioned by contiguous blocks of inverted lists, as ``ShardedIVFPQIndex``: every rank holds the
+    coarse centroids (``set_coarse``, or ``optimize`` on the same sample on every rank) and the vectors of ITS lists; a row
+    travels to the rank owning its list at ``add``.  Probes of the batch are selected once and exchanged; each rank scans
+    the probed lists it owns; the answer equals ``IVFIndex`` on one GPU (its distances are exact per pair and its ties
+    fall to the id, so the order the rows arrived in does not matter)."""
+
+    def __init__(self, dimension, metric="euclidean", nlist=256, nprobe=8, group=None):
+        self._setup(IVFIndex(dimension, metric, nlist, nprobe), group)
+        self.kc = int(nlist)
+        self.nprobe = int(nprobe)
+
+    def set_list_bounds(self, bounds):
+        """Block boundaries of the list partition ([world + 1], identical on every rank; before the first ``add``).
+        Default: equal-count blocks."""
+        b = np.asarray(bounds, dtype=np.int64)
+        if b.size != self.world + 1 or b[0] != 0 or b[-1] != self.kc or (np.diff(b) < 0).any():
+            raise ValueError("bounds must be [world + 1] ascending list ids from 0 to nlist")
+        self.bounds = b
+
+    def set_coarse(self, centroids):
+        self.local.set_coarse(centroids)
+        self.kc = int(self.local.get_coarse().shape[0])
+
+    def optimize(self, training_vectors, kmeans_cfg: KMeansCfg | None = None):
+        """Trains the coarse quantiser on ``training_vectors`` -- the same sample (and seed) on every rank, so every rank
+        holds the same centroids.  Before the first ``add``."""
+        if training_vectors is None:
+            raise ValueError("a sharded IVF-Flat index trains on an explicit sample, the same on every rank")
+        self.local.optimize(training_vectors, kmeans_cfg)
+        self.kc = int(self.local.get_coarse().shape[0])
+
+    train = optimize
