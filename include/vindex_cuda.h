@@ -50,7 +50,7 @@
  *   VIX_DISABLE_TC, VIX_DISABLE_PQ_TC, VIX_DISABLE_LUT_IMAGE
  *                            exact CUDA-core kernels instead of the tensor-core shortlists / per-query tables built inside
  *                            the scan instead of batch-wide (the parity tests compare both ways)
- *   VIX_NO_P2P=1             vix_sharded_*: NCCL all-gathers instead of peer memory; VIX_NCCL_PATH: the libnccl to dlopen
+ *   VIX_NO_P2P=1             vix_sharded_* / vix_replicated_*: NCCL all-gathers instead of peer memory; VIX_NCCL_PATH: the libnccl to dlopen
  *
  * Each declaration cites the reference interface it replaces (paths relative to
  * /root/reference/Sources/VectorIndex unless another root is given).
@@ -512,7 +512,7 @@ int vix_comm_rank(const vix_comm_t* c);
 int vix_comm_world(const vix_comm_t* c);
 int vix_comm_uses_peer_memory(const vix_comm_t* c);        /* 1 peer memory, 0 NCCL all-gathers, -1 not decided yet */
 /* measurement aid: CUDA events around the three phases of the LAST vix_sharded_search, vix_sharded_search_filtered or
- * vix_sharded_range_search on this communicator -- probe selection + exchange | fused scan (range: local scan and sort;
+ * vix_sharded_range_search (or replicated search, see vix_replicated_search) on this communicator -- probe selection + exchange | fused scan (range: local scan and sort;
  * k > VIX_MAX_K: seed, bound exchange, collect and cut at k) | result exchange + merge (range: + decode; k > VIX_MAX_K:
  * + cut at k) (ms; waits for that call to finish) */
 int vix_comm_trace(vix_comm_t* c, int enabled);
@@ -554,6 +554,72 @@ int vix_sharded_range_search(vix_index_t* h, vix_comm_t* c, const float* queries
 int vix_sharded_search_filtered(vix_index_t* h, vix_comm_t* c, const float* queries, int64_t nq, int k, int nprobe,
                                 const uint64_t* filter_words /* nullable */, int64_t filter_capacity, int filter_mode,
                                 float* out_dist, int64_t* out_ids);
+
+/* ---- multi-GPU replicas: every rank holds the WHOLE index and answers its share of the batch --------------------------
+ * For an index that fits one GPU this is the faster layout (no probe exchange, no merge: a query's answer never depends on
+ * the other queries of its batch).  The calls take the vix_comm_t of the sharded calls and a handle whose shard_world is 0
+ * or 1 (VIX_ERR_INVALID_PARAM otherwise).  All four are collective: every rank calls them in the same order with the same
+ * nq, k, radius, nprobe and filter.
+ *   vix_replicated_add              x / ids: the rows THIS rank contributes (any rows; n may be 0; explicit ids).  Each rank
+ *                                   prepares its own rows (IVF-PQ: list assignment and codes; IVF-Flat: assignment; flat:
+ *                                   nothing), the counts are all-gathered, and a row with no nearest list (IVF kinds) or an id
+ *                                   outside [0, 2^32 - 1) on ANY rank makes every rank return VIX_ERR_INVALID_PARAM naming that
+ *                                   rank, before any row travels: no rank stores a row of the call.  The prepared rows
+ *                                   (IVF-PQ m + 12 bytes, IVF-Flat 4 d + 12, flat 4 d + 8) are all-gathered over peer memory
+ *                                   (the range region, grown collectively) or NCCL grouped send / receive, and every replica
+ *                                   appends all of them rank by rank, rank 0's first: every replica holds identical lists, rows
+ *                                   in identical slots.  An IVF-PQ index must be trained, an IVF-Flat index needs its
+ *                                   centroids (VIX_ERR_NOT_TRAINED).
+ *   vix_replicated_search[_filtered] rank r answers rows vix_sharded_query_block(nq, r, world) with the one-GPU search
+ *                                   (vix_index_search / _filtered: the list-major scan when the block's shape allows it, the
+ *                                   two-pass route for VIX_MAX_K < k <= VIX_MAX_K_LARGE); from a host pointer only that block
+ *                                   of queries crosses PCIe.  Its [cnt x k] block is stored into every peer's region at the
+ *                                   block's row offset, one barrier (NCCL: an all-gather), and every rank receives the whole
+ *                                   [nq x k] answer.  k <= VIX_MAX_K with device outputs in asynchronous mode: no host
+ *                                   synchronisation; a rank whose local search failed then raises the pipeline error that the
+ *                                   next synchronising call on every rank reports (VIX_ERR_CUDA).  Otherwise (host outputs,
+ *                                   synchronous mode, or k > VIX_MAX_K, whose blocks travel through the range region, grown
+ *                                   collectively) the call synchronises and every rank returns the failing rank's code.
+ *   vix_replicated_range_search     each rank range-searches its block; row starts and sorted keys travel as in
+ *                                   vix_sharded_range_search (statuses, global total, collective growth, allocation verdict:
+ *                                   VIX_ERR_OOM on every rank when the answer does not fit on one); the rows of different ranks
+ *                                   belong to different queries, so the global CSR is the ranks' rows concatenated (no merge).
+ *   remove                          no collective call: every replica calls vix_index_remove with the same ids (the remaining
+ *                                   rows keep their order, so the replicas stay identical).
+ *   a rank that only needs ITS block (no assembly) calls vix_index_search on the rows vix_sharded_query_block gives it.
+ * Contract: the collective answer equals the one-GPU call (vix_index_search, vix_index_search_filtered,
+ * vix_index_range_search) on the whole batch, over an index holding the rows in the order the replicas append them, bit for
+ * bit: ids, distance bits with the sign of zero, -1 / NaN padding, rows stored twice and lists probed twice, and
+ * search(k)[:, :k2] == search(k2).  It rests on one fact, which tests/test_replicated.py pins for every kind, metric, route
+ * and filter: a query's answer does not depend on the other queries of its batch.  One rank is the one-GPU call.
+ * Refusals, on every rank alike and before any exchange, with the codes of the sharded calls: a NaN radius, a bad
+ * filter_mode or negative filter_capacity (VIX_ERR_INVALID_PARAM); nprobe outside 1 .. VIX_MAX_K after the default
+ * (VIX_ERR_INVALID_K; read by IVF indexes with centroids only, as on one GPU); k > VIX_MAX_K_LARGE (VIX_ERR_INVALID_K); k >
+ * VIX_MAX_K with nq >= 2^31 - 1 (VIX_ERR_INVALID_PARAM); an untrained IVF-PQ index (VIX_ERR_NOT_TRAINED) or one with cosine
+ * (VIX_ERR_UNSUPPORTED).  vix_comm_trace records three phases: queries in | local search | assembly (range: exchange and
+ * concatenation).  VIX_SCAN_DEBUG=1 prints one "[vix replicated] world W, peer P, kind K, op knn|range|add, block B, total
+ * T, grown 0|1" line per call and rank at world > 1 (B: this rank's queries or rows, T: entries of the answer or rows
+ * appended). */
+int vix_replicated_add(vix_index_t* h, vix_comm_t* c, const float* x, const int64_t* ids, int64_t n);
+int vix_replicated_search(vix_index_t* h, vix_comm_t* c, const float* queries, int64_t nq, int k, int nprobe,
+                          float* out_dist, int64_t* out_ids);
+int vix_replicated_search_filtered(vix_index_t* h, vix_comm_t* c, const float* queries, int64_t nq, int k, int nprobe,
+                                   const uint64_t* filter_words /* nullable */, int64_t filter_capacity, int filter_mode,
+                                   float* out_dist, int64_t* out_ids);
+int vix_replicated_range_search(vix_index_t* h, vix_comm_t* c, const float* queries, int64_t nq, float radius, int nprobe,
+                                const uint64_t* filter_words /* nullable */, int64_t filter_capacity, int filter_mode,
+                                vix_range_result_t** out);
+
+/* Test hook: the assembly of the replicated calls on one GPU, over blocks the caller passes (host or device pointers; world
+ * 1 .. 256; rank r's block is vix_sharded_query_block(nq, r, world)).  out_range == NULL: k-NN -- dist_all / ids_all [nq x
+ * k] hold the ranks' [count_r x k] blocks rank by rank (raw bits; lims_all is not read); every emulated rank stores its
+ * block into the other ranks' buffers as the exchange does, and out_dist / out_ids receive the last rank's buffer.
+ * Otherwise range search -- lims_all: every rank's block row starts (count_r + 1 each, rank by rank: nq + world in all);
+ * dist_all / ids_all: their rows (API distances, ids) rank by rank; they are keyed, laid out as the exchange holds them and
+ * concatenated and decoded (kind and metric: the sign of zero distances, IP -0 but IVF-Flat +0) into a new result object. */
+int vix_debug_replica_assemble(const int64_t* lims_all /* nullable for k-NN */, const float* dist_all, const int64_t* ids_all,
+                               int world, int64_t nq, int k, int metric, int kind, float* out_dist, int64_t* out_ids,
+                               vix_range_result_t** out_range /* nullable */);
 
 /* f-1  The IVF-PQ query with its optional last step (docs/kernel-specs/DONE_22_adc_scan.md:873-878, "7. Optional: exact
  * rerank (kernel #40)"; IVFIndex.swift:1380-1439): ADC search for the rerank_r best candidates per query (k <= rerank_r <=

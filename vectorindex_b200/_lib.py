@@ -96,7 +96,8 @@ _EXPORTS = [
     "vix_comm_unique_id", "vix_comm_create", "vix_comm_destroy", "vix_comm_rank", "vix_comm_world",
     "vix_comm_uses_peer_memory", "vix_comm_trace", "vix_comm_trace_get", "vix_sharded_query_block", "vix_sharded_add", "vix_sharded_search",
     "vix_sharded_search_filtered", "vix_sharded_range_search", "vix_debug_shard_range_merge", "vix_debug_shard_knn_merge",
-    "vix_debug_shard_flat_merge", "vix_debug_sharded_emulate",
+    "vix_debug_shard_flat_merge", "vix_debug_sharded_emulate", "vix_replicated_add", "vix_replicated_search",
+    "vix_replicated_search_filtered", "vix_replicated_range_search", "vix_debug_replica_assemble",
     "vix_index_encode", "vix_index_add_encoded", "vix_debug_tc_scores_f32", "vix_debug_tc_codes", "vix_debug_tc_seed", "vix_debug_shard_merge", "vix_accel_rank_candidates_f32",
     "cpq_encode_u8_f32", "cpq_encode_u8_f32_with_csq", "cpq_encode_u4_f32", "cpq_encode_residual_u8_f32",
     "cpq_encode_residual_u8_f32_with_csq", "cpq_encode_residual_u4_f32", "cpq_pack_u4_bulk", "cpq_unpack_u4_bulk",

@@ -16,7 +16,7 @@
 //
 // NCCL is bound at run time (dlopen of libnccl.so.2: inside a PyTorch process that is the copy torch already loaded),
 // so the library itself has no link-time dependency on it and single-GPU hosts never touch it.
-#include "vix_index.cuh"
+#include "vix_comm.cuh"
 #include "vix_scan.cuh"
 #include "vix_topk.cuh"
 #include "vix_group.cuh"
@@ -36,25 +36,10 @@
 
 namespace vix {
 
-// ------------------------------------------------------------------------------------------------ NCCL binding
-struct NcclApi {
-    void* lib = nullptr;
-    ncclResult_t (*GetUniqueId)(ncclUniqueId*) = nullptr;
-    ncclResult_t (*CommInitRank)(ncclComm_t*, int, ncclUniqueId, int) = nullptr;
-    ncclResult_t (*CommDestroy)(ncclComm_t) = nullptr;
-    ncclResult_t (*AllGather)(const void*, void*, size_t, ncclDataType_t, ncclComm_t, cudaStream_t) = nullptr;
-    ncclResult_t (*AllReduce)(const void*, void*, size_t, ncclDataType_t, ncclRedOp_t, ncclComm_t, cudaStream_t) = nullptr;
-    ncclResult_t (*Send)(const void*, size_t, ncclDataType_t, int, ncclComm_t, cudaStream_t) = nullptr;
-    ncclResult_t (*Recv)(void*, size_t, ncclDataType_t, int, ncclComm_t, cudaStream_t) = nullptr;
-    ncclResult_t (*GroupStart)() = nullptr;
-    ncclResult_t (*GroupEnd)() = nullptr;
-    const char* (*GetErrorString)(ncclResult_t) = nullptr;
-};
-
-static NcclApi g_nccl;
+NcclApi g_nccl;
 static std::mutex g_nccl_mu;
 
-static int nccl_load() {
+int nccl_load() {
     std::lock_guard<std::mutex> lk(g_nccl_mu);
     if (g_nccl.lib) return VIX_OK;
     const char* env = getenv("VIX_NCCL_PATH");
@@ -87,58 +72,11 @@ static int nccl_load() {
     return VIX_OK;
 }
 
-#define VIX_NCCL(expr)                                                                                  \
-    do {                                                                                                \
-        ncclResult_t _r = (expr);                                                                       \
-        if (_r != ncclSuccess) {                                                                        \
-            ::vix::set_error("NCCL error %d (%s): %s", (int)_r, g_nccl.GetErrorString(_r), #expr);     \
-            return VIX_ERR_CUDA;                                                                        \
-        }                                                                                               \
-    } while (0)
-
 }  // namespace vix
 
 using namespace vix;
 
-// ------------------------------------------------------------------------------------------------ communicator
-struct vix_comm {
-    ncclComm_t comm = nullptr;
-    int rank = 0, world = 1, device = 0;
-    std::mutex mu;
-    // exchange memory: one region per rank, every region mapped into every rank (cudaIpc).  Same layout everywhere:
-    //   [flags: one word per peer][queries: world x per x d f32][probes: world x per x nprobe i32][results: world x nq x k u64]
-    //   [bounds: nq f32 -- the list-major scan's per-query bounds the OTHER ranks found; all bits set (a NaN) = none]
-    int peer_state = -1;                    // -1 undecided, 0 NCCL all-gathers, 1 peer memory
-    void* local = nullptr;
-    size_t local_bytes = 0;
-    std::vector<void*> peer;                // base of every rank's region in THIS process (peer[rank] == local)
-    void** peer_dev = nullptr;              // device copy
-    uint32_t epoch = 0;                     // barriers passed so far
-    size_t off_queries = 0, off_probes = 0, off_results = 0, off_bounds = 0;
-    int64_t cap_nq = 0, cap_per = 0;
-    int cap_d = 0, cap_nprobe = 0, cap_k = 0;
-    // NCCL path: plain local buffers with the same roles
-    void* gather_probes = nullptr; size_t gather_probes_bytes = 0;
-    void* gather_keys = nullptr; size_t gather_keys_bytes = 0;
-    // range search (and k-NN search beyond VIX_MAX_K): a second region, mapped like the first (peer memory only), grown
-    // collectively and geometrically:
-    //   [lims: world x (nq + 2) i64 -- each rank's local CSR row starts + its status]
-    //   [bounds: world x nq u32 -- each rank's k-NN seed bounds; apart from the lims, which a fast peer may already store
-    //    while this rank still reads the bounds]
-    //   [keys: the global answer's sorted keys, rank by rank]
-    void* range_local = nullptr;
-    std::vector<void*> range_peer;
-    void** range_peer_dev = nullptr;
-    size_t range_off_bounds = 0, range_off_keys = 0;
-    int64_t range_cap_nq = 0, range_cap_keys = 0;
-    // optional phase events of the last search (vix_comm_trace): start | probes exchanged | scanned | merged
-    bool trace = false;
-    cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
-};
-
 namespace vix {
-
-constexpr size_t kFlagBytes = 4096;         // flags[world] (u32), padded
 
 static void close_peers(vix_comm* c) {
     for (int p = 0; p < (int)c->peer.size(); ++p)
@@ -151,16 +89,9 @@ static void close_peers(vix_comm* c) {
     c->peer_dev = nullptr;
 }
 
-// rows of the batch whose probe lists a rank computes: blocks of `per` rows (a multiple of 4, so that every block of
-// queries / probes is a whole number of 16-byte pieces)
-static int64_t block_rows(int64_t nq, int world) {
-    int64_t per = (nq + world - 1) / world;
-    return (per + 3) & ~(int64_t)3;
-}
-
 // Collective: make every rank's region large enough for (nq, d, nprobe, k) and map it everywhere.  All ranks call this
 // with the same arguments, so they agree on whether to reallocate.  Returns with c->peer_state decided.
-static int ensure_region(vix_comm* c, int64_t nq, int d, int nprobe, int k) {
+int ensure_region(vix_comm* c, int64_t nq, int d, int nprobe, int k) {
     if (c->peer_state == 0) return VIX_OK;
     if (c->peer_state == 1 && nq <= c->cap_nq && d <= c->cap_d && nprobe <= c->cap_nprobe && k <= c->cap_k) return VIX_OK;
     cudaStream_t s = ctx().stream;
@@ -349,7 +280,7 @@ __global__ void take_bounds_kernel(float* __restrict__ thr, int64_t nq, uint32_t
     thr[q] = fminf(thr[q], __uint_as_float(v));             // fminf(x, NaN) = x
 }
 
-static int peer_barrier(vix_comm* c) {
+int peer_barrier(vix_comm* c) {
     c->epoch += 1;
     peer_barrier_kernel<<<1, 32 * ((c->world + 31) / 32), 0, ctx().stream>>>(c->peer_dev, c->world, c->rank, c->epoch,
                                                                               pipeline_error_flag());
@@ -646,7 +577,7 @@ __global__ void min_knn_bounds_kernel(const uint32_t* __restrict__ slots, int wo
 
 // lims_all [world][nq + 2] on the device -> glims [nq + 1] (device) and meta (host: base [world + 1], longest row, statuses
 // [world]).  Synchronises the stream: the size of the global answer.
-static int shard_range_lims(const int64_t* lims_all, int world, int64_t nq, int64_t* glims, std::vector<int64_t>& meta) {
+int shard_range_lims(const int64_t* lims_all, int world, int64_t nq, int64_t* glims, std::vector<int64_t>& meta) {
     cudaStream_t s = ctx().stream;
     Scratch<int64_t> dmeta;
     const size_t nm = 2 * (size_t)world + 2;
@@ -710,10 +641,10 @@ static int merge_flat_keys(const u64* keys_all, int world, int64_t nq, int k, in
 // The sign one GPU gives a zero distance (the keys hold +0): k-NN of the IVF-PQ scan with inner product -0, of the IVF-Flat
 // scan +0 (it keys the distance itself); the flat engine's mapping (flat_knn_decode) restores its own.  Range search: the
 // flat engine's and the IVF-PQ scan's inner product -0, IVF-Flat +0.
-static int knn_neg_zero(const vix_index* h) { return h->p.kind == VIX_INDEX_IVF_PQ && h->p.metric == VIX_METRIC_IP; }
-static int range_neg_zero(const vix_index* h) { return h->p.kind != VIX_INDEX_IVF_FLAT && h->p.metric == VIX_METRIC_IP; }
+int knn_neg_zero(const vix_index* h) { return h->p.kind == VIX_INDEX_IVF_PQ && h->p.metric == VIX_METRIC_IP; }
+int range_neg_zero(const vix_index* h) { return h->p.kind != VIX_INDEX_IVF_FLAT && h->p.metric == VIX_METRIC_IP; }
 
-static const char* kind_name(const vix_index* h) {
+const char* kind_name(const vix_index* h) {
     return h->p.kind == VIX_INDEX_FLAT ? "flat" : h->p.kind == VIX_INDEX_IVF_FLAT ? "ivfflat" : "ivfpq";
 }
 
@@ -745,7 +676,7 @@ static void close_range_peers(vix_comm* c) {
 // Collective (peer memory only): make every rank's range region hold nq rows of lims and `keys` keys, growing it
 // geometrically.  Every rank passes the same (nq, keys) -- the batch, and the global total all ranks computed -- so they
 // agree on whether to grow.  A rank that cannot allocate or map makes every rank return VIX_ERR_OOM with no region left.
-static int ensure_range_region(vix_comm* c, int64_t nq, int64_t keys, bool* grown) {
+int ensure_range_region(vix_comm* c, int64_t nq, int64_t keys, bool* grown) {
     if (c->range_local && nq <= c->range_cap_nq && keys <= c->range_cap_keys) return VIX_OK;
     cudaStream_t s = ctx().stream;
     const int world = c->world;
@@ -968,7 +899,7 @@ static int exchange_probes(vix_index* h, vix_comm* c, const float* queries, int6
 }
 
 // filter arguments of the C ABI -> FilterArgs over a staged copy of the words (f == nullptr when there is no filter)
-static int stage_filter(const uint64_t* words, int64_t capacity, int mode, In<uint64_t>& staged, FilterArgs& f,
+int stage_filter(const uint64_t* words, int64_t capacity, int mode, In<uint64_t>& staged, FilterArgs& f,
                         const FilterArgs*& fp) {
     fp = nullptr;
     if (!words) return VIX_OK;
@@ -1133,34 +1064,18 @@ static int sharded_search(vix_index* h, vix_comm* c, const float* queries, int64
     return finish(dd.is_host() || di.is_host());
 }
 
-// The last step of sharded_range_exchange: range search decodes the merged rows into a new result object (*out); k-NN
-// search beyond VIX_MAX_K (out == nullptr) cuts them at k into [nq x k] (dist, ids: device), after checking on the exchanged
-// row starts that no row whose bound is finite came out shorter than k.
-// neg_zero: the kind's zero sign (knn_neg_zero / range_neg_zero); flat_metric >= 0: the flat kind's k-NN keys (score word,
-// user id), merged by shard_flat_merge with that metric's mapping.
-struct ShardTail {
-    vix_range_result** out = nullptr;
-    int k = 0;
-    const uint32_t* bound = nullptr;
-    float* dist = nullptr;
-    int64_t* ids = nullptr;
-    int neg_zero = 0;
-    int flat_metric = -1;
-};
-// what the exchange reports for the VIX_SCAN_DEBUG lines: this rank's entries, the merged entries, the longest merged row
-struct ShardTotals { int64_t mine = 0, total = 0, max_row = 0; bool grown = false; };
 
 // The step after each rank's local pass: its sorted keys and lims (rc: its status) -> every rank's lims and status (peer
 // region + barrier, or all-gather) -> global row starts and total (synchronises) -> the keys of every rank (peer region +
 // barrier, or grouped send / receive) -> merge, then the tail's last step.
-static int sharded_range_exchange(vix_index* h, vix_comm* c, int64_t nq, int rc, RangeKeys& rk, bool grown, const ShardTail& t,
+int sharded_range_exchange(vix_index* h, vix_comm* c, int64_t nq, int rc, RangeKeys& rk, bool grown, const ShardTail& t,
                                   ShardTotals* st) {
     cudaStream_t s = ctx().stream;
     const int world = c->world, rank = c->rank;
     const int64_t L = nq + 2;
     const bool peer = c->peer_state == 1;
     const bool knn = t.out == nullptr;
-    const char* who = knn ? "vix_sharded_search" : "vix_sharded_range_search";
+    const char* who = t.concat ? "vix_replicated_range_search" : knn ? "vix_sharded_search" : "vix_sharded_range_search";
     Scratch<int64_t> mine, lims_all, glims, dbase;
     VIX_TRY(mine.alloc((size_t)L));
     VIX_TRY(lims_all.alloc((size_t)world * L));
@@ -1257,12 +1172,13 @@ static int sharded_range_exchange(vix_index* h, vix_comm* c, int64_t nq, int rc,
         }
         keys = kall.ptr;
     }
-    const int mr = !knn ? shard_range_merge(keys, dbase.ptr, lims_all.ptr, world, nq, glims.ptr, total, t.neg_zero, r)
+    const int mr = t.concat ? replica_range_concat(keys, glims.ptr, nq, total, t.neg_zero, r)
+                 : !knn ? shard_range_merge(keys, dbase.ptr, lims_all.ptr, world, nq, glims.ptr, total, t.neg_zero, r)
                  : t.flat_metric >= 0 ? shard_flat_merge(keys, dbase.ptr, lims_all.ptr, world, nq, glims.ptr, total, t.k, t.flat_metric,
                                                           t.dist, t.ids)
                  : shard_knn_merge(keys, dbase.ptr, lims_all.ptr, world, nq, glims.ptr, total, t.k, t.neg_zero, t.dist, t.ids);
     if (mr != VIX_OK) return fail(mr);
-    if (getenv("VIX_SCAN_DEBUG") && !knn)
+    if (getenv("VIX_SCAN_DEBUG") && !knn && !t.concat)
         fprintf(stderr, "[vix sharded range] world %d, peer %d, local %lld, total %lld, max_row %lld, grown %d, kind %s\n", world,
                 peer ? 1 : 0, (long long)mine_n, (long long)total, (long long)max_row, grown ? 1 : 0, kind_name(h));
     st->mine = mine_n; st->total = total; st->max_row = max_row; st->grown = grown;

@@ -1066,3 +1066,156 @@ class ShardedIVFFlatIndex(_ShardedExactIndex):
         self.kc = int(self.local.get_coarse().shape[0])
 
     train = optimize
+
+
+class _ReplicatedIndex:
+    """Replicas over the ranks of a ``torch.distributed`` NCCL group, behind the library's C ABI: every rank holds the WHOLE
+    index and answers its block of each batch (``query_block``) with the one-GPU search; the blocks are assembled on the
+    device (vix_replicated_add / vix_replicated_search_filtered / vix_replicated_range_search over a ``vix_comm_t``).  The
+    answer on every rank is the local index's answer on one GPU holding the rows in the order the replicas append them (rank
+    0's contributions first), bit for bit.  ``gather=False`` returns this rank's block only and skips the assembly (no
+    exchange: the local index's search on the rows ``query_block(nq)``).  One rank is the local index."""
+
+    def _setup(self, local, group):
+        _ShardedExactIndex._setup(self, local, group)
+
+    def _native(self):
+        return _ShardedExactIndex._native(self)
+
+    def _pinned(self, tag, shape, dtype):
+        return ShardedIVFPQIndex._pinned(self, tag, shape, dtype)
+
+    @property
+    def count(self) -> int:
+        """rows every replica holds"""
+        return self.local.count
+
+    def query_block(self, nq: int):
+        """Rows of a batch of ``nq`` queries THIS rank answers: (first row, rows)."""
+        first, cnt = C.c_int64(0), C.c_int64(0)
+        check(lib().vix_sharded_query_block(C.c_int64(int(nq)), C.c_int(self.rank), C.c_int(self.world), C.byref(first),
+                                            C.byref(cnt)))
+        return int(first.value), int(cnt.value)
+
+    def add(self, vectors, ids):
+        """Collective: the rows THIS rank contributes (any rows; n may be 0; explicit ids).  Every replica appends every
+        rank's rows, rank 0's first."""
+        comm = self._native()
+        if comm is None:
+            self.local.batch_insert(vectors, ids)
+            return
+        x = as_input(vectors, np.float32)
+        self.local._check_dim(x, "add")
+        i = as_input(ids, np.int64)
+        check(lib().vix_replicated_add(self.local._h, comm._c, ptr(x, np.float32), ptr(i, np.int64), C.c_int64(int(x.shape[0]))))
+
+    def remove(self, ids) -> int:
+        """Every replica passes the SAME ids and removes the rows locally (no exchange: the remaining rows keep their order,
+        so the replicas stay identical); returns the rows removed, the same on every replica."""
+        return self.local.batch_remove(ids)
+
+    def batch_search(self, queries, k, nprobe=0, out=None, filter=None, gather=True):
+        """Collective: every rank passes the same queries, k (up to ``VIX_MAX_K_LARGE``), nprobe and ``filter`` (an
+        :class:`IDFilter`) and receives the whole [nq x k] (distances, ids).  Host queries: only this rank's block crosses
+        PCIe, and the result lands in pinned memory; ``out``: optional (distances f32, ids int64) arrays to write into.
+        ``gather=False``: this rank's block only (rows ``query_block(nq)``), with no exchange."""
+        import torch
+        q = as_input(queries, np.float32)
+        self.local._check_dim(q, "batch_search")
+        if not gather:
+            lo, cnt = self.query_block(int(q.shape[0]))
+            return self.local.batch_search(q[lo:lo + cnt], k, nprobe, filter=filter, out=out)
+        comm = self._native()
+        if comm is None:
+            return self.local.batch_search(q, k, nprobe, filter=filter, out=out)
+        nq, kk = int(q.shape[0]), max(int(k), 0)
+        host = not _lib._is_torch(queries)
+        if out is not None:
+            dist_, ids = out
+        elif host and nq and kk:
+            dist_, ids = self._pinned("d", (nq, kk), torch.float32), self._pinned("i", (nq, kk), torch.int64)
+        else:
+            dist_, ids = empty_like_input(q, (nq, kk), np.float32), empty_like_input(q, (nq, kk), np.int64)
+        if nq and kk:
+            words = filter.words if filter is not None else None
+            check(lib().vix_replicated_search_filtered(self.local._h, comm._c, ptr(q, np.float32), C.c_int64(nq), C.c_int(k),
+                                                       C.c_int(nprobe), ptr(words, np.uint64),
+                                                       C.c_int64(filter.capacity if filter is not None else 0),
+                                                       C.c_int(filter.mode if filter is not None else 0),
+                                                       ptr(dist_, np.float32), ptr(ids, np.int64)))
+        if out is None and host and nq and kk:
+            return dist_.numpy().copy(), ids.numpy().copy()
+        return dist_, ids
+
+    def range_search(self, queries, radius: float, nprobe: int = 0, filter=None, gather=True):
+        """Collective: every stored vector within ``radius`` of each query, as the local index's ``range_search`` on one GPU:
+        CSR ``(lims int64 [nq + 1], distances f32 [total], ids int64 [total])``, numpy for host queries, torch tensors on the
+        queries' device for CUDA tensors.  ``gather=False``: this rank's block only, with no exchange."""
+        q = as_input(queries, np.float32)
+        self.local._check_dim(q, "range_search")
+        if not gather:
+            lo, cnt = self.query_block(int(q.shape[0]))
+            return self.local.range_search(q[lo:lo + cnt], radius, nprobe=nprobe, filter=filter)
+        comm = self._native()
+        if comm is None:
+            return self.local.range_search(q, radius, nprobe=nprobe, filter=filter)
+        nq = int(q.shape[0])
+        res = C.c_void_p(0)
+        try:
+            words = filter.words if filter is not None else None
+            check(lib().vix_replicated_range_search(self.local._h, comm._c, ptr(q, np.float32), C.c_int64(nq),
+                                                    C.c_float(float(radius)), C.c_int(nprobe), ptr(words, np.uint64),
+                                                    C.c_int64(filter.capacity if filter is not None else 0),
+                                                    C.c_int(filter.mode if filter is not None else 0), C.byref(res)))
+            total = int(lib().vix_range_result_total(res))
+            lims = empty_like_input(q, (nq + 1,), np.int64)
+            dist_ = empty_like_input(q, (total,), np.float32)
+            ids = empty_like_input(q, (total,), np.int64)
+            check(lib().vix_range_result_get(res, ptr(lims, np.int64), ptr(dist_, np.float32) if total else None,
+                                             ptr(ids, np.int64) if total else None))
+            return lims, dist_, ids
+        finally:
+            lib().vix_range_result_destroy(res)
+
+
+class ReplicatedFlatIndex(_ReplicatedIndex):
+    """Flat index replicated on every rank (see :class:`_ReplicatedIndex`)."""
+
+    def __init__(self, dimension, metric="euclidean", group=None):
+        self._setup(FlatIndex(dimension, metric), group)
+
+
+class ReplicatedIVFFlatIndex(_ReplicatedIndex):
+    """IVF-Flat index replicated on every rank.  Every rank holds the same coarse centroids (``set_coarse``, or ``optimize``
+    on the same sample on every rank) before the first ``add``."""
+
+    def __init__(self, dimension, metric="euclidean", nlist=256, nprobe=8, group=None):
+        self._setup(IVFIndex(dimension, metric, nlist, nprobe), group)
+
+    def set_coarse(self, centroids):
+        self.local.set_coarse(centroids)
+
+    def optimize(self, training_vectors, kmeans_cfg: KMeansCfg | None = None):
+        if training_vectors is None:
+            raise ValueError("a replicated IVF-Flat index trains on an explicit sample, the same on every rank")
+        self.local.optimize(training_vectors, kmeans_cfg)
+
+    train = optimize
+
+
+class ReplicatedNativeIVFPQIndex(_ReplicatedIndex):
+    """IVF-PQ index replicated on every rank, entirely inside the library (``ReplicatedIVFPQIndex`` is the older layout whose
+    add and final all-gather run through ``torch.distributed``, and which has no range search or filters).  Every rank holds
+    the same coarse centroids and codebooks (``set_parameters``, or ``optimize`` on the same sample on every rank)."""
+
+    def __init__(self, dimension, metric="euclidean", nlist=256, nprobe=8, m=16, ks=256, group=None):
+        self._setup(IVFPQIndex(dimension, metric, nlist, nprobe, m, ks), group)
+
+    def set_parameters(self, coarse, codebooks, centroid_norms=None):
+        self.local.set_coarse(coarse)
+        self.local.set_codebooks(codebooks, centroid_norms)
+
+    def optimize(self, training_vectors, kmeans_cfg: KMeansCfg | None = None, pq_cfg: PQTrainCfg | None = None):
+        self.local.optimize(training_vectors, kmeans_cfg, pq_cfg)
+
+    train = optimize
